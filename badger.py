@@ -27,7 +27,7 @@ def parse_args(args):
     parser.add_argument("--barcodes", "-b", help="(README spelling) tsv file containing the observed cell barcodes; "
                         "same as --reads", type=str, dest="bar_file", default=None)
     parser.add_argument("--threshold", "-t", help="Maximal accepted difference between barcodes "
-                        "(1 and 2 run the sorted / joined searches; >= 3 runs the dense all-pairs kernel, meant for small inputs)",
+                        "(1 runs the sorted search, 2 and 3 the joined searches on multi-block seeds; >= 4 runs the dense all-pairs kernel, meant for small inputs)",
                         type=int, dest="threshold", default=1)
     parser.add_argument("--reads", "-r", help="TSV from barcode extraction",
                         type=str, dest="reads", default=None)

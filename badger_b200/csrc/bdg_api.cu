@@ -18,6 +18,7 @@
 #include "../../include/badger_b200.h"
 #include "bdg_kernels.cuh"
 #include "bdg_join.cuh"
+#include "bdg_join3.cuh"
 #include "bdg_tsv.hpp"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -105,6 +106,8 @@ struct DevCtx {
     // (one set per stream: the conditions of a block set run back to back on one stream)
     Buf jn_rows[2], jn_cols[2], jn_tab[2], jn_tabc[2], jn_hist[2], jn_cub[2], jn_counts[2], jn_offs[2], jn_rank[2], jn_lut, jn_weigh;
     int scheme_serial = 0;                                    // which scheme sits in this device's constant memory (0: none)
+    Buf jn3_scheme;                                           // t = 3 join: device copy of the seed table (bdg_seed3.cuh)
+    int scheme3_serial = 0;
     cudaEvent_t ev_cond[bdg::SEED_MAX_CONDS] = {};            // bdg_edges_build_into: "condition c has appended its edges"
     cudaEvent_t ev_pre[2] = {nullptr, nullptr}, ev_join[2] = {nullptr, nullptr};   // streaming form: scratch set k is bucketed / its join has finished
     unsigned long long* snap_host = nullptr;                  // mapped page-locked: the edge count after every condition
@@ -166,10 +169,25 @@ void build_plan(size_t N, int part, int nparts, int workers, Plan& p, uint64_t c
 constexpr size_t PLAN_HDR = 128;  // per launch: [work cursor u64 | tile-list count u64 | 8 x u64 statistics | pad]
 constexpr size_t HDR_LIST = 8, HDR_STATS = 16;
 int g_edge_mode = -1;             // -1: BDG_EDGE_MODE or default (by threshold and size); 0 dense; 1 sparse; 2 join
+constexpr size_t JOIN3_MIN_N = 90000;   // t = 3: join from this many distinct barcodes upwards (measured crossover, DESIGN.md 3.8)
 
-// 0 dense, 1 sparse, 2 join.  The join form exists for t = 2 only and pays off once the key buckets fill (DESIGN.md 3).
+// 0 dense, 1 sparse, 2 join.  The join form exists for t = 2 and t = 3 and pays off once the key buckets fill (DESIGN.md 3).
+// t = 3 has no sparse form: it runs the join when asked for (mode 2) or from BDG_JOIN3_MIN_N distinct barcodes upwards, else dense.
 int edge_mode_for(int t, size_t N)
 {
+    if (t == 3) {
+        int m = g_edge_mode;
+        if (m < 0) {
+            const char* e = getenv("BDG_EDGE_MODE");
+            if (e && !strcmp(e, "join")) m = 2;
+            else if (!e || (strcmp(e, "dense") && strcmp(e, "sparse"))) {
+                size_t min_n = JOIN3_MIN_N;
+                if (const char* j = getenv("BDG_JOIN3_MIN_N")) min_n = (size_t)std::max(0ll, atoll(j));
+                m = N >= min_n ? 2 : 0;
+            }
+        }
+        return (m == 2 && N < (1ull << 28)) ? 2 : 0;
+    }
     if (t != 1 && t != 2) return 0;
     int m = g_edge_mode;
     if (m < 0) {
@@ -533,6 +551,266 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
     return BDG_OK;
 }
 
+// ---- the t = 3 seed scheme (bdg_seed3.cuh): built once on the host, copied to the device memory of every device that uses it ----
+bdg::Seed3Scheme g_scheme3;
+int g_scheme3_serial = 0;
+
+int scheme3_ready()
+{
+    std::lock_guard<std::mutex> lock(g_scheme_mutex);
+    if (g_scheme3_serial) return BDG_OK;
+    int bases[bdg::SEED3_MAX_BLOCKS] = {3, 2, 2, 2, 2, 2, 2};
+    int nb = 7;
+    if (const char* e = getenv("BDG_JOIN3_BLOCKS")) {         // e.g. "3,3,3,2,2,2": development aid
+        nb = 0;
+        for (const char* p = e; *p && nb < bdg::SEED3_MAX_BLOCKS;) {
+            bases[nb++] = atoi(p);
+            while (*p && *p != ',') p++;
+            if (*p == ',') p++;
+        }
+    }
+    if (!bdg::seed3_scheme_build(g_scheme3, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN3_BLOCKS is not a usable block layout (4..7 blocks of >= 2 bases, 15 bases in all)");
+    g_scheme3_serial = 1;
+    return BDG_OK;
+}
+
+// Join form at t = 3 (bdg_join3.cuh): the structure of launch_edges_join over the t = 3 seed table.  Its conditions are many
+// (475 in the default layout) but come in few block sets (35), so the per-condition pieces that t = 2 keeps in fixed arrays are
+// sized by SEED3_MAX_CONDS here, the work estimate runs block set by block set (one row table and the set's column tables at a
+// time), and the streaming form snapshots the edge count once per block set rather than once per condition.
+int launch_edges_join3(const uint32_t* d_sorted, size_t N, int part, int nparts, uint32_t* d_a, uint32_t* d_b, uint8_t* d_d, size_t cap,
+                       unsigned long long* d_count, cudaStream_t caller, DevCtx* ws, const JoinStream* js = nullptr)
+{
+    if (int rc = scheme3_ready()) return rc;
+    const bdg::Seed3Scheme& S = g_scheme3;
+    auto ensure = [&](Buf& b, size_t bytes) -> int {
+        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
+            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
+        return BDG_OK;
+    };
+    if (ws->scheme3_serial != g_scheme3_serial) {
+        if (int e = ensure(ws->jn3_scheme, sizeof(bdg::Seed3Scheme))) return e;
+        CU_TRY(cudaMemcpyAsync(ws->jn3_scheme.p, &g_scheme3, sizeof(g_scheme3), cudaMemcpyHostToDevice, caller));
+        CU_TRY(cudaStreamSynchronize(caller));              // the host copy above is read asynchronously
+        ws->scheme3_serial = g_scheme3_serial;
+    }
+    const bdg::Seed3Scheme* d_scheme = (const bdg::Seed3Scheme*)ws->jn3_scheme.p;
+    int rs = (N >> S.ka[0].key_bits) < 48 ? 8 : 32;
+    if (const char* e = getenv("BDG_JOIN_RS")) rs = atoi(e) == 8 ? 8 : 32;
+    int owner_first = 0;                                    // hand-over walk after the exact distance (DESIGN.md 3.8)
+    if (const char* e = getenv("BDG_JOIN3_OWNER_FIRST")) owner_first = atoi(e) != 0;
+    const uint32_t n_slabs = (uint32_t)((N + bdg::JROWS - 1) / bdg::JROWS);
+    const bool trace = getenv("BDG_TRACE") != nullptr;
+    std::vector<long long> weight(S.nconds, 1);
+    const double t_weigh = trace ? (cudaStreamSynchronize(caller), now_ms()) : 0.0;
+    if (nparts > 1 || trace) {
+        // Pairs of every condition estimated from bucket sizes over a sample, block set by block set; the cost model of the t = 2
+        // form (launch_edges_join) is reused as it stands: time ~ pairs x (1.45 symmetric, 1 shifted) + 2.4 x N.
+        int max_set = 1, max_bits = 0;
+        for (int k = 0; k < S.nsets; k++) max_set = std::max(max_set, (int)(S.set_first[k + 1] - S.set_first[k]));
+        for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
+        const uint32_t tab = 1u << max_bits;
+        const uint32_t stride = (uint32_t)std::max<size_t>(1, (N + (1u << 17) - 1) >> 17);
+        const size_t hist_bytes = (size_t)max_set * tab * 4;
+        if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * (size_t)bdg::SEED3_MAX_CONDS)) return e;
+        uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
+        unsigned long long* d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
+        CU_TRY(cudaMemsetAsync(d_pairs, 0, 8 * (size_t)S.nconds, caller));
+        const uint32_t m = (uint32_t)((N + stride - 1) / stride);
+        for (int k = 0; k < S.nsets; k++) {
+            const int c0 = S.set_first[k], c1 = S.set_first[k + 1];
+            CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)(c1 - c0) * tab * 4, caller));
+            bdg::join3_weigh_hist_kernel<<<(int)std::min<uint32_t>((m + 255) / 256, (uint32_t)ws->sms * 8), 256, 0, caller>>>(d_sorted, (uint32_t)N, stride, d_scheme, c0, c1, tab, d_hist);
+            bdg::join3_weigh_sum_kernel<<<dim3((tab + 1023) / 1024, c1 - c0), 256, 0, caller>>>(d_hist, tab, c0, d_pairs);
+            g_launches += 2;
+        }
+        std::vector<unsigned long long> pairs(S.nconds), cost(S.nconds);
+        CU_TRY(cudaMemcpyAsync(pairs.data(), d_pairs, 8 * (size_t)S.nconds, cudaMemcpyDeviceToHost, caller));
+        CU_TRY(cudaStreamSynchronize(caller));
+        unsigned long long top = 1;
+        for (int c = 0; c < S.nconds; c++) {
+            cost[c] = pairs[c] * stride * stride * (S.cond[c].self ? 29 : 20) + 48ull * N;
+            top = std::max(top, cost[c]);
+        }
+        for (int c = 0; c < S.nconds; c++) weight[c] = (long long)std::max<unsigned long long>(1, cost[c] * 4096 / top);
+        if (trace) {
+            fprintf(stderr, "[bdg] join3 work estimate: %.3f ms\n", now_ms() - t_weigh);
+            fprintf(stderr, "[bdg] join3 estimated pairs:");
+            for (int c = 0; c < S.nconds; c++) fprintf(stderr, " %llu", pairs[c] * stride * stride);
+            fprintf(stderr, "\n");
+        }
+    }
+    // block sets alternately from the front and the back of the table, as at t = 2
+    std::vector<int> order;
+    for (int i = 0, lo = 0, hi = S.nsets - 1; lo <= hi; i++) {
+        const int k = (i & 1) ? hi-- : lo++;
+        for (int c = S.set_first[k]; c < S.set_first[k + 1]; c++) order.push_back(c);
+    }
+    long long W = 0;
+    for (int c = 0; c < S.nconds; c++) W += weight[c];
+    const long long piece_lo = (long long)part * W, piece_hi = (long long)(part + 1) * W;
+    const size_t plan_bytes = PLAN_HDR * bdg::MAX_PASSES + 8 * (size_t)bdg::SEED3_MAX_CONDS;
+    if (int e = ensure(ws->plan, plan_bytes)) return e;
+    char* d_plan = (char*)ws->plan.p;
+    CU_TRY(cudaMemsetAsync(d_plan, 0, plan_bytes, caller));
+    for (int p = 0; p < bdg::MAX_PASSES; p++) ws->host_stats[p][0] = ws->host_stats[p][1] = 0;
+    unsigned long long* d_cursors = (unsigned long long*)(d_plan + PLAN_HDR * bdg::MAX_PASSES);
+    int max_bits = 0;
+    for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
+    const size_t max_keys = (size_t)1 << max_bits;
+    size_t tmp_a = 0, tmp_b = 0;
+    CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_a, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(max_keys + 1), caller));
+    CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(n_slabs + 1), caller));
+    const size_t tmp_bytes = std::max(tmp_a, tmp_b);
+    for (int k = 0; k < 2; k++) {
+        if (int e = ensure(ws->jn_hist[k], (max_keys + 1) * 4 * 2)) return e;
+        if (int e = ensure(ws->jn_tab[k], (max_keys + 1) * 4)) return e;
+        if (int e = ensure(ws->jn_tabc[k], (max_keys + 1) * 4)) return e;
+        if (int e = ensure(ws->jn_rows[k], N * 4)) return e;
+        if (int e = ensure(ws->jn_cols[k], N * 4)) return e;
+        if (int e = ensure(ws->jn_rank[k], N * 4)) return e;
+        if (int e = ensure(ws->jn_cub[k], tmp_bytes)) return e;
+        if (int e = ensure(ws->jn_counts[k], ((size_t)n_slabs + 1) * 4)) return e;
+        if (int e = ensure(ws->jn_offs[k], ((size_t)n_slabs + 1) * 4)) return e;
+    }
+    const void* kern = rs == 8 ? (const void*)bdg::join3_kernel<8> : (const void*)bdg::join3_kernel<32>;
+    int grid = 0;
+    if (int rc = grid_for(kern, &grid, bdg::ENT)) return rc;
+    if (const char* e = getenv("BDG_JOIN_CTAS")) grid = std::min(grid, ws->sms * std::max(1, atoi(e)));
+    const int gb = (int)std::min<size_t>((N + 255) / 256, (size_t)ws->sms * 8);
+    const int bb = (int)std::min<size_t>(((size_t)n_slabs + 256) / 256, (size_t)ws->sms * 8);
+    const bool fork = !js && !getenv("BDG_EDGE_SERIAL");
+    const bool ahead = js && !getenv("BDG_EDGE_SERIAL");
+    if (fork || ahead) CU_TRY(cudaEventRecord(ws->ev_start, caller));
+    bool set_joined[2] = {false, false};
+    bool aux_used = false;
+    int n_snaps = 0;
+    if (js && !ws->snap_host) {
+        CU_TRY(cudaHostAlloc((void**)&ws->snap_host, sizeof(unsigned long long) * bdg::SEED_MAX_CONDS, cudaHostAllocMapped));
+        CU_TRY(cudaHostGetDevicePointer((void**)&ws->snap_dev, ws->snap_host, 0));
+        for (int c = 0; c < bdg::SEED_MAX_CONDS; c++) CU_TRY(cudaEventCreateWithFlags(&ws->ev_cond[c], cudaEventDisableTiming));
+        for (int q = 0; q < 2; q++) { CU_TRY(cudaEventCreateWithFlags(&ws->ev_pre[q], cudaEventDisableTiming)); CU_TRY(cudaEventCreateWithFlags(&ws->ev_join[q], cudaEventDisableTiming)); }
+    }
+    bdg::EdgeOut o{d_a, d_b, d_d, d_count, (unsigned long long)cap};
+    long long start = 0;
+    int cur_set = -1, k = 1;
+    int row_set[2] = {-1, -1};
+    double t_prev = 0;
+    if (trace) { cudaStreamSynchronize(caller); t_prev = now_ms(); }
+    std::vector<int> mine;                                  // the conditions this part works on, in order, with their row ranges
+    std::vector<long long> m_lo, m_hi, m_clo, m_chi;
+    for (int c : order) {
+        const long long w = weight[c];
+        const long long c_lo = start * nparts, c_hi = (start + w) * nparts;
+        start += w;
+        const long long lo = std::max(c_lo, piece_lo), hi = std::min(c_hi, piece_hi);
+        if (lo >= hi) continue;
+        mine.push_back(c); m_lo.push_back(lo); m_hi.push_back(hi); m_clo.push_back(c_lo); m_chi.push_back(c_hi);
+    }
+    for (size_t oi = 0; oi < mine.size(); oi++) {
+        const int c = mine[oi];
+        const int set = S.cond[c].set;
+        if (nparts > 1 || ahead || set != cur_set) k ^= 1;
+        cur_set = set;
+        const bool new_set = row_set[k] != set;
+        row_set[k] = set;
+        cudaStream_t st = (fork && k == 1) ? ws->aux[1] : caller;
+        cudaStream_t sp = ahead ? ws->aux[1] : st;
+        if (fork && k == 1 && !aux_used) { CU_TRY(cudaStreamWaitEvent(st, ws->ev_start, 0)); aux_used = true; }
+        if (ahead) {
+            if (!aux_used) { CU_TRY(cudaStreamWaitEvent(sp, ws->ev_start, 0)); aux_used = true; }
+            if (set_joined[k]) CU_TRY(cudaStreamWaitEvent(sp, ws->ev_join[k], 0));
+        }
+        auto bucket_side = [&](const bdg::SeedKey& key, Buf& dst, Buf& table) -> int {
+            const size_t nkeys = (size_t)1 << key.key_bits;
+            uint32_t* hist = (uint32_t*)ws->jn_hist[k].p;
+            uint32_t* rank = (uint32_t*)ws->jn_rank[k].p;
+            size_t bytes = ws->jn_cub[k].cap;
+            CU_TRY(cudaMemsetAsync(hist, 0, (nkeys + 1) * 4, sp));
+            bdg::join_hist_rank_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, hist, rank);
+            CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)hist, (uint32_t*)table.p, (int)(nkeys + 1), sp));
+            bdg::join_scatter_rank_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, (const uint32_t*)table.p, rank, (uint32_t*)dst.p);
+            g_launches += 2;
+            return BDG_OK;
+        };
+        if (new_set) { if (int e = bucket_side(S.ka[S.set_first[set]], ws->jn_rows[k], ws->jn_tab[k])) return e; }
+        bdg::Join3Args A3{};
+        bdg::JoinArgs& A = A3.j;
+        A.rows = (const uint32_t*)ws->jn_rows[k].p;
+        A.rowstart = (const uint32_t*)ws->jn_tab[k].p;
+        A.nkeys = 1u << S.ka[c].key_bits;
+        if (S.cond[c].self) {
+            A.cols = A.rows;
+            A.colstart = (const uint32_t*)ws->jn_tab[k].p;
+        } else {
+            if (int e = bucket_side(S.kb[c], ws->jn_cols[k], ws->jn_tabc[k])) return e;
+            A.cols = (const uint32_t*)ws->jn_cols[k].p;
+            A.colstart = (const uint32_t*)ws->jn_tabc[k].p;
+        }
+        A.offs = (const uint32_t*)ws->jn_offs[k].p;
+        A.cursor = d_cursors + c;
+        A.stats = (unsigned long long*)(d_plan + HDR_STATS);
+        A.N = (uint32_t)N;
+        A.n_slabs = n_slabs;
+        A.cond = c;
+        A.self = S.cond[c].self;
+        A.f0 = (uint32_t)(m_lo[oi] - m_clo[oi]); A.f1 = (uint32_t)(m_hi[oi] - m_clo[oi]); A.fden = (uint32_t)(m_chi[oi] - m_clo[oi]);
+        A.T = bdg::qgram_threshold(3);
+        A.one = 1u;
+        A.mone = 0xFFFFFFFFu;
+        A3.ka = S.ka[c];
+        A3.kb = S.kb[c];
+        A3.scheme = d_scheme;
+        A3.owner_first = owner_first;
+        bdg::join3_band_kernel<<<bb, 256, 0, sp>>>(A3, (uint32_t*)ws->jn_counts[k].p);
+        size_t bytes = ws->jn_cub[k].cap;
+        CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)ws->jn_counts[k].p, (uint32_t*)ws->jn_offs[k].p, (int)(n_slabs + 1), sp));
+        if (ahead) {
+            CU_TRY(cudaEventRecord(ws->ev_pre[k], sp));
+            CU_TRY(cudaStreamWaitEvent(st, ws->ev_pre[k], 0));
+        }
+        if (rs == 8) bdg::join3_kernel<8><<<grid, bdg::ENT, 0, st>>>(A3, o);
+        else bdg::join3_kernel<32><<<grid, bdg::ENT, 0, st>>>(A3, o);
+        g_launches += 3;
+        CU_TRY(cudaGetLastError());
+        if (ahead) { CU_TRY(cudaEventRecord(ws->ev_join[k], st)); set_joined[k] = true; }
+        if (trace) {
+            CU_TRY(cudaStreamSynchronize(st));
+            const double now = now_ms();
+            fprintf(stderr, "[bdg] join3 cond %3d (set %2d, %s, rows %u/%u..%u/%u, weight %lld): %.3f ms\n", c, set, S.cond[c].self ? "sym" : "shf",
+                    A.f0, A.fden, A.f1, A.fden, weight[c], now - t_prev);
+            t_prev = now;
+        }
+        if (js && (oi + 1 == mine.size() || S.cond[mine[oi + 1]].set != set)) {      // the last condition of a block set
+            bdg::join_snapshot_kernel<<<1, 1, 0, st>>>(d_count, ws->snap_dev + n_snaps);
+            g_launches++;
+            CU_TRY(cudaEventRecord(ws->ev_cond[n_snaps], st));
+            n_snaps++;
+        }
+    }
+    if (aux_used) {
+        CU_TRY(cudaEventRecord(ws->ev_done[1], ws->aux[1]));
+        CU_TRY(cudaStreamWaitEvent(caller, ws->ev_done[1], 0));
+    }
+    if (trace) { cudaStreamSynchronize(caller); fprintf(stderr, "[bdg] join3 part %d of %d: %.3f ms from entry to the last condition\n", part, nparts, now_ms() - t_weigh); }
+    if (js) {
+        cudaStream_t cp = ws->aux[2];
+        size_t done = 0;
+        for (int q = 0; q < n_snaps; q++) {
+            CU_TRY(cudaEventSynchronize(ws->ev_cond[q]));
+            const size_t upto = (size_t)std::min<unsigned long long>(ws->snap_host[q], js->h_cap);
+            if (upto > done) {
+                CU_TRY(cudaMemcpyAsync(js->h_a + done, d_a + done, (upto - done) * 4, cudaMemcpyDeviceToHost, cp));
+                CU_TRY(cudaMemcpyAsync(js->h_b + done, d_b + done, (upto - done) * 4, cudaMemcpyDeviceToHost, cp));
+                CU_TRY(cudaMemcpyAsync(js->h_d + done, d_d + done, upto - done, cudaMemcpyDeviceToHost, cp));
+                done = upto;
+            }
+        }
+        CU_TRY(cudaStreamSynchronize(cp));
+    }
+    return BDG_OK;
+}
+
 // Launch the edge construction of one part on the current device / stream.  d_count is zeroed on the stream.
 // ws: the device's grow-only workspaces (plan, rotated keys, sort scratch); one in-flight call per device.
 int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts, uint32_t* d_a, uint32_t* d_b,
@@ -544,7 +822,8 @@ int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts
     CU_TRY(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), st));
     if (t <= 0 || N < 2) return BDG_OK;   // D >= 1 for distinct barcodes: no edges (barcode_graph.py:245)
     const int mode = edge_mode_for(t, N);
-    if (mode == 2) return launch_edges_join(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js);
+    if (mode == 2) return t == 3 ? launch_edges_join3(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js)
+                                 : launch_edges_join(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js);
     const bool sparse = mode == 1;
     const int passes = sparse ? bdg::n_passes(t) : 1;
     const void* kern = sparse ? (t == 1 ? (const void*)bdg::sparse_tile_kernel<1, 0, false> : (const void*)bdg::sparse_tile_kernel<2, 0, false>)
@@ -859,6 +1138,7 @@ void bdg_shutdown(void)
             c.jn_cub[k].release(); c.jn_counts[k].release(); c.jn_offs[k].release();
         }
         c.jn_lut.release(); c.jn_weigh.release(); for (auto& b : c.jn_rank) b.release();
+        c.jn3_scheme.release();
         if (c.snap_host) { cudaFreeHost(c.snap_host); c.snap_host = nullptr; for (auto& e : c.ev_cond) if (e) cudaEventDestroy(e);
                            for (int q = 0; q < 2; q++) { if (c.ev_pre[q]) cudaEventDestroy(c.ev_pre[q]); if (c.ev_join[q]) cudaEventDestroy(c.ev_join[q]); } }
     }

@@ -41,7 +41,7 @@ enum {
 /* How the edge construction is dealt to parts (GPUs / ranks); the parts' edge lists are disjoint and their union is the full edge
  * set, so they are simply concatenated (no exchange step).  Replaces the 10 000-barcode chunks dealt to worker processes in
  * barcode_graph.py:26,164-189.
- *   join form (t = 2): the seed conditions are laid on a line by estimated work and the line is cut into nparts equal pieces; a
+ *   join form (t = 2, 3): the seed conditions are laid on a line by estimated work and the line is cut into nparts equal pieces; a
  *     part buckets and joins only the conditions its piece touches, a condition on a cut is shared by row range, cut at a bucket
  *     boundary (the same on every part, because it depends on the bucket sizes only);
  *   sparse / dense forms: rows of the (rotated) sort order in tiles of BDG_ROW_TILE rows, boustrophedon: tile I belongs to part
@@ -193,14 +193,15 @@ int bdg_kmer_index_info(const bdg_kmer_index* ix, int* posted, double* kernel_ms
  * extremely dense inputs): call bdg_edges_build_part once (it grows the list) or use dense mode, then repeat. */
 int bdg_dev_edges_build(const uint32_t* d_sorted, size_t N, int t, int part, int nparts, uint32_t* d_a,
                         uint32_t* d_b, uint8_t* d_d, size_t cap, unsigned long long* d_count, void* stream);
-/* How the edge set is searched for t = 1, 2 (results are identical; DESIGN.md "edge construction"):
- *   2 join (t = 2 only): sort-merge joins on multi-block seeds - per seed condition the array is sorted by the condition's
- *     key, equal-key buckets are paired and only those pairs are tested (bdg_join.cuh); the default for t = 2 from
- *     BDG_JOIN_MIN_N (150 000) distinct barcodes upwards;
+/* How the edge set is searched (results are identical; DESIGN.md "edge construction"):
+ *   2 join (t = 2, 3): sort-merge joins on multi-block seeds - per seed condition the array is sorted by the condition's
+ *     key, equal-key buckets are paired and only those pairs are tested (bdg_join.cuh, bdg_join3.cuh); the default for t = 2
+ *     from BDG_JOIN_MIN_N (150 000) distinct barcodes upwards, for t = 3 from BDG_JOIN3_MIN_N (90 000) upwards;
  *   1 sparse (default otherwise): one pass per prefilter block over the array sorted by a rotated key, pairs are decided
  *     tile by tile from key intervals and scored only inside the tiles that can hold a candidate;
  *   0 dense: one pass, the low-block conditions are scored for every pair (the all-pairs kernel);
- *  -1 back to the default / BDG_EDGE_MODE=dense|sparse|join.  t >= 3 always runs dense without a block prefilter. */
+ *  -1 back to the default / BDG_EDGE_MODE=dense|sparse|join.  t = 3 has no sparse form: modes 0 and 1 run it dense, below
+ *     BDG_JOIN3_MIN_N too; t >= 4 always runs dense without a block prefilter. */
 int bdg_set_edge_mode(int mode);
 /* Work statistics of the last bdg_dev_edges_build / bdg_edges_build* launch on the current device, summed over
  * its passes: out5[0] column sub-tiles whose key interval was tested, out5[1] sub-tiles that could hold a
@@ -210,7 +211,8 @@ int bdg_set_edge_mode(int mode);
 int bdg_dev_edges_stats(unsigned long long* out5, void* stream);
 /* The kernels' eight raw counters of the last edge launch on the current device, summed over its passes.  Join form: [0] work
  * units, [2] pairs tested, [3] candidates handed to the exact stage, [6] candidates with D <= 2, [7] pairs whose 6-mer score was
- * computed; [4] / [5] sum / max over the warps of their busy time in ns.  Synchronises the stream. */
+ * computed (t = 3: [6] candidates with D <= 3, [7] of those this condition owns; with BDG_JOIN3_OWNER_FIRST=1 the hand-over
+ * runs first and [6] counts only the owned ones); [4] / [5] sum / max over the warps of their busy time in ns.  Synchronises the stream. */
 int bdg_dev_edges_stats_raw(unsigned long long* out8, void* stream);
 /* Development aid: out[2p], out[2p+1] = sum and max over the warps of pass p of (warp exit - first warp start), ns. */
 int bdg_dev_edges_balance(unsigned long long* out6, void* stream);
