@@ -18,7 +18,6 @@
 #include "../../include/badger_b200.h"
 #include "bdg_kernels.cuh"
 #include "bdg_join.cuh"
-#include "bdg_join3.cuh"
 #include "bdg_tsv.hpp"
 
 #include <cub/device/device_radix_sort.cuh>
@@ -101,16 +100,17 @@ struct DevCtx {
     Buf top16;                                                // first node of every high half of the barcode (the node of an edge end is searched in that run)
     Buf io[4];                                                // host-buffer calls of pack16 / membership: inputs, outputs, check flag
     Buf nn[9];                                                // sparse nearest: rotated keys + payload (in/out) of queries and targets, scratch
-    // join form of the t = 2 edge construction (bdg_join.cuh): barcodes in the key order of every condition's row side / column
-    // side, first column of every key, scratch keys (in / sorted) and radix-sort scratch, units per slab and their prefix sums
-    // (one set per stream: the conditions of a block set run back to back on one stream)
+    // join form of the t = 2 and t = 3 edge construction (bdg_join.cuh): barcodes in the key order of every condition's row side /
+    // column side, first column of every key, bucket sizes and every barcode's place in its bucket, scan scratch, units per slab
+    // and their prefix sums (one set per stream: the conditions of a block set run back to back on one stream); the t = 2
+    // hand-over table and the work-estimate histograms
     Buf jn_rows[2], jn_cols[2], jn_tab[2], jn_tabc[2], jn_hist[2], jn_cub[2], jn_counts[2], jn_offs[2], jn_rank[2], jn_lut, jn_weigh;
-    int scheme_serial = 0;                                    // which scheme sits in this device's constant memory (0: none)
+    int scheme_serial = 0;                                    // which t = 2 scheme sits in this device's constant memory (0: none)
     Buf jn3_scheme;                                           // t = 3 join: device copy of the seed table (bdg_seed3.cuh)
     int scheme3_serial = 0;
-    cudaEvent_t ev_cond[bdg::SEED_MAX_CONDS] = {};            // bdg_edges_build_into: "condition c has appended its edges"
+    cudaEvent_t ev_snap[bdg::JOIN_MAX_SNAPS] = {};            // bdg_edges_build_into: "the edges up to snapshot q are appended"
     cudaEvent_t ev_pre[2] = {nullptr, nullptr}, ev_join[2] = {nullptr, nullptr};   // streaming form: scratch set k is bucketed / its join has finished
-    unsigned long long* snap_host = nullptr;                  // mapped page-locked: the edge count after every condition
+    unsigned long long* snap_host = nullptr;                  // mapped page-locked: the edge count at every snapshot
     unsigned long long* snap_dev = nullptr;
 };
 std::vector<DevCtx> g_ctx;
@@ -171,65 +171,69 @@ constexpr size_t HDR_LIST = 8, HDR_STATS = 16;
 int g_edge_mode = -1;             // -1: BDG_EDGE_MODE or default (by threshold and size); 0 dense; 1 sparse; 2 join
 constexpr size_t JOIN3_MIN_N = 90000;   // t = 3: join from this many distinct barcodes upwards (measured crossover, DESIGN.md 3.8)
 
-// 0 dense, 1 sparse, 2 join.  The join form exists for t = 2 and t = 3 and pays off once the key buckets fill (DESIGN.md 3).
-// t = 3 has no sparse form: it runs the join when asked for (mode 2) or from BDG_JOIN3_MIN_N distinct barcodes upwards, else dense.
+// 0 dense, 1 sparse, 2 join.  The join form exists for t = 2 and t = 3 and pays off once the key buckets fill (DESIGN.md 3);
+// below that t = 2 runs sparse and t = 3, which has no sparse form, dense.
 int edge_mode_for(int t, size_t N)
 {
-    if (t == 3) {
-        int m = g_edge_mode;
-        if (m < 0) {
-            const char* e = getenv("BDG_EDGE_MODE");
-            if (e && !strcmp(e, "join")) m = 2;
-            else if (!e || (strcmp(e, "dense") && strcmp(e, "sparse"))) {
-                size_t min_n = JOIN3_MIN_N;
-                if (const char* j = getenv("BDG_JOIN3_MIN_N")) min_n = (size_t)std::max(0ll, atoll(j));
-                m = N >= min_n ? 2 : 0;
-            }
-        }
-        return (m == 2 && N < (1ull << 28)) ? 2 : 0;
-    }
-    if (t != 1 && t != 2) return 0;
     int m = g_edge_mode;
     if (m < 0) {
         const char* e = getenv("BDG_EDGE_MODE");
         if (e && !strcmp(e, "dense")) m = 0;
         else if (e && !strcmp(e, "sparse")) m = 1;
         else if (e && !strcmp(e, "join")) m = 2;
-        else {
-            size_t min_n = 150000;
-            if (const char* j = getenv("BDG_JOIN_MIN_N")) min_n = (size_t)std::max(0ll, atoll(j));
-            m = (t == 2 && N >= min_n) ? 2 : 1;
-        }
+        else if (t == 2 || t == 3) {
+            size_t min_n = t == 2 ? 150000 : JOIN3_MIN_N;
+            if (const char* j = getenv(t == 2 ? "BDG_JOIN_MIN_N" : "BDG_JOIN3_MIN_N")) min_n = (size_t)std::max(0ll, atoll(j));
+            m = N >= min_n ? 2 : t == 2 ? 1 : 0;
+        } else m = t == 1 ? 1 : 0;
     }
-    if (m == 2 && (t != 2 || N >= (1ull << 28))) m = 1;
+    if (m == 2 && (t < 2 || t > 3 || N >= (1ull << 28))) m = t == 3 ? 0 : 1;
+    if (m == 1 && t != 1 && t != 2) m = 0;
     return m;
 }
 
-// ---- the seed scheme of the join form: built once on the host (bdg_seed.cuh), copied to every device that uses it ----
+// ---- the seed schemes of the join form: built once on the host (bdg_seed.cuh, bdg_seed3.cuh), copied to every device that uses them ----
 bdg::SeedScheme g_scheme;
 std::vector<uint8_t> g_scheme_lut;
-int g_scheme_serial = 0;
+bdg::Seed3Scheme g_scheme3;
+int g_scheme_serial = 0, g_scheme3_serial = 0;
 
 std::mutex g_scheme_mutex;        // the devices of one build call arrive on their own host threads
 
+template <int T>
+const auto& join_scheme()
+{
+    if constexpr (T == 2) return g_scheme; else return g_scheme3;
+}
+
+// The block layout of the threshold-T table is BDG_JOIN_BLOCKS / BDG_JOIN3_BLOCKS (e.g. "4,4,4,3" / "3,3,3,2,2,2": development
+// aids), else five blocks of 3 bases at t = 2 and 3,2,2,2,2,2,2 at t = 3.
+template <int T>
 int scheme_ready()
 {
     std::lock_guard<std::mutex> lock(g_scheme_mutex);
-    if (g_scheme_serial) return BDG_OK;
-    int bases[bdg::SEED_MAX_BLOCKS] = {3, 3, 3, 3, 3};
-    int nb = 5;
-    if (const char* e = getenv("BDG_JOIN_BLOCKS")) {          // e.g. "4,4,4,3": development aid
+    int& serial = T == 2 ? g_scheme_serial : g_scheme3_serial;
+    if (serial) return BDG_OK;
+    const int max_blocks = T == 2 ? bdg::SEED_MAX_BLOCKS : bdg::SEED3_MAX_BLOCKS;
+    int bases[bdg::SEED3_MAX_BLOCKS] = {3, 3, 3, 3, 3, 3, 3};
+    int nb = T == 2 ? 5 : 7;
+    if (T == 3) std::fill(bases + 1, bases + nb, 2);
+    if (const char* e = getenv(T == 2 ? "BDG_JOIN_BLOCKS" : "BDG_JOIN3_BLOCKS")) {
         nb = 0;
-        for (const char* p = e; *p && nb < bdg::SEED_MAX_BLOCKS;) {
+        for (const char* p = e; *p && nb < max_blocks;) {
             bases[nb++] = atoi(p);
             while (*p && *p != ',') p++;
             if (*p == ',') p++;
         }
     }
-    if (!bdg::seed_scheme_build(g_scheme, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN_BLOCKS is not a usable block layout (3..6 blocks, 15 bases in all)");
-    g_scheme_lut.assign((size_t)1 << g_scheme.nflags, 0);
-    bdg::seed_lut_build(g_scheme, g_scheme_lut.data());
-    g_scheme_serial = 1;
+    if constexpr (T == 2) {
+        if (!bdg::seed_scheme_build(g_scheme, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN_BLOCKS is not a usable block layout (3..6 blocks, 15 bases in all)");
+        g_scheme_lut.assign((size_t)1 << g_scheme.nflags, 0);
+        bdg::seed_lut_build(g_scheme, g_scheme_lut.data());
+    } else {
+        if (!bdg::seed3_scheme_build(g_scheme3, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN3_BLOCKS is not a usable block layout (4..7 blocks of >= 2 bases, 15 bases in all)");
+    }
+    serial = 1;
     return BDG_OK;
 }
 
@@ -268,15 +272,16 @@ double now_ms()
     return ts.tv_sec * 1e3 + ts.tv_nsec * 1e-6;
 }
 
-// Join form (t = 2), bdg_join.cuh.  The seed conditions are laid on a line by weight (their estimated work, see below) and the
-// line is cut into nparts equal pieces: a part sorts and
-// joins only the conditions its piece touches, a condition on a cut is shared by row range (cut at a bucket boundary).  Per condition: counting sort by the
-// key (rows once per block set, columns for the shifted conditions; its prefix sums are colstart) -> units per slab -> prefix sums ->
-// one persistent join launch.  The conditions of a block set follow one another and share the row order.  Consecutive block sets alternate between the caller's stream and an auxiliary one, so that one
-// condition's sorts and the tail of its join overlap the neighbour's join.
+// Join form (t = 2 and t = 3), bdg_join.cuh.  The seed conditions are laid on a line by weight (their estimated work, see below)
+// and the line is cut into nparts equal pieces: a part sorts and joins only the conditions its piece touches, a condition on a
+// cut is shared by row range (cut at a bucket boundary).  Per condition: counting sort by the key (rows once per block set,
+// columns for the shifted conditions; its prefix sums are colstart) -> units per slab -> prefix sums -> one persistent join
+// launch.  The conditions of a block set follow one another and share the row order.  Consecutive block sets alternate between
+// the caller's stream and an auxiliary one, so that one condition's sorts and the tail of its join overlap the neighbour's join.
 // Host buffers the finished edges are copied into WHILE later conditions still run (bdg_edges_build_into): the conditions
-// then run on one stream, a snapshot of the edge count follows every join launch, and the ranges between two snapshots -
-// final, because their launches have ended - leave on the copy stream.
+// then run on one stream, a snapshot of the edge count follows every condition (t = 2) or the last condition of every block
+// set (t = 3, whose 475 conditions are short), and the ranges between two snapshots - final, because their launches have
+// ended - leave on the copy stream.
 struct JoinStream {
     uint32_t* h_a;
     uint32_t* h_b;
@@ -284,65 +289,97 @@ struct JoinStream {
     size_t h_cap;
 };
 
+template <int T>
 int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, uint32_t* d_a, uint32_t* d_b, uint8_t* d_d, size_t cap,
-                      unsigned long long* d_count, cudaStream_t caller, DevCtx* ws, const JoinStream* js = nullptr)
+                      unsigned long long* d_count, cudaStream_t caller, DevCtx* ws, const JoinStream* js)
 {
-    if (int rc = scheme_ready()) return rc;
-    const bdg::SeedScheme& S = g_scheme;
+    if (int rc = scheme_ready<T>()) return rc;
+    const auto& S = join_scheme<T>();
     auto ensure = [&](Buf& b, size_t bytes) -> int {
         if (cudaError_t e = (cudaError_t)b.ensure(bytes))
             return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
         return BDG_OK;
     };
-    if (ws->scheme_serial != g_scheme_serial) {
-        if (int e = ensure(ws->jn_lut, g_scheme_lut.size())) return e;
-        CU_TRY(cudaMemcpyToSymbolAsync(bdg::c_scheme, &g_scheme, sizeof(g_scheme), 0, cudaMemcpyHostToDevice, caller));
-        CU_TRY(cudaMemcpyAsync(ws->jn_lut.p, g_scheme_lut.data(), g_scheme_lut.size(), cudaMemcpyHostToDevice, caller));
-        CU_TRY(cudaStreamSynchronize(caller));              // the host copies above are read asynchronously
-        ws->scheme_serial = g_scheme_serial;
+    if constexpr (T == 2) {                                 // the table to constant memory, the hand-over table beside it
+        if (ws->scheme_serial != g_scheme_serial) {
+            if (int e = ensure(ws->jn_lut, g_scheme_lut.size())) return e;
+            CU_TRY(cudaMemcpyToSymbolAsync(bdg::c_scheme, &g_scheme, sizeof(g_scheme), 0, cudaMemcpyHostToDevice, caller));
+            CU_TRY(cudaMemcpyAsync(ws->jn_lut.p, g_scheme_lut.data(), g_scheme_lut.size(), cudaMemcpyHostToDevice, caller));
+            CU_TRY(cudaStreamSynchronize(caller));          // the host copies above are read asynchronously
+            ws->scheme_serial = g_scheme_serial;
+        }
+    } else {                                                // too large for constant memory: a device copy
+        if (ws->scheme3_serial != g_scheme3_serial) {
+            if (int e = ensure(ws->jn3_scheme, sizeof(g_scheme3))) return e;
+            CU_TRY(cudaMemcpyAsync(ws->jn3_scheme.p, &g_scheme3, sizeof(g_scheme3), cudaMemcpyHostToDevice, caller));
+            CU_TRY(cudaStreamSynchronize(caller));          // the host copy above is read asynchronously
+            ws->scheme3_serial = g_scheme3_serial;
+        }
     }
     // rows per sub-slab: 8 when the key buckets are short (fewer rows then span fewer foreign buckets), else 32
     int rs = (N >> S.ka[0].key_bits) < 48 ? 8 : 32;
     if (const char* e = getenv("BDG_JOIN_RS")) rs = atoi(e) == 8 ? 8 : 32;
     const uint32_t n_slabs = (uint32_t)((N + bdg::JROWS - 1) / bdg::JROWS);
+    const bool trace = getenv("BDG_TRACE") != nullptr;
     // Weights of the conditions for the deal to the parts: one part takes everything; several parts estimate every condition's
     // pairs from bucket sizes over a sample (identical integer arithmetic on every part) and add the bucketing of its sides.
-    long long weight[bdg::SEED_MAX_CONDS];
-    for (int c = 0; c < S.nconds; c++) weight[c] = 1;
-    const double t_weigh = getenv("BDG_TRACE") ? (cudaStreamSynchronize(caller), now_ms()) : 0.0;
-    if (nparts > 1 || getenv("BDG_TRACE")) {                 // (traced runs print the estimate beside the measured time of every condition)
-        uint32_t maxtab = 4;
-        for (int c = 0; c < S.nconds; c++) maxtab = std::max(maxtab, 1u << S.ka[c].key_bits);
-        bdg::WeighSlots slots{};
-        for (int c = 0; c < S.nconds; c++) {
-            slots.row[c] = S.cond[c].row_sort == c ? (uint8_t)slots.n++ : slots.row[S.cond[c].row_sort];
-            slots.col[c] = S.cond[c].self ? slots.row[c] : (uint8_t)slots.n++;
-        }
+    std::vector<long long> weight(S.nconds, 1);
+    const double t_weigh = trace ? (cudaStreamSynchronize(caller), now_ms()) : 0.0;
+    if (nparts > 1 || trace) {                              // (traced runs print the estimate beside the measured time of every condition)
         const uint32_t stride = (uint32_t)std::max<size_t>(1, (N + (1u << 17) - 1) >> 17);
-        const size_t hist_bytes = (size_t)slots.n * maxtab * 4;
-        if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * bdg::SEED_MAX_CONDS)) return e;
-        uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
-        unsigned long long* d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
-        CU_TRY(cudaMemsetAsync(ws->jn_weigh.p, 0, hist_bytes + 8 * bdg::SEED_MAX_CONDS, caller));
         const uint32_t m = (uint32_t)((N + stride - 1) / stride);
-        bdg::join_weigh_hist_kernel<<<(int)std::min<uint32_t>((m + 255) / 256, (uint32_t)ws->sms * 8), 256, 0, caller>>>(d_sorted, (uint32_t)N, stride, S.nconds, maxtab, slots, d_hist);
-        bdg::join_weigh_sum_kernel<<<dim3((maxtab / 4 + 1023) / 1024, S.nconds), 256, 0, caller>>>(d_hist, maxtab, slots, d_pairs);
-        g_launches += 2;
-        unsigned long long pairs[bdg::SEED_MAX_CONDS];
-        CU_TRY(cudaMemcpyAsync(pairs, d_pairs, 8 * S.nconds, cudaMemcpyDeviceToHost, caller));
+        const int hb = (int)std::min<uint32_t>((m + 255) / 256, (uint32_t)ws->sms * 8);
+        unsigned long long* d_pairs = nullptr;
+        if constexpr (T == 2) {                             // all tables in one pass
+            uint32_t maxtab = 4;
+            for (int c = 0; c < S.nconds; c++) maxtab = std::max(maxtab, 1u << S.ka[c].key_bits);
+            bdg::WeighSlots slots{};
+            for (int c = 0; c < S.nconds; c++) {
+                slots.row[c] = S.cond[c].row_sort == c ? (uint8_t)slots.n++ : slots.row[S.cond[c].row_sort];
+                slots.col[c] = S.cond[c].self ? slots.row[c] : (uint8_t)slots.n++;
+            }
+            const size_t hist_bytes = (size_t)slots.n * maxtab * 4;
+            if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * bdg::SEED_MAX_CONDS)) return e;
+            uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
+            d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
+            CU_TRY(cudaMemsetAsync(ws->jn_weigh.p, 0, hist_bytes + 8 * bdg::SEED_MAX_CONDS, caller));
+            bdg::join_weigh_hist_kernel<<<hb, 256, 0, caller>>>(d_sorted, (uint32_t)N, stride, S.nconds, maxtab, slots, d_hist);
+            bdg::join_weigh_sum_kernel<<<dim3((maxtab / 4 + 1023) / 1024, S.nconds), 256, 0, caller>>>(d_hist, maxtab, slots, d_pairs);
+            g_launches += 2;
+        } else {                                            // block set by block set: one row table and the set's column tables at a time
+            int max_set = 1, max_bits = 0;
+            for (int k = 0; k < S.nsets; k++) max_set = std::max(max_set, (int)(S.set_first[k + 1] - S.set_first[k]));
+            for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
+            const uint32_t tab = 1u << max_bits;
+            const size_t hist_bytes = (size_t)max_set * tab * 4;
+            if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * (size_t)bdg::SEED3_MAX_CONDS)) return e;
+            uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
+            d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
+            CU_TRY(cudaMemsetAsync(d_pairs, 0, 8 * (size_t)S.nconds, caller));
+            for (int k = 0; k < S.nsets; k++) {
+                const int c0 = S.set_first[k], c1 = S.set_first[k + 1];
+                CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)(c1 - c0) * tab * 4, caller));
+                bdg::join3_weigh_hist_kernel<<<hb, 256, 0, caller>>>(d_sorted, (uint32_t)N, stride, (const bdg::Seed3Scheme*)ws->jn3_scheme.p, c0, c1, tab, d_hist);
+                bdg::join3_weigh_sum_kernel<<<dim3((tab + 1023) / 1024, c1 - c0), 256, 0, caller>>>(d_hist, tab, c0, d_pairs);
+                g_launches += 2;
+            }
+        }
+        std::vector<unsigned long long> pairs(S.nconds), cost(S.nconds);
+        CU_TRY(cudaMemcpyAsync(pairs.data(), d_pairs, 8 * (size_t)S.nconds, cudaMemcpyDeviceToHost, caller));
         CU_TRY(cudaStreamSynchronize(caller));
-        // Cost model fitted to the per-condition times of a traced C4 run (BDG_TRACE; 25 conditions, rms error 8 %):
+        // Cost model fitted to the per-condition times of a traced t = 2 C4 run (BDG_TRACE; 25 conditions, rms error 8 %), and
+        // reused at t = 3 without refitting:
         //   time ~ pairs x (1.45 for a symmetric condition, 1 for a shifted one) + 2.4 x N.
         // A symmetric condition's pairs are counted once (n (n - 1) / 2) and hold most of the really close pairs of barcode data -
         // the ones that cost an exact distance, a hand-over check and a score sit on diagonal 0; the N term is the bucketing and
         // the per-slab bookkeeping.  Scaled to <= 4096 so that the cut arithmetic stays small.
-        unsigned long long cost[bdg::SEED_MAX_CONDS], top = 1;
+        unsigned long long top = 1;
         for (int c = 0; c < S.nconds; c++) {
             cost[c] = pairs[c] * stride * stride * (S.cond[c].self ? 29 : 20) + 48ull * N;
             top = std::max(top, cost[c]);
         }
         for (int c = 0; c < S.nconds; c++) weight[c] = (long long)std::max<unsigned long long>(1, cost[c] * 4096 / top);
-        if (getenv("BDG_TRACE")) {
+        if (trace) {
             fprintf(stderr, "[bdg] join work estimate: %.3f ms\n", now_ms() - t_weigh);
             fprintf(stderr, "[bdg] join weights (part %d of %d):", part, nparts);
             for (int c = 0; c < S.nconds; c++) fprintf(stderr, " %lld", weight[c]);
@@ -354,25 +391,27 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
     // Order of the conditions along the line: block set by block set (a set shares its row order), the sets taken alternately
     // from the front and from the back of the table.  A pair that meets several conditions is emitted by the first one in TABLE
     // order, so the early sets own most of the edges; alternating spreads the edges (their scores, stores and PCIe bytes) over
-    // the parts.
-    int order[bdg::SEED_MAX_CONDS], n_order = 0;
+    // the parts.  This part keeps the conditions its piece of the line touches, with their row ranges.
+    struct Piece { int c, set; long long lo, hi, c_lo, c_hi; };
+    std::vector<Piece> mine;
     {
-        int set_first[bdg::SEED_MAX_CONDS], set_last[bdg::SEED_MAX_CONDS], n_sets = 0;
-        for (int c = 0; c < S.nconds; c++) {
-            if (S.cond[c].row_sort == c) { set_first[n_sets] = c; set_last[n_sets] = c; n_sets++; }
-            else set_last[n_sets - 1] = c;
-        }
-        for (int i = 0, lo = 0, hi = n_sets - 1; lo <= hi; i++) {
-            const int k = (i & 1) ? hi-- : lo++;
-            for (int c = set_first[k]; c <= set_last[k]; c++) order[n_order++] = c;
+        long long W = 0, start = 0;
+        for (int c = 0; c < S.nconds; c++) W += weight[c];
+        const long long piece_lo = (long long)part * W, piece_hi = (long long)(part + 1) * W;   // cond c covers [start_c * nparts, (start_c + w_c) * nparts)
+        for (int i = 0, lo = 0, hi = S.nsets - 1; lo <= hi; i++) {
+            const int set = (i & 1) ? hi-- : lo++;
+            for (int c = S.set_first[set]; c < S.set_first[set + 1]; c++) {
+                const long long c_lo = start * nparts, c_hi = (start + weight[c]) * nparts;
+                start += weight[c];
+                const long long p_lo = std::max(c_lo, piece_lo), p_hi = std::min(c_hi, piece_hi);
+                if (p_lo < p_hi) mine.push_back({c, set, p_lo, p_hi, c_lo, c_hi});
+            }
         }
     }
-    long long W = 0;
-    for (int c = 0; c < S.nconds; c++) W += weight[c];
-    const long long piece_lo = (long long)part * W, piece_hi = (long long)(part + 1) * W;      // cond c covers [start_c * nparts, (start_c + w_c) * nparts)
-    if (int e = ensure(ws->plan, PLAN_HDR * bdg::MAX_PASSES + 8 * bdg::SEED_MAX_CONDS)) return e;
+    const size_t plan_bytes = PLAN_HDR * bdg::MAX_PASSES + 8 * (size_t)S.nconds;
+    if (int e = ensure(ws->plan, plan_bytes)) return e;
     char* d_plan = (char*)ws->plan.p;
-    CU_TRY(cudaMemsetAsync(d_plan, 0, PLAN_HDR * bdg::MAX_PASSES + 8 * bdg::SEED_MAX_CONDS, caller));
+    CU_TRY(cudaMemsetAsync(d_plan, 0, plan_bytes, caller));
     for (int p = 0; p < bdg::MAX_PASSES; p++) ws->host_stats[p][0] = ws->host_stats[p][1] = 0;
     unsigned long long* d_cursors = (unsigned long long*)(d_plan + PLAN_HDR * bdg::MAX_PASSES);
     int max_bits = 0;
@@ -382,62 +421,49 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
     CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_a, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(max_keys + 1), caller));
     CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(n_slabs + 1), caller));
     const size_t tmp_bytes = std::max(tmp_a, tmp_b);
-    bool ranked = true;                                     // counting sort with one atomic per barcode (its place in the bucket is kept)
-    if (const char* e = getenv("BDG_JOIN_RANK")) ranked = atoi(e) != 0;
     for (int k = 0; k < 2; k++) {                           // one scratch set per stream
-        if (int e = ensure(ws->jn_hist[k], (max_keys + 1) * 4 * 2)) return e;       // bucket sizes | fill cursors
+        if (int e = ensure(ws->jn_hist[k], (max_keys + 1) * 4)) return e;
         if (int e = ensure(ws->jn_tab[k], (max_keys + 1) * 4)) return e;
         if (int e = ensure(ws->jn_tabc[k], (max_keys + 1) * 4)) return e;
         if (int e = ensure(ws->jn_rows[k], N * 4)) return e;
         if (int e = ensure(ws->jn_cols[k], N * 4)) return e;
-        if (ranked) { if (int e = ensure(ws->jn_rank[k], N * 4)) return e; }
+        if (int e = ensure(ws->jn_rank[k], N * 4)) return e;
         if (int e = ensure(ws->jn_cub[k], tmp_bytes)) return e;
         if (int e = ensure(ws->jn_counts[k], ((size_t)n_slabs + 1) * 4)) return e;
         if (int e = ensure(ws->jn_offs[k], ((size_t)n_slabs + 1) * 4)) return e;
     }
-    int occ = 6;                                            // resident CTAs per SM the kernel is compiled for (registers per thread follow)
-    if (const char* e = getenv("BDG_JOIN_OCC")) occ = atoi(e) == 4 ? 4 : (atoi(e) == 5 ? 5 : 6);
-    const void* kern = rs == 8 ? (occ == 4 ? (const void*)bdg::join_kernel<8, 4> : occ == 5 ? (const void*)bdg::join_kernel<8, 5> : (const void*)bdg::join_kernel<8, 6>)
-                               : (occ == 4 ? (const void*)bdg::join_kernel<32, 4> : occ == 5 ? (const void*)bdg::join_kernel<32, 5> : (const void*)bdg::join_kernel<32, 6>);
+    const auto kern = rs == 8 ? bdg::join_kernel<T, 8> : bdg::join_kernel<T, 32>;
     int grid = 0;
-    if (int rc = grid_for(kern, &grid, bdg::ENT)) return rc;
+    if (int rc = grid_for((const void*)kern, &grid, bdg::ENT)) return rc;
     if (const char* e = getenv("BDG_JOIN_CTAS")) grid = std::min(grid, ws->sms * std::max(1, atoi(e)));   // CTAs per SM of a join launch
     const int gb = (int)std::min<size_t>((N + 255) / 256, (size_t)ws->sms * 8);
     const int bb = (int)std::min<size_t>(((size_t)n_slabs + 256) / 256, (size_t)ws->sms * 8);
     // Two ways to keep the bucketing of one condition out of the way of the joins.  The resident form forks: its two streams
     // carry whole conditions (bucketing + join) and overlap each other.  The streaming form (js) must be able to say "edges
-    // [0, n) are complete" after every condition, so its joins stay on ONE stream in order, and only the bucketing of the next
+    // [0, n) are complete" after every snapshot, so its joins stay on ONE stream in order, and only the bucketing of the next
     // condition runs ahead on a second stream, into the other scratch set.
     const bool fork = !js && !getenv("BDG_EDGE_SERIAL");
     const bool ahead = js && !getenv("BDG_EDGE_SERIAL");
     if (fork || ahead) CU_TRY(cudaEventRecord(ws->ev_start, caller));
     bool set_joined[2] = {false, false};                     // ahead: a join on scratch set k is in flight / done (ev_join[k] recorded)
     bool aux_used = false;
-    int streamed[bdg::SEED_MAX_CONDS], n_streamed = 0;
+    int n_snaps = 0;
     if (js && !ws->snap_host) {
-        CU_TRY(cudaHostAlloc((void**)&ws->snap_host, sizeof(unsigned long long) * bdg::SEED_MAX_CONDS, cudaHostAllocMapped));
+        CU_TRY(cudaHostAlloc((void**)&ws->snap_host, sizeof(unsigned long long) * bdg::JOIN_MAX_SNAPS, cudaHostAllocMapped));
         CU_TRY(cudaHostGetDevicePointer((void**)&ws->snap_dev, ws->snap_host, 0));
-        for (int c = 0; c < bdg::SEED_MAX_CONDS; c++) CU_TRY(cudaEventCreateWithFlags(&ws->ev_cond[c], cudaEventDisableTiming));
+        for (int q = 0; q < bdg::JOIN_MAX_SNAPS; q++) CU_TRY(cudaEventCreateWithFlags(&ws->ev_snap[q], cudaEventDisableTiming));
         for (int q = 0; q < 2; q++) { CU_TRY(cudaEventCreateWithFlags(&ws->ev_pre[q], cudaEventDisableTiming)); CU_TRY(cudaEventCreateWithFlags(&ws->ev_join[q], cudaEventDisableTiming)); }
     }
     bdg::EdgeOut o{d_a, d_b, d_d, d_count, (unsigned long long)cap};
-    long long start = 0;
     int cur_set = -1, k = 1;                                 // k: scratch set / stream of the current condition
     int row_set[2] = {-1, -1};                               // block set whose row order the scratch set holds
-    const bool trace = getenv("BDG_TRACE") != nullptr;
     double t_prev = 0;
     if (trace) { cudaStreamSynchronize(caller); t_prev = now_ms(); }
-    for (int oi = 0; oi < n_order; oi++) {
-        const int c = order[oi];
-        const long long w = weight[c];
-        const long long c_lo = start * nparts, c_hi = (start + w) * nparts;
-        start += w;
-        const long long lo = std::max(c_lo, piece_lo), hi = std::min(c_hi, piece_hi);
-        if (lo >= hi) continue;
+    for (size_t oi = 0; oi < mine.size(); oi++) {
+        const int c = mine[oi].c, set = mine[oi].set;
         // The whole job alternates its two streams block set by block set (a set sorts its rows once).  A part of several has few
         // conditions, often of one set: it alternates condition by condition, so that the bucketing of one condition runs beside
         // the join of the other, and sorts the rows again when the stream's row order is of another set.
-        const int set = S.cond[c].row_sort;
         if (nparts > 1 || ahead || set != cur_set) k ^= 1;
         cur_set = set;
         const bool new_set = row_set[k] != set;
@@ -453,277 +479,6 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
         auto bucket_side = [&](const bdg::SeedKey& key, Buf& dst, Buf& table) -> int {
             const size_t nkeys = (size_t)1 << key.key_bits;
             uint32_t* hist = (uint32_t*)ws->jn_hist[k].p;
-            uint32_t* fill = hist + (nkeys + 1);
-            size_t bytes = ws->jn_cub[k].cap;
-            if (ranked) {
-                uint32_t* rank = (uint32_t*)ws->jn_rank[k].p;
-                CU_TRY(cudaMemsetAsync(hist, 0, (nkeys + 1) * 4, sp));
-                bdg::join_hist_rank_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, hist, rank);
-                CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)hist, (uint32_t*)table.p, (int)(nkeys + 1), sp));
-                bdg::join_scatter_rank_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, (const uint32_t*)table.p, rank, (uint32_t*)dst.p);
-            } else {
-                CU_TRY(cudaMemsetAsync(hist, 0, (nkeys + 1) * 4 * 2, sp));
-                bdg::join_hist_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, hist);
-                CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)hist, (uint32_t*)table.p, (int)(nkeys + 1), sp));
-                bdg::join_scatter_kernel<<<gb, 256, 0, sp>>>(d_sorted, (uint32_t)N, key, (const uint32_t*)table.p, fill, (uint32_t*)dst.p);
-            }
-            g_launches += 2;
-            return BDG_OK;
-        };
-        if (new_set) { if (int e = bucket_side(S.ka[c], ws->jn_rows[k], ws->jn_tab[k])) return e; }      // the stream's row order: this block set
-        bdg::JoinArgs A{};
-        A.rows = (const uint32_t*)ws->jn_rows[k].p;
-        A.rowstart = (const uint32_t*)ws->jn_tab[k].p;
-        A.nkeys = 1u << S.ka[c].key_bits;
-        if (S.cond[c].self) {
-            A.cols = A.rows;
-            A.colstart = (const uint32_t*)ws->jn_tab[k].p;
-        } else {
-            if (int e = bucket_side(S.kb[c], ws->jn_cols[k], ws->jn_tabc[k])) return e;
-            A.cols = (const uint32_t*)ws->jn_cols[k].p;
-            A.colstart = (const uint32_t*)ws->jn_tabc[k].p;
-        }
-        A.offs = (const uint32_t*)ws->jn_offs[k].p;
-        A.lut = (const uint8_t*)ws->jn_lut.p;
-        A.cursor = d_cursors + c;
-        A.stats = (unsigned long long*)(d_plan + HDR_STATS);
-        A.N = (uint32_t)N;
-        A.n_slabs = n_slabs;
-        A.cond = c;
-        A.self = S.cond[c].self;
-        A.f0 = (uint32_t)(lo - c_lo); A.f1 = (uint32_t)(hi - c_lo); A.fden = (uint32_t)(c_hi - c_lo);
-        A.T = bdg::qgram_threshold(2);
-        A.one = 1u;
-        A.mone = 0xFFFFFFFFu;
-        bdg::join_band_kernel<<<bb, 256, 0, sp>>>(A, (uint32_t*)ws->jn_counts[k].p);
-        size_t bytes = ws->jn_cub[k].cap;
-        CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)ws->jn_counts[k].p, (uint32_t*)ws->jn_offs[k].p, (int)(n_slabs + 1), sp));
-        if (ahead) {
-            CU_TRY(cudaEventRecord(ws->ev_pre[k], sp));
-            CU_TRY(cudaStreamWaitEvent(st, ws->ev_pre[k], 0));
-        }
-        if (rs == 8) {
-            if (occ == 4) bdg::join_kernel<8, 4><<<grid, bdg::ENT, 0, st>>>(A, o);
-            else if (occ == 5) bdg::join_kernel<8, 5><<<grid, bdg::ENT, 0, st>>>(A, o);
-            else bdg::join_kernel<8, 6><<<grid, bdg::ENT, 0, st>>>(A, o);
-        } else {
-            if (occ == 4) bdg::join_kernel<32, 4><<<grid, bdg::ENT, 0, st>>>(A, o);
-            else if (occ == 5) bdg::join_kernel<32, 5><<<grid, bdg::ENT, 0, st>>>(A, o);
-            else bdg::join_kernel<32, 6><<<grid, bdg::ENT, 0, st>>>(A, o);
-        }
-        g_launches += 3;
-        CU_TRY(cudaGetLastError());
-        if (ahead) { CU_TRY(cudaEventRecord(ws->ev_join[k], st)); set_joined[k] = true; }
-        if (trace) {                                        // development aid: per-condition wall time (serialises the streams)
-            CU_TRY(cudaStreamSynchronize(st));
-            const double now = now_ms();
-            fprintf(stderr, "[bdg] join cond %2d (%s, rows %u/%u..%u/%u, weight %lld): %.3f ms\n", c, S.cond[c].self ? "sym" : "shf", A.f0, A.fden, A.f1, A.fden,
-                    weight[c], now - t_prev);
-            t_prev = now;
-        }
-        if (js) {
-            bdg::join_snapshot_kernel<<<1, 1, 0, st>>>(d_count, ws->snap_dev + c);
-            g_launches++;
-            CU_TRY(cudaEventRecord(ws->ev_cond[c], st));
-            streamed[n_streamed++] = c;
-        }
-    }
-    if (aux_used) {
-        CU_TRY(cudaEventRecord(ws->ev_done[1], ws->aux[1]));
-        CU_TRY(cudaStreamWaitEvent(caller, ws->ev_done[1], 0));
-    }
-    if (trace) { cudaStreamSynchronize(caller); fprintf(stderr, "[bdg] join part %d of %d: %.3f ms from entry to the last condition\n", part, nparts, now_ms() - t_weigh); }
-    if (js) {                                               // everything is enqueued: follow the conditions and copy what they have finished
-        cudaStream_t cp = ws->aux[2];
-        size_t done = 0;
-        for (int k = 0; k < n_streamed; k++) {
-            CU_TRY(cudaEventSynchronize(ws->ev_cond[streamed[k]]));
-            const size_t upto = (size_t)std::min<unsigned long long>(ws->snap_host[streamed[k]], js->h_cap);
-            if (upto > done) {
-                CU_TRY(cudaMemcpyAsync(js->h_a + done, d_a + done, (upto - done) * 4, cudaMemcpyDeviceToHost, cp));
-                CU_TRY(cudaMemcpyAsync(js->h_b + done, d_b + done, (upto - done) * 4, cudaMemcpyDeviceToHost, cp));
-                CU_TRY(cudaMemcpyAsync(js->h_d + done, d_d + done, upto - done, cudaMemcpyDeviceToHost, cp));
-                done = upto;
-            }
-        }
-        CU_TRY(cudaStreamSynchronize(cp));
-    }
-    return BDG_OK;
-}
-
-// ---- the t = 3 seed scheme (bdg_seed3.cuh): built once on the host, copied to the device memory of every device that uses it ----
-bdg::Seed3Scheme g_scheme3;
-int g_scheme3_serial = 0;
-
-int scheme3_ready()
-{
-    std::lock_guard<std::mutex> lock(g_scheme_mutex);
-    if (g_scheme3_serial) return BDG_OK;
-    int bases[bdg::SEED3_MAX_BLOCKS] = {3, 2, 2, 2, 2, 2, 2};
-    int nb = 7;
-    if (const char* e = getenv("BDG_JOIN3_BLOCKS")) {         // e.g. "3,3,3,2,2,2": development aid
-        nb = 0;
-        for (const char* p = e; *p && nb < bdg::SEED3_MAX_BLOCKS;) {
-            bases[nb++] = atoi(p);
-            while (*p && *p != ',') p++;
-            if (*p == ',') p++;
-        }
-    }
-    if (!bdg::seed3_scheme_build(g_scheme3, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN3_BLOCKS is not a usable block layout (4..7 blocks of >= 2 bases, 15 bases in all)");
-    g_scheme3_serial = 1;
-    return BDG_OK;
-}
-
-// Join form at t = 3 (bdg_join3.cuh): the structure of launch_edges_join over the t = 3 seed table.  Its conditions are many
-// (475 in the default layout) but come in few block sets (35), so the per-condition pieces that t = 2 keeps in fixed arrays are
-// sized by SEED3_MAX_CONDS here, the work estimate runs block set by block set (one row table and the set's column tables at a
-// time), and the streaming form snapshots the edge count once per block set rather than once per condition.
-int launch_edges_join3(const uint32_t* d_sorted, size_t N, int part, int nparts, uint32_t* d_a, uint32_t* d_b, uint8_t* d_d, size_t cap,
-                       unsigned long long* d_count, cudaStream_t caller, DevCtx* ws, const JoinStream* js = nullptr)
-{
-    if (int rc = scheme3_ready()) return rc;
-    const bdg::Seed3Scheme& S = g_scheme3;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    if (ws->scheme3_serial != g_scheme3_serial) {
-        if (int e = ensure(ws->jn3_scheme, sizeof(bdg::Seed3Scheme))) return e;
-        CU_TRY(cudaMemcpyAsync(ws->jn3_scheme.p, &g_scheme3, sizeof(g_scheme3), cudaMemcpyHostToDevice, caller));
-        CU_TRY(cudaStreamSynchronize(caller));              // the host copy above is read asynchronously
-        ws->scheme3_serial = g_scheme3_serial;
-    }
-    const bdg::Seed3Scheme* d_scheme = (const bdg::Seed3Scheme*)ws->jn3_scheme.p;
-    int rs = (N >> S.ka[0].key_bits) < 48 ? 8 : 32;
-    if (const char* e = getenv("BDG_JOIN_RS")) rs = atoi(e) == 8 ? 8 : 32;
-    int owner_first = 0;                                    // hand-over walk after the exact distance (DESIGN.md 3.8)
-    if (const char* e = getenv("BDG_JOIN3_OWNER_FIRST")) owner_first = atoi(e) != 0;
-    const uint32_t n_slabs = (uint32_t)((N + bdg::JROWS - 1) / bdg::JROWS);
-    const bool trace = getenv("BDG_TRACE") != nullptr;
-    std::vector<long long> weight(S.nconds, 1);
-    const double t_weigh = trace ? (cudaStreamSynchronize(caller), now_ms()) : 0.0;
-    if (nparts > 1 || trace) {
-        // Pairs of every condition estimated from bucket sizes over a sample, block set by block set; the cost model of the t = 2
-        // form (launch_edges_join) is reused as it stands: time ~ pairs x (1.45 symmetric, 1 shifted) + 2.4 x N.
-        int max_set = 1, max_bits = 0;
-        for (int k = 0; k < S.nsets; k++) max_set = std::max(max_set, (int)(S.set_first[k + 1] - S.set_first[k]));
-        for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
-        const uint32_t tab = 1u << max_bits;
-        const uint32_t stride = (uint32_t)std::max<size_t>(1, (N + (1u << 17) - 1) >> 17);
-        const size_t hist_bytes = (size_t)max_set * tab * 4;
-        if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * (size_t)bdg::SEED3_MAX_CONDS)) return e;
-        uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
-        unsigned long long* d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
-        CU_TRY(cudaMemsetAsync(d_pairs, 0, 8 * (size_t)S.nconds, caller));
-        const uint32_t m = (uint32_t)((N + stride - 1) / stride);
-        for (int k = 0; k < S.nsets; k++) {
-            const int c0 = S.set_first[k], c1 = S.set_first[k + 1];
-            CU_TRY(cudaMemsetAsync(d_hist, 0, (size_t)(c1 - c0) * tab * 4, caller));
-            bdg::join3_weigh_hist_kernel<<<(int)std::min<uint32_t>((m + 255) / 256, (uint32_t)ws->sms * 8), 256, 0, caller>>>(d_sorted, (uint32_t)N, stride, d_scheme, c0, c1, tab, d_hist);
-            bdg::join3_weigh_sum_kernel<<<dim3((tab + 1023) / 1024, c1 - c0), 256, 0, caller>>>(d_hist, tab, c0, d_pairs);
-            g_launches += 2;
-        }
-        std::vector<unsigned long long> pairs(S.nconds), cost(S.nconds);
-        CU_TRY(cudaMemcpyAsync(pairs.data(), d_pairs, 8 * (size_t)S.nconds, cudaMemcpyDeviceToHost, caller));
-        CU_TRY(cudaStreamSynchronize(caller));
-        unsigned long long top = 1;
-        for (int c = 0; c < S.nconds; c++) {
-            cost[c] = pairs[c] * stride * stride * (S.cond[c].self ? 29 : 20) + 48ull * N;
-            top = std::max(top, cost[c]);
-        }
-        for (int c = 0; c < S.nconds; c++) weight[c] = (long long)std::max<unsigned long long>(1, cost[c] * 4096 / top);
-        if (trace) {
-            fprintf(stderr, "[bdg] join3 work estimate: %.3f ms\n", now_ms() - t_weigh);
-            fprintf(stderr, "[bdg] join3 estimated pairs:");
-            for (int c = 0; c < S.nconds; c++) fprintf(stderr, " %llu", pairs[c] * stride * stride);
-            fprintf(stderr, "\n");
-        }
-    }
-    // block sets alternately from the front and the back of the table, as at t = 2
-    std::vector<int> order;
-    for (int i = 0, lo = 0, hi = S.nsets - 1; lo <= hi; i++) {
-        const int k = (i & 1) ? hi-- : lo++;
-        for (int c = S.set_first[k]; c < S.set_first[k + 1]; c++) order.push_back(c);
-    }
-    long long W = 0;
-    for (int c = 0; c < S.nconds; c++) W += weight[c];
-    const long long piece_lo = (long long)part * W, piece_hi = (long long)(part + 1) * W;
-    const size_t plan_bytes = PLAN_HDR * bdg::MAX_PASSES + 8 * (size_t)bdg::SEED3_MAX_CONDS;
-    if (int e = ensure(ws->plan, plan_bytes)) return e;
-    char* d_plan = (char*)ws->plan.p;
-    CU_TRY(cudaMemsetAsync(d_plan, 0, plan_bytes, caller));
-    for (int p = 0; p < bdg::MAX_PASSES; p++) ws->host_stats[p][0] = ws->host_stats[p][1] = 0;
-    unsigned long long* d_cursors = (unsigned long long*)(d_plan + PLAN_HDR * bdg::MAX_PASSES);
-    int max_bits = 0;
-    for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
-    const size_t max_keys = (size_t)1 << max_bits;
-    size_t tmp_a = 0, tmp_b = 0;
-    CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_a, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(max_keys + 1), caller));
-    CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(n_slabs + 1), caller));
-    const size_t tmp_bytes = std::max(tmp_a, tmp_b);
-    for (int k = 0; k < 2; k++) {
-        if (int e = ensure(ws->jn_hist[k], (max_keys + 1) * 4 * 2)) return e;
-        if (int e = ensure(ws->jn_tab[k], (max_keys + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_tabc[k], (max_keys + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_rows[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_cols[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_rank[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_cub[k], tmp_bytes)) return e;
-        if (int e = ensure(ws->jn_counts[k], ((size_t)n_slabs + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_offs[k], ((size_t)n_slabs + 1) * 4)) return e;
-    }
-    const void* kern = rs == 8 ? (const void*)bdg::join3_kernel<8> : (const void*)bdg::join3_kernel<32>;
-    int grid = 0;
-    if (int rc = grid_for(kern, &grid, bdg::ENT)) return rc;
-    if (const char* e = getenv("BDG_JOIN_CTAS")) grid = std::min(grid, ws->sms * std::max(1, atoi(e)));
-    const int gb = (int)std::min<size_t>((N + 255) / 256, (size_t)ws->sms * 8);
-    const int bb = (int)std::min<size_t>(((size_t)n_slabs + 256) / 256, (size_t)ws->sms * 8);
-    const bool fork = !js && !getenv("BDG_EDGE_SERIAL");
-    const bool ahead = js && !getenv("BDG_EDGE_SERIAL");
-    if (fork || ahead) CU_TRY(cudaEventRecord(ws->ev_start, caller));
-    bool set_joined[2] = {false, false};
-    bool aux_used = false;
-    int n_snaps = 0;
-    if (js && !ws->snap_host) {
-        CU_TRY(cudaHostAlloc((void**)&ws->snap_host, sizeof(unsigned long long) * bdg::SEED_MAX_CONDS, cudaHostAllocMapped));
-        CU_TRY(cudaHostGetDevicePointer((void**)&ws->snap_dev, ws->snap_host, 0));
-        for (int c = 0; c < bdg::SEED_MAX_CONDS; c++) CU_TRY(cudaEventCreateWithFlags(&ws->ev_cond[c], cudaEventDisableTiming));
-        for (int q = 0; q < 2; q++) { CU_TRY(cudaEventCreateWithFlags(&ws->ev_pre[q], cudaEventDisableTiming)); CU_TRY(cudaEventCreateWithFlags(&ws->ev_join[q], cudaEventDisableTiming)); }
-    }
-    bdg::EdgeOut o{d_a, d_b, d_d, d_count, (unsigned long long)cap};
-    long long start = 0;
-    int cur_set = -1, k = 1;
-    int row_set[2] = {-1, -1};
-    double t_prev = 0;
-    if (trace) { cudaStreamSynchronize(caller); t_prev = now_ms(); }
-    std::vector<int> mine;                                  // the conditions this part works on, in order, with their row ranges
-    std::vector<long long> m_lo, m_hi, m_clo, m_chi;
-    for (int c : order) {
-        const long long w = weight[c];
-        const long long c_lo = start * nparts, c_hi = (start + w) * nparts;
-        start += w;
-        const long long lo = std::max(c_lo, piece_lo), hi = std::min(c_hi, piece_hi);
-        if (lo >= hi) continue;
-        mine.push_back(c); m_lo.push_back(lo); m_hi.push_back(hi); m_clo.push_back(c_lo); m_chi.push_back(c_hi);
-    }
-    for (size_t oi = 0; oi < mine.size(); oi++) {
-        const int c = mine[oi];
-        const int set = S.cond[c].set;
-        if (nparts > 1 || ahead || set != cur_set) k ^= 1;
-        cur_set = set;
-        const bool new_set = row_set[k] != set;
-        row_set[k] = set;
-        cudaStream_t st = (fork && k == 1) ? ws->aux[1] : caller;
-        cudaStream_t sp = ahead ? ws->aux[1] : st;
-        if (fork && k == 1 && !aux_used) { CU_TRY(cudaStreamWaitEvent(st, ws->ev_start, 0)); aux_used = true; }
-        if (ahead) {
-            if (!aux_used) { CU_TRY(cudaStreamWaitEvent(sp, ws->ev_start, 0)); aux_used = true; }
-            if (set_joined[k]) CU_TRY(cudaStreamWaitEvent(sp, ws->ev_join[k], 0));
-        }
-        auto bucket_side = [&](const bdg::SeedKey& key, Buf& dst, Buf& table) -> int {
-            const size_t nkeys = (size_t)1 << key.key_bits;
-            uint32_t* hist = (uint32_t*)ws->jn_hist[k].p;
             uint32_t* rank = (uint32_t*)ws->jn_rank[k].p;
             size_t bytes = ws->jn_cub[k].cap;
             CU_TRY(cudaMemsetAsync(hist, 0, (nkeys + 1) * 4, sp));
@@ -733,9 +488,8 @@ int launch_edges_join3(const uint32_t* d_sorted, size_t N, int part, int nparts,
             g_launches += 2;
             return BDG_OK;
         };
-        if (new_set) { if (int e = bucket_side(S.ka[S.set_first[set]], ws->jn_rows[k], ws->jn_tab[k])) return e; }
-        bdg::Join3Args A3{};
-        bdg::JoinArgs& A = A3.j;
+        if (new_set) { if (int e = bucket_side(S.ka[S.set_first[set]], ws->jn_rows[k], ws->jn_tab[k])) return e; }      // the stream's row order: this block set
+        bdg::JoinArgsT<T> A{};
         A.rows = (const uint32_t*)ws->jn_rows[k].p;
         A.rowstart = (const uint32_t*)ws->jn_tab[k].p;
         A.nkeys = 1u << S.ka[c].key_bits;
@@ -754,37 +508,39 @@ int launch_edges_join3(const uint32_t* d_sorted, size_t N, int part, int nparts,
         A.n_slabs = n_slabs;
         A.cond = c;
         A.self = S.cond[c].self;
-        A.f0 = (uint32_t)(m_lo[oi] - m_clo[oi]); A.f1 = (uint32_t)(m_hi[oi] - m_clo[oi]); A.fden = (uint32_t)(m_chi[oi] - m_clo[oi]);
-        A.T = bdg::qgram_threshold(3);
+        A.f0 = (uint32_t)(mine[oi].lo - mine[oi].c_lo); A.f1 = (uint32_t)(mine[oi].hi - mine[oi].c_lo); A.fden = (uint32_t)(mine[oi].c_hi - mine[oi].c_lo);
+        A.T = bdg::qgram_threshold(T);
         A.one = 1u;
         A.mone = 0xFFFFFFFFu;
-        A3.ka = S.ka[c];
-        A3.kb = S.kb[c];
-        A3.scheme = d_scheme;
-        A3.owner_first = owner_first;
-        bdg::join3_band_kernel<<<bb, 256, 0, sp>>>(A3, (uint32_t*)ws->jn_counts[k].p);
+        if constexpr (T == 2) {
+            A.lut = (const uint8_t*)ws->jn_lut.p;
+        } else {
+            A.ka = S.ka[c];
+            A.kb = S.kb[c];
+            A.scheme = (const bdg::Seed3Scheme*)ws->jn3_scheme.p;
+        }
+        bdg::join_band_kernel<T><<<bb, 256, 0, sp>>>(A, (uint32_t*)ws->jn_counts[k].p);
         size_t bytes = ws->jn_cub[k].cap;
         CU_TRY(cub::DeviceScan::ExclusiveSum(ws->jn_cub[k].p, bytes, (const uint32_t*)ws->jn_counts[k].p, (uint32_t*)ws->jn_offs[k].p, (int)(n_slabs + 1), sp));
         if (ahead) {
             CU_TRY(cudaEventRecord(ws->ev_pre[k], sp));
             CU_TRY(cudaStreamWaitEvent(st, ws->ev_pre[k], 0));
         }
-        if (rs == 8) bdg::join3_kernel<8><<<grid, bdg::ENT, 0, st>>>(A3, o);
-        else bdg::join3_kernel<32><<<grid, bdg::ENT, 0, st>>>(A3, o);
+        kern<<<grid, bdg::ENT, 0, st>>>(A, o);
         g_launches += 3;
         CU_TRY(cudaGetLastError());
         if (ahead) { CU_TRY(cudaEventRecord(ws->ev_join[k], st)); set_joined[k] = true; }
-        if (trace) {
+        if (trace) {                                        // development aid: per-condition wall time (serialises the streams)
             CU_TRY(cudaStreamSynchronize(st));
             const double now = now_ms();
-            fprintf(stderr, "[bdg] join3 cond %3d (set %2d, %s, rows %u/%u..%u/%u, weight %lld): %.3f ms\n", c, set, S.cond[c].self ? "sym" : "shf",
+            fprintf(stderr, "[bdg] join cond %3d (set %2d, %s, rows %u/%u..%u/%u, weight %lld): %.3f ms\n", c, set, S.cond[c].self ? "sym" : "shf",
                     A.f0, A.fden, A.f1, A.fden, weight[c], now - t_prev);
             t_prev = now;
         }
-        if (js && (oi + 1 == mine.size() || S.cond[mine[oi + 1]].set != set)) {      // the last condition of a block set
+        if (js && (T == 2 || oi + 1 == mine.size() || mine[oi + 1].set != set)) {
             bdg::join_snapshot_kernel<<<1, 1, 0, st>>>(d_count, ws->snap_dev + n_snaps);
             g_launches++;
-            CU_TRY(cudaEventRecord(ws->ev_cond[n_snaps], st));
+            CU_TRY(cudaEventRecord(ws->ev_snap[n_snaps], st));
             n_snaps++;
         }
     }
@@ -792,12 +548,12 @@ int launch_edges_join3(const uint32_t* d_sorted, size_t N, int part, int nparts,
         CU_TRY(cudaEventRecord(ws->ev_done[1], ws->aux[1]));
         CU_TRY(cudaStreamWaitEvent(caller, ws->ev_done[1], 0));
     }
-    if (trace) { cudaStreamSynchronize(caller); fprintf(stderr, "[bdg] join3 part %d of %d: %.3f ms from entry to the last condition\n", part, nparts, now_ms() - t_weigh); }
-    if (js) {
+    if (trace) { cudaStreamSynchronize(caller); fprintf(stderr, "[bdg] join part %d of %d: %.3f ms from entry to the last condition\n", part, nparts, now_ms() - t_weigh); }
+    if (js) {                                               // everything is enqueued: follow the snapshots and copy what they have finished
         cudaStream_t cp = ws->aux[2];
         size_t done = 0;
         for (int q = 0; q < n_snaps; q++) {
-            CU_TRY(cudaEventSynchronize(ws->ev_cond[q]));
+            CU_TRY(cudaEventSynchronize(ws->ev_snap[q]));
             const size_t upto = (size_t)std::min<unsigned long long>(ws->snap_host[q], js->h_cap);
             if (upto > done) {
                 CU_TRY(cudaMemcpyAsync(js->h_a + done, d_a + done, (upto - done) * 4, cudaMemcpyDeviceToHost, cp));
@@ -822,8 +578,8 @@ int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts
     CU_TRY(cudaMemsetAsync(d_count, 0, sizeof(unsigned long long), st));
     if (t <= 0 || N < 2) return BDG_OK;   // D >= 1 for distinct barcodes: no edges (barcode_graph.py:245)
     const int mode = edge_mode_for(t, N);
-    if (mode == 2) return t == 3 ? launch_edges_join3(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js)
-                                 : launch_edges_join(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js);
+    if (mode == 2) return t == 3 ? launch_edges_join<3>(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js)
+                                 : launch_edges_join<2>(d_sorted, N, part, nparts, d_a, d_b, d_d, cap, d_count, st, ws, js);
     const bool sparse = mode == 1;
     const int passes = sparse ? bdg::n_passes(t) : 1;
     const void* kern = sparse ? (t == 1 ? (const void*)bdg::sparse_tile_kernel<1, 0, false> : (const void*)bdg::sparse_tile_kernel<2, 0, false>)
@@ -1139,7 +895,7 @@ void bdg_shutdown(void)
         }
         c.jn_lut.release(); c.jn_weigh.release(); for (auto& b : c.jn_rank) b.release();
         c.jn3_scheme.release();
-        if (c.snap_host) { cudaFreeHost(c.snap_host); c.snap_host = nullptr; for (auto& e : c.ev_cond) if (e) cudaEventDestroy(e);
+        if (c.snap_host) { cudaFreeHost(c.snap_host); c.snap_host = nullptr; for (auto& e : c.ev_snap) if (e) cudaEventDestroy(e);
                            for (int q = 0; q < 2; q++) { if (c.ev_pre[q]) cudaEventDestroy(c.ev_pre[q]); if (c.ev_join[q]) cudaEventDestroy(c.ev_join[q]); } }
     }
     g_ctx.clear();

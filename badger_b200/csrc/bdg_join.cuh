@@ -1,4 +1,4 @@
-// bdg_join.cuh -- edge construction at t = 2 by sort-merge joins on multi-block seeds (bdg_seed.cuh); sm_100a.
+// bdg_join.cuh -- edge construction at t = 2 and t = 3 by sort-merge joins on multi-block seeds (bdg_seed.cuh, bdg_seed3.cuh); sm_100a.
 // Reference semantics: index.py:77-93 (candidate filter S >= T) + barcode_graph.py:233-249 (3-way edit-distance verify, emit).
 //
 // Per condition c of the seed scheme the N barcodes are bucketed by the condition's join key (the kernels read a key off a
@@ -7,22 +7,31 @@
 // are then adjacent on both sides: row i pairs with the column run colstart[key(i)] .. colstart[key(i) + 1].
 //   join_hist_rank_kernel / join_scatter_rank_kernel  counting sort by the join key (one digit; cub's scan turns the bucket
 //                          sizes into colstart, the first column of every key value) with one atomic per barcode: the counting
-//                          pass keeps the place its atomic returned.  (join_hist_kernel / join_scatter_kernel: the two-atomic
-//                          form, BDG_JOIN_RANK=0.)
-//   join_band_kernel       per slab of 32 consecutive rows: number of work units (runs of <= JUNIT columns) it needs
+//                          pass keeps the place its atomic returned.
+//   join_band_kernel<T>    per slab of 32 consecutive rows: number of work units (runs of <= JUNIT columns) it needs
 //   (cub::DeviceScan::ExclusiveSum: unit index -> slab)
-//   join_kernel<RS>        one persistent launch per condition: warps pull batches of units from an atomic cursor, stage the
+//   join_kernel<T, RS>     one persistent launch per condition: warps pull batches of units from an atomic cursor, stage the
 //                          unit's columns in their own slice of shared memory (y, y >> 2, y << 2, key) and test
 //                          (row, column) pairs: quick test of bdg_core.cuh + key equality, one hit bit per pair; hits go
-//                          through the warp's queue to the exact stage on full warps (dist_small, hand-over table, then
-//                          the 6-mer score in a second queue), edges are appended with one atomic per warp.
+//                          through the warp's queue to the exact stage on full warps, edges are appended with one atomic per warp.
 // A unit's 32 rows are worked through as 32/RS sub-slabs of RS rows x 32/RS column phases, each against its own column run:
 // RS = 32 when the key buckets are long, RS = 8 when they are short (fewer rows span fewer foreign buckets).
-// The conditions are dealt to the parts (GPUs / ranks) by estimated work (join_weigh_*), a condition on a part boundary is split
-// by row range at a bucket boundary (join_cut), so a part sorts only the conditions it works on.  No block-level barrier anywhere.
+// What differs between the thresholds T is the per-pair stage:
+//   T = 2  quick test on the diagonals -1..1 (quick_marks), two marks dropped; exact stage join_process: dist_small, the
+//          hand-over table over seed_flags, then the 6-mer score in two queues (the middle diagonals, then the other eighteen).
+//   T = 3  quick test on the diagonals -2..2 (quick3_marks; the +-2 words are derived from the staged +-1 ones), three marks
+//          dropped; exact stage join3_process: dist3_min (Myers' bit-vector pass; D <= 3 has no case analysis), the hand-over
+//          walk seed3_first, then the 6-mer score through one queue.  The t = 3 scheme is too large for constant memory next to
+//          the t = 2 one: the kernels read the condition's two keys from their arguments and the hand-over tables from a device
+//          copy of the Seed3Scheme.
+// The conditions are dealt to the parts (GPUs / ranks) by estimated work (join_weigh_*, join3_weigh_*), a condition on a part
+// boundary is split by row range at a bucket boundary (join_cut), so a part sorts only the conditions it works on.  No
+// block-level barrier anywhere.
 #pragma once
+#include <type_traits>
 #include "bdg_edges.cuh"
 #include "bdg_seed.cuh"
+#include "bdg_seed3.cuh"
 
 namespace bdg {
 
@@ -30,9 +39,11 @@ constexpr int JCH = 128;           // columns staged at a time
 constexpr int JPAD = 32;           // slack behind the staged columns (steps may start up to one step early)
 constexpr int JUNIT = 2048;        // columns per work unit
 constexpr int JBATCH = 4;          // units per cursor fetch
-constexpr int JQCAP = 120;         // candidate queue entries per warp (with the other arrays: 6 CTAs of 8 warps per SM)
-constexpr int JQ2CAP = 64;         // entries of each of the two scoring queues
+constexpr int JQCAP = 120;         // candidate queue entries per warp (with the other arrays: 6 CTAs of 8 warps per SM at t = 2)
+constexpr int JQ2CAP = 64;         // entries of each scoring queue (two at t = 2, one at t = 3)
 constexpr int JROWS = 32;          // rows per slab
+// edge-count snapshots of the streaming form: one after every condition at t = 2, one after every block set at t = 3
+constexpr int JOIN_MAX_SNAPS = SEED_MAX_CONDS > SEED3_MAX_SETS ? SEED_MAX_CONDS : SEED3_MAX_SETS;
 
 __constant__ SeedScheme c_scheme;
 
@@ -41,9 +52,9 @@ struct JoinArgs {
     const uint32_t* cols;          // ... of the column-side key (== rows for a symmetric condition)
     const uint32_t* colstart;      // (1 << key_bits) + 1 lower bounds into cols
     const uint32_t* offs;          // exclusive prefix sums of the units per slab: n_slabs + 1 entries
-    const uint8_t* lut;            // hand-over table over seed_flags
+    const uint8_t* lut;            // t = 2: hand-over table over seed_flags
     unsigned long long* cursor;    // batches handed out by this launch
-    unsigned long long* stats;     // [0] units, [2] pairs tested, [3] candidates, [6] pairs with D <= 2, [7] pairs scored, [4]/[5] warp times
+    unsigned long long* stats;     // [0] units, [2] pairs tested, [3] candidates, [6] pairs with D <= t, [7] of those owned and scored, [4]/[5] warp times
     uint32_t N, n_slabs;
     int cond, self;
     const uint32_t* rowstart;      // (1 << key_bits) + 1 lower bounds into rows (== colstart for a symmetric condition)
@@ -53,27 +64,33 @@ struct JoinArgs {
     uint32_t one, mone;            // runtime 1 / -1: u * one + mone is u - 1 on the FMA pipe
 };
 
+// t = 3: the keys and the hand-over tables travel with the launch (the t = 2 ones sit in c_scheme)
+struct Join3Args : JoinArgs {
+    SeedKey ka, kb;                // the condition's row-side / column-side key
+    const Seed3Scheme* scheme;     // device copy: hand-over tables
+};
+
+template <int T>
+using JoinArgsT = std::conditional_t<T == 2, JoinArgs, Join3Args>;
+
+template <int T>
+__device__ __forceinline__ const SeedKey& join_ka(const JoinArgsT<T>& A)
+{
+    if constexpr (T == 2) return c_scheme.ka[A.cond]; else return A.ka;
+}
+
+template <int T>
+__device__ __forceinline__ const SeedKey& join_kb(const JoinArgsT<T>& A)
+{
+    if constexpr (T == 2) return c_scheme.kb[A.cond]; else return A.kb;
+}
+
 // ---- bucketing by join key: a counting sort in three launches (the key has <= 20 bits, so ONE digit: no radix passes) ----
-//   join_hist_kernel     bucket sizes (one global atomic per barcode; the 2^key_bits counters stay in L2)
+//   join_hist_rank_kernel     bucket sizes (one global atomic per barcode; the 2^key_bits counters stay in L2); each barcode
+//                             keeps what its atomic returned, its place inside its bucket
 //   (cub::DeviceScan::ExclusiveSum over the counters: colstart, the first position of every key value)
-//   join_scatter_kernel  every barcode to the next free slot of its bucket
+//   join_scatter_rank_kernel  every barcode to start[key] + place
 // The order inside a bucket is whatever the atomics give: the join pairs whole buckets, so it does not matter.
-__global__ void join_hist_kernel(const uint32_t* __restrict__ in, uint32_t n, SeedKey k, uint32_t* __restrict__ hist)
-{
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) atomicAdd(&hist[seed_key(__ldg(&in[i]), k)], 1u);
-}
-
-__global__ void join_scatter_kernel(const uint32_t* __restrict__ in, uint32_t n, SeedKey k, const uint32_t* __restrict__ start, uint32_t* __restrict__ fill,
-                                    uint32_t* __restrict__ out)
-{
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
-        const uint32_t v = __ldg(&in[i]), key = seed_key(v, k);
-        out[__ldg(&start[key]) + atomicAdd(&fill[key], 1u)] = v;
-    }
-}
-
-// The same sort with ONE atomic per barcode: the counting pass keeps what its atomic returned (the barcode's place inside its
-// bucket), the scatter is then a plain gather of start[key] + place.
 __global__ void join_hist_rank_kernel(const uint32_t* __restrict__ in, uint32_t n, SeedKey k, uint32_t* __restrict__ hist, uint32_t* __restrict__ rank)
 {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) rank[i] = atomicAdd(&hist[seed_key(__ldg(&in[i]), k)], 1u);
@@ -108,6 +125,7 @@ __device__ __forceinline__ uint32_t join_cut(const uint32_t* __restrict__ rowsta
 // Bucket sizes of every condition over a SAMPLE of the barcodes (every stride-th one): the number of (row, column) pairs a
 // condition has to test is sum_k rows_k * cols_k (a symmetric one: sum_k n_k (n_k - 1) / 2), and the sample's sum times
 // stride^2 estimates it.  Integer counts over the same sample on every part, so every part computes the same deal.
+// t = 2 samples all its tables in one pass; t = 3 goes block set by block set, because its 475 tables do not fit at once.
 struct WeighSlots { uint8_t row[SEED_MAX_CONDS], col[SEED_MAX_CONDS]; int n; };   // table of a condition's row / column key (a block set shares its row table)
 
 __global__ void join_weigh_hist_kernel(const uint32_t* __restrict__ in, uint32_t n, uint32_t stride, int nconds, uint32_t tab, const WeighSlots ws,
@@ -145,6 +163,35 @@ __global__ void join_weigh_sum_kernel(const uint32_t* __restrict__ hist, uint32_
     if ((threadIdx.x & 31) == 0 && mine) atomicAdd(&out[c], mine);
 }
 
+// Work estimate of the t = 3 conditions c0 .. c1 - 1 of one block set: table 0 holds the row key of the set (its first,
+// symmetric, condition), table c - c0 the column key of condition c.
+__global__ void join3_weigh_hist_kernel(const uint32_t* __restrict__ in, uint32_t n, uint32_t stride, const Seed3Scheme* __restrict__ S, int c0, int c1,
+                                        uint32_t tab, uint32_t* __restrict__ hist)
+{
+    const uint32_t m = (n + stride - 1) / stride;
+    for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < m; j += gridDim.x * blockDim.x) {
+        const uint32_t x = __ldg(&in[(uint64_t)j * stride]);
+        atomicAdd(&hist[seed_key(x, S->ka[c0])], 1u);
+        for (int c = c0 + 1; c < c1; c++) atomicAdd(&hist[(size_t)(c - c0) * tab + seed_key(x, S->kb[c])], 1u);
+    }
+}
+
+// grid (x, c1 - c0): pairs of condition c0 + blockIdx.y over the sample
+__global__ void join3_weigh_sum_kernel(const uint32_t* __restrict__ hist, uint32_t tab, int c0, unsigned long long* __restrict__ out)
+{
+    const int q = blockIdx.y;
+    const uint32_t* __restrict__ hr = hist;
+    const uint32_t* __restrict__ hc = hist + (size_t)q * tab;
+    unsigned long long mine = 0;
+    for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < tab; k += gridDim.x * blockDim.x) {
+        const unsigned long long r = __ldg(&hr[k]);
+        if (q == 0) mine += r * (r - (r ? 1 : 0)) / 2;
+        else if (r) mine += r * __ldg(&hc[k]);
+    }
+    for (int o = 16; o; o >>= 1) mine += __shfl_down_sync(FULL, mine, o);
+    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(&out[c0 + q], mine);
+}
+
 // the edge count as it stands when the stream reaches this point (bdg_edges_build_into copies the finished edges out meanwhile)
 __global__ void join_snapshot_kernel(const unsigned long long* __restrict__ count, volatile unsigned long long* __restrict__ snap)
 {
@@ -153,9 +200,10 @@ __global__ void join_snapshot_kernel(const unsigned long long* __restrict__ coun
 
 // units of every slab of 32 rows: its column run (first key's bucket .. last key's bucket; a symmetric condition pairs
 // each couple once - column index > row index - so its run starts behind the slab's first row) in pieces of JUNIT columns
-__global__ void join_band_kernel(const JoinArgs A, uint32_t* __restrict__ counts)
+template <int T>
+__global__ void join_band_kernel(const JoinArgsT<T> A, uint32_t* __restrict__ counts)
 {
-    const SeedKey& ka = c_scheme.ka[A.cond];
+    const SeedKey& ka = join_ka<T>(A);
     const uint32_t r0 = join_cut(A.rowstart, A.nkeys, A.N, A.f0, A.fden), r1 = join_cut(A.rowstart, A.nkeys, A.N, A.f1, A.fden);
     for (uint32_t s = blockIdx.x * blockDim.x + threadIdx.x; s <= A.n_slabs; s += gridDim.x * blockDim.x) {
         uint32_t cnt = 0;
@@ -174,15 +222,16 @@ __global__ void join_band_kernel(const JoinArgs A, uint32_t* __restrict__ counts
 
 struct JoinCtx {
     uint2* q;                      // candidates (x, y): row value, column value
-    uint2* q2;                     // (a, b) with D <= 2 that still need the 6-mer score
+    uint2* q2;                     // (a, b) with D <= t owned by this pass that still need the 6-mer score
     uint8_t* q2d;
-    const uint8_t* lut;
+    const uint8_t* lut;            // t = 2: hand-over table
     int lane, T, cond, shifted;    // shifted: 1 for a condition with a shifted diagonal (its two value orders are two hand-over indices)
-    unsigned long long n_d2, n_score;
+    unsigned long long n_near, n_owned;   // pairs with D <= t; of those, owned by this pass and handed to the score
+    const Seed3Scheme* scheme;     // t = 3: hand-over tables
 };
 
-// exact stage on a batch of candidates of one condition (one per lane): D by case analysis, hand-over table, survivors into the
-// scoring queue, full batches of that queue through the 6-mer score.  A real call, not inlined: one copy of the exact distance
+// t = 2 exact stage on a batch of candidates of one condition (one per lane): D by case analysis, hand-over table, survivors into
+// the scoring queue, full batches of that queue through the 6-mer score.  A real call, not inlined: one copy of the exact distance
 // and of the score loop keeps the kernel's hot code inside the instruction cache (ncu: the fully inlined form spent most of its
 // issue slots waiting for instructions).  Everything travels in registers: returns the two queue fills (8 bits each) | pairs
 // with D <= 2 << 16 | pairs handed to the score << 24.
@@ -235,6 +284,43 @@ __device__ __noinline__ uint32_t join_process(uint2* q2, uint8_t* q2d, const uin
     return (uint32_t)n1 | ((uint32_t)n2 << 8) | (n_d2 << 16) | ((uint32_t)__popc(m) << 24);
 }
 
+// t = 3 exact stage on a batch of candidates (one per lane): D, hand-over walk, survivors into the scoring queue, full batches of
+// that queue through the 6-mer score.  Not inlined, as at t = 2: one copy of the bit-vector pass, the walk and the score loop.
+// The walk runs after the distance, on the candidates within D <= 3 only (DESIGN.md 3.8).
+// Returns the queue fill | pairs with D <= 3 << 16 | pairs owned by this pass << 24, the packing of join_process.
+__device__ __noinline__ uint32_t join3_process(uint2* q2, uint8_t* q2d, const Seed3Scheme* S, int want0, int want1, int T, const EdgeOut out,
+                                               uint2 e, bool active, int n1)
+{
+    const int lane = threadIdx.x & 31;
+    const uint32_t a = min(e.x, e.y), b = max(e.x, e.y);
+    const int want = e.x > e.y ? want1 : want0;
+    bool ok = active && a != b;
+    int d = 4;
+    if (ok) { d = dist3_min(a, b); ok = d <= 3; }
+    const uint32_t n_d3 = (uint32_t)__popc(__ballot_sync(FULL, ok));
+    if (ok) ok = seed3_first(*S, a, b) == want;          // emitted by the first (condition, orientation) the pair meets
+    const uint32_t n_own = (uint32_t)__popc(__ballot_sync(FULL, ok));
+    const unsigned m = __ballot_sync(FULL, ok);
+    if (m) {
+        if (ok) {                                        // fewer than 32 entries wait on entry, so 32 more always fit
+            const int slot = n1 + __popc(m & ((1u << lane) - 1u));
+            q2[slot] = make_uint2(a, b);
+            q2d[slot] = (uint8_t)d;
+        }
+        n1 += __popc(m);
+        __syncwarp();
+        if (n1 >= 32) {
+            n1 -= 32;
+            const uint2 v = q2[n1 + lane];
+            const uint8_t vd = q2d[n1 + lane];
+            emit_warp(qgram_score_compact(v.x, v.y) >= T, v.x, v.y, vd, out);
+            __syncwarp();
+        }
+    }
+    return (uint32_t)n1 | (n_d3 << 16) | (n_own << 24);
+}
+
+template <int T>
 __device__ __forceinline__ void join_drain(JoinCtx& c, const EdgeOut& out, int& qn, int& q2n, bool all)
 {
     __syncwarp();
@@ -242,16 +328,18 @@ __device__ __forceinline__ void join_drain(JoinCtx& c, const EdgeOut& out, int& 
         const int take = min(qn, 32);
         qn -= take;
         const uint2 e = c.lane < take ? c.q[qn + c.lane] : make_uint2(0u, 0u);
-        const uint32_t r = join_process(c.q2, c.q2d, c.lut, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n);
+        uint32_t r;
+        if constexpr (T == 2) r = join_process(c.q2, c.q2d, c.lut, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n);
+        else r = join3_process(c.q2, c.q2d, c.scheme, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n);
         q2n = (int)(r & 0xFFFFu);
-        c.n_d2 += (r >> 16) & 255u;
-        c.n_score += r >> 24;
+        c.n_near += (r >> 16) & 255u;
+        c.n_owned += r >> 24;
         __syncwarp();
     }
 }
 
 // append the hits of a group of 8 steps: bit 4 * st + kk of h = column colbase + st * STEP + kk of the staged sub-tile
-template <int STEP>
+template <int T, int STEP>
 __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t* sb0, int colbase, int& qn, int& q2n, JoinCtx& c, const EdgeOut& out)
 {
     const int cnt = __popc(h);
@@ -270,7 +358,7 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
             c.q[slot++] = make_uint2(x, sb0[colbase + (j >> 2) * STEP + (j & 3)]);
         }
         qn += total;
-        join_drain(c, out, qn, q2n, false);
+        join_drain<T>(c, out, qn, q2n, false);
         return;
     }
     for (;;) {                                           // burst larger than the queue: one hit per lane and round
@@ -283,19 +371,20 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
             c.q[qn + __popc(m & ((1u << c.lane) - 1u))] = make_uint2(x, sb0[colbase + (j >> 2) * STEP + (j & 3)]);
         }
         qn += __popc(m);                                 // qn < 32 before every round, so the round's <= 32 entries fit
-        join_drain(c, out, qn, q2n, false);
+        join_drain<T>(c, out, qn, q2n, false);
     }
 }
 
-template <int RS, int OCC>
-__global__ void __launch_bounds__(ENT, OCC) join_kernel(const JoinArgs A, const EdgeOut out)
+// T = 2 is compiled for 6 resident CTAs per SM (40 registers), T = 3 for 4: its exact stage needs the registers
+template <int T, int RS>
+__global__ void __launch_bounds__(ENT, T == 2 ? 6 : 4) join_kernel(const JoinArgsT<T> A, const EdgeOut out)
 {
     constexpr int PH = 32 / RS;                          // column phases of a warp
     constexpr int STEP = 4 * PH;                         // columns per inner step
     __shared__ __align__(16) uint32_t s_b[EW][4][JCH + JPAD];   // y, y >> 2, y << 2, key of the staged columns
     __shared__ uint2 s_q[EW][JQCAP];
-    __shared__ uint2 s_q2[EW][2 * JQ2CAP];              // pairs that need their score | pairs that need the far diagonals
-    __shared__ uint8_t s_q2d[EW][2 * JQ2CAP];
+    __shared__ uint2 s_q2[EW][T == 2 ? 2 * JQ2CAP : JQ2CAP];   // pairs that need their score | (t = 2) pairs that need the far diagonals
+    __shared__ uint8_t s_q2d[EW][T == 2 ? 2 * JQ2CAP : JQ2CAP];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int r = lane & (RS - 1), ph = lane / RS;
     uint32_t* const sb0 = s_b[wid][0];
@@ -303,13 +392,15 @@ __global__ void __launch_bounds__(ENT, OCC) join_kernel(const JoinArgs A, const 
     uint32_t* const sbM = s_b[wid][2];
     uint32_t* const sbK = s_b[wid][3];
     JoinCtx c;
-    c.q = s_q[wid]; c.q2 = s_q2[wid]; c.q2d = s_q2d[wid]; c.lut = A.lut; c.lane = lane; c.T = A.T; c.cond = A.cond; c.shifted = A.self ? 0 : 1; c.n_d2 = 0; c.n_score = 0;
+    c.q = s_q[wid]; c.q2 = s_q2[wid]; c.q2d = s_q2d[wid];
+    if constexpr (T == 2) c.lut = A.lut; else c.scheme = A.scheme;
+    c.lane = lane; c.T = A.T; c.cond = A.cond; c.shifted = A.self ? 0 : 1; c.n_near = 0; c.n_owned = 0;
     int qn = 0, q2n = 0;
     const uint32_t mone = A.mone;
     const unsigned long long t_start = global_ns();
     unsigned long long n_units = 0, n_pairs = 0, n_cand = 0;
-    const SeedKey& ka = c_scheme.ka[A.cond];
-    const SeedKey& kb = c_scheme.kb[A.cond];
+    const SeedKey& ka = join_ka<T>(A);
+    const SeedKey& kb = join_kb<T>(A);
     const bool self = A.self != 0;
     const uint32_t total_units = __ldg(&A.offs[A.n_slabs]);
     const uint32_t n_batches = (total_units + JBATCH - 1) / JBATCH;
@@ -390,9 +481,11 @@ __global__ void __launch_bounds__(ENT, OCC) join_kernel(const JoinArgs A, const 
                                 const uint4 BK = *reinterpret_cast<const uint4*>(&sbK[off]);
 #pragma unroll
                                 for (int kk = 0; kk < 4; kk++) {
-                                    uint32_t w = quick_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk));
-                                    w &= w * A.one + mone;   // drop the two lowest marks (IMAD keeps the -1 off the ALU pipe)
+                                    uint32_t w = T == 2 ? quick_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk))
+                                                        : quick3_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk));
+                                    w &= w * A.one + mone;   // drop the t lowest marks (IMAD keeps the -1 off the ALU pipe)
                                     w &= w * A.one + mone;
+                                    if constexpr (T == 3) w &= w * A.one + mone;
                                     bool hit = w == 0 && pick4(BK, kk) == kq;
                                     if (self) hit = hit && base + (uint32_t)(off + kk) > iq;
                                     h |= (hit ? 1u : 0u) << (st * 4 + kk);
@@ -401,15 +494,15 @@ __global__ void __launch_bounds__(ENT, OCC) join_kernel(const JoinArgs A, const 
                         }
                         if (__any_sync(FULL, h != 0)) {
                             n_cand += __popc(h);
-                            join_push<STEP>(h, xq, sb0, g0 + 4 * ph, qn, q2n, c, out);
+                            join_push<T, STEP>(h, xq, sb0, g0 + 4 * ph, qn, q2n, c, out);
                         }
                     }
                 }
             }
         }
     }
-    join_drain(c, out, qn, q2n, true);
-    {                                                    // what is left in the two scoring queues: fewer than 32 each
+    join_drain<T>(c, out, qn, q2n, true);
+    {                                                    // what is left in the scoring queues: fewer than 32 each
         const int n1 = q2n & 255, n2 = q2n >> 8;
         bool ok = false;
         uint32_t a = 0, b = 0;
@@ -420,20 +513,22 @@ __global__ void __launch_bounds__(ENT, OCC) join_kernel(const JoinArgs A, const 
             ok = qgram_score_compact(a, b) >= A.T;
         }
         emit_warp(ok, a, b, d, out);
-        ok = false;
-        if (lane < n2) {
-            const uint2 e = c.q2[JQ2CAP + lane];
-            const uint8_t fd = c.q2d[JQ2CAP + lane];
-            a = e.x; b = e.y; d = fd & 3;
-            ok = (int)(fd >> 2) + qgram_score_far(a, b) >= A.T;
+        if constexpr (T == 2) {                          // the far diagonals of the undecided
+            ok = false;
+            if (lane < n2) {
+                const uint2 e = c.q2[JQ2CAP + lane];
+                const uint8_t fd = c.q2d[JQ2CAP + lane];
+                a = e.x; b = e.y; d = fd & 3;
+                ok = (int)(fd >> 2) + qgram_score_far(a, b) >= A.T;
+            }
+            emit_warp(ok, a, b, d, out);
         }
-        emit_warp(ok, a, b, d, out);
     }
     if (A.stats) {
         for (int o = 16; o; o >>= 1) n_cand += __shfl_down_sync(FULL, n_cand, o);           // per-lane counts
         if (lane == 0) {                                                                  // the others are uniform per warp
             atomicAdd(&A.stats[0], n_units); atomicAdd(&A.stats[2], n_pairs * (unsigned long long)RS); atomicAdd(&A.stats[3], n_cand);
-            atomicAdd(&A.stats[6], c.n_d2); atomicAdd(&A.stats[7], c.n_score);
+            atomicAdd(&A.stats[6], c.n_near); atomicAdd(&A.stats[7], c.n_owned);
             warp_exit_stats(A.stats, t_start);
         }
     }

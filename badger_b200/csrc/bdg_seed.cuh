@@ -66,6 +66,8 @@ struct SeedScheme {
     int nflags;                                            // bits of seed_flags: 3 per block
     uint32_t hi_mask, lo_mask;                             // top bit of every block / the other bits of the blocks
     uint32_t fmask[SEED_MAX_BLOCKS], fnet[SEED_MAX_BLOCKS]; // seed_flags: where block k's three flags sit in the zero-field word, and how far they move down
+    int nsets;                                             // block sets, as in Seed3Scheme: the conditions of set s are
+    uint16_t set_first[SEED_MAX_CONDS + 1];                // set_first[s] .. set_first[s + 1] - 1
 };
 
 // x[fields of condition c] == y[the same fields moved by their diagonals]
@@ -137,6 +139,7 @@ inline bool seed_scheme_build(SeedScheme& s, const int* bases, int nblocks)
             if (popc(sub) != nf) continue;
             int blk[SEED_MAX_FIELDS], q = 0;
             for (int k = 0; k < nblocks; k++) if (sub & (1u << k)) blk[q++] = k;
+            s.set_first[s.nsets++] = (uint16_t)s.nconds;        // every set has its symmetric condition, so it is never empty
             for (uint32_t dm = 0; dm < (1u << nf); dm++) {      // bit f: diagonal of field f
                 bool ok = true;
                 if (blk[0] == 0 && (dm & 1u)) ok = false;                                     // block 0 sits on diagonal 0
@@ -171,6 +174,7 @@ inline bool seed_scheme_build(SeedScheme& s, const int* bases, int nblocks)
             }
         }
     }
+    s.set_first[s.nsets] = (uint16_t)s.nconds;
     for (int c = 0; c < s.nconds; c++) s.nself += s.cond[c].self;
     return true;
 }

@@ -1,4 +1,4 @@
-// bdg_seed3.cuh -- multi-block seeds for the t = 3 edge construction by sort-merge joins (bdg_join3.cuh).
+// bdg_seed3.cuh -- multi-block seeds for the t = 3 edge construction by sort-merge joins (bdg_join.cuh).
 //
 // What is searched (reference index.py:77-93 + barcode_graph.py:233-249): pairs a < b with D(a,b) <= 3 and S(a,b) >= 4
 // (T(3) = 4, the same candidate threshold as t = 2).  The necessary condition extends the t = 2 one of bdg_seed.cuh:
@@ -36,7 +36,6 @@ constexpr int SEED3_MAX_BLOCKS = 7;
 constexpr int SEED3_MAX_CONDS = 640;
 constexpr int SEED3_MAX_SETS = 35;                 // C(7, 4): block sets of the largest layout
 constexpr int SEED3_NONE = 0xFFFF;
-static_assert(SEED3_MAX_SETS <= SEED_MAX_CONDS, "the streaming form keeps one edge-count snapshot per block set in the t = 2 slots");
 
 struct Seed3Cond {
     uint8_t nf;                       // number of blocks in the condition (B - 3)

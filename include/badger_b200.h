@@ -195,7 +195,7 @@ int bdg_dev_edges_build(const uint32_t* d_sorted, size_t N, int t, int part, int
                         uint32_t* d_b, uint8_t* d_d, size_t cap, unsigned long long* d_count, void* stream);
 /* How the edge set is searched (results are identical; DESIGN.md "edge construction"):
  *   2 join (t = 2, 3): sort-merge joins on multi-block seeds - per seed condition the array is sorted by the condition's
- *     key, equal-key buckets are paired and only those pairs are tested (bdg_join.cuh, bdg_join3.cuh); the default for t = 2
+ *     key, equal-key buckets are paired and only those pairs are tested (bdg_join.cuh); the default for t = 2
  *     from BDG_JOIN_MIN_N (150 000) distinct barcodes upwards, for t = 3 from BDG_JOIN3_MIN_N (90 000) upwards;
  *   1 sparse (default otherwise): one pass per prefilter block over the array sorted by a rotated key, pairs are decided
  *     tile by tile from key intervals and scored only inside the tiles that can hold a candidate;
@@ -210,9 +210,8 @@ int bdg_set_edge_mode(int mode);
  * mode only).  Synchronises the stream.  (bench.py's roofline numerator.) */
 int bdg_dev_edges_stats(unsigned long long* out5, void* stream);
 /* The kernels' eight raw counters of the last edge launch on the current device, summed over its passes.  Join form: [0] work
- * units, [2] pairs tested, [3] candidates handed to the exact stage, [6] candidates with D <= 2, [7] pairs whose 6-mer score was
- * computed (t = 3: [6] candidates with D <= 3, [7] of those this condition owns; with BDG_JOIN3_OWNER_FIRST=1 the hand-over
- * runs first and [6] counts only the owned ones); [4] / [5] sum / max over the warps of their busy time in ns.  Synchronises the stream. */
+ * units, [2] pairs tested, [3] candidates handed to the exact stage, [6] candidates with D <= t, [7] of those, the ones this
+ * condition owns, whose 6-mer score was computed; [4] / [5] sum / max over the warps of their busy time in ns.  Synchronises the stream. */
 int bdg_dev_edges_stats_raw(unsigned long long* out8, void* stream);
 /* Development aid: out[2p], out[2p+1] = sum and max over the warps of pass p of (warp exit - first warp start), ns. */
 int bdg_dev_edges_balance(unsigned long long* out6, void* stream);

@@ -72,6 +72,8 @@ int shim_scheme(const int* bases, int nblocks)          // returns the number of
 int shim_scheme_nself(void) { return g_scheme.nself; }
 int shim_scheme_key_bits(int c) { return g_scheme.ka[c].key_bits; }
 int shim_scheme_row_sort(int c) { return g_scheme.cond[c].row_sort; }
+int shim_scheme_nsets(void) { return g_scheme.nsets; }
+int shim_scheme_set_first(int k) { return g_scheme.set_first[k]; }
 // first (condition, orientation) by the definition and by the table over the block-match flags
 void shim_scheme_first(const uint32_t* a, const uint32_t* b, size_t n, uint8_t* slow, uint8_t* fast)
 {

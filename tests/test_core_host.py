@@ -447,6 +447,11 @@ def test_seed_scheme_tables(shim):
             assert shim.shim_scheme_row_sort(c) <= c
             fired |= pred.astype(bool) & (first == 2 * c)
         assert fired.sum() > 1000
+        # the block sets as the driver walks them: consecutive runs of conditions that share their row order
+        set_first = [shim.shim_scheme_set_first(k) for k in range(shim.shim_scheme_nsets() + 1)]
+        assert set_first[0] == 0 and set_first[-1] == nc and all(x < y for x, y in zip(set_first, set_first[1:]))
+        for k in range(len(set_first) - 1):
+            assert all(shim.shim_scheme_row_sort(c) == set_first[k] for c in range(set_first[k], set_first[k + 1]))
 
 
 @pytest.mark.parametrize("name", ["4", "5", "6"])

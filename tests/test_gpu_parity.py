@@ -30,8 +30,8 @@ MODES = {"dense": 0, "sparse": 1, "join": 2}
 @pytest.fixture(params=["sparse", "dense", "join"])
 def mode(request):
     """Every search strategy of the edge construction (include/badger_b200.h bdg_set_edge_mode) must give the
-    reference's edge set.  The join form exists for t = 2 only: asked for at another threshold, the library takes the
-    sparse / dense route, and the edge set must still be the reference's."""
+    reference's edge set.  The join form exists for t = 2 and t = 3: asked for at another threshold, the library takes
+    the sparse / dense route, and the edge set must still be the reference's."""
     L = badger_b200.lib()
     badger_b200._lib.check(L.bdg_set_edge_mode(MODES[request.param]))
     yield request.param

@@ -1,4 +1,4 @@
-"""Edge construction at t = 3 by the join form (bdg_join3.cuh) against the CPU oracle: forced with bdg_set_edge_mode(2) and
+"""Edge construction at t = 3 by the join form (bdg_join.cuh) against the CPU oracle: forced with bdg_set_edge_mode(2) and
 BDG_JOIN3_MIN_N=0 so that small inputs take it too."""
 import os
 
@@ -111,14 +111,6 @@ def test_join3_edge_buffer_regrow(monkeypatch):
     badger_b200._lib.check(badger_b200.lib().bdg_set_edge_mode(2))
     got = edge_rows(*ops.edges_build(s, 3))
     assert np.array_equal(got, want)
-
-
-def test_join3_owner_first_same_edges(monkeypatch):
-    """The two orders of the exact stage (hand-over walk before / after the distance) give the same edge set."""
-    s = clustered_set(58, 200, 10000, 0.08)
-    want = edge_rows(*ops.edges_build(s, 3))
-    monkeypatch.setenv("BDG_JOIN3_OWNER_FIRST", "1")
-    assert np.array_equal(edge_rows(*ops.edges_build(s, 3)), want)
 
 
 @pytest.mark.parametrize("nparts", [1, 2, 3, 8])

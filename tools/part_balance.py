@@ -51,12 +51,13 @@ def main():
     whole, edges = timed(0, 1)
     print("%s N=%d t=%d: whole job %.3f ms, %d edges" % (cfg_name, n, t, whole, edges))
     for nparts in (2, 4, 8):
-        ms, tot = [], 0
+        ms, es = [], []
         for p in range(nparts):
             m, e = timed(p, nparts)
-            ms.append(m); tot += e
-        print("nparts=%d  parts %s  max %.3f ms  sum %.3f ms  efficiency %.3f  edges %s" % (
-            nparts, " ".join("%.2f" % x for x in ms), max(ms), sum(ms), whole / (nparts * max(ms)), "ok" if tot == edges else "MISMATCH %d" % tot))
+            ms.append(m); es.append(e)
+        print("nparts=%d  parts %s  max %.3f ms  sum %.3f ms  efficiency %.3f  edges %s  per part %s" % (
+            nparts, " ".join("%.2f" % x for x in ms), max(ms), sum(ms), whole / (nparts * max(ms)),
+            "ok" if sum(es) == edges else "MISMATCH %d" % sum(es), " ".join(str(e) for e in es)))
 
 
 if __name__ == "__main__":

@@ -1,4 +1,4 @@
-"""Edge construction at t = 3 on one GPU: the join form (bdg_join3.cuh) against the dense all-pairs kernel.
+"""Edge construction at t = 3 on one GPU: the join form (bdg_join.cuh) against the dense all-pairs kernel.
 
 Random subsets of the C4 set (the C4 synthetic data, 4.57e6 distinct barcodes) at growing sizes, both forms while the dense one
 finishes in seconds, then the join alone up to the full set.  Per size and form: device time per step (CUDA events around
@@ -7,7 +7,7 @@ candidates, candidates with D <= 3, owned pairs).  Where both forms run, their e
 One JSON line per measurement on stdout, appended to --out as well when given.
 
   python tools/t3_time.py [--dense 25000,50000,100000,200000] [--join 25000,50000,100000,200000,1000000,full] [--steps 3]
-Environment: BDG_JOIN3_BLOCKS / BDG_JOIN3_OWNER_FIRST pick the layout / the order of the exact stage (read once per process)."""
+Environment: BDG_JOIN3_BLOCKS picks the layout (read once per process)."""
 import argparse
 import ctypes as C
 import json
@@ -99,8 +99,7 @@ def main():
                 r, edges = run(torch, L, s, mode, args.steps, flush)
                 res[form] = edges
                 rec = dict(form=form, N=int(s.size), t=3, ms=round(r["ms"], 3), ms_all=r["ms_all"], edges=r["edges"],
-                           layout=os.environ.get("BDG_JOIN3_BLOCKS", "3,2,2,2,2,2,2"), owner_first=os.environ.get("BDG_JOIN3_OWNER_FIRST", "0"),
-                           gpu=label)
+                           layout=os.environ.get("BDG_JOIN3_BLOCKS", "3,2,2,2,2,2,2"), gpu=label)
                 if form == "join":
                     raw = r["raw"]
                     rec.update(units=raw[0], pairs_tested=raw[2], candidates=raw[3], cand_d_le3=raw[6], owned=raw[7],
