@@ -82,6 +82,12 @@ def lib():
     L.bdg_dev_pack16.argtypes = [_vp, _sz, _vp, _vp, _vp]
     L.bdg_dev_member_sorted.argtypes = [_vp, _sz, _vp, _sz, _vp, _vp]
     L.bdg_dev_nearest_bounded.argtypes = [_vp, _sz, _vp, _sz, _i, _vp, _vp, _vp, _vp]
+    L.bdg_dev_dedup_reads.argtypes = [_vp, _vp, _sz, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong), _vp]
+    L.bdg_dev_dedup_fetch.argtypes = [C.c_ulonglong, _vp, _vp, _vp, _vp, _vp]
+    L.bdg_dev_pack16_sorted.argtypes = [_vp, _sz, _vp, C.POINTER(_sz), _vp]
+    L.bdg_dev_centres_above.argtypes = [C.c_ulonglong, _sz, _vp, _sz, _vp, _vp, _vp, _sz, C.POINTER(_sz), C.POINTER(C.c_double), _vp]
+    L.bdg_dev_edges_copy.argtypes = [_vp, _vp, _vp, _vp, _vp]
+    L.bdg_dev_assign_reads32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, C.POINTER(_sz), _vp]
     L.bdg_part_pairs.argtypes = [_sz, _i, _i]
     L.bdg_part_pairs.restype = C.c_ulonglong
     L.bdg_dev_pipe_probe.argtypes = [_i, _i, _i, _vp, C.POINTER(C.c_ulonglong), _vp]
@@ -102,7 +108,8 @@ def lib():
     for name in ("bdg_init", "bdg_host_alloc", "bdg_pack16", "bdg_dedup_first_seen", "bdg_edges_build", "bdg_edges_build_part", "bdg_edges_build_resident", "bdg_edges_build_into", "bdg_edges_copy", "bdg_cluster_levels", "bdg_cluster_levels_from_edges", "bdg_member_sorted",
                  "bdg_nearest_bounded", "bdg_kmer_score", "bdg_kmer_index_create", "bdg_kmer_index_query", "bdg_dev_edges_build", "bdg_set_edge_mode", "bdg_dev_edges_stats", "bdg_dev_edges_stats_raw", "bdg_dev_edges_balance", "bdg_dev_pack16", "bdg_dev_member_sorted",
                  "bdg_dev_nearest_bounded", "bdg_dev_pipe_probe", "bdg_tsv_open", "bdg_tsv_barcodes", "bdg_tsv_write_assignments", "bdg_lines16_open", "bdg_dedup_reads", "bdg_assign_reads", "bdg_pack16_sorted", "bdg_assign_reads32", "bdg_dedup_fetch", "bdg_centres_above", "bdg_centres_rest", "bdg_cluster_resident",
-                 "bdg_tsv_write_assignments32"):
+                 "bdg_tsv_write_assignments32", "bdg_dev_dedup_reads", "bdg_dev_dedup_fetch", "bdg_dev_pack16_sorted", "bdg_dev_centres_above",
+                 "bdg_dev_edges_copy", "bdg_dev_assign_reads32"):
         getattr(L, name).restype = _i
     _lib = L
     return L
@@ -113,15 +120,26 @@ def check(rc: int) -> None:
         raise BadgerB200Error(rc, (lib().bdg_last_error() or b"").decode(errors="replace"))
 
 
+_first_device = 0        # the first device of the last successful init (a call that initialises the library itself claims all, from 0)
+
+
 def init(device_ids=None) -> int:
     """bdg_init: claim the listed CUDA devices (default: all visible). Returns the device count."""
+    global _first_device
     L = lib()
-    if device_ids is None:
+    if not device_ids:
         check(L.bdg_init(None, 0))
+        _first_device = 0
     else:
         arr = (C.c_int * len(device_ids))(*device_ids)
         check(L.bdg_init(arr, len(device_ids)))
+        _first_device = int(device_ids[0])
     return L.bdg_device_count()
+
+
+def first_device() -> int:
+    """The CUDA device the read map and the bdg_dev_* correction-step calls live on: the first device given to init()."""
+    return _first_device
 
 
 def ptr(a: np.ndarray):

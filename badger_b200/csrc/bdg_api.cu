@@ -112,6 +112,7 @@ struct DevCtx {
     cudaEvent_t ev_pre[2] = {nullptr, nullptr}, ev_join[2] = {nullptr, nullptr};   // streaming form: scratch set k is bucketed / its join has finished
     unsigned long long* snap_host = nullptr;                  // mapped page-locked: the edge count at every snapshot
     unsigned long long* snap_dev = nullptr;
+    cudaEvent_t ev_caller = nullptr;                          // bdg_dev_* correction-step calls: orders this device's stream against the caller's
 };
 std::vector<DevCtx> g_ctx;
 
@@ -786,6 +787,41 @@ size_t edge_cap_guess(size_t N, int t, int nparts)
     return std::max<size_t>(1u << 16, per_row * N / (size_t)nparts + 1024);
 }
 
+// The bdg_dev_* forms of the correction step read and write caller memory on the first claimed device, where the read map lives.
+int check_on_first(const void* p, const char* what)
+{
+    cudaPointerAttributes a;
+    if (cudaPointerGetAttributes(&a, p) != cudaSuccess) {
+        (void)cudaGetLastError();
+        return fail(BDG_ERR_ARG, "%s is not a CUDA pointer", what);
+    }
+    if ((a.type != cudaMemoryTypeDevice && a.type != cudaMemoryTypeManaged) || a.device != g_ctx[0].dev)
+        return fail(BDG_ERR_ARG, "%s is not memory of device %d (the first claimed device)", what, g_ctx[0].dev);
+    return BDG_OK;
+}
+
+// Stream order of a bdg_dev_* call that runs on the library's stream of the first device: begin() holds that stream until the
+// work the caller queued on its own stream so far is done (it produces the inputs and frees the output buffers); the
+// destructor, on every return path, holds the caller's stream until the library's work is done (it writes the outputs and
+// reads the inputs).
+struct CallerOrder {
+    DevCtx& c;
+    cudaStream_t caller;
+    bool armed = false;
+    CallerOrder(DevCtx& c_, void* stream) : c(c_), caller((cudaStream_t)stream) {}
+    int begin()
+    {
+        CU_TRY(cudaEventRecord(c.ev_caller, caller));
+        CU_TRY(cudaStreamWaitEvent(c.stream, c.ev_caller, 0));
+        armed = true;
+        return BDG_OK;
+    }
+    ~CallerOrder()
+    {
+        if (armed && cudaEventRecord(c.ev_caller, c.stream) == cudaSuccess) cudaStreamWaitEvent(caller, c.ev_caller, 0);
+    }
+};
+
 }  // namespace
 
 // Handle of one edge construction: the edges stay in the devices' grow-only workspaces until the caller copies them
@@ -841,6 +877,7 @@ int bdg_init(const int* device_ids, int n_devices)
         c.sms = prop.multiProcessorCount;
         CU_TRY(cudaStreamCreateWithFlags(&c.stream, cudaStreamNonBlocking));
         CU_TRY(cudaEventCreateWithFlags(&c.ev_start, cudaEventDisableTiming));
+        CU_TRY(cudaEventCreateWithFlags(&c.ev_caller, cudaEventDisableTiming));
         for (int p = 1; p < bdg::MAX_PASSES; p++) {
             CU_TRY(cudaStreamCreateWithFlags(&c.aux[p], cudaStreamNonBlocking));
             CU_TRY(cudaEventCreateWithFlags(&c.ev_done[p], cudaEventDisableTiming));
@@ -881,6 +918,7 @@ void bdg_shutdown(void)
             if (c.ev_done[p]) cudaEventDestroy(c.ev_done[p]);
         }
         if (c.ev_start) cudaEventDestroy(c.ev_start);
+        if (c.ev_caller) cudaEventDestroy(c.ev_caller);
         for (auto& b : c.dd) b.release();
         for (auto& b : c.nn) b.release();
         for (auto& b : c.io) b.release();
@@ -1151,17 +1189,12 @@ int bdg_dedup_first_seen(const uint32_t* ranks, size_t R, uint32_t* distinct, ui
 }
 
 // ---- f-1 + f-2 on the device: masked dedup that keeps the read map resident, and the per-read gather that uses it ------
-int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos,
-                    uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+// ranks / valid are host arrays (kind = cudaMemcpyHostToDevice) or device arrays on c.dev (cudaMemcpyDeviceToDevice): the masked
+// compaction reads device ranks in place; the valid bytes are always copied, because the per-read gather reads them again.
+static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* valid, size_t R_all, cudaMemcpyKind kind, uint32_t* distinct,
+                            uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid,
+                            unsigned long long* token)
 {
-    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_distinct = 0; *n_valid = 0; *token = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R_all > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
     cudaStream_t st = c.stream;
     c.map_token = 0;
     c.cl_token = 0;
@@ -1184,11 +1217,15 @@ int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, u
         size_t tmp = 0;
         CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, d_excl, (int)R_all, st));
         if (int e = ensure(c.as[3], tmp)) return e;
-        CU_TRY(cudaMemcpyAsync(c.as[0].p, ranks, R_all * 4, cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaMemcpyAsync(c.as[1].p, valid, R_all, cudaMemcpyHostToDevice, st));
+        const uint32_t* d_ranks = ranks;
+        if (kind == cudaMemcpyHostToDevice) {
+            CU_TRY(cudaMemcpyAsync(c.as[0].p, ranks, R_all * 4, kind, st));
+            d_ranks = (const uint32_t*)c.as[0].p;
+        }
+        CU_TRY(cudaMemcpyAsync(c.as[1].p, valid, R_all, kind, st));
         CU_TRY(cub::DeviceScan::ExclusiveSum(c.as[3].p, tmp, flags, d_excl, (int)R_all, st));
         const int blocks = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
-        bdg::compact_valid_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)c.as[0].p, d_valid, d_excl, (uint32_t)R_all, (uint32_t*)c.dd[0].p);
+        bdg::compact_valid_kernel<<<blocks, 256, 0, st>>>(d_ranks, d_valid, d_excl, (uint32_t)R_all, (uint32_t*)c.dd[0].p);
         g_launches++;
         uint32_t last_excl = 0;
         uint8_t last_valid = 0;
@@ -1197,7 +1234,7 @@ int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, u
         CU_TRY(cudaStreamSynchronize(st));
         n_reads = (size_t)last_excl + (last_valid ? 1 : 0);
     } else {
-        CU_TRY(cudaMemcpyAsync(c.dd[0].p, ranks, R_all * 4, cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaMemcpyAsync(c.dd[0].p, ranks, R_all * 4, kind, st));
     }
     *n_valid = n_reads;
     c.map_rows = R_all; c.map_reads = n_reads; c.map_distinct = 0;
@@ -1209,38 +1246,86 @@ int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, u
     return BDG_OK;
 }
 
-// What bdg_dedup_reads left on the device, on demand (any pointer may be NULL): the arrays of its output list.
+int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos,
+                    uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+{
+    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *n_valid = 0; *token = 0;
+    if (R_all == 0) return BDG_OK;
+    if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R_all > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    return dedup_reads_core(c, ranks, valid, R_all, cudaMemcpyHostToDevice, distinct, counts, sorted_pos, sorted_distinct, n_distinct, n_valid, token);
+}
+
+int bdg_dev_dedup_reads(const uint32_t* d_ranks, const uint8_t* d_valid, size_t R_all, size_t* n_distinct, size_t* n_valid,
+                        unsigned long long* token, void* stream)
+{
+    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *n_valid = 0; *token = 0;
+    if (R_all == 0) return BDG_OK;
+    if (!d_ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R_all > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int rc = check_on_first(d_ranks, "ranks")) return rc;
+    if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    return dedup_reads_core(c, d_ranks, d_valid, R_all, cudaMemcpyDeviceToDevice, nullptr, nullptr, nullptr, nullptr, n_distinct, n_valid, token);
+}
+
+// What bdg_dedup_reads left on the device, on demand (any pointer may be NULL): the arrays of its output list, to the host
+// (kind = cudaMemcpyDeviceToHost, the call waits for the copies) or to device memory on c.dev (stream-ordered, no wait).
+static int dedup_fetch_core(DevCtx& c, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, cudaMemcpyKind kind)
+{
+    const size_t n = c.map_distinct;
+    if (distinct) CU_TRY(cudaMemcpyAsync(distinct, c.dd[2].p, n * 4, kind, c.stream));
+    if (counts) CU_TRY(cudaMemcpyAsync(counts, c.dd[0].p, n * 4, kind, c.stream));
+    if (sorted_pos) CU_TRY(cudaMemcpyAsync(sorted_pos, c.dd[1].p, n * 4, kind, c.stream));
+    if (sorted_distinct) CU_TRY(cudaMemcpyAsync(sorted_distinct, c.dd[6].p, n * 4, kind, c.stream));
+    if (kind == cudaMemcpyDeviceToHost) CU_TRY(cudaStreamSynchronize(c.stream));
+    return BDG_OK;
+}
+
 int bdg_dedup_fetch(unsigned long long token, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct)
 {
     if (int rc = need_ctx()) return rc;
     DevCtx& c = g_ctx[0];
     if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
     CU_TRY(cudaSetDevice(c.dev));
-    const size_t n = c.map_distinct;
-    if (distinct) CU_TRY(cudaMemcpyAsync(distinct, c.dd[2].p, n * 4, cudaMemcpyDeviceToHost, c.stream));
-    if (counts) CU_TRY(cudaMemcpyAsync(counts, c.dd[0].p, n * 4, cudaMemcpyDeviceToHost, c.stream));
-    if (sorted_pos) CU_TRY(cudaMemcpyAsync(sorted_pos, c.dd[1].p, n * 4, cudaMemcpyDeviceToHost, c.stream));
-    if (sorted_distinct) CU_TRY(cudaMemcpyAsync(sorted_distinct, c.dd[6].p, n * 4, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
-    return BDG_OK;
+    return dedup_fetch_core(c, distinct, counts, sorted_pos, sorted_distinct, cudaMemcpyDeviceToHost);
+}
+
+int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t* d_counts, uint32_t* d_sorted_pos, uint32_t* d_sorted_distinct,
+                        void* stream)
+{
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    CU_TRY(cudaSetDevice(c.dev));
+    uint32_t* outs[4] = {d_distinct, d_counts, d_sorted_pos, d_sorted_distinct};
+    for (uint32_t* p : outs)
+        if (p && c.map_distinct) if (int rc = check_on_first(p, "output")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    return dedup_fetch_core(c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice);
 }
 
 // ---- a-6 / centre selection, barcode_graph.py:252-267, over the distinct barcodes a dedup call left on the device ----
 // cutoff = max(mean(counts of the first n_cells barcodes in first-seen order) / 5, 5) (:255-256); the barcodes with
 // count > cutoff in count-descending order, ties in first-seen order (the head of `bc_by_counts`, :253), with their counts and
 // - when a whitelist is given - their membership (:264).  The short walk over that head stays with the caller.
-int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* sorted_wl, size_t W, uint32_t* top_ranks, uint32_t* top_counts,
-                      uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
+// sorted_wl is a host array (wl_on_device false: uploaded into io[0]) or device memory on c.dev, read in place.
+static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_wl, bool wl_on_device, size_t W, uint32_t* top_ranks,
+                              uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
 {
-    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_above = 0; *cutoff = 0.0;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
     const size_t N = c.map_distinct;
     const size_t first = std::min(n_cells, N);
     if (first == 0) return fail(BDG_ERR_ARG, "mean requires at least one data point");
-    CU_TRY(cudaSetDevice(c.dev));
     cudaStream_t st = c.stream;
     auto ensure = [&](Buf& b, size_t bytes) -> int {
         if (cudaError_t e = (cudaError_t)b.ensure(bytes))
@@ -1290,16 +1375,20 @@ int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* 
     if (top_hits) {
         if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
         if (W && !sorted_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
-        if (int e = ensure(c.io[0], std::max<size_t>(W, 1) * 4)) return e;
         if (int e = ensure(c.io[3], 8)) return e;
         unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
-        CU_TRY(cudaMemcpyAsync(c.io[0].p, sorted_wl, W * 4, cudaMemcpyHostToDevice, st));
+        const uint32_t* d_wl = sorted_wl;
+        if (!wl_on_device) {
+            if (int e = ensure(c.io[0], std::max<size_t>(W, 1) * 4)) return e;
+            CU_TRY(cudaMemcpyAsync(c.io[0].p, sorted_wl, W * 4, cudaMemcpyHostToDevice, st));
+            d_wl = (const uint32_t*)c.io[0].p;
+        }
         CU_TRY(cudaMemsetAsync(d_bad, 0xFF, 8, st));
         if (W > 1) {
-            bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, st>>>((const uint32_t*)c.io[0].p, (uint32_t)W, d_bad);
+            bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, st>>>(d_wl, (uint32_t)W, d_bad);
             g_launches++;
         }
-        if (int rc = bdg_dev_member_sorted((const uint32_t*)c.io[0].p, W, (const uint32_t*)c.ce[4].p, nsel, (uint8_t*)c.ce[6].p, st)) return rc;
+        if (int rc = bdg_dev_member_sorted(d_wl, W, (const uint32_t*)c.ce[4].p, nsel, (uint8_t*)c.ce[6].p, st)) return rc;
         unsigned long long first_bad = ~0ull;
         CU_TRY(cudaMemcpyAsync(top_hits, c.ce[6].p, nsel, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaMemcpyAsync(&first_bad, d_bad, 8, cudaMemcpyDeviceToHost, st));
@@ -1313,6 +1402,33 @@ int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* 
     CU_TRY(cudaMemcpyAsync(top_counts, c.ce[5].p, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     return BDG_OK;
+}
+
+int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* sorted_wl, size_t W, uint32_t* top_ranks, uint32_t* top_counts,
+                      uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
+{
+    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_above = 0; *cutoff = 0.0;
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    CU_TRY(cudaSetDevice(c.dev));
+    return centres_above_core(c, n_cells, sorted_wl, false, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
+}
+
+int bdg_dev_centres_above(unsigned long long token, size_t n_cells, const uint32_t* d_sorted_wl, size_t W, uint32_t* top_ranks,
+                          uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff, void* stream)
+{
+    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_above = 0; *cutoff = 0.0;
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    CU_TRY(cudaSetDevice(c.dev));
+    if (top_hits && W) if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    return centres_above_core(c, n_cells, d_sorted_wl, true, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
 }
 
 // The stretch of `bc_by_counts` right behind the head bdg_centres_above returns (barcode_graph.py:273-276 runs into it when too few
@@ -1365,41 +1481,33 @@ int bdg_centres_rest(unsigned long long token, double cutoff, size_t need, uint3
     return BDG_OK;
 }
 
-// bdg_assign_reads with a 5-byte result per row (centre barcode + "has a centre" byte).  centre_idx == NULL: the clustering a
-// bdg_cluster_resident call left on the device is used in place (nothing is uploaded).
-int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size_t N, uint32_t* centre_per_row, uint8_t* has_centre, size_t R_all,
-                       size_t* n_assigned)
+static int ensure_buf(Buf& b, size_t bytes)
 {
-    if (n_assigned) *n_assigned = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!centre_per_row || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
+    if (cudaError_t e = (cudaError_t)b.ensure(bytes))
+        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
+    return BDG_OK;
+}
+
+static int check_assign_args(DevCtx& c, unsigned long long token, bool resident, size_t N, size_t R_all)
+{
     if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
     if (N != c.map_distinct || R_all != c.map_rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
-    if (!centre_idx && N && c.cl_token != token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
-    CU_TRY(cudaSetDevice(c.dev));
+    if (resident && N && c.cl_token != token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
+    return BDG_OK;
+}
+
+// The per-read gather on c.stream: d_ci (device, on c.dev) is the centre index per node, NULL for the resident clustering result;
+// the 5-byte result goes to d_out / d_oh (device, R_all rows) and the number of rows with a centre to the counter in as[7].
+static int assign_reads32_core(DevCtx& c, const int32_t* d_ci, size_t N, uint32_t* d_out, uint8_t* d_oh, size_t R_all)
+{
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    // as[4] centre index per node (upload), as[5] centre value + has byte per distinct barcode, as[6] result per row, as[7] counter
-    if (int e = ensure(c.as[5], std::max<size_t>(N, 1) * 5)) return e;
-    if (int e = ensure(c.as[6], R_all * 5)) return e;
-    if (int e = ensure(c.as[7], 8)) return e;
-    const int32_t* d_ci = (const int32_t*)c.cl[1].p;
-    if (centre_idx) {
-        if (int e = ensure(c.as[4], std::max<size_t>(N, 1) * 4)) return e;
-        CU_TRY(cudaMemcpyAsync(c.as[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-        d_ci = (const int32_t*)c.as[4].p;
-    }
+    // as[5] centre value + has byte per distinct barcode, as[7] counter
+    if (int e = ensure_buf(c.as[5], std::max<size_t>(N, 1) * 5)) return e;
+    if (int e = ensure_buf(c.as[7], 8)) return e;
+    if (!d_ci) d_ci = (const int32_t*)c.cl[1].p;
     CU_TRY(cudaMemsetAsync(c.as[7].p, 0, 8, st));
     uint32_t* d_cv = (uint32_t*)c.as[5].p;
     uint8_t* d_ch = (uint8_t*)c.as[5].p + std::max<size_t>(N, 1) * 4;
-    uint32_t* d_out = (uint32_t*)c.as[6].p;
-    uint8_t* d_oh = (uint8_t*)c.as[6].p + R_all * 4;
     if (N) {
         const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
         bdg::centre_of_distinct32_kernel<<<nb, 256, 0, st>>>(d_ci, (const uint32_t*)c.dd[1].p /* first-seen -> node */,
@@ -1411,12 +1519,64 @@ int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size
                                                    (unsigned long long*)c.as[7].p);
     g_launches += 2;
     CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+// bdg_assign_reads with a 5-byte result per row (centre barcode + "has a centre" byte).  centre_idx == NULL: the clustering a
+// bdg_cluster_resident call left on the device is used in place (nothing is uploaded).
+int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size_t N, uint32_t* centre_per_row, uint8_t* has_centre, size_t R_all,
+                       size_t* n_assigned)
+{
+    if (n_assigned) *n_assigned = 0;
+    if (R_all == 0) return BDG_OK;
+    if (!centre_per_row || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (int rc = check_assign_args(c, token, !centre_idx, N, R_all)) return rc;
+    CU_TRY(cudaSetDevice(c.dev));
+    cudaStream_t st = c.stream;
+    // as[4] centre index per node (upload), as[6] result per row
+    if (int e = ensure_buf(c.as[6], R_all * 5)) return e;
+    const int32_t* d_ci = nullptr;
+    if (centre_idx) {
+        if (int e = ensure_buf(c.as[4], std::max<size_t>(N, 1) * 4)) return e;
+        CU_TRY(cudaMemcpyAsync(c.as[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+        d_ci = (const int32_t*)c.as[4].p;
+    }
+    uint32_t* d_out = (uint32_t*)c.as[6].p;
+    uint8_t* d_oh = (uint8_t*)c.as[6].p + R_all * 4;
+    if (int rc = assign_reads32_core(c, d_ci, N, d_out, d_oh, R_all)) return rc;
     unsigned long long cnt = 0;
     CU_TRY(cudaMemcpyAsync(centre_per_row, d_out, R_all * 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(has_centre, d_oh, R_all, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(&cnt, c.as[7].p, 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     if (n_assigned) *n_assigned = (size_t)cnt;
+    return BDG_OK;
+}
+
+int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx, size_t N, uint32_t* d_centre_per_row, uint8_t* d_has_centre,
+                           size_t R_all, size_t* n_assigned, void* stream)
+{
+    if (n_assigned) *n_assigned = 0;
+    if (R_all == 0) return BDG_OK;
+    if (!d_centre_per_row || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (int rc = check_assign_args(c, token, !d_centre_idx, N, R_all)) return rc;
+    CU_TRY(cudaSetDevice(c.dev));
+    if (d_centre_idx && N) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
+    if (int rc = check_on_first(d_centre_per_row, "centre_per_row")) return rc;
+    if (int rc = check_on_first(d_has_centre, "has_centre")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    if (int rc = assign_reads32_core(c, N ? d_centre_idx : nullptr, N, d_centre_per_row, d_has_centre, R_all)) return rc;
+    if (n_assigned) {
+        unsigned long long cnt = 0;
+        CU_TRY(cudaMemcpyAsync(&cnt, c.as[7].p, 8, cudaMemcpyDeviceToHost, c.stream));
+        CU_TRY(cudaStreamSynchronize(c.stream));
+        *n_assigned = (size_t)cnt;
+    }
     return BDG_OK;
 }
 
@@ -1484,31 +1644,18 @@ int bdg_pack16(const char* seqs, size_t R, uint32_t* out, uint8_t* valid)
 
 // badger.py:82-88 for the array pipeline: the whitelist records packed (a-1), the invalid ones dropped, sorted and made
 // distinct on the device (cub radix sort + unique); out_sorted has room for R entries, *n receives the number kept.
-int bdg_pack16_sorted(const char* seqs, size_t R, uint32_t* out_sorted, size_t* n)
+// d_seqs: the R records on c.dev; the distinct packed barcodes stay in ce[2], *n receives their number.
+static int pack16_sorted_core(DevCtx& c, const char* d_seqs, size_t R, size_t* n)
 {
-    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n = 0;
-    if (R == 0) return BDG_OK;
-    if (!seqs || !out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    // io[0] letters, io[1] ranks, io[2] validity; ce[0] kept ranks, ce[1] sorted, ce[2] distinct, ce[7] count, ce[8] cub scratch
-    if (int e = ensure(c.io[0], R * 16)) return e;
+    auto ensure = ensure_buf;
+    // io[1] ranks, io[2] validity; ce[0] kept ranks, ce[1] sorted, ce[2] distinct, ce[7] count, ce[8] cub scratch
     if (int e = ensure(c.io[1], R * 4)) return e;
     if (int e = ensure(c.io[2], R)) return e;
     for (int k = 0; k < 3; k++) if (int e = ensure(c.ce[k], R * 4)) return e;
     if (int e = ensure(c.ce[7], 64)) return e;
     uint32_t* d_n = (uint32_t*)c.ce[7].p;
-    CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, st));
-    if (int rc = bdg_dev_pack16((const char*)c.io[0].p, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, st)) return rc;
+    if (int rc = bdg_dev_pack16(d_seqs, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, st)) return rc;
     size_t t1 = 0, t2 = 0, t3 = 0;
     CU_TRY(cub::DeviceSelect::Flagged(nullptr, t1, (const uint32_t*)c.io[1].p, (const uint8_t*)c.io[2].p, (uint32_t*)c.ce[0].p, d_n, (int)R, st));
     CU_TRY(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[1].p, (int)R, 0, 32, st));
@@ -1524,9 +1671,48 @@ int bdg_pack16_sorted(const char* seqs, size_t R, uint32_t* out_sorted, size_t* 
     uint32_t distinct = 0;
     CU_TRY(cudaMemcpyAsync(&distinct, d_n, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    CU_TRY(cudaMemcpyAsync(out_sorted, c.ce[2].p, (size_t)distinct * 4, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
     *n = distinct;
+    return BDG_OK;
+}
+
+int bdg_pack16_sorted(const char* seqs, size_t R, uint32_t* out_sorted, size_t* n)
+{
+    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n = 0;
+    if (R == 0) return BDG_OK;
+    if (!seqs || !out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int e = ensure_buf(c.io[0], R * 16)) return e;     // io[0] letters
+    CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, c.stream));
+    size_t kept = 0;
+    if (int rc = pack16_sorted_core(c, (const char*)c.io[0].p, R, &kept)) return rc;
+    CU_TRY(cudaMemcpyAsync(out_sorted, c.ce[2].p, kept * 4, cudaMemcpyDeviceToHost, c.stream));
+    CU_TRY(cudaStreamSynchronize(c.stream));
+    *n = kept;
+    return BDG_OK;
+}
+
+int bdg_dev_pack16_sorted(const char* d_seqs, size_t R, uint32_t* d_out_sorted, size_t* n, void* stream)
+{
+    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n = 0;
+    if (R == 0) return BDG_OK;
+    if (!d_seqs || !d_out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int rc = check_on_first(d_seqs, "records")) return rc;
+    if (int rc = check_on_first(d_out_sorted, "out_sorted")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    size_t kept = 0;
+    if (int rc = pack16_sorted_core(c, d_seqs, R, &kept)) return rc;
+    CU_TRY(cudaMemcpyAsync(d_out_sorted, c.ce[2].p, kept * 4, cudaMemcpyDeviceToDevice, c.stream));
+    *n = kept;
     return BDG_OK;
 }
 
@@ -1758,16 +1944,23 @@ size_t bdg_edges_count(const bdg_edges* e)
     return n;
 }
 
+static int check_edges_handle(const bdg_edges* e)
+{
+    for (size_t g = 0; g < e->ctx.size(); g++)
+        if (e->ctx[g] < 0 || (size_t)e->ctx[g] >= g_ctx.size() || g_ctx[e->ctx[g]].generation != e->gen[g])
+            return fail(BDG_ERR_ARG, "stale edge handle: a later edge build on the same device has reused its buffers");
+    return BDG_OK;
+}
+
 int bdg_edges_copy(const bdg_edges* e, uint32_t* a, uint32_t* b, uint8_t* d)
 {
     if (!e) return fail(BDG_ERR_ARG, "NULL edge handle");
     const size_t n = bdg_edges_count(e);
     if (n && (!a || !b || !d)) return fail(BDG_ERR_ARG, "NULL output pointer");
+    if (int rc = check_edges_handle(e)) return rc;
     const double tc0 = now_ms();
     size_t off = 0;
     for (size_t g = 0; g < e->ctx.size(); g++) {
-        if (e->ctx[g] < 0 || (size_t)e->ctx[g] >= g_ctx.size() || g_ctx[e->ctx[g]].generation != e->gen[g])
-            return fail(BDG_ERR_ARG, "stale edge handle: a later edge build on the same device has reused its buffers");
         DevCtx& c = g_ctx[e->ctx[g]];
         const size_t k = e->count[g];
         if (k) {
@@ -1782,6 +1975,42 @@ int bdg_edges_copy(const bdg_edges* e, uint32_t* a, uint32_t* b, uint8_t* d)
         if (e->count[g]) { CU_TRY(cudaSetDevice(g_ctx[e->ctx[g]].dev)); CU_TRY(cudaStreamSynchronize(g_ctx[e->ctx[g]].stream)); }
     if (!g_ctx.empty()) cudaSetDevice(g_ctx[0].dev);
     if (getenv("BDG_TRACE")) fprintf(stderr, "[bdg] edges_copy %zu edges %.3f ms\n", n, now_ms() - tc0);
+    return BDG_OK;
+}
+
+// Every part is copied on the first device's stream (peer copies for parts on other devices; the builds have finished when the
+// handle is returned).  The part's own stream then waits for the copy too, so that a later build there cannot overwrite the
+// edges while they are still being read.
+int bdg_dev_edges_copy(const bdg_edges* e, uint32_t* d_a, uint32_t* d_b, uint8_t* d_d, void* stream)
+{
+    if (!e) return fail(BDG_ERR_ARG, "NULL edge handle");
+    const size_t n = bdg_edges_count(e);
+    if (n && (!d_a || !d_b || !d_d)) return fail(BDG_ERR_ARG, "NULL output pointer");
+    if (int rc = check_edges_handle(e)) return rc;
+    if (n == 0) return BDG_OK;
+    DevCtx& c0 = g_ctx[0];
+    CU_TRY(cudaSetDevice(c0.dev));
+    if (int rc = check_on_first(d_a, "a")) return rc;
+    if (int rc = check_on_first(d_b, "b")) return rc;
+    if (int rc = check_on_first(d_d, "d")) return rc;
+    CallerOrder order(c0, stream);
+    if (int rc = order.begin()) return rc;
+    size_t off = 0;
+    for (size_t g = 0; g < e->ctx.size(); g++) {
+        DevCtx& c = g_ctx[e->ctx[g]];
+        const size_t k = e->count[g];
+        if (k) {
+            CU_TRY(cudaMemcpyPeerAsync(d_a + off, c0.dev, c.ea.p, c.dev, k * 4, c0.stream));
+            CU_TRY(cudaMemcpyPeerAsync(d_b + off, c0.dev, c.eb.p, c.dev, k * 4, c0.stream));
+            CU_TRY(cudaMemcpyPeerAsync(d_d + off, c0.dev, c.ed.p, c.dev, k, c0.stream));
+        }
+        off += k;
+    }
+    CU_TRY(cudaEventRecord(c0.ev_caller, c0.stream));
+    for (size_t g = 0; g < e->ctx.size(); g++) {
+        DevCtx& c = g_ctx[e->ctx[g]];
+        if (e->count[g] && &c != &c0) CU_TRY(cudaStreamWaitEvent(c.stream, c0.ev_caller, 0));
+    }
     return BDG_OK;
 }
 

@@ -33,16 +33,16 @@ class _Token:
         return True
 
 
-def select_centres(rm, n_cells, interval, whitelist_sorted, true_barcodes):
+def select_centres(rm, n_cells, interval, whitelist_sorted, true_barcodes, centres_above=ops.centres_above):
     """barcode_graph.py:252-277 with the counting, the count-ordered head of the barcode list and its whitelist membership on
-    the device (ops.centres_above, and ops.centres_rest if the top-up loop has to go below the cutoff): no per-barcode array is
+    the device (centres_above, and ops.centres_rest if the top-up loop has to go below the cutoff): no per-barcode array is
     downloaded."""
     from statistics import StatisticsError
     from .barcode_graph import walk_centres
     if rm.n_distinct == 0 or n_cells <= 0:
         raise StatisticsError("mean requires at least one data point")
     tb = None if true_barcodes is None else [int(x) for x in true_barcodes]
-    cutoff, top, _, hits = ops.centres_above(rm, n_cells, None if tb else whitelist_sorted)
+    cutoff, top, _, hits = centres_above(rm, n_cells, None if tb else whitelist_sorted)
     have_list = whitelist_sorted is not None
     if hits is None and have_list and not tb:
         hits = np.zeros(0, bool)
@@ -61,11 +61,9 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
     the iteration order of that very set of strings in this process, which is what badger_b200.BarcodeGraph meets too).
 
     Without high_sens nothing per-barcode ever reaches the host: the distinct barcodes, their counts, the edges, the
-    clustering result and the read map stay on the device between the stages."""
+    clustering result and the read map stay on the device between the stages.  (badger_b200.device.assign_packed is the
+    same step with the per-read arrays in CUDA tensors.)"""
     T = timings if timings is not None else {}
-
-    def tick(name, t0):
-        T[name] = T.get(name, 0.0) + time.perf_counter() - t0
 
     def result(c32, has):
         if form == "u32":
@@ -85,18 +83,38 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
 
     t0 = time.perf_counter()
     rm = ops.dedup_reads(ranks, valid)                    # valid rows compacted on the device; everything stays there
-    tick("dedup_first_seen", t0)
+    _tick(T, "dedup_first_seen", t0)
     info["valid_reads"] = int(rm.n_valid)
     if rm.n_valid == 0:
         return result(np.zeros(R, np.uint32), np.zeros(R, np.uint8)), info
+
+    def gather(ci):
+        c32, has, n_assigned = ops.assign_reads32(rm, ci)     # per-read gather on the device
+        return result(c32, has), n_assigned
+
+    return run_stages(rm, info, T, gather, threshold=threshold, n_cells=n_cells, interval=interval, whitelist_sorted=whitelist_sorted,
+                      true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order, centres_above=ops.centres_above), info
+
+
+def _tick(T, name, t0):
+    T[name] = T.get(name, 0.0) + time.perf_counter() - t0
+
+
+def run_stages(rm, info, T, gather, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order,
+               centres_above):
+    """The stages after the dedup of a read map `rm` with at least one valid read: edges, centres, clustering, --high_sens,
+    and last `gather(centre_idx)` -> (result, rows with a centre) over the read map, with centre_idx None for the clustering
+    left on the device.  Fills `info` and the timings `T`; returns what `gather` returned first.  centres_above is
+    ops.centres_above or a function of the same signature that takes the whitelist in another form."""
     t0 = time.perf_counter()
     handle = ops.edges_handle_resident(rm, threshold)     # the ascending array is already on the device: no upload, peer copies to the other GPUs
-    tick("edges", t0)
+    _tick(T, "edges", t0)
     info.update(distinct=int(rm.n_distinct), edges=int(handle.count))
 
     t0 = time.perf_counter()
-    centres = np.asarray(list(dict.fromkeys(select_centres(rm, n_cells, interval, whitelist_sorted, true_barcodes))), dtype=np.uint32)
-    tick("centres", t0)
+    centres = np.asarray(list(dict.fromkeys(select_centres(rm, n_cells, interval, whitelist_sorted, true_barcodes, centres_above))),
+                         dtype=np.uint32)
+    _tick(T, "centres", t0)
     info["centres"] = int(centres.size)
 
     if not high_sens:
@@ -105,19 +123,19 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
         handle.free()
         # badger.py:131 `len(counts) - len(edges.keys())`: the keys are the nodes with an edge plus every centre cluster() touched
         info["disconnected"] = int(rm.n_distinct) - (int(n_has_edge) + int(centres.size))
-        tick("cluster", t0)
+        _tick(T, "cluster", t0)
         t0 = time.perf_counter()
-        c32, has, n_assigned = ops.assign_reads32(rm, None)
-        tick("gather", t0)
+        out, n_assigned = gather(None)
+        _tick(T, "gather", t0)
         info["assigned_reads"] = int(n_assigned)
-        return result(c32, has), info
+        return out
 
     t0 = time.perf_counter()
     s, spos = rm.sorted_distinct, rm.sorted_pos
     ci, lv, has_edge = handle.cluster_levels(centres, 2, want_has_edge=True)   # consumes the handle's edges (no copy to the host)
     handle.free()
     info["disconnected"] = int(rm.n_distinct) - (int(has_edge.sum()) + int(centres.size))
-    tick("cluster", t0)
+    _tick(T, "cluster", t0)
     # barcode_graph.py:370-385 on node positions: every node without a centre looks for the nearest used centre
     t0 = time.perf_counter()
     todo = np.nonzero(ci < 0)[0]
@@ -143,10 +161,10 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
         am, _ = ops.nearest_bounded(s[todo], targets, 2)
         hit = am >= 0
         ci[todo[hit]] = np.searchsorted(s, targets[am[hit]]).astype(np.int32)
-    tick("high_sens", t0)
+    _tick(T, "high_sens", t0)
 
     t0 = time.perf_counter()
-    c32, has, n_assigned = ops.assign_reads32(rm, ci)     # per-read gather on the device
-    tick("gather", t0)
+    out, n_assigned = gather(ci)
+    _tick(T, "gather", t0)
     info["assigned_reads"] = int(n_assigned)
-    return result(c32, has), info
+    return out

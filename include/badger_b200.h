@@ -10,7 +10,8 @@
  * Conventions
  *   - plain pointers and sizes only; host entry points take HOST buffers (read-only during the call) and
  *     do their own host<->device copies; bdg_dev_* entry points take DEVICE pointers on the current CUDA
- *     device plus a cudaStream_t passed as void*, and are asynchronous on that stream.
+ *     device plus a cudaStream_t passed as void*, and are asynchronous on that stream (the correction-step ones
+ *     take pointers on the first claimed device and order their work against that stream; see below).
  *   - every int-returning function returns BDG_OK (0) or a negative error code; bdg_last_error() gives the
  *     text.  There is NO CPU fallback: without a usable CUDA device every compute call fails with
  *     BDG_ERR_NODEVICE.
@@ -218,6 +219,34 @@ int bdg_dev_edges_balance(unsigned long long* out6, void* stream);
 int bdg_dev_pack16(const char* d_seqs, size_t R, uint32_t* d_out, uint8_t* d_valid, void* stream);
 int bdg_dev_member_sorted(const uint32_t* d_sorted_wl, size_t W, const uint32_t* d_q, size_t Q, uint8_t* d_hit,
                           void* stream);
+
+/* ---- the correction step with the per-read arrays in caller device memory ------------------------------------------------
+ * Device forms of bdg_dedup_reads / bdg_dedup_fetch / bdg_pack16_sorted / bdg_centres_above / bdg_edges_copy / bdg_assign_reads32:
+ * the same kernels and results, but the per-read and per-barcode arrays are read from and written to caller memory on the FIRST
+ * device given to bdg_init (where the read map lives); a pointer to any other memory is BDG_ERR_ARG.  The work runs on the
+ * library's stream of that device, ordered after everything queued on `stream` before the call, and `stream` is ordered after
+ * the work of the call: the inputs may be produced, and the outputs consumed, by kernels on `stream` without a synchronisation.
+ * A call synchronises only where its host form does to learn a size (*n_valid / *n_distinct, *n, *n_above, *n_assigned); only
+ * such sizes and scalars cross PCIe.  Tokens have the life cycle of the host forms. */
+/* bdg_dedup_reads with every output pointer NULL; d_valid may be NULL (all rows valid).  The valid bytes are copied into the
+ * library's workspace (the per-read gather reads them again), so the caller's arrays are free once the call returns. */
+int bdg_dev_dedup_reads(const uint32_t* d_ranks, const uint8_t* d_valid, size_t R_all, size_t* n_distinct, size_t* n_valid,
+                        unsigned long long* token, void* stream);
+/* bdg_dedup_fetch into device buffers of n_distinct entries; any pointer may be NULL. */
+int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t* d_counts, uint32_t* d_sorted_pos,
+                        uint32_t* d_sorted_distinct, void* stream);
+/* bdg_pack16_sorted over R records of 16 bytes on the device (16-byte aligned); d_out_sorted has room for R entries. */
+int bdg_dev_pack16_sorted(const char* d_seqs, size_t R, uint32_t* d_out_sorted, size_t* n, void* stream);
+/* bdg_centres_above with the sorted whitelist on the device; top_ranks / top_counts / top_hits stay HOST buffers (the head of a few
+ * thousand entries is walked on the host). */
+int bdg_dev_centres_above(unsigned long long token, size_t n_cells, const uint32_t* d_sorted_wl, size_t W, uint32_t* top_ranks,
+                          uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff, void* stream);
+/* bdg_edges_copy into device buffers of bdg_edges_count(e) entries; the parts of a multi-device handle arrive by peer copies. */
+int bdg_dev_edges_copy(const bdg_edges* e, uint32_t* d_a, uint32_t* d_b, uint8_t* d_d, void* stream);
+/* bdg_assign_reads32 with a device centre_idx (NULL: the clustering bdg_cluster_resident left on the device) and device outputs
+ * of R_all rows.  n_assigned may be NULL: the call then does not wait for the gather. */
+int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx, size_t N, uint32_t* d_centre_per_row,
+                           uint8_t* d_has_centre, size_t R_all, size_t* n_assigned, void* stream);
 int bdg_dev_nearest_bounded(const uint32_t* d_q, size_t Q, const uint32_t* d_targets, size_t W, int max_d,
                             uint32_t* d_keys /* Q words of scratch */, int32_t* d_argmin, uint8_t* d_dist,
                             void* stream);
