@@ -88,6 +88,12 @@ def lib():
     L.bdg_dev_centres_above.argtypes = [C.c_ulonglong, _sz, _vp, _sz, _vp, _vp, _vp, _sz, C.POINTER(_sz), C.POINTER(C.c_double), _vp]
     L.bdg_dev_edges_copy.argtypes = [_vp, _vp, _vp, _vp, _vp]
     L.bdg_dev_assign_reads32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, C.POINTER(_sz), _vp]
+    L.bdg_dev_dedup_merge.argtypes = [C.c_ulonglong, _vp, _vp, _vp, _vp, _vp, _i, _i, C.POINTER(_sz), C.POINTER(C.c_ulonglong), _vp]
+    L.bdg_dev_index_edges.argtypes = [_vp, _sz, _vp, _vp, _sz, _vp, _vp, _vp]
+    L.bdg_dev_cluster_init.argtypes = [_vp, _sz, _vp, _sz, _vp, _vp, _vp, _vp, _vp]
+    L.bdg_dev_cluster_mark.argtypes = [_vp, _vp, _sz, _vp, _vp, _vp]
+    L.bdg_dev_cluster_claim.argtypes = [_vp, _vp, _sz, _i, _vp, _vp, _vp, _vp, _vp]
+    L.bdg_dev_cluster_resolve.argtypes = [_vp, _vp, _vp, _vp, _sz, _i, _vp]
     L.bdg_part_pairs.argtypes = [_sz, _i, _i]
     L.bdg_part_pairs.restype = C.c_ulonglong
     L.bdg_dev_pipe_probe.argtypes = [_i, _i, _i, _vp, C.POINTER(C.c_ulonglong), _vp]
@@ -109,7 +115,8 @@ def lib():
                  "bdg_nearest_bounded", "bdg_kmer_score", "bdg_kmer_index_create", "bdg_kmer_index_query", "bdg_dev_edges_build", "bdg_set_edge_mode", "bdg_dev_edges_stats", "bdg_dev_edges_stats_raw", "bdg_dev_edges_balance", "bdg_dev_pack16", "bdg_dev_member_sorted",
                  "bdg_dev_nearest_bounded", "bdg_dev_pipe_probe", "bdg_tsv_open", "bdg_tsv_barcodes", "bdg_tsv_write_assignments", "bdg_lines16_open", "bdg_dedup_reads", "bdg_assign_reads", "bdg_pack16_sorted", "bdg_assign_reads32", "bdg_dedup_fetch", "bdg_centres_above", "bdg_centres_rest", "bdg_cluster_resident",
                  "bdg_tsv_write_assignments32", "bdg_dev_dedup_reads", "bdg_dev_dedup_fetch", "bdg_dev_pack16_sorted", "bdg_dev_centres_above",
-                 "bdg_dev_edges_copy", "bdg_dev_assign_reads32"):
+                 "bdg_dev_edges_copy", "bdg_dev_assign_reads32", "bdg_dev_dedup_merge", "bdg_dev_index_edges", "bdg_dev_cluster_init",
+                 "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve"):
         getattr(L, name).restype = _i
     _lib = L
     return L

@@ -93,6 +93,7 @@ struct DevCtx {
     unsigned long long cl_token = 0;                          // read-map token the clustering result resident in cl[1] / cl[2] belongs to (0: none)
     Buf ce[9];                                                // centre selection: positions above the cutoff, sort keys / values, results, scratch
     Buf as[8];                                                // masked dedup + per-read gather: all ranks, valid bytes, their scan, scratch, centre idx / value, result, counter
+    Buf mg[12];                                               // merge of the parts' dedup results (bdg_dev_dedup_merge), see there
     unsigned long long map_token = 0, map_serial = 0;         // read map left on the device by bdg_dedup_reads (0: none)
     size_t map_rows = 0, map_reads = 0, map_distinct = 0;
     bool map_masked = false;
@@ -1315,6 +1316,111 @@ int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t
     return dedup_fetch_core(c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice);
 }
 
+static int ensure_buf(Buf& b, size_t bytes);
+
+// ---- the dedup results of P parts (one process per GPU) reduced to the global distinct set (bdg_kernels.cuh, merge_*) ----
+// The work arrays live in mg[] until the end, so that a failed check leaves the token's read map as it was; only then do the
+// global arrays move to where the token's consumers read them (dd[0] counts, dd[1] first-seen -> ascending, dd[2] distinct,
+// dd[6] ascending) and the read map dd[7] is rewritten in place.  as[1] / as[2] (the valid rows) are not touched.
+static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first, const size_t* starts,
+                            const size_t* sizes, int n_parts, int my_part, size_t* n_distinct, unsigned long long* merged_token)
+{
+    cudaStream_t st = c.stream;
+    std::vector<uint64_t> h_starts(n_parts);
+    std::vector<uint32_t> h_offs(n_parts + 1, 0);
+    size_t total = 0;
+    for (int p = 0; p < n_parts; p++) {
+        h_starts[p] = starts[p];
+        h_offs[p] = (uint32_t)total;
+        total += sizes[p];
+        if (total >= 0x80000000ull) return fail(BDG_ERR_ARG, "the parts hold 2^31 or more barcodes in all");
+    }
+    h_offs[n_parts] = (uint32_t)total;
+    if (total == 0) return fail(BDG_ERR_ARG, "no part holds a barcode");
+    const uint32_t T = (uint32_t)total, n_mine = (uint32_t)sizes[my_part], off_mine = h_offs[my_part];
+    // mg[0] part starts, [1] part offsets, [2] keys, [3] entry index, [4] sorted keys, [5] sorted index, [6] counts, [7] first keys,
+    // [8] heads / run order, [9] scan / sorted first keys, [10] run key | count | first | own run | position of run | local -> global, [11] scratch
+    if (int e = ensure_buf(c.mg[0], (size_t)n_parts * 8)) return e;
+    if (int e = ensure_buf(c.mg[1], ((size_t)n_parts + 1) * 4 + 4)) return e;
+    for (int k = 2; k < 10; k++) if (int e = ensure_buf(c.mg[k], total * 4)) return e;
+    if (int e = ensure_buf(c.mg[10], (5 * total + std::max<size_t>(n_mine, 1)) * 4)) return e;
+    uint32_t *d_key = (uint32_t*)c.mg[2].p, *d_idx = (uint32_t*)c.mg[3].p, *d_sk = (uint32_t*)c.mg[4].p, *d_si = (uint32_t*)c.mg[5].p;
+    uint32_t *d_cnt = (uint32_t*)c.mg[6].p, *d_fst = (uint32_t*)c.mg[7].p, *d_head = (uint32_t*)c.mg[8].p, *d_scan = (uint32_t*)c.mg[9].p;
+    uint32_t *d_rk = (uint32_t*)c.mg[10].p, *d_rc = d_rk + total, *d_rf = d_rc + total, *d_mrun = d_rf + total, *d_prun = d_mrun + total,
+             *d_loc = d_prun + total;
+    unsigned int* d_bad = (unsigned int*)((uint32_t*)c.mg[1].p + n_parts + 1);
+    size_t tmp1 = 0, tmp2 = 0;
+    CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
+    CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp2, d_head, d_scan, (int)T, st));
+    if (int e = ensure_buf(c.mg[11], std::max(tmp1, tmp2))) return e;
+    CU_TRY(cudaMemcpyAsync(c.mg[0].p, h_starts.data(), (size_t)n_parts * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(c.mg[1].p, h_offs.data(), ((size_t)n_parts + 1) * 4, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemsetAsync(d_bad, 0, 4, st));
+    const int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)c.sms * 8);
+    bdg::merge_gather_kernel<<<blocks, 256, 0, st>>>(d_keys, d_counts, d_first, (const uint64_t*)c.mg[0].p, (const uint32_t*)c.mg[1].p, (uint32_t)n_parts,
+                                                     T, (uint32_t)my_part, (const uint32_t*)c.dd[6].p, d_key, d_idx, d_cnt, d_fst, d_bad);
+    CU_TRY(cub::DeviceRadixSort::SortPairs(c.mg[11].p, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
+    bdg::dedup_heads_kernel<<<blocks, 256, 0, st>>>(d_sk, T, d_head);
+    CU_TRY(cub::DeviceScan::InclusiveSum(c.mg[11].p, tmp2, d_head, d_scan, (int)T, st));
+    bdg::merge_runs_kernel<<<blocks, 256, 0, st>>>(d_sk, d_si, d_head, d_scan, T, d_cnt, d_fst, off_mine, n_mine, d_rk, d_rc, d_rf, d_mrun);
+    g_launches += 3;
+    CU_TRY(cudaGetLastError());
+    uint32_t n_runs = 0;
+    unsigned int bad = 0;
+    CU_TRY(cudaMemcpyAsync(&n_runs, d_scan + (T - 1), 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    if (bad) return fail(BDG_ERR_ARG, "the list of part %d is not the distinct list of the read map the token names", my_part);
+    // runs by first key (unique: every key names one barcode of one part): d_scan := sorted first keys, d_head := order
+    bdg::iota_kernel<<<blocks, 256, 0, st>>>(d_idx, n_runs);
+    CU_TRY(cub::DeviceRadixSort::SortPairs(c.mg[11].p, tmp1, d_rf, d_scan, d_idx, d_head, (int)n_runs, 0, 32, st));
+    // d_key / d_cnt are free: distinct and counts in first-seen order
+    bdg::merge_finish_kernel<<<blocks, 256, 0, st>>>(d_head, d_rk, d_rc, n_runs, d_key, d_cnt, d_prun);
+    g_launches += 2;
+    if (n_mine) {
+        const int lb = (int)std::min<size_t>((n_mine + 255) / 256, (size_t)c.sms * 8);
+        const int rb = (int)std::min<size_t>((c.map_reads + 255) / 256, (size_t)c.sms * 8);
+        bdg::merge_local_kernel<<<lb, 256, 0, st>>>((const uint32_t*)c.dd[1].p, d_mrun, d_prun, n_mine, d_loc);
+        bdg::merge_remap_kernel<<<rb, 256, 0, st>>>((uint32_t*)c.dd[7].p, (uint32_t)c.map_reads, d_loc);
+        g_launches += 2;
+    }
+    CU_TRY(cudaGetLastError());
+    // growing a dd[] buffer frees its old memory: the kernels above that read dd[1] / dd[6] must have finished
+    CU_TRY(cudaStreamSynchronize(st));
+    for (int k : {0, 1, 2, 6}) if (int e = ensure_buf(c.dd[k], (size_t)n_runs * 4)) return e;
+    CU_TRY(cudaMemcpyAsync(c.dd[0].p, d_cnt, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(c.dd[1].p, d_head, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));   // order[pos] = run = ascending position
+    CU_TRY(cudaMemcpyAsync(c.dd[2].p, d_key, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(c.dd[6].p, d_rk, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));    // runs are numbered in key order
+    c.map_distinct = n_runs;
+    c.cl_token = 0;
+    c.map_token = ++c.map_serial;
+    *n_distinct = n_runs;
+    *merged_token = c.map_token;
+    return BDG_OK;
+}
+
+int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first, const size_t* starts,
+                        const size_t* sizes, int n_parts, int my_part, size_t* n_distinct, unsigned long long* merged_token, void* stream)
+{
+    if (!n_distinct || !merged_token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *merged_token = 0;
+    if (n_parts < 1 || my_part < 0 || my_part >= n_parts || !starts || !sizes) return fail(BDG_ERR_ARG, "need 0 <= my_part < n_parts and the parts' starts / sizes");
+    if (!d_keys || !d_counts || !d_first) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    // token 0: this part has no valid read (the dedup call issued no token); its list must then be empty
+    if (token != 0 && token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    if (sizes[my_part] != (token ? c.map_distinct : 0))
+        return fail(BDG_ERR_ARG, "part %d has %zu barcodes, the read map of the token %zu", my_part, sizes[my_part], token ? c.map_distinct : (size_t)0);
+    CU_TRY(cudaSetDevice(c.dev));
+    for (const uint32_t* p : {d_keys, d_counts, d_first}) if (int rc = check_on_first(p, "merge input")) return rc;
+    if (token == 0) { c.map_token = 0; c.map_rows = 0; c.map_reads = 0; c.map_masked = false; }
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    return dedup_merge_core(c, d_keys, d_counts, d_first, starts, sizes, n_parts, my_part, n_distinct, merged_token);
+}
+
 // ---- a-6 / centre selection, barcode_graph.py:252-267, over the distinct barcodes a dedup call left on the device ----
 // cutoff = max(mean(counts of the first n_cells barcodes in first-seen order) / 5, 5) (:255-256); the barcodes with
 // count > cutoff in count-descending order, ties in first-seen order (the head of `bc_by_counts`, :253), with their counts and
@@ -2020,22 +2126,68 @@ void bdg_edges_free(bdg_edges* e) { delete e; }
 // ---- f-3  cluster(): barcode_graph.py:279-301 -------------------------------------------------------------
 // d_ea / d_eb hold barcode VALUES on entry and node indices on return (converted in place).
 // centre_idx / level may be NULL: the result then only stays on the device (cl[1] / cl[2]) for bdg_assign_reads*.
-// values -> node indices of the E edges (ea, eb) on device c (its own copy of the sorted array), written to (oa, ob); on c.stream
-static int index_edges(DevCtx& c, size_t N, const uint32_t* d_ea, const uint32_t* d_eb, size_t E, uint32_t* d_oa, uint32_t* d_ob)
+// The phases of cluster() over node arrays the caller owns, each on the stream it is given: cluster_on_device runs them on one
+// device; the bdg_dev_cluster_* entry points expose them to one process per GPU, which reduces the claims between the ranks.
+// values -> node indices of the E edges (ea, eb) against d_sorted[N] on device c (top16: its search table), written to (oa, ob)
+static int index_edges(DevCtx& c, const uint32_t* d_sorted, size_t N, const uint32_t* d_ea, const uint32_t* d_eb, size_t E, uint32_t* d_oa,
+                       uint32_t* d_ob, cudaStream_t st)
 {
     if (cudaError_t e = (cudaError_t)c.top16.ensure(65537 * 4))
         return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation: %s", cudaGetErrorString(e));
     const int nb = (int)std::min<size_t>((N + 256) / 256, (size_t)c.sms * 8);
-    bdg::top_start_kernel<<<nb, 256, 0, c.stream>>>((const uint32_t*)c.sorted.p, (uint32_t)N, (uint32_t*)c.top16.p);
+    bdg::top_start_kernel<<<nb, 256, 0, st>>>(d_sorted, (uint32_t)N, (uint32_t*)c.top16.p);
     if (E) {
         const int eb = (int)std::min<size_t>((E + 255) / 256, (size_t)c.sms * 16);
-        bdg::cluster_index_kernel<<<eb, 256, 0, c.stream>>>((const uint32_t*)c.sorted.p, (const uint32_t*)c.top16.p, d_ea, d_eb, E, d_oa, d_ob);
+        bdg::cluster_index_kernel<<<eb, 256, 0, st>>>(d_sorted, (const uint32_t*)c.top16.p, d_ea, d_eb, E, d_oa, d_ob);
     }
     g_launches += 2;
     CU_TRY(cudaGetLastError());
     return BDG_OK;
 }
 
+static int node_blocks(size_t N, int sms) { return (int)std::min<size_t>((N + 255) / 256, (size_t)sms * 8); }
+static int edge_blocks(size_t E, int sms) { return (int)std::min<size_t>((E + 255) / 256, (size_t)sms * 16); }
+
+// every node free (centre -2, level 255, no claim), then the centres (barcode values d_cen[C]; unobserved ones have no node) seeded
+static int cluster_init(const uint32_t* d_sorted, size_t N, const uint32_t* d_cen, size_t C, int32_t* d_ci, uint8_t* d_lv, int32_t* d_min,
+                        int32_t* d_max, int sms, cudaStream_t st)
+{
+    bdg::cluster_init_kernel<<<node_blocks(N, sms), 256, 0, st>>>(d_ci, d_lv, d_min, d_max, (uint32_t)N);
+    if (C) bdg::cluster_seed_kernel<<<node_blocks(C, sms), 256, 0, st>>>(d_sorted, (uint32_t)N, d_cen, (uint32_t)C, d_ci, d_lv);
+    g_launches += 2;
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+static int cluster_mark(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, uint8_t* d_lv, unsigned int* d_bad, int sms, cudaStream_t st)
+{
+    if (E == 0) return BDG_OK;
+    bdg::cluster_mark_kernel<<<edge_blocks(E, sms), 256, 0, st>>>(d_ia, d_ib, E, d_lv, d_bad);
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+static int cluster_claim(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, int round, const int32_t* d_ci, const uint8_t* d_lv, int32_t* d_min,
+                         int32_t* d_max, int sms, cudaStream_t st)
+{
+    if (E == 0) return BDG_OK;
+    bdg::cluster_claim_kernel<<<edge_blocks(E, sms), 256, 0, st>>>(d_ia, d_ib, E, round, d_ci, d_lv, d_min, d_max);
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+static int cluster_resolve(int32_t* d_ci, uint8_t* d_lv, int32_t* d_min, int32_t* d_max, size_t N, int round, int sms, cudaStream_t st)
+{
+    bdg::cluster_resolve_kernel<<<node_blocks(N, sms), 256, 0, st>>>(d_ci, d_lv, d_min, d_max, (uint32_t)N, round);
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+// d_ea / d_eb hold barcode VALUES on entry and node indices on return (converted in place) unless `indexed`.
+// centre_idx / level may be NULL: the result then only stays on the device (cl[1] / cl[2]) for bdg_assign_reads*.
 static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint32_t* d_ea, uint32_t* d_eb, size_t E,
                              const uint32_t* centres, size_t C, int rounds, int32_t* centre_idx, uint8_t* level, size_t* n_has_edge = nullptr,
                              bool indexed = false)
@@ -2058,25 +2210,20 @@ static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint
     uint32_t* d_cen = (uint32_t*)c.cl[0].p;
     int32_t *d_ci = (int32_t*)c.cl[1].p, *d_min = (int32_t*)c.cl[3].p, *d_max = (int32_t*)c.cl[4].p;
     uint8_t* d_lv = (uint8_t*)c.cl[2].p;
-    const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
-    const int eb = (int)std::min<size_t>((E + 255) / 256, (size_t)c.sms * 16);
+    const int nb = node_blocks(N, c.sms);
     const bool trace = getenv("BDG_TRACE") != nullptr;
     double tr0 = 0, tr1 = 0, tr2 = 0;
     if (trace) { cudaStreamSynchronize(st); tr0 = now_ms(); }
     CU_TRY(cudaMemcpyAsync(d_cen, centres, C * 4, cudaMemcpyHostToDevice, st));
-    bdg::cluster_init_kernel<<<nb, 256, 0, st>>>(d_ci, d_lv, d_min, d_max, (uint32_t)N);
-    if (C) bdg::cluster_seed_kernel<<<(int)std::min<size_t>((C + 255) / 256, (size_t)c.sms * 8), 256, 0, st>>>(d_sorted, (uint32_t)N, d_cen, (uint32_t)C, d_ci, d_lv);
-    g_launches += 2;
+    if (int rc = cluster_init(d_sorted, N, d_cen, C, d_ci, d_lv, d_min, d_max, c.sms, st)) return rc;
     if (E) {
         if (!indexed)                                       // (d_sorted is c.sorted on every path that reaches here)
-            if (int e = index_edges(c, N, d_ea, d_eb, E, d_ea, d_eb)) return e;
-        bdg::cluster_mark_kernel<<<eb, 256, 0, st>>>(d_ea, d_eb, E, d_lv, d_bad);
-        g_launches++;
+            if (int e = index_edges(c, d_sorted, N, d_ea, d_eb, E, d_ea, d_eb, st)) return e;
+        if (int rc = cluster_mark(d_ea, d_eb, E, d_lv, d_bad, c.sms, st)) return rc;
         if (trace) { cudaStreamSynchronize(st); tr1 = now_ms(); }
         for (int r = 1; r <= rounds; r++) {
-            bdg::cluster_claim_kernel<<<eb, 256, 0, st>>>(d_ea, d_eb, E, r, d_ci, d_lv, d_min, d_max);
-            bdg::cluster_resolve_kernel<<<nb, 256, 0, st>>>(d_ci, d_lv, d_min, d_max, (uint32_t)N, r);
-            g_launches += 2;
+            if (int rc = cluster_claim(d_ea, d_eb, E, r, d_ci, d_lv, d_min, d_max, c.sms, st)) return rc;
+            if (int rc = cluster_resolve(d_ci, d_lv, d_min, d_max, N, r, c.sms, st)) return rc;
         }
     }
     CU_TRY(cudaGetLastError());
@@ -2176,12 +2323,12 @@ static int cluster_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, s
             if (k == 0) continue;
             if (&src == &c) {
                 CU_TRY(cudaSetDevice(c.dev));
-                if (int rc = index_edges(c, N, (const uint32_t*)c.ea.p, (const uint32_t*)c.eb.p, k, (uint32_t*)c.gather_a.p + off, (uint32_t*)c.gather_b.p + off)) return rc;
+                if (int rc = index_edges(c, (const uint32_t*)c.sorted.p, N, (const uint32_t*)c.ea.p, (const uint32_t*)c.eb.p, k, (uint32_t*)c.gather_a.p + off, (uint32_t*)c.gather_b.p + off, c.stream)) return rc;
             } else {
                 CU_TRY(cudaSetDevice(src.dev));
                 if (cudaError_t err = (cudaError_t)src.gather_a.ensure(k * 4)) return fail(BDG_ERR_OOM, "index buffer: %s", cudaGetErrorString(err));
                 if (cudaError_t err = (cudaError_t)src.gather_b.ensure(k * 4)) return fail(BDG_ERR_OOM, "index buffer: %s", cudaGetErrorString(err));
-                if (int rc = index_edges(src, N, (const uint32_t*)src.ea.p, (const uint32_t*)src.eb.p, k, (uint32_t*)src.gather_a.p, (uint32_t*)src.gather_b.p)) return rc;
+                if (int rc = index_edges(src, (const uint32_t*)src.sorted.p, N, (const uint32_t*)src.ea.p, (const uint32_t*)src.eb.p, k, (uint32_t*)src.gather_a.p, (uint32_t*)src.gather_b.p, src.stream)) return rc;
                 CU_TRY(cudaMemcpyPeerAsync((uint32_t*)c.gather_a.p + off, c.dev, src.gather_a.p, src.dev, k * 4, src.stream));
                 CU_TRY(cudaMemcpyPeerAsync((uint32_t*)c.gather_b.p + off, c.dev, src.gather_b.p, src.dev, k * 4, src.stream));
             }
@@ -2199,6 +2346,66 @@ static int cluster_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, s
     // the handle's edge VALUES are turned into node indices in place: the handle is consumed (stale afterwards)
     c.generation++;
     return cluster_on_device(c, (const uint32_t*)c.sorted.p, N, (uint32_t*)c.ea.p, (uint32_t*)c.eb.p, e->count[0], centres, C, rounds, centre_idx, level, n_has_edge);
+}
+
+// ---- the phases of cluster() on caller-owned node arrays (one process per GPU; include/badger_b200.h) ----
+static DevCtx* claimed_current(int* rc)
+{
+    DevCtx* c = ctx_of_current_device();
+    *rc = c ? BDG_OK : fail(BDG_ERR_NODEVICE, "the current device was not claimed by bdg_init");
+    return c;
+}
+
+int bdg_dev_index_edges(const uint32_t* d_sorted, size_t N, const uint32_t* d_ea, const uint32_t* d_eb, size_t E, uint32_t* d_ia, uint32_t* d_ib,
+                        void* stream)
+{
+    if (!d_sorted || (E && (!d_ea || !d_eb || !d_ia || !d_ib))) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (N == 0 || N > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "need 0 < N < 2^31");
+    int rc = 0;
+    DevCtx* c = claimed_current(&rc);
+    if (rc) return rc;
+    return index_edges(*c, d_sorted, N, d_ea, d_eb, E, d_ia, d_ib, (cudaStream_t)stream);
+}
+
+int bdg_dev_cluster_init(const uint32_t* d_sorted, size_t N, const uint32_t* d_centres, size_t C, int32_t* d_centre_idx, uint8_t* d_level,
+                         int32_t* d_cmin, int32_t* d_cmax, void* stream)
+{
+    if (!d_sorted || !d_centre_idx || !d_level || !d_cmin || !d_cmax || (C && !d_centres)) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (N == 0 || N > 0x7FFFFFFFull || C > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "need 0 < N < 2^31 and C < 2^32");
+    int rc = 0;
+    DevCtx* c = claimed_current(&rc);
+    if (rc) return rc;
+    return cluster_init(d_sorted, N, d_centres, C, d_centre_idx, d_level, d_cmin, d_cmax, c->sms, (cudaStream_t)stream);
+}
+
+int bdg_dev_cluster_mark(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, uint8_t* d_level, unsigned int* d_bad, void* stream)
+{
+    if (E && (!d_ia || !d_ib || !d_level || !d_bad)) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    int rc = 0;
+    DevCtx* c = claimed_current(&rc);
+    if (rc) return rc;
+    return cluster_mark(d_ia, d_ib, E, d_level, d_bad, c->sms, (cudaStream_t)stream);
+}
+
+int bdg_dev_cluster_claim(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, int round, const int32_t* d_centre_idx, const uint8_t* d_level,
+                          int32_t* d_cmin, int32_t* d_cmax, void* stream)
+{
+    if (E && (!d_ia || !d_ib || !d_centre_idx || !d_level || !d_cmin || !d_cmax)) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (round < 1 || round > 253) return fail(BDG_ERR_ARG, "round must be in 1..253");
+    int rc = 0;
+    DevCtx* c = claimed_current(&rc);
+    if (rc) return rc;
+    return cluster_claim(d_ia, d_ib, E, round, d_centre_idx, d_level, d_cmin, d_cmax, c->sms, (cudaStream_t)stream);
+}
+
+int bdg_dev_cluster_resolve(int32_t* d_centre_idx, uint8_t* d_level, int32_t* d_cmin, int32_t* d_cmax, size_t N, int round, void* stream)
+{
+    if (!d_centre_idx || !d_level || !d_cmin || !d_cmax) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (N == 0 || N > 0x7FFFFFFFull || round < 1 || round > 253) return fail(BDG_ERR_ARG, "need 0 < N < 2^31 and round in 1..253");
+    int rc = 0;
+    DevCtx* c = claimed_current(&rc);
+    if (rc) return rc;
+    return cluster_resolve(d_centre_idx, d_level, d_cmin, d_cmax, N, round, c->sms, (cudaStream_t)stream);
 }
 
 int bdg_member_sorted(const uint32_t* sorted_wl, size_t W, const uint32_t* q, size_t Q, uint8_t* hit)

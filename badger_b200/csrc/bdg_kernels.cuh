@@ -380,6 +380,89 @@ __global__ void dedup_scatter_kernel(const uint32_t* __restrict__ si, const uint
 }
 
 // ---------------------------------------------------------------------------------------------------
+// Merge of the dedup results of P parts (one process per GPU, bdg_dev_dedup_merge): every part brings its distinct barcodes
+// ascending, their counts and their local first-seen positions.  The first sighting of a barcode over all parts is the
+// smallest (part, local position), one 32-bit key: offset of the part (the sizes of the parts before it) + position.
+//   merge_gather_kernel   the P lists (part p at starts[p], offs[p+1]-offs[p] entries) -> one concatenation with the first
+//                         key of every entry; the entries of part `mine` are compared with the caller's own list
+//   (radix sort by barcode, dedup_heads_kernel, inclusive scan: runs of equal barcodes, at most P entries each)
+//   merge_runs_kernel     per run: barcode, summed count, smallest first key; for the entries of part `mine`, the run
+//   (radix sort of the runs by first key: the global first-seen order)
+//   merge_finish_kernel   distinct / counts in first-seen order and the first-seen position of every run
+//   merge_local_kernel    local first-seen position of part `mine` -> global first-seen position
+//   merge_remap_kernel    the read -> barcode map of part `mine` rewritten through that table
+// ---------------------------------------------------------------------------------------------------
+__global__ void merge_gather_kernel(const uint32_t* __restrict__ keys, const uint32_t* __restrict__ counts, const uint32_t* __restrict__ first,
+                                    const uint64_t* __restrict__ starts, const uint32_t* __restrict__ offs, uint32_t P, uint32_t total,
+                                    uint32_t mine, const uint32_t* __restrict__ own_sorted, uint32_t* __restrict__ out_key,
+                                    uint32_t* __restrict__ out_idx, uint32_t* __restrict__ out_count, uint32_t* __restrict__ out_first,
+                                    unsigned int* __restrict__ bad)
+{
+    for (uint32_t j = blockIdx.x * blockDim.x + threadIdx.x; j < total; j += gridDim.x * blockDim.x) {
+        uint32_t lo = 0, hi = P;                               // part p with offs[p] <= j < offs[p + 1]
+        while (hi - lo > 1) {
+            const uint32_t mid = (lo + hi) >> 1;
+            if (__ldg(&offs[mid]) <= j) lo = mid; else hi = mid;
+        }
+        const uint32_t q = j - __ldg(&offs[lo]);
+        const uint64_t src = __ldg(&starts[lo]) + q;
+        const uint32_t k = __ldg(&keys[src]);
+        out_key[j] = k;
+        out_idx[j] = j;
+        out_count[j] = __ldg(&counts[src]);
+        out_first[j] = __ldg(&offs[lo]) + __ldg(&first[src]);
+        if (lo == mine && __ldg(&own_sorted[q]) != k) *bad = 1u;
+    }
+}
+
+__global__ void merge_runs_kernel(const uint32_t* __restrict__ sk, const uint32_t* __restrict__ si, const uint32_t* __restrict__ head,
+                                  const uint32_t* __restrict__ scan_incl, uint32_t n, const uint32_t* __restrict__ count,
+                                  const uint32_t* __restrict__ first, uint32_t mine_off, uint32_t mine_n, uint32_t* __restrict__ run_key,
+                                  uint32_t* __restrict__ run_count, uint32_t* __restrict__ run_first, uint32_t* __restrict__ mine_run)
+{
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        if (!__ldg(&head[i])) continue;
+        const uint32_t r = __ldg(&scan_incl[i]) - 1u;
+        uint32_t c = 0, f = 0xFFFFFFFFu;
+        for (uint32_t j = i; j < n && (j == i || !__ldg(&head[j])); j++) {
+            const uint32_t e = __ldg(&si[j]);
+            c += __ldg(&count[e]);
+            f = min(f, __ldg(&first[e]));
+            if (e - mine_off < mine_n) mine_run[e - mine_off] = r;   // (unsigned: e < mine_off wraps above mine_n)
+        }
+        run_key[r] = __ldg(&sk[i]);
+        run_count[r] = c;
+        run_first[r] = f;
+    }
+}
+
+// order[pos] = run with the pos-th smallest first key
+__global__ void merge_finish_kernel(const uint32_t* __restrict__ order, const uint32_t* __restrict__ run_key, const uint32_t* __restrict__ run_count,
+                                    uint32_t n_runs, uint32_t* __restrict__ distinct, uint32_t* __restrict__ counts, uint32_t* __restrict__ pos_of_run)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n_runs; p += gridDim.x * blockDim.x) {
+        const uint32_t r = __ldg(&order[p]);
+        distinct[p] = __ldg(&run_key[r]);
+        counts[p] = __ldg(&run_count[r]);
+        pos_of_run[r] = p;
+    }
+}
+
+// own_sorted_pos[q] = ascending position of the part's q-th barcode in first-seen order (its own list)
+__global__ void merge_local_kernel(const uint32_t* __restrict__ own_sorted_pos, const uint32_t* __restrict__ mine_run,
+                                   const uint32_t* __restrict__ pos_of_run, uint32_t n, uint32_t* __restrict__ global_pos)
+{
+    for (uint32_t q = blockIdx.x * blockDim.x + threadIdx.x; q < n; q += gridDim.x * blockDim.x)
+        global_pos[q] = __ldg(&pos_of_run[__ldg(&mine_run[__ldg(&own_sorted_pos[q])])]);
+}
+
+__global__ void merge_remap_kernel(uint32_t* __restrict__ read_to_distinct, uint32_t n, const uint32_t* __restrict__ global_pos)
+{
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
+        read_to_distinct[i] = __ldg(&global_pos[read_to_distinct[i]]);
+}
+
+// ---------------------------------------------------------------------------------------------------
 // Rows f-1 / f-2 with the per-read arrays staying on the device: bdg_dedup_reads compacts the valid rows (valid bytes +
 // their exclusive scan), dedups them as above and keeps read -> first-seen position resident; bdg_assign_reads then
 // turns the clustering result into the centre of every input row (barcode_graph.py:322-329 + 395-404) with two

@@ -96,44 +96,47 @@ def pack16_sorted(records: torch.Tensor) -> torch.Tensor:
     return out[:int(n.value)]
 
 
-def _edge_cap(n, t):
+def _edge_cap(n, t, nparts=1):
     """First guess of the edge buffer size; BDG_EDGE_CAP_PER_ROW overrides the edges per row, as for the host builds."""
     per_row = int(os.environ.get("BDG_EDGE_CAP_PER_ROW", 16 if t <= 1 else 64))
-    return max(1 << 16, max(per_row, 1) * n + 1024)
+    return max(1 << 16, max(per_row, 1) * n // nparts + 1024)
 
 
-def edges(sorted_unique: torch.Tensor, t: int):
+def edges(sorted_unique: torch.Tensor, t: int, *, part: int = 0, nparts: int = 1):
     """index.py:77-93 + barcode_graph.py:224-249 (ops.edges_build) on the first device: (a, b, d), every undirected edge once with
     a < b, order unspecified; a / b in the dtype of sorted_unique, d uint8.  sorted_unique must be strictly increasing as uint32
     (not checked here; ops.edges_build checks it).  Waits once for the edge count; when the first guess of the buffer size was
-    too small, the build runs again with the exact size (the edge set is deterministic)."""
+    too small, the build runs again with the exact size (the edge set is deterministic).  part / nparts: only the edges of that
+    part of the construction (include/badger_b200.h BDG_ROW_TILE); the nparts parts are disjoint and their union is the edge set."""
     _ready()
     _check(sorted_unique, "sorted_unique", BARCODE_DTYPES)
+    if not 0 <= part < nparts:
+        raise ValueError("part %d of %d parts" % (part, nparts))
     dev, n, L = sorted_unique.device, sorted_unique.numel(), lib()
     count = torch.zeros(1, dtype=torch.int64, device=dev)
-    cap = _edge_cap(n, t)
+    cap = _edge_cap(n, t, nparts)
     with torch.cuda.device(dev):
         for _ in range(2):
             a = torch.empty(cap, dtype=sorted_unique.dtype, device=dev)
             b = torch.empty(cap, dtype=sorted_unique.dtype, device=dev)
             d = torch.empty(cap, dtype=torch.uint8, device=dev)
-            check(L.bdg_dev_edges_build(_ptr(sorted_unique), n, int(t), 0, 1, a.data_ptr(), b.data_ptr(), d.data_ptr(), cap,
-                                        count.data_ptr(), _stream()))
+            check(L.bdg_dev_edges_build(_ptr(sorted_unique), n, int(t), int(part), int(nparts), a.data_ptr(), b.data_ptr(), d.data_ptr(),
+                                        cap, count.data_ptr(), _stream()))
             k = int(count.item())
             if k < 0:
                 # bit 63: a sparse pass listed more candidate tiles than the device's tile list holds (adversarial, extremely dense
                 # inputs).  The host build grows the list and its result is the edge set: copy that one out.
-                return _edges_host_build(sorted_unique, t)
+                return _edges_host_build(sorted_unique, t, part, nparts)
             if k <= cap:
                 return a[:k], b[:k], d[:k]
             cap = k
     raise _lib.BadgerB200Error(_lib.BDG_ERR_CUDA, "edge construction did not settle after growing its buffers (count %d)" % k)
 
 
-def _edges_host_build(sorted_unique, t):
+def _edges_host_build(sorted_unique, t, part, nparts):
     s = sorted_unique.cpu().numpy().view(np.uint32)
     h = C.c_void_p()
-    check(lib().bdg_edges_build_part(_lib.ptr(s), s.size, int(t), 0, 1, C.byref(h)))
+    check(lib().bdg_edges_build_part(_lib.ptr(s), s.size, int(t), int(part), int(nparts), C.byref(h)))
     try:
         return edges_copy(h, sorted_unique.dtype)
     finally:

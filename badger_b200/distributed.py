@@ -1,0 +1,228 @@
+"""The correction step over a torch.distributed process group, one process per GPU: every rank keeps its own reads.
+
+    every rank                                   what crosses between the ranks
+      device.dedup_reads of its own reads          -
+      its distinct list, counts, first sightings   all-gather (sizes, then the three lists padded to the longest)
+      bdg_dev_dedup_merge                          -   (the global distinct set, the same on every rank; the rank's read map
+                                                        now points at global first-seen positions)
+      device.edges, part `rank` of `world`         all-reduce of the edge count; the edges stay on the rank that found them
+      pipeline.select_centres                      -   (identical inputs on every rank: identical centres)
+      cluster_levels: mark, two rounds             all-reduce of the levels (min), then per round of the claims (min / max)
+      --high_sens on rank 0                        broadcast of the patched node -> centre array
+      bdg_dev_assign_reads32 of its own rows       all-reduce of the rows with a centre
+
+Nothing per read is exchanged.  Concatenated in rank order, the results equal those of device.assign_packed (and
+pipeline.assign_packed(form="u32")) run in one process on the concatenation of the ranks' inputs in rank order.
+
+Every call is collective: all ranks of the group make it, with the same scalar arguments.  Which collectives run depends only on
+those arguments and on values reduced over the group, never on a rank's own reads, so a rank with no rows, or with no valid row,
+takes part like any other.  Collectives run on CUDA tensors in the order of torch.cuda.current_stream() (NCCL or gloo).
+"""
+from __future__ import annotations
+
+import ctypes as C
+import time
+
+import numpy as np
+import torch
+import torch.distributed as dist
+
+from . import _lib, pipeline
+from . import device as bd
+from ._lib import check, lib
+
+ROUNDS = 2          # barcode_graph.py:279-301 runs two rounds
+
+
+class _Group:
+    """Rank, world size and the collectives of one call; without an initialised process group a world of one, whose collectives
+    return their input.  `traffic` counts the bytes every collective delivered to this rank, by name."""
+
+    def __init__(self, group, traffic=None):
+        self.on = dist.is_available() and dist.is_initialized()
+        self.pg = group
+        self.rank = dist.get_rank(group) if self.on else 0
+        self.world = dist.get_world_size(group) if self.on else 1
+        self.traffic = traffic if traffic is not None else {}
+
+    def _count(self, name, nbytes):
+        self.traffic[name] = self.traffic.get(name, 0) + int(nbytes)
+
+    def all_gather(self, t, name):
+        """[world, *t.shape]: the tensors of all ranks in rank order."""
+        out = torch.empty((self.world,) + tuple(t.shape), dtype=t.dtype, device=t.device)
+        if self.on:
+            dist.all_gather(list(out.unbind(0)), t, group=self.pg)
+        else:
+            out[0].copy_(t)
+        self._count(name, out.numel() * out.element_size())
+        return out
+
+    def all_reduce(self, t, op, name):
+        if self.on:
+            dist.all_reduce(t, op=op, group=self.pg)
+        self._count(name, t.numel() * t.element_size())
+        return t
+
+    def broadcast_from_first(self, t, name):
+        if self.on:
+            dist.broadcast(t, src=dist.get_global_rank(self.pg, 0) if self.pg is not None else 0, group=self.pg)
+        self._count(name, t.numel() * t.element_size())
+        return t
+
+
+def _lists(rm, dev):
+    """int32[3, n]: the rank's distinct barcodes ascending, their counts and their local first-seen positions."""
+    n = rm.n_distinct
+    out = torch.empty((3, n), dtype=torch.int32, device=dev)
+    if n:
+        sp = rm.sorted_pos                                            # first-seen -> ascending position
+        out[0] = rm.sorted_distinct.view(torch.int32)
+        out[1, sp] = rm.counts.to(torch.int32)
+        out[2, sp] = torch.arange(n, dtype=torch.int32, device=dev)
+    return out
+
+
+def dedup_merge(rm, group=None, *, _g=None):
+    """The distinct barcodes of every rank's read map `rm` (device.dedup_reads) merged into the global ones: a DeviceReadMap
+    whose distinct / counts / sorted_pos / sorted_distinct are those of one dedup over the concatenation of all ranks' reads in
+    rank order (the same on every rank), and whose read map holds this rank's rows.  rm's token dies.  Returns (merged, valid
+    reads of all ranks, rows of all ranks); merged is None on every rank when no rank has a valid read."""
+    g = _g or _Group(group)
+    dev = bd._device()
+    local = _lists(rm, dev)
+    meta = torch.tensor([rm.n_distinct, rm.n_valid, rm.rows], dtype=torch.int64, device=dev)
+    metas = g.all_gather(meta, "sizes").cpu()                         # host wait: the sizes decide the shapes below
+    sizes = [int(x) for x in metas[:, 0]]
+    total_valid, total_rows = int(metas[:, 1].sum()), int(metas[:, 2].sum())
+    if total_valid == 0:
+        return None, total_valid, total_rows
+    width = max(sizes)
+    mine = torch.zeros((3, width), dtype=torch.int32, device=dev)
+    mine[:, :rm.n_distinct] = local
+    parts = g.all_gather(mine, "lists")                               # [world, 3, width]
+    base, row = parts.data_ptr(), 4 * width
+    starts = (C.c_size_t * g.world)(*[3 * width * p for p in range(g.world)])
+    n, tok = C.c_size_t(0), C.c_ulonglong(0)
+    with torch.cuda.device(dev):
+        check(lib().bdg_dev_dedup_merge(rm.token, base, base + row, base + 2 * row, starts, (C.c_size_t * g.world)(*sizes), g.world,
+                                        g.rank, C.byref(n), C.byref(tok), bd._stream()))
+    return bd.DeviceReadMap(int(n.value), rm.n_valid, rm.rows, int(tok.value), rm.dtype), total_valid, total_rows
+
+
+def cluster_levels(sorted_distinct: torch.Tensor, ea: torch.Tensor, eb: torch.Tensor, centres, rounds: int = ROUNDS, *, group=None,
+                   _g=None):
+    """barcode_graph.py:279-301 over the union of the ranks' edge lists (every rank passes its own; each edge on one rank only),
+    with the nodes (sorted_distinct, the same on every rank) and the centres (barcode values, the same on every rank) replicated.
+    Returns (centre_idx int32[N], level uint8[N]) tensors, equal on every rank: as ops.cluster_levels, except that level 254 marks
+    the nodes with an edge that no round reached.  The claims of every round are reduced over the group (minimum and maximum of
+    the claiming centres), which is the reference's same-round conflict rule over the union."""
+    g = _g or _Group(group)
+    bd._check(sorted_distinct, "sorted_distinct", bd.BARCODE_DTYPES)
+    bd._check(ea, "ea", (sorted_distinct.dtype,))
+    bd._check(eb, "eb", (sorted_distinct.dtype,))
+    dev, N, E = sorted_distinct.device, sorted_distinct.numel(), ea.numel()
+    if eb.numel() != E:
+        raise ValueError("ea has %d edges, eb %d" % (E, eb.numel()))
+    cen = torch.from_numpy(np.ascontiguousarray(centres, dtype=np.uint32).view(np.int32)).to(dev)
+    ci = torch.empty(N, dtype=torch.int32, device=dev)
+    lv = torch.empty(N, dtype=torch.uint8, device=dev)
+    cmin, cmax = torch.empty_like(ci), torch.empty_like(ci)
+    ia, ib = torch.empty(E, dtype=torch.int32, device=dev), torch.empty(E, dtype=torch.int32, device=dev)
+    bad = torch.zeros(1, dtype=torch.int32, device=dev)
+    L, st, p = lib(), bd._stream(), bd._ptr
+    with torch.cuda.device(dev):
+        check(L.bdg_dev_cluster_init(sorted_distinct.data_ptr(), N, p(cen), cen.numel(), ci.data_ptr(), lv.data_ptr(), cmin.data_ptr(),
+                                     cmax.data_ptr(), st))
+        check(L.bdg_dev_index_edges(sorted_distinct.data_ptr(), N, p(ea), p(eb), E, p(ia), p(ib), st))
+        check(L.bdg_dev_cluster_mark(p(ia), p(ib), E, lv.data_ptr(), bad.data_ptr(), st))
+        g.all_reduce(lv, dist.ReduceOp.MIN, "levels")                 # 255 -> 254 wherever any rank has an edge; centres keep 0
+        g.all_reduce(bad, dist.ReduceOp.MAX, "levels")
+        for r in range(1, int(rounds) + 1):
+            check(L.bdg_dev_cluster_claim(p(ia), p(ib), E, r, ci.data_ptr(), lv.data_ptr(), cmin.data_ptr(), cmax.data_ptr(), st))
+            g.all_reduce(cmin, dist.ReduceOp.MIN, "claims")
+            g.all_reduce(cmax, dist.ReduceOp.MAX, "claims")
+            check(L.bdg_dev_cluster_resolve(ci.data_ptr(), lv.data_ptr(), cmin.data_ptr(), cmax.data_ptr(), N, r, st))
+    if int(bad.item()):
+        raise _lib.BadgerB200Error(_lib.BDG_ERR_ARG, "an edge end point is not in the barcode array")
+    return ci, lv
+
+
+def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, threshold, n_cells, interval=25, whitelist_sorted=None,
+                  true_barcodes=None, high_sens=False, centre_order=None, group=None, timings=None):
+    """device.assign_packed over the ranks of `group` (None: the default group; no initialised process group: a world of one).
+    Called on every rank with that rank's reads (ranks / valid: CUDA tensors on the first device given to badger_b200.init, as
+    for device.assign_packed) and the same scalar arguments; whitelist_sorted and true_barcodes are the same on every rank.
+    Returns ((centre, has_centre), info) for the rank's own rows.  Concatenated in rank order, the results of all ranks equal
+    device.assign_packed run in one process on the concatenation of their inputs in rank order (first-seen order therefore
+    starts with rank 0's reads), and `info` - the same on every rank - equals its `info`.
+
+    With high_sens, rank 0 runs the per-barcode --high_sens work of pipeline.assign_packed on the host and broadcasts the result;
+    centre_order="set" is the set order of rank 0's process.  timings: a dict that receives the host time of every stage, each
+    stage ended by a device synchronise, and under "collective_bytes" the bytes each kind of collective delivered to this rank."""
+    bd._ready()
+    bd._check(ranks, "ranks", bd.BARCODE_DTYPES)
+    if whitelist_sorted is not None:
+        bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
+    if isinstance(true_barcodes, torch.Tensor):
+        true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+    T = timings if timings is not None else {}
+    g = _Group(group, T.setdefault("collective_bytes", {}) if timings is not None else None)
+    R, dev = ranks.numel(), ranks.device
+
+    def tick(name, t0):
+        if timings is not None:
+            torch.cuda.synchronize(dev)
+        pipeline._tick(T, name, t0)
+
+    t0 = time.perf_counter()
+    rm = bd.dedup_reads(ranks, valid)
+    tick("dedup_first_seen", t0)
+
+    t0 = time.perf_counter()
+    merged, total_valid, total_rows = dedup_merge(rm, _g=g)
+    tick("exchange_merge", t0)
+    info = {"reads": total_rows, "valid_reads": total_valid}
+    if merged is None:
+        return (torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)), info
+    N = merged.n_distinct
+
+    t0 = time.perf_counter()
+    s = merged.sorted_distinct                                        # the global nodes, ascending, on every rank
+    a, b, _ = bd.edges(s, threshold, part=g.rank, nparts=g.world)
+    n_edges = g.all_reduce(torch.tensor([a.numel()], dtype=torch.int64, device=dev), dist.ReduceOp.SUM, "counts")
+    info.update(distinct=int(N), edges=int(n_edges.item()))
+    tick("edges", t0)
+
+    t0 = time.perf_counter()
+    centres = np.asarray(list(dict.fromkeys(pipeline.select_centres(merged, n_cells, interval, whitelist_sorted, true_barcodes,
+                                                                    bd.centres_above))), dtype=np.uint32)
+    info["centres"] = int(centres.size)
+    tick("centres", t0)
+
+    t0 = time.perf_counter()
+    ci, lv = cluster_levels(s, a, b, centres, _g=g)
+    del a, b
+    n_has_edge = int(((lv != 255) & (lv != 0)).sum().item())
+    # badger.py:131 `len(counts) - len(edges.keys())`: the keys are the nodes with an edge plus every centre cluster() touched
+    info["disconnected"] = int(N) - (n_has_edge + int(centres.size))
+    tick("cluster", t0)
+
+    if high_sens:
+        t0 = time.perf_counter()
+        if g.rank == 0:
+            patched = pipeline.high_sens_patch(ci.cpu().numpy(), merged.host.sorted_distinct, merged.host.sorted_pos, centre_order)
+            ci.copy_(torch.from_numpy(patched))
+        g.broadcast_from_first(ci, "high_sens")
+        tick("high_sens", t0)
+
+    t0 = time.perf_counter()
+    centre = torch.zeros(R, dtype=ranks.dtype, device=dev)
+    has = torch.zeros(R, dtype=torch.bool, device=dev)
+    if rm.n_valid:
+        with torch.cuda.device(dev):
+            check(lib().bdg_dev_assign_reads32(merged.token, ci.data_ptr(), N, centre.data_ptr(), has.data_ptr(), R, None, bd._stream()))
+    n_assigned = g.all_reduce(has.sum(dtype=torch.int64).reshape(1), dist.ReduceOp.SUM, "counts")
+    info["assigned_reads"] = int(n_assigned.item())
+    tick("gather", t0)
+    return (centre, has), info

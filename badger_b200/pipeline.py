@@ -136,8 +136,21 @@ def run_stages(rm, info, T, gather, *, threshold, n_cells, interval, whitelist_s
     handle.free()
     info["disconnected"] = int(rm.n_distinct) - (int(has_edge.sum()) + int(centres.size))
     _tick(T, "cluster", t0)
-    # barcode_graph.py:370-385 on node positions: every node without a centre looks for the nearest used centre
     t0 = time.perf_counter()
+    ci = high_sens_patch(ci, s, spos, centre_order)
+    _tick(T, "high_sens", t0)
+
+    t0 = time.perf_counter()
+    out, n_assigned = gather(ci)
+    _tick(T, "gather", t0)
+    info["assigned_reads"] = int(n_assigned)
+    return out
+
+
+def high_sens_patch(ci, s, spos, centre_order):
+    """barcode_graph.py:370-385 on node positions: every node without a centre (ci < 0) takes the nearest used centre within
+    distance 2, tried in the order centre_order names (see assign_packed).  ci: the clustering result (int32[N], patched in
+    place and returned); s: the distinct barcodes ascending; spos: their first-seen -> ascending positions."""
     todo = np.nonzero(ci < 0)[0]
     used_nodes = ops.sorted_unique(ci[ci >= 0])                              # set(assignments.values()), as nodes (ascending = by value)
     if centre_order is None:
@@ -161,10 +174,4 @@ def run_stages(rm, info, T, gather, *, threshold, n_cells, interval, whitelist_s
         am, _ = ops.nearest_bounded(s[todo], targets, 2)
         hit = am >= 0
         ci[todo[hit]] = np.searchsorted(s, targets[am[hit]]).astype(np.int32)
-    _tick(T, "high_sens", t0)
-
-    t0 = time.perf_counter()
-    out, n_assigned = gather(ci)
-    _tick(T, "gather", t0)
-    info["assigned_reads"] = int(n_assigned)
-    return out
+    return ci

@@ -247,6 +247,45 @@ int bdg_dev_edges_copy(const bdg_edges* e, uint32_t* d_a, uint32_t* d_b, uint8_t
  * of R_all rows.  n_assigned may be NULL: the call then does not wait for the gather. */
 int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx, size_t N, uint32_t* d_centre_per_row,
                            uint8_t* d_has_centre, size_t R_all, size_t* n_assigned, void* stream);
+
+/* ---- the correction step over P processes, one per GPU (badger_b200.distributed) ------------------------------------------
+ * Every process dedups its own reads (bdg_dev_dedup_reads), the processes exchange their distinct lists, and each reduces the
+ * P lists to the global distinct set with bdg_dev_dedup_merge.  The reads of part 0 come first, then those of part 1, ...:
+ * the global first sighting of a barcode is the smallest (part, local first-seen position).
+ * d_keys / d_counts / d_first: device memory on the first claimed device; part p's list has sizes[p] entries at index starts[p]
+ * (host arrays of n_parts): its distinct barcodes ASCENDING, their counts, and their local first-seen positions.  The list of
+ * my_part must be the one of the read map `token` names (checked: size, and every barcode on the device); token 0 stands for a
+ * part without a valid read, whose list is empty.  The parts hold fewer than 2^31 barcodes in all.
+ * On success *merged_token names a read map that holds THIS part's reads and the GLOBAL barcodes (N = *n_distinct):
+ *   distinct (dd[2])  in global first-seen order          counts (dd[0])  summed over the parts, in that order
+ *   sorted_pos (dd[1]) global first-seen -> ascending     sorted_distinct (dd[6]) ascending
+ *   the read -> barcode map (dd[7]) points at global first-seen positions; the valid rows are those of the dedup call.
+ * bdg_dev_dedup_fetch, bdg_dev_centres_above, bdg_centres_rest and bdg_dev_assign_reads32 (with a device centre_idx over the N
+ * global nodes) take the merged token as they take a dedup token; `token` itself dies.  On error the token stays as it was. */
+int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first,
+                        const size_t* starts, const size_t* sizes, int n_parts, int my_part, size_t* n_distinct,
+                        unsigned long long* merged_token, void* stream);
+/* The phases of bdg_cluster_levels over node arrays the caller owns, on `stream` of the current (claimed) device and without a
+ * synchronisation, so that processes can reduce the claims between the phases.  Nodes are positions in d_sorted[N]
+ * (0 < N < 2^31); d_centre_idx / d_level as for bdg_cluster_levels, except that level 254 marks a node with an edge that no
+ * round reached; d_cmin / d_cmax (int32[N]) hold the claims of the running round.
+ *   index_edges  edge end points (barcode values) -> node indices (in place when d_ia == d_ea); an end point that is not a node
+ *                turns both ends of its edge into 0xFFFFFFFF, which cluster_mark reports through *d_bad != 0
+ *   cluster_init every node free, no claims; the centres (barcode values, d_centres[C]) that are nodes seeded at level 0
+ *   cluster_mark level 255 -> 254 at both ends of every edge
+ *   cluster_claim (round r = 1, 2, ...)  every edge from a node joined at level r-1 to a free node records its centre in the free
+ *                node's min / max: over several edge lists, reduce d_cmin by minimum and d_cmax by maximum before the resolve
+ *   cluster_resolve (round r)  a claimed node joins when min == max and is evicted otherwise; clears the claims
+ * The reference runs rounds 1 and 2. */
+int bdg_dev_index_edges(const uint32_t* d_sorted, size_t N, const uint32_t* d_ea, const uint32_t* d_eb, size_t E, uint32_t* d_ia,
+                        uint32_t* d_ib, void* stream);
+int bdg_dev_cluster_init(const uint32_t* d_sorted, size_t N, const uint32_t* d_centres, size_t C, int32_t* d_centre_idx,
+                         uint8_t* d_level, int32_t* d_cmin, int32_t* d_cmax, void* stream);
+int bdg_dev_cluster_mark(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, uint8_t* d_level, unsigned int* d_bad, void* stream);
+int bdg_dev_cluster_claim(const uint32_t* d_ia, const uint32_t* d_ib, size_t E, int round, const int32_t* d_centre_idx,
+                          const uint8_t* d_level, int32_t* d_cmin, int32_t* d_cmax, void* stream);
+int bdg_dev_cluster_resolve(int32_t* d_centre_idx, uint8_t* d_level, int32_t* d_cmin, int32_t* d_cmax, size_t N, int round,
+                            void* stream);
 int bdg_dev_nearest_bounded(const uint32_t* d_q, size_t Q, const uint32_t* d_targets, size_t W, int max_d,
                             uint32_t* d_keys /* Q words of scratch */, int32_t* d_argmin, uint8_t* d_dist,
                             void* stream);
