@@ -94,6 +94,10 @@ def lib():
     L.bdg_dev_cluster_mark.argtypes = [_vp, _vp, _sz, _vp, _vp, _vp]
     L.bdg_dev_cluster_claim.argtypes = [_vp, _vp, _sz, _i, _vp, _vp, _vp, _vp, _vp]
     L.bdg_dev_cluster_resolve.argtypes = [_vp, _vp, _vp, _vp, _sz, _i, _vp]
+    L.bdg_dev_whitelist_check.argtypes = [_vp, _sz, _vp]
+    L.bdg_dev_kmer_index_create.argtypes = [_vp, _sz, _vp, C.POINTER(_vp)]
+    L.bdg_dev_kmer_index_query.argtypes = [_vp, _vp, _sz, _i, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz), _vp]
+    L.bdg_dev_kmer_score.argtypes = [_vp, _sz, _vp, _sz, _i, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz), _vp]
     L.bdg_part_pairs.argtypes = [_sz, _i, _i]
     L.bdg_part_pairs.restype = C.c_ulonglong
     L.bdg_dev_pipe_probe.argtypes = [_i, _i, _i, _vp, C.POINTER(C.c_ulonglong), _vp]
@@ -116,7 +120,8 @@ def lib():
                  "bdg_dev_nearest_bounded", "bdg_dev_pipe_probe", "bdg_tsv_open", "bdg_tsv_barcodes", "bdg_tsv_write_assignments", "bdg_lines16_open", "bdg_dedup_reads", "bdg_assign_reads", "bdg_pack16_sorted", "bdg_assign_reads32", "bdg_dedup_fetch", "bdg_centres_above", "bdg_centres_rest", "bdg_cluster_resident",
                  "bdg_tsv_write_assignments32", "bdg_dev_dedup_reads", "bdg_dev_dedup_fetch", "bdg_dev_pack16_sorted", "bdg_dev_centres_above",
                  "bdg_dev_edges_copy", "bdg_dev_assign_reads32", "bdg_dev_dedup_merge", "bdg_dev_index_edges", "bdg_dev_cluster_init",
-                 "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve"):
+                 "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve", "bdg_dev_whitelist_check",
+                 "bdg_dev_kmer_index_create", "bdg_dev_kmer_index_query", "bdg_dev_kmer_score"):
         getattr(L, name).restype = _i
     _lib = L
     return L

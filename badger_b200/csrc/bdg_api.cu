@@ -2439,6 +2439,31 @@ int bdg_member_sorted(const uint32_t* sorted_wl, size_t W, const uint32_t* q, si
     return BDG_OK;
 }
 
+// The check bdg_member_sorted makes on its whitelist, for a whitelist in device memory (bdg_dev_member_sorted does not check).
+int bdg_dev_whitelist_check(const uint32_t* d_sorted_wl, size_t W, void* stream)
+{
+    if (W <= 1) return BDG_OK;
+    if (!d_sorted_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
+    if (int e = ensure_buf(c.io[3], 8)) return e;
+    unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    CU_TRY(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
+    bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, c.stream>>>(d_sorted_wl, (uint32_t)W, d_bad);
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    unsigned long long first_bad = ~0ull;
+    CU_TRY(cudaMemcpyAsync(&first_bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
+    CU_TRY(cudaStreamSynchronize(c.stream));
+    if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "whitelist not sorted at index %llu", first_bad);
+    return BDG_OK;
+}
+
 int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, size_t W, int max_d, int32_t* argmin, uint8_t* dist)
 {
     if (Q == 0) return BDG_OK;
@@ -2486,7 +2511,9 @@ int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, si
 }
 
 // ---- a-5  KmerIndexer / QGramIndex: the known strings stay on the device between queries ------------------
-static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, bdg_kmer_index** out)
+// wl: the W strings in host memory (kind = cudaMemcpyHostToDevice) or in device memory on the first claimed device
+// (cudaMemcpyDeviceToDevice, read on that device's stream, which the device form has ordered after the caller's).
+static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, cudaMemcpyKind kind, bdg_kmer_index** out)
 {
     if (!out || (W && !wl)) return fail(BDG_ERR_ARG, "NULL pointer argument");
     *out = nullptr;
@@ -2501,7 +2528,7 @@ static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, bdg_km
         delete ix;
         return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", W * 4, cudaGetErrorString(e));
     }
-    cudaError_t e = cudaMemcpyAsync(ix->wl.p, wl, W * 4, cudaMemcpyHostToDevice, g_ctx[0].stream);
+    cudaError_t e = cudaMemcpyAsync(ix->wl.p, wl, W * 4, kind, g_ctx[0].stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(g_ctx[0].stream);
     if (e != cudaSuccess) { bdg_kmer_index_free(ix); return fail(BDG_ERR_CUDA, "upload of the index failed: %s", cudaGetErrorString(e)); }
     // posting lists of the strings' 6-mers (kmer_indexer.py:29-32): worth it once a bucket is a small share of the strings
@@ -2544,7 +2571,24 @@ static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, bdg_km
     return BDG_OK;
 }
 
-int bdg_kmer_index_create(const uint32_t* wl, size_t W, bdg_kmer_index** out) { return kmer_index_create(wl, W, true, out); }
+int bdg_kmer_index_create(const uint32_t* wl, size_t W, bdg_kmer_index** out)
+{
+    return kmer_index_create(wl, W, true, cudaMemcpyHostToDevice, out);
+}
+
+int bdg_dev_kmer_index_create(const uint32_t* d_known, size_t W, void* stream, bdg_kmer_index** out)
+{
+    if (!out || (W && !d_known)) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    *out = nullptr;
+    if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (W) if (int rc = check_on_first(d_known, "known")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    return kmer_index_create(d_known, W, true, cudaMemcpyDeviceToDevice, out);
+}
 
 int bdg_kmer_index_info(const bdg_kmer_index* ix, int* posted, double* kernel_ms)
 {
@@ -2568,14 +2612,45 @@ void bdg_kmer_index_free(bdg_kmer_index* ix)
     delete ix;
 }
 
+// The query proper, on c (the context of the index's device): d_q (Q queries) on that device, hits appended to d_hq / d_hw / d_cnt
+// / d_mult, of which only the first cap are stored.  Waits once, for *tot (the number of hits, which may exceed cap).
+static int kmer_query_core(bdg_kmer_index* ix, DevCtx& c, const uint32_t* d_q, size_t Q, int min_kmers, size_t cap, uint32_t* d_hq,
+                           uint32_t* d_hw, uint8_t* d_cnt, unsigned long long* d_mult, unsigned long long* tot)
+{
+    const size_t W = ix->W;
+    if (int e = ensure_buf(ix->outb[5], 8)) return e;
+    unsigned long long* d_total = (unsigned long long*)ix->outb[5].p;
+    CU_TRY(cudaMemsetAsync(d_total, 0, 8, c.stream));
+    CU_TRY(cudaEventRecord(ix->ev[0], c.stream));
+    if (ix->posted) {                                       // walk the buckets of the queries' own 6-mers
+        const unsigned blocks = (unsigned)std::min<unsigned long long>((unsigned long long)Q * 11, (unsigned long long)c.sms * 64);
+        bdg::kmer_post_kernel<<<blocks, bdg::NT, 0, c.stream>>>(d_q, (uint32_t)Q, (const uint32_t*)ix->wl.p, (const uint32_t*)ix->kstart.p,
+                                                              (const uint32_t*)ix->post.p, std::max(min_kmers, 1), (unsigned long long)cap, d_hq, d_hw,
+                                                              d_cnt, d_mult, d_total);
+    } else {
+        const uint32_t gy_total = (uint32_t)((Q + bdg::KS_QB - 1) / bdg::KS_QB);
+        const uint32_t gx = (uint32_t)((W + bdg::NT - 1) / bdg::NT);
+        if (gy_total > 65535u) return fail(BDG_ERR_ARG, "Q too large for one call (> 65535*256 queries)");
+        bdg::kmer_score_kernel<<<dim3(gx, gy_total), bdg::NT, 0, c.stream>>>(d_q, (uint32_t)Q, (const uint32_t*)ix->wl.p, (uint32_t)W, min_kmers,
+                                                                          (unsigned long long)cap, d_hq, d_hw, d_cnt, d_mult, d_total);
+    }
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaEventRecord(ix->ev[1], c.stream));
+    ix->timed = true;
+    *tot = 0;
+    CU_TRY(cudaMemcpyAsync(tot, d_total, 8, cudaMemcpyDeviceToHost, c.stream));
+    CU_TRY(cudaStreamSynchronize(c.stream));
+    return BDG_OK;
+}
+
 int bdg_kmer_index_query(bdg_kmer_index* ix, const uint32_t* q, size_t Q, int min_kmers, size_t cap, uint32_t* hit_q, uint32_t* hit_w,
                          uint8_t* cnt, uint64_t* mult, size_t* total)
 {
     if (!total) return fail(BDG_ERR_ARG, "NULL total pointer");
     *total = 0;
     if (!ix) return fail(BDG_ERR_ARG, "NULL index handle");
-    const size_t W = ix->W;
-    if (Q == 0 || W == 0) return BDG_OK;
+    if (Q == 0 || ix->W == 0) return BDG_OK;
     if (!q || (cap && (!hit_q || !hit_w || !cnt || !mult))) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (Q > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
     DevCtx* c = nullptr;
@@ -2583,35 +2658,15 @@ int bdg_kmer_index_query(bdg_kmer_index* ix, const uint32_t* q, size_t Q, int mi
     if (!c) return fail(BDG_ERR_NODEVICE, "the device the index lives on is no longer claimed (bdg_shutdown?)");
     CU_TRY(cudaSetDevice(c->dev));
     const size_t capa = std::max<size_t>(cap, 1);
-    const size_t sizes[6] = {Q * 4, capa * 4, capa * 4, capa, capa * 8, 8};     // queries, hit_q, hit_w, cnt, mult, total
-    for (int k = 0; k < 6; k++)
-        if (cudaError_t e = (cudaError_t)ix->outb[k].ensure(sizes[k]))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", sizes[k], cudaGetErrorString(e));
+    const size_t sizes[5] = {Q * 4, capa * 4, capa * 4, capa, capa * 8};     // queries, hit_q, hit_w, cnt, mult
+    for (int k = 0; k < 5; k++)
+        if (int e = ensure_buf(ix->outb[k], sizes[k])) return e;
     uint32_t *d_q = (uint32_t*)ix->outb[0].p, *d_hq = (uint32_t*)ix->outb[1].p, *d_hw = (uint32_t*)ix->outb[2].p;
     uint8_t* d_cnt = (uint8_t*)ix->outb[3].p;
-    unsigned long long *d_mult = (unsigned long long*)ix->outb[4].p, *d_total = (unsigned long long*)ix->outb[5].p;
-    CU_TRY(cudaMemsetAsync(d_total, 0, 8, c->stream));
+    unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
     CU_TRY(cudaMemcpyAsync(d_q, q, Q * 4, cudaMemcpyHostToDevice, c->stream));
-    CU_TRY(cudaEventRecord(ix->ev[0], c->stream));
-    if (ix->posted) {                                       // walk the buckets of the queries' own 6-mers
-        const unsigned blocks = (unsigned)std::min<unsigned long long>((unsigned long long)Q * 11, (unsigned long long)c->sms * 64);
-        bdg::kmer_post_kernel<<<blocks, bdg::NT, 0, c->stream>>>(d_q, (uint32_t)Q, (const uint32_t*)ix->wl.p, (const uint32_t*)ix->kstart.p,
-                                                               (const uint32_t*)ix->post.p, std::max(min_kmers, 1), (unsigned long long)cap, d_hq, d_hw,
-                                                               d_cnt, d_mult, d_total);
-    } else {
-        const uint32_t gy_total = (uint32_t)((Q + bdg::KS_QB - 1) / bdg::KS_QB);
-        const uint32_t gx = (uint32_t)((W + bdg::NT - 1) / bdg::NT);
-        if (gy_total > 65535u) return fail(BDG_ERR_ARG, "Q too large for one call (> 65535*256 queries)");
-        bdg::kmer_score_kernel<<<dim3(gx, gy_total), bdg::NT, 0, c->stream>>>(d_q, (uint32_t)Q, (const uint32_t*)ix->wl.p, (uint32_t)W, min_kmers,
-                                                                           (unsigned long long)cap, d_hq, d_hw, d_cnt, d_mult, d_total);
-    }
-    g_launches++;
-    CU_TRY(cudaGetLastError());
-    CU_TRY(cudaEventRecord(ix->ev[1], c->stream));
-    ix->timed = true;
     unsigned long long tot = 0;
-    CU_TRY(cudaMemcpyAsync(&tot, d_total, 8, cudaMemcpyDeviceToHost, c->stream));
-    CU_TRY(cudaStreamSynchronize(c->stream));
+    if (int rc = kmer_query_core(ix, *c, d_q, Q, min_kmers, cap, d_hq, d_hw, d_cnt, d_mult, &tot)) return rc;
     const size_t n = (size_t)std::min<unsigned long long>(tot, cap);
     if (n) {
         CU_TRY(cudaMemcpyAsync(hit_q, d_hq, n * 4, cudaMemcpyDeviceToHost, c->stream));
@@ -2625,6 +2680,42 @@ int bdg_kmer_index_query(bdg_kmer_index* ix, const uint32_t* q, size_t Q, int mi
     return BDG_OK;
 }
 
+int bdg_dev_kmer_index_query(bdg_kmer_index* ix, const uint32_t* d_q, size_t Q, int min_kmers, size_t cap, uint32_t* d_hit_q, uint32_t* d_hit_w,
+                             uint8_t* d_cnt, uint8_t* d_pos, size_t* total, void* stream)
+{
+    if (!total) return fail(BDG_ERR_ARG, "NULL total pointer");
+    *total = 0;
+    if (!ix) return fail(BDG_ERR_ARG, "NULL index handle");
+    if (Q == 0 || ix->W == 0) return BDG_OK;
+    if (!d_q || (cap && (!d_hit_q || !d_hit_w || !d_cnt || !d_pos))) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (Q > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
+    if (g_ctx.empty() || g_ctx[0].dev != ix->dev)
+        return fail(BDG_ERR_ARG, "the index lives on device %d, which is not the first claimed device", ix->dev);
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int rc = check_on_first(d_q, "queries")) return rc;
+    if (cap) {
+        const void* outs[4] = {d_hit_q, d_hit_w, d_cnt, d_pos};
+        for (const void* p : outs) if (int rc = check_on_first(p, "output")) return rc;
+    }
+    // the position counts are unpacked from library scratch into d_pos; the other outputs are written by the kernels in place
+    if (int e = ensure_buf(ix->outb[4], std::max<size_t>(cap, 1) * 8)) return e;
+    unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    unsigned long long tot = 0;
+    if (int rc = kmer_query_core(ix, c, d_q, Q, min_kmers, cap, d_hit_q, d_hit_w, d_cnt, d_mult, &tot)) return rc;
+    *total = (size_t)tot;
+    if (tot > cap) return fail(BDG_ERR_CAPACITY, "%llu hits but room for %zu", tot, cap);
+    if (tot) {
+        const unsigned blocks = (unsigned)std::min<unsigned long long>((tot * 11 + 255) / 256, (unsigned long long)c.sms * 16);
+        bdg::kmer_unpack_kernel<<<blocks, 256, 0, c.stream>>>(d_mult, tot, d_pos);
+        g_launches++;
+        CU_TRY(cudaGetLastError());
+    }
+    return BDG_OK;
+}
+
 int bdg_kmer_score(const uint32_t* q, size_t Q, const uint32_t* wl, size_t W, int min_kmers, size_t cap, uint32_t* hit_q,
                    uint32_t* hit_w, uint8_t* cnt, uint64_t* mult, size_t* total)
 {
@@ -2633,9 +2724,32 @@ int bdg_kmer_score(const uint32_t* q, size_t Q, const uint32_t* wl, size_t W, in
     if (Q == 0 || W == 0) return BDG_OK;
     if (!q || !wl || (cap && (!hit_q || !hit_w || !cnt || !mult))) return fail(BDG_ERR_ARG, "NULL pointer argument");
     bdg_kmer_index* ix = nullptr;
-    if (int rc = kmer_index_create(wl, W, Q >= 64, &ix)) return rc;       // a one-off call with few queries: the scan costs less than the lists
+    if (int rc = kmer_index_create(wl, W, Q >= 64, cudaMemcpyHostToDevice, &ix)) return rc;       // a one-off call with few queries: the scan costs less than the lists
     const int rc = bdg_kmer_index_query(ix, q, Q, min_kmers, cap, hit_q, hit_w, cnt, mult, total);
     bdg_kmer_index_free(ix);
+    return rc;
+}
+
+int bdg_dev_kmer_score(const uint32_t* d_q, size_t Q, const uint32_t* d_wl, size_t W, int min_kmers, size_t cap, uint32_t* d_hit_q,
+                       uint32_t* d_hit_w, uint8_t* d_cnt, uint8_t* d_pos, size_t* total, void* stream)
+{
+    if (!total) return fail(BDG_ERR_ARG, "NULL total pointer");
+    *total = 0;
+    if (Q == 0 || W == 0) return BDG_OK;
+    if (!d_q || !d_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    CU_TRY(cudaSetDevice(c.dev));
+    if (int rc = check_on_first(d_wl, "wl")) return rc;
+    bdg_kmer_index* ix = nullptr;
+    {
+        CallerOrder order(c, stream);
+        if (int rc = order.begin()) return rc;
+        if (int rc = kmer_index_create(d_wl, W, Q >= 64, cudaMemcpyDeviceToDevice, &ix)) return rc;   // the rule of bdg_kmer_score
+    }
+    const int rc = bdg_dev_kmer_index_query(ix, d_q, Q, min_kmers, cap, d_hit_q, d_hit_w, d_cnt, d_pos, total, stream);
+    bdg_kmer_index_free(ix);          // cudaFree waits for the unpack kernel that still reads the index's scratch
     return rc;
 }
 

@@ -4,6 +4,7 @@
 //   edges_kernel<MODE>   (bdg_edges.cuh) all-pairs edge construction over the sorted barcodes   INT-ALU bound
 //   nearest_kernel       Q x W bounded plain edit distance, first minimum per query           INT-ALU bound
 //   kmer_score_kernel    Q x W shared-6-mer product counts with per-position multiplicities   INT-ALU bound
+//   kmer_unpack_kernel   packed position counts -> uint8[hits][11] (device form of a-5)        HBM bound
 //   member_kernel        sorted-whitelist membership (smem pivots + L2-resident search)       HBM/L2 bound
 //   pack16_kernel        16 ASCII bases -> 2-bit packed uint32 + validity                     HBM bound
 //   pipe_probe_kernel    LOP3 / IMAD / POPC issue-rate probe for the integer roofline
@@ -208,6 +209,16 @@ __global__ void __launch_bounds__(NT) kmer_score_kernel(const uint32_t* __restri
                 mult[pos] = mu;
             }
         }
+    }
+}
+
+// kmer_unpack_kernel (a-5, device form): the 4-bit position counts of n hits (mult, nibble p = query position p) as uint8[n][11],
+// the layout of the host operator's result.  One thread per output byte, so the writes are coalesced.
+__global__ void kmer_unpack_kernel(const unsigned long long* __restrict__ mult, uint64_t n, uint8_t* __restrict__ pos)
+{
+    for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n * 11; i += (uint64_t)gridDim.x * blockDim.x) {
+        const uint64_t h = i / 11;
+        pos[i] = (uint8_t)((__ldg(&mult[h]) >> (4 * (i - h * 11))) & 15u);
     }
 }
 

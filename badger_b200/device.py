@@ -1,5 +1,6 @@
 """The correction step on CUDA tensors: the operators of ``ops`` and ``pipeline.assign_packed`` for callers whose barcodes are
-already on the GPU (a torch pipeline, or letters read into a CUDA tensor and packed with ``pack16``).
+already on the GPU (a torch pipeline, or letters read into a CUDA tensor and packed with ``pack16``), and the whitelist
+operators ``member_sorted``, ``nearest_bounded``, ``kmer_score`` and ``KmerIndex``, whose per-query and per-hit arrays stay there.
 
 Tensors live on the first device given to ``badger_b200.init`` (where the library keeps the read map) and every call runs in
 order with ``torch.cuda.current_stream()`` of that device: inputs produced there, and outputs consumed there, need no
@@ -255,3 +256,99 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
                               whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens,
                               centre_order=centre_order, centres_above=centres_above)
     return out, info
+
+
+# ---------------------------------------------------------------------------------------------- the whitelist operators
+def member_sorted(sorted_wl: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
+    """ops.member_sorted on tensors: bool[Q], hit[i] = q[i] is in sorted_wl.  sorted_wl must be ascending as uint32; it is
+    checked as the host form checks it (one 8-byte wait), and an unsorted whitelist raises the same error."""
+    _ready()
+    _check(sorted_wl, "sorted_wl", BARCODE_DTYPES)
+    _check(q, "q", BARCODE_DTYPES)
+    Q, W = q.numel(), sorted_wl.numel()
+    hit = torch.empty(Q, dtype=torch.bool, device=q.device)
+    if Q:
+        with torch.cuda.device(q.device):
+            check(lib().bdg_dev_whitelist_check(_ptr(sorted_wl), W, _stream()))
+            check(lib().bdg_dev_member_sorted(_ptr(sorted_wl), W, q.data_ptr(), Q, hit.data_ptr(), _stream()))
+    return hit
+
+
+def nearest_bounded(q: torch.Tensor, targets_in_order: torch.Tensor, max_d: int = 2):
+    """ops.nearest_bounded on tensors: (argmin int32[Q], dist uint8[Q]), the first index of the minimum plain edit distance over
+    the targets in their given order, kept when it is <= max_d; -1 / 255 otherwise."""
+    _ready()
+    _check(q, "q", BARCODE_DTYPES)
+    _check(targets_in_order, "targets_in_order", BARCODE_DTYPES)
+    Q, W, dev = q.numel(), targets_in_order.numel(), q.device
+    am = torch.empty(Q, dtype=torch.int32, device=dev)
+    dist = torch.empty(Q, dtype=torch.uint8, device=dev)
+    if Q:
+        keys = torch.empty(Q, dtype=torch.int32, device=dev)      # the packed (distance, index) minimum of every query
+        with torch.cuda.device(dev):
+            check(lib().bdg_dev_nearest_bounded(q.data_ptr(), Q, _ptr(targets_in_order), W, int(max_d), keys.data_ptr(), am.data_ptr(),
+                                                dist.data_ptr(), _stream()))
+    return am, dist
+
+
+def _int32_sized(t, name):
+    if t.numel() >= 1 << 31:
+        raise ValueError("%s has %d entries; the hit indices are int32, so fewer than 2^31 are allowed" % (name, t.numel()))
+
+
+def _kmer_query(call, q, n_known, min_kmers, cap, hint=None):
+    """ops._kmer_query on tensors: the hits land in tensors sized for `cap` (returned as views of their first `hits` rows).  A
+    first guess that is too small costs one repeated launch with the exact size; hint carries the room needed from call to call."""
+    _check(q, "q", BARCODE_DTYPES)
+    _int32_sized(q, "q")
+    Q, dev = q.numel(), q.device
+    if cap is None:
+        cap = hint[0] if hint and hint[0] else max(1 << 16, min(4 * n_known, 2048 * max(Q, 1)))
+    for attempt in range(2):
+        hq = torch.empty(cap, dtype=torch.int32, device=dev)
+        hw = torch.empty(cap, dtype=torch.int32, device=dev)
+        cnt = torch.empty(cap, dtype=torch.uint8, device=dev)
+        pos = torch.empty((cap, 11), dtype=torch.uint8, device=dev)
+        total = C.c_size_t(0)
+        with torch.cuda.device(dev):
+            rc = call(_ptr(q), Q, int(min_kmers), cap, _ptr(hq), _ptr(hw), _ptr(cnt), _ptr(pos), C.byref(total), _stream())
+        if rc == _lib.BDG_ERR_CAPACITY and attempt == 0:
+            cap = int(total.value)
+            continue
+        check(rc)
+        n = int(total.value)
+        if hint is not None:
+            hint[0] = max(1 << 16, n + n // 8)
+        return hq[:n], hw[:n], cnt[:n], pos[:n]
+
+
+def kmer_score(q: torch.Tensor, wl: torch.Tensor, min_kmers: int = 1, cap: int | None = None):
+    """ops.kmer_score on tensors: (hit_q int32, hit_w int32, cnt uint8, pos uint8[hits, 11]) for every (query, string) pair with
+    cnt >= min_kmers, order unspecified.  A one-off index: posting lists from 64 queries upwards, as bdg_kmer_score."""
+    _ready()
+    _check(wl, "wl", BARCODE_DTYPES)
+    _int32_sized(wl, "wl")
+    L, w = lib(), wl
+    return _kmer_query(lambda *a: L.bdg_dev_kmer_score(a[0], a[1], _ptr(w), w.numel(), *a[2:]), q, wl.numel(), min_kmers, cap)
+
+
+class KmerIndex(ops.KmerIndex):
+    """ops.KmerIndex built from a tensor of known strings on the first device: query(q, min_kmers, cap) takes and returns tensors
+    (see kmer_score); info() / free() as there.  The index stays on the device it was built on, which must still be the first
+    device given to badger_b200.init when it is queried."""
+
+    def __init__(self, known: torch.Tensor):
+        _ready()
+        _check(known, "known", BARCODE_DTYPES)
+        _int32_sized(known, "known")
+        self.size = int(known.numel())
+        self._h = C.c_void_p()
+        with torch.cuda.device(known.device):
+            check(lib().bdg_dev_kmer_index_create(_ptr(known), self.size, _stream(), C.byref(self._h)))
+        self._room = [0]
+
+    def query(self, q: torch.Tensor, min_kmers: int = 1, cap: int | None = None):
+        if self._h is None:
+            raise ValueError("the index was freed")
+        L = lib()
+        return _kmer_query(lambda *a: L.bdg_dev_kmer_index_query(self._h, *a), q, self.size, min_kmers, cap, self._room)

@@ -289,6 +289,23 @@ int bdg_dev_cluster_resolve(int32_t* d_centre_idx, uint8_t* d_level, int32_t* d_
 int bdg_dev_nearest_bounded(const uint32_t* d_q, size_t Q, const uint32_t* d_targets, size_t W, int max_d,
                             uint32_t* d_keys /* Q words of scratch */, int32_t* d_argmin, uint8_t* d_dist,
                             void* stream);
+
+/* ---- the whitelist operators (a-5, a-6) with the strings and the results in caller device memory --------------------------
+ * Pointers on the first claimed device (else BDG_ERR_ARG); the work runs on the library's stream of that device, ordered as the
+ * correction-step device forms above.  bdg_dev_member_sorted and bdg_dev_nearest_bounded run on `stream` itself.
+ *   whitelist_check  the sortedness check of bdg_member_sorted (BDG_ERR_ARG "whitelist not sorted at index i"); waits for 8 bytes
+ *   kmer_index_create  bdg_kmer_index_create from W strings on the device (same posting-list rule, BDG_KMER_POST_MIN_W)
+ *   kmer_index_query   bdg_kmer_index_query into device buffers of cap hits: d_hit_q, d_hit_w, d_cnt as there, d_pos as
+ *                      uint8[cap][11] (the position counts of query positions 0..10, unpacked).  The index must live on the first
+ *                      claimed device.  Waits once, for *total; when *total > cap: BDG_ERR_CAPACITY, d_pos untouched and nothing
+ *                      beyond cap entries written.
+ *   kmer_score         bdg_kmer_score on the device: a one-off index (posting lists from 64 queries upwards) and one query. */
+int bdg_dev_whitelist_check(const uint32_t* d_sorted_wl, size_t W, void* stream);
+int bdg_dev_kmer_index_create(const uint32_t* d_known, size_t W, void* stream, bdg_kmer_index** out);
+int bdg_dev_kmer_index_query(bdg_kmer_index* ix, const uint32_t* d_q, size_t Q, int min_kmers, size_t cap, uint32_t* d_hit_q,
+                             uint32_t* d_hit_w, uint8_t* d_cnt, uint8_t* d_pos, size_t* total, void* stream);
+int bdg_dev_kmer_score(const uint32_t* d_q, size_t Q, const uint32_t* d_wl, size_t W, int min_kmers, size_t cap, uint32_t* d_hit_q,
+                       uint32_t* d_hit_w, uint8_t* d_cnt, uint8_t* d_pos, size_t* total, void* stream);
 /* Number of pairs the edge kernel decides for this part: sum over owned rows i of (N-1-i). */
 unsigned long long bdg_part_pairs(size_t N, int part, int nparts);
 /* Kernel launches issued by this process so far (bench.py's gpu_launches). */
