@@ -1019,6 +1019,25 @@ int bdg_dev_edges_stats_raw(unsigned long long* out8, void* stream)
     return BDG_OK;
 }
 
+// Development aid (tools/join_lane_stats.py): the lane-use counters of the join kernel (bdg_join.cuh g_join_lane), only in a build
+// with -DBDG_JOIN_LANE_STATS; summed over every join launch on the current device since the last reset.
+int bdg_join_lane_stats(unsigned long long* out8, int reset)
+{
+    if (!out8) return fail(BDG_ERR_ARG, "NULL pointer argument");
+#ifdef BDG_JOIN_LANE_STATS
+    CU_TRY(cudaDeviceSynchronize());
+    CU_TRY(cudaMemcpyFromSymbol(out8, bdg::g_join_lane, 8 * sizeof(unsigned long long)));
+    if (reset) {
+        const unsigned long long zero[8] = {};
+        CU_TRY(cudaMemcpyToSymbol(bdg::g_join_lane, zero, sizeof(zero)));
+    }
+    return BDG_OK;
+#else
+    (void)reset;
+    return fail(BDG_ERR_UNSUPPORTED, "built without the join lane counters (make EXTRA=-DBDG_JOIN_LANE_STATS)");
+#endif
+}
+
 // Development aid (tools/sweep_edges.py): per pass, sum and max over warps of the warp's exit time in ns
 // measured from the first warp's start - the load-balance picture of the last edge launch.
 int bdg_dev_edges_balance(unsigned long long* out /* 2 * MAX_PASSES */, void* stream)

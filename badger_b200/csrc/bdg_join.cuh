@@ -18,7 +18,8 @@
 // RS = 32 when the key buckets are long, RS = 8 when they are short (fewer rows span fewer foreign buckets).
 // What differs between the thresholds T is the per-pair stage:
 //   T = 2  quick test on the diagonals -1..1 (quick_marks), two marks dropped; exact stage join_process: dist_small, the
-//          hand-over table over seed_flags, then the 6-mer score in two queues (the middle diagonals, then the other eighteen).
+//          hand-over table over seed_flags on full batches of close pairs, then the 6-mer score in two queues (the middle
+//          diagonals, then the other eighteen).
 //   T = 3  quick test on the diagonals -2..2 (quick3_marks; the +-2 words are derived from the staged +-1 ones), three marks
 //          dropped; exact stage join3_process: dist3_min (Myers' bit-vector pass; D <= 3 has no case analysis), the hand-over
 //          walk seed3_first, then the 6-mer score through one queue.  The t = 3 scheme is too large for constant memory next to
@@ -39,13 +40,27 @@ constexpr int JCH = 128;           // columns staged at a time
 constexpr int JPAD = 32;           // slack behind the staged columns (steps may start up to one step early)
 constexpr int JUNIT = 2048;        // columns per work unit
 constexpr int JBATCH = 4;          // units per cursor fetch
-constexpr int JQCAP = 120;         // candidate queue entries per warp (with the other arrays: 6 CTAs of 8 warps per SM at t = 2)
-constexpr int JQ2CAP = 64;         // entries of each scoring queue (two at t = 2, one at t = 3)
+constexpr int JQCAP = 120;         // candidate queue entries per warp (with the other arrays: 5 CTAs of 8 warps per SM at t = 2)
+constexpr int JQ2CAP = 64;         // entries of each exact-stage queue (t = 2: close pairs and two scoring queues; t = 3: one scoring queue)
 constexpr int JROWS = 32;          // rows per slab
 // edge-count snapshots of the streaming form: one after every condition at t = 2, one after every block set at t = 3
 constexpr int JOIN_MAX_SNAPS = SEED_MAX_CONDS > SEED3_MAX_SETS ? SEED_MAX_CONDS : SEED3_MAX_SETS;
 
 __constant__ SeedScheme c_scheme;
+
+#ifdef BDG_JOIN_LANE_STATS
+// Development build (make EXTRA=-DBDG_JOIN_LANE_STATS; read with bdg_join_lane_stats): how full the warps of the candidate push and
+// of the exact stages run.  [0] push rounds, [1] hits pushed, [2] candidate batches through dist_small, [3] their candidates,
+// [4] of those batches, the ones with a pair at D <= 2, [5] batches through the hand-over check, [6] their pairs.
+__device__ unsigned long long g_join_lane[8];
+#define BDG_LANE_ADD(k, v)                                                                                           \
+    do {                                                                                                             \
+        const unsigned long long v_ = (unsigned long long)(v);                                                      \
+        if ((threadIdx.x & 31) == 0) atomicAdd(&g_join_lane[k], v_);                                                 \
+    } while (0)
+#else
+#define BDG_LANE_ADD(k, v) do { } while (0)
+#endif
 
 struct JoinArgs {
     const uint32_t* rows;          // barcodes in the order of the row-side key of the condition
@@ -230,58 +245,92 @@ struct JoinCtx {
     const Seed3Scheme* scheme;     // t = 3: hand-over tables
 };
 
-// t = 2 exact stage on a batch of candidates of one condition (one per lane): D by case analysis, hand-over table, survivors into
-// the scoring queue, full batches of that queue through the 6-mer score.  A real call, not inlined: one copy of the exact distance
-// and of the score loop keeps the kernel's hot code inside the instruction cache (ncu: the fully inlined form spent most of its
-// issue slots waiting for instructions).  Everything travels in registers: returns the two queue fills (8 bits each) | pairs
-// with D <= 2 << 16 | pairs handed to the score << 24.
+// t = 2 exact stage: three stages chained by per-warp queues in q2 / q2d, each run on full batches of 32 only (except the flush):
+//   candidates (one per lane) -> dist_small -> pairs with D <= 2 into the close-pair queue;
+//   32 close pairs -> seed_flags + hand-over table -> pairs this pass owns into the scoring queue;
+//   32 owned pairs -> 6-mer score of the middle diagonals; the undecided wait for the other eighteen in a second scoring queue.
+// Only about a quarter of the candidates are close: behind its own queue the hand-over check runs on full warps instead of on
+// every candidate batch that holds one close pair (nearly all of them).
+// Every queue holds fewer than 32 entries when a stage starts and a stage adds at most 32, so JQ2CAP = 64 entries never overflow.
+// A real call, not inlined: one copy of the exact distance and of the score loop keeps the kernel's hot code inside the instruction
+// cache (ncu: the fully inlined form spent most of its issue slots waiting for instructions).  Everything travels in registers:
+// q2n packs the three fills (JFILL_BITS each, see below); returns the new fills | pairs with D <= 2 << 16 | pairs handed to the
+// score << 24.
 // want0 / want1: the hand-over index this pass owns for a candidate with row value < / > column value (the same for a symmetric
-// condition, whose buckets are in no particular order).
+// condition, whose buckets are in no particular order).  flush: run the hand-over check on a partial batch of close pairs (the end
+// of a launch; no candidates then).
+constexpr int JFILL_BITS = 5;      // a queue fill between calls is < 32
+constexpr int JQ_NEAR = 0, JQ_FAR = JQ2CAP, JQ_CLOSE = 2 * JQ2CAP;   // t = 2: the three queues of q2 / q2d
+
+__device__ __forceinline__ int jfill(int q2n, int k) { return (q2n >> (k * JFILL_BITS)) & ((1 << JFILL_BITS) - 1); }
+
 __device__ __noinline__ uint32_t join_process(uint2* q2, uint8_t* q2d, const uint8_t* lut, int want0, int want1, int T, const EdgeOut out, uint2 e, bool active,
-                                              int q2n)
+                                              int q2n, bool flush)
 {
-    // q2 holds two queues: entries [0, 64) pairs that still need their score, entries [64, 128) pairs whose three middle
-    // diagonals did not reach the threshold and need the other eighteen; q2n = fill of the first | fill of the second << 8
+    // q2 holds three queues: entries [JQ_NEAR, +64) owned pairs that still need their score, [JQ_FAR, +64) pairs whose three middle
+    // diagonals did not reach the threshold and need the other eighteen, [JQ_CLOSE, +64) pairs with D <= 2 before the hand-over check
     const int lane = threadIdx.x & 31;
-    int n1 = q2n & 255, n2 = q2n >> 8;
+    const unsigned lt = (1u << lane) - 1u;
+    int n1 = jfill(q2n, 0), n2 = jfill(q2n, 1), nc = jfill(q2n, 2);
     const uint32_t a = min(e.x, e.y), b = max(e.x, e.y);
     bool ok = active && a != b;
     int d = 3;
     if (ok) { d = dist_small(a, b, false, true); ok = d <= 2; }
-    const uint32_t n_d2 = (uint32_t)__popc(__ballot_sync(FULL, ok));
-    if (ok) ok = __ldg(&lut[seed_flags(c_scheme, a, b)]) == (uint8_t)(e.x > e.y ? want1 : want0);   // emitted by the first (condition, orientation) the pair meets
-    const unsigned m = __ballot_sync(FULL, ok);
-    if (m == 0) return (uint32_t)q2n | (n_d2 << 16);
-    if (ok) {                                            // fewer than 32 entries wait on entry, so 32 more always fit
-        const int slot = n1 + __popc(m & ((1u << lane) - 1u));
+    const unsigned mc = __ballot_sync(FULL, ok);
+    if (ok) {                                            // D (1 or 2) and the orientation: want0 / want1 depend on the original order
+        const int slot = JQ_CLOSE + nc + __popc(mc & lt);
         q2[slot] = make_uint2(a, b);
-        q2d[slot] = (uint8_t)d;
+        q2d[slot] = (uint8_t)(d | (e.x > e.y ? 4 : 0));
     }
-    n1 += __popc(m);
-    __syncwarp();
-    while (n1 >= 32) {                                   // full batches: score of the middle diagonals; what they decide is emitted
-        n1 -= 32;
-        const uint2 mv = q2[n1 + lane];
-        const uint8_t md = q2d[n1 + lane];
-        const int near = qgram_score_near(mv.x, mv.y);
-        emit_warp(near >= T, mv.x, mv.y, md, out);
-        const unsigned rest = __ballot_sync(FULL, near < T);
-        if (near < T) {
-            const int slot = JQ2CAP + n2 + __popc(rest & ((1u << lane) - 1u));
-            q2[slot] = mv;
-            q2d[slot] = (uint8_t)(md | (near << 2));     // distance (1 or 2) and the part of the score that is known
-        }
-        n2 += __popc(rest);
+    nc += __popc(mc);
+    if (!flush) { BDG_LANE_ADD(2, 1); BDG_LANE_ADD(3, __popc(__ballot_sync(FULL, active))); BDG_LANE_ADD(4, mc != 0); }
+    uint32_t n_own = 0;
+    if (nc >= 32 || (flush && nc > 0)) {                 // hand-over check on a full batch of close pairs
         __syncwarp();
-        if (n2 >= 32) {                                  // a full batch of the undecided: the other eighteen diagonals
-            n2 -= 32;
-            const uint2 fv = q2[JQ2CAP + n2 + lane];
-            const uint8_t fd = q2d[JQ2CAP + n2 + lane];
-            emit_warp((int)(fd >> 2) + qgram_score_far(fv.x, fv.y) >= T, fv.x, fv.y, fd & 3, out);
+        const int take = min(nc, 32);
+        nc -= take;
+        bool own = false;
+        uint2 v = make_uint2(0u, 0u);
+        uint8_t vd = 0;
+        if (lane < take) {
+            v = q2[JQ_CLOSE + nc + lane];
+            vd = q2d[JQ_CLOSE + nc + lane];
+            own = __ldg(&lut[seed_flags(c_scheme, v.x, v.y)]) == (uint8_t)((vd & 4) ? want1 : want0);   // emitted by the first (condition, orientation) the pair meets
+        }
+        const unsigned m = __ballot_sync(FULL, own);
+        n_own = (uint32_t)__popc(m);
+        BDG_LANE_ADD(5, 1); BDG_LANE_ADD(6, take);
+        if (own) {
+            const int slot = JQ_NEAR + n1 + __popc(m & lt);
+            q2[slot] = v;
+            q2d[slot] = (uint8_t)(vd & 3);
+        }
+        n1 += __popc(m);
+        __syncwarp();
+        if (n1 >= 32) {                                  // full batch: score of the middle diagonals; what they decide is emitted
+            n1 -= 32;
+            const uint2 mv = q2[JQ_NEAR + n1 + lane];
+            const uint8_t md = q2d[JQ_NEAR + n1 + lane];
+            const int near = qgram_score_near(mv.x, mv.y);
+            emit_warp(near >= T, mv.x, mv.y, md, out);
+            const unsigned rest = __ballot_sync(FULL, near < T);
+            if (near < T) {
+                const int slot = JQ_FAR + n2 + __popc(rest & lt);
+                q2[slot] = mv;
+                q2d[slot] = (uint8_t)(md | (near << 2));     // distance (1 or 2) and the part of the score that is known
+            }
+            n2 += __popc(rest);
             __syncwarp();
+            if (n2 >= 32) {                              // a full batch of the undecided: the other eighteen diagonals
+                n2 -= 32;
+                const uint2 fv = q2[JQ_FAR + n2 + lane];
+                const uint8_t fd = q2d[JQ_FAR + n2 + lane];
+                emit_warp((int)(fd >> 2) + qgram_score_far(fv.x, fv.y) >= T, fv.x, fv.y, fd & 3, out);
+                __syncwarp();
+            }
         }
     }
-    return (uint32_t)n1 | ((uint32_t)n2 << 8) | (n_d2 << 16) | ((uint32_t)__popc(m) << 24);
+    return (uint32_t)(n1 | (n2 << JFILL_BITS) | (nc << (2 * JFILL_BITS))) | ((uint32_t)__popc(mc) << 16) | (n_own << 24);
 }
 
 // t = 3 exact stage on a batch of candidates (one per lane): D, hand-over walk, survivors into the scoring queue, full batches of
@@ -329,12 +378,20 @@ __device__ __forceinline__ void join_drain(JoinCtx& c, const EdgeOut& out, int& 
         qn -= take;
         const uint2 e = c.lane < take ? c.q[qn + c.lane] : make_uint2(0u, 0u);
         uint32_t r;
-        if constexpr (T == 2) r = join_process(c.q2, c.q2d, c.lut, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n);
+        if constexpr (T == 2) r = join_process(c.q2, c.q2d, c.lut, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n, false);
         else r = join3_process(c.q2, c.q2d, c.scheme, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, e, c.lane < take, q2n);
         q2n = (int)(r & 0xFFFFu);
         c.n_near += (r >> 16) & 255u;
         c.n_owned += r >> 24;
         __syncwarp();
+    }
+    if constexpr (T == 2) {
+        if (all) {                                       // the close pairs still waiting: a partial batch through the hand-over check
+            const uint32_t r = join_process(c.q2, c.q2d, c.lut, 2 * c.cond, 2 * c.cond + c.shifted, c.T, out, make_uint2(0u, 0u), false, q2n, true);
+            q2n = (int)(r & 0xFFFFu);
+            c.n_owned += r >> 24;
+            __syncwarp();
+        }
     }
 }
 
@@ -351,6 +408,7 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
     }
     const int total = __shfl_sync(FULL, incl, 31);
     if (qn + total <= JQCAP) {
+        BDG_LANE_ADD(0, __reduce_max_sync(FULL, (unsigned)cnt)); BDG_LANE_ADD(1, total);
         int slot = qn + incl - cnt;
         while (h) {
             const int j = __ffs(h) - 1;
@@ -365,6 +423,7 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
         const bool has = h != 0;
         const unsigned m = __ballot_sync(FULL, has);
         if (m == 0) break;
+        BDG_LANE_ADD(0, 1); BDG_LANE_ADD(1, __popc(m));
         if (has) {
             const int j = __ffs(h) - 1;
             h &= h - 1;
@@ -375,16 +434,17 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
     }
 }
 
-// T = 2 is compiled for 6 resident CTAs per SM (40 registers), T = 3 for 4: its exact stage needs the registers
+// T = 2 is compiled for 5 resident CTAs per SM (48 registers; its three exact-stage queues take 41 KB of shared memory per CTA),
+// T = 3 for 4: its exact stage needs the registers
 template <int T, int RS>
-__global__ void __launch_bounds__(ENT, T == 2 ? 6 : 4) join_kernel(const JoinArgsT<T> A, const EdgeOut out)
+__global__ void __launch_bounds__(ENT, T == 2 ? 5 : 4) join_kernel(const JoinArgsT<T> A, const EdgeOut out)
 {
     constexpr int PH = 32 / RS;                          // column phases of a warp
     constexpr int STEP = 4 * PH;                         // columns per inner step
     __shared__ __align__(16) uint32_t s_b[EW][4][JCH + JPAD];   // y, y >> 2, y << 2, key of the staged columns
     __shared__ uint2 s_q[EW][JQCAP];
-    __shared__ uint2 s_q2[EW][T == 2 ? 2 * JQ2CAP : JQ2CAP];   // pairs that need their score | (t = 2) pairs that need the far diagonals
-    __shared__ uint8_t s_q2d[EW][T == 2 ? 2 * JQ2CAP : JQ2CAP];
+    __shared__ uint2 s_q2[EW][T == 2 ? 3 * JQ2CAP : JQ2CAP];   // pairs that need their score | (t = 2) pairs that need the far diagonals | close pairs
+    __shared__ uint8_t s_q2d[EW][T == 2 ? 3 * JQ2CAP : JQ2CAP];
     const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
     const int r = lane & (RS - 1), ph = lane / RS;
     uint32_t* const sb0 = s_b[wid][0];
@@ -503,7 +563,7 @@ __global__ void __launch_bounds__(ENT, T == 2 ? 6 : 4) join_kernel(const JoinArg
     }
     join_drain<T>(c, out, qn, q2n, true);
     {                                                    // what is left in the scoring queues: fewer than 32 each
-        const int n1 = q2n & 255, n2 = q2n >> 8;
+        const int n1 = T == 2 ? jfill(q2n, 0) : q2n, n2 = T == 2 ? jfill(q2n, 1) : 0;
         bool ok = false;
         uint32_t a = 0, b = 0;
         int d = 0;
@@ -516,8 +576,8 @@ __global__ void __launch_bounds__(ENT, T == 2 ? 6 : 4) join_kernel(const JoinArg
         if constexpr (T == 2) {                          // the far diagonals of the undecided
             ok = false;
             if (lane < n2) {
-                const uint2 e = c.q2[JQ2CAP + lane];
-                const uint8_t fd = c.q2d[JQ2CAP + lane];
+                const uint2 e = c.q2[JQ_FAR + lane];
+                const uint8_t fd = c.q2d[JQ_FAR + lane];
                 a = e.x; b = e.y; d = fd & 3;
                 ok = (int)(fd >> 2) + qgram_score_far(a, b) >= A.T;
             }

@@ -35,7 +35,8 @@ enum {
     BDG_ERR_ARG = -3,      /* bad argument (NULL, unsorted input, size limit) */
     BDG_ERR_NODEVICE = -4, /* no CUDA device / library not initialised on one */
     BDG_ERR_CAPACITY = -5, /* caller-provided output capacity too small; *total holds the need */
-    BDG_ERR_UNSUPPORTED = -6, /* bdg_tsv_open: the file uses a construct the native reader refuses (take the pandas route) */
+    BDG_ERR_UNSUPPORTED = -6, /* bdg_tsv_open: the file uses a construct the native reader refuses (take the pandas route);
+                                 bdg_join_lane_stats: the build does not count */
     BDG_ERR_IO = -7        /* a file could not be opened, mapped or written */
 };
 
@@ -216,6 +217,11 @@ int bdg_dev_edges_stats(unsigned long long* out5, void* stream);
 int bdg_dev_edges_stats_raw(unsigned long long* out8, void* stream);
 /* Development aid: out[2p], out[2p+1] = sum and max over the warps of pass p of (warp exit - first warp start), ns. */
 int bdg_dev_edges_balance(unsigned long long* out6, void* stream);
+/* Development aid: lane use of the join kernel, summed over its launches on the current device since the last reset (reset != 0
+ * clears them after the read): out8[0] push rounds, [1] hits pushed, [2] candidate batches through the exact distance, [3] their
+ * candidates, [4] those batches with a pair at D <= t, [5] batches through the hand-over check, [6] their pairs.  Only in a build
+ * with -DBDG_JOIN_LANE_STATS; otherwise BDG_ERR_UNSUPPORTED.  Synchronises the device. */
+int bdg_join_lane_stats(unsigned long long* out8, int reset);
 int bdg_dev_pack16(const char* d_seqs, size_t R, uint32_t* d_out, uint8_t* d_valid, void* stream);
 int bdg_dev_member_sorted(const uint32_t* d_sorted_wl, size_t W, const uint32_t* d_q, size_t Q, uint8_t* d_hit,
                           void* stream);
