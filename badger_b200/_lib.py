@@ -99,6 +99,15 @@ def lib():
     L.bdg_dev_kmer_index_create.argtypes = [_vp, _sz, _vp, C.POINTER(_vp)]
     L.bdg_dev_kmer_index_query.argtypes = [_vp, _vp, _sz, _i, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz), _vp]
     L.bdg_dev_kmer_score.argtypes = [_vp, _sz, _vp, _sz, _i, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz), _vp]
+    L.bdg_tally_create.argtypes = [C.POINTER(_vp)]
+    L.bdg_tally_free.argtypes = [_vp]
+    L.bdg_tally_free.restype = None
+    L.bdg_tally_add.argtypes = [_vp, _vp, _vp, _sz, C.POINTER(_sz)]
+    L.bdg_dev_tally_add.argtypes = [_vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]
+    L.bdg_tally_finish.argtypes = [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong)]
+    L.bdg_dev_tally_finish.argtypes = [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong), _vp]
+    L.bdg_assign_lookup32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, _vp, _vp, C.POINTER(_sz), C.POINTER(_sz)]
+    L.bdg_dev_assign_lookup32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, _vp, _vp, C.POINTER(_sz), C.POINTER(_sz), _vp]
     L.bdg_part_pairs.argtypes = [_sz, _i, _i]
     L.bdg_part_pairs.restype = C.c_ulonglong
     L.bdg_dev_pipe_probe.argtypes = [_i, _i, _i, _vp, C.POINTER(C.c_ulonglong), _vp]
@@ -122,7 +131,8 @@ def lib():
                  "bdg_tsv_write_assignments32", "bdg_dev_dedup_reads", "bdg_dev_dedup_fetch", "bdg_dev_pack16_sorted", "bdg_dev_centres_above",
                  "bdg_dev_edges_copy", "bdg_dev_assign_reads32", "bdg_dev_dedup_merge", "bdg_dev_index_edges", "bdg_dev_cluster_init",
                  "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve", "bdg_dev_whitelist_check",
-                 "bdg_dev_kmer_index_create", "bdg_dev_kmer_index_query", "bdg_dev_kmer_score"):
+                 "bdg_dev_kmer_index_create", "bdg_dev_kmer_index_query", "bdg_dev_kmer_score", "bdg_tally_create", "bdg_tally_add",
+                 "bdg_dev_tally_add", "bdg_tally_finish", "bdg_dev_tally_finish", "bdg_assign_lookup32", "bdg_dev_assign_lookup32"):
         getattr(L, name).restype = _i
     _lib = L
     return L

@@ -94,6 +94,7 @@ struct DevCtx {
     Buf ce[9];                                                // centre selection: positions above the cutoff, sort keys / values, results, scratch
     Buf as[8];                                                // masked dedup + per-read gather: all ranks, valid bytes, their scan, scratch, centre idx / value, result, counter
     Buf mg[12];                                               // merge of the parts' dedup results (bdg_dev_dedup_merge), see there
+    Buf lk[5];                                                // per-read lookup (bdg_assign_lookup32): counters, and the host form's ranks, valid bytes, result, centre idx
     unsigned long long map_token = 0, map_serial = 0;         // read map left on the device by bdg_dedup_reads (0: none)
     size_t map_rows = 0, map_reads = 0, map_distinct = 0;
     bool map_masked = false;
@@ -926,6 +927,7 @@ void bdg_shutdown(void)
         for (auto& b : c.cl) b.release();
         c.gather_a.release(); c.gather_b.release(); c.top16.release();
         for (auto& b : c.as) b.release();
+        for (auto& b : c.lk) b.release();
         for (auto& b : c.ce) b.release();
         for (auto& b : c.rot_sorted) b.release();
         for (int k = 0; k < 2; k++) {
@@ -1440,6 +1442,202 @@ int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const 
     return dedup_merge_core(c, d_keys, d_counts, d_first, starts, sizes, n_parts, my_part, n_distinct, merged_token);
 }
 
+}  // extern "C"
+
+// ---- the tally: reads deduplicated batch by batch into a running distinct set (bdg_kernels.cuh, tally_*) -------------------
+// The set lives in the handle's own buffers, ascending by barcode, with a 64-bit count and a 64-bit first-sighting key per
+// barcode: the rows added before the batch + the barcode's first-seen position in the batch, so that the keys sort in the
+// first-seen order of the concatenated batches.  add merges a batch into the other half of the double buffer and swaps; a
+// refused batch leaves the set as it was.  finish sorts the set by first-sighting key and installs the read-map arrays of a
+// dedup call without rows (dd[0] counts, dd[1] first-seen -> ascending, dd[2] distinct, dd[6] ascending).
+struct bdg_tally {
+    int dev = -1;                                   // the first claimed device when the tally was created
+    Buf key[2], cnt[2], fst[2];                     // the running set and the half the next batch is merged into
+    Buf m_key, m_cnt, m_fst, m_head, m_scan;        // the merged order of set and batch, head flags and their scan; order at finish
+    Buf scratch, flag;                              // cub scratch; overflow flag + set size read back after a merge
+    int cur = 0;
+    size_t n = 0;                                   // distinct barcodes in the set
+    unsigned long long rows = 0, valid = 0;         // rows and valid rows added
+    bool over = false;                              // some barcode was counted 2^32 times or more
+    bool finished = false;
+};
+
+namespace {
+
+int tally_ready(bdg_tally* h, DevCtx** out)
+{
+    if (!h) return fail(BDG_ERR_ARG, "NULL tally handle");
+    if (g_ctx.empty() || g_ctx[0].dev != h->dev)
+        return fail(BDG_ERR_ARG, "the tally lives on device %d, which is not the first claimed device", h->dev);
+    *out = &g_ctx[0];
+    CU_TRY(cudaSetDevice(h->dev));
+    return BDG_OK;
+}
+
+int tally_add_core(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, cudaMemcpyKind kind, size_t* n_valid)
+{
+    if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
+    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    size_t nb = 0, nv = 0;
+    unsigned long long tok = 0;
+    const int rc = dedup_reads_core(c, ranks, valid, R, kind, nullptr, nullptr, nullptr, nullptr, &nb, &nv, &tok);
+    c.map_token = 0;                                // the batch's read map is not handed out
+    if (rc) return rc;
+    if (n_valid) *n_valid = nv;
+    if (nv == 0) { h->rows += R; return BDG_OK; }
+    cudaStream_t st = c.stream;
+    const int nx = h->cur ^ 1;
+    const size_t na = h->n, M = na + nb;            // na < 2^31 and nb < 2^31: M < 2^32
+    for (Buf* b : {&h->m_key, &h->m_head, &h->m_scan, &h->key[nx]}) if (int e = ensure_buf(*b, M * 4)) return e;
+    for (Buf* b : {&h->m_cnt, &h->m_fst, &h->cnt[nx], &h->fst[nx]}) if (int e = ensure_buf(*b, M * 8)) return e;
+    if (int e = ensure_buf(h->flag, 16)) return e;
+    size_t tmp = 0;
+    CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
+    if (int e = ensure_buf(h->scratch, tmp)) return e;
+    unsigned int* d_flag = (unsigned int*)h->flag.p;
+    CU_TRY(cudaMemsetAsync(d_flag, 0, 4, st));
+    bdg::tally_merge_kernel<<<(unsigned)((M + bdg::TALLY_TILE - 1) / bdg::TALLY_TILE), bdg::NT, 0, st>>>(
+        (const uint32_t*)h->key[h->cur].p, (const unsigned long long*)h->cnt[h->cur].p, (const unsigned long long*)h->fst[h->cur].p, na,
+        (const uint32_t*)c.dd[6].p /* batch runs ascending */, (const uint32_t*)c.dd[0].p /* counts, first-seen order */,
+        (const uint32_t*)c.dd[4].p /* run -> first-seen position */, nb, h->rows, (uint32_t*)h->m_key.p, (unsigned long long*)h->m_cnt.p,
+        (unsigned long long*)h->m_fst.p, (uint32_t*)h->m_head.p);
+    CU_TRY(cub::DeviceScan::InclusiveSum(h->scratch.p, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
+    const int blocks = (int)std::min<size_t>((M + 255) / 256, (size_t)c.sms * 8);
+    bdg::tally_compact_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)h->m_key.p, (const unsigned long long*)h->m_cnt.p,
+                                                      (const unsigned long long*)h->m_fst.p, (const uint32_t*)h->m_head.p,
+                                                      (const uint32_t*)h->m_scan.p, M, (uint32_t*)h->key[nx].p,
+                                                      (unsigned long long*)h->cnt[nx].p, (unsigned long long*)h->fst[nx].p, d_flag);
+    g_launches += 2;
+    CU_TRY(cudaGetLastError());
+    uint32_t n_out = 0, over = 0;
+    CU_TRY(cudaMemcpyAsync(&n_out, (const uint32_t*)h->m_scan.p + (M - 1), 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&over, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    if (n_out > 0x7FFFFFFFu)
+        return fail(BDG_ERR_ARG, "the batch would take the tally to %u distinct barcodes; fewer than 2^31 are allowed (the set keeps the batches before it)", n_out);
+    h->cur = nx;
+    h->n = n_out;
+    h->rows += R;
+    h->valid += nv;
+    h->over = h->over || over != 0;
+    return BDG_OK;
+}
+
+int tally_finish_core(DevCtx& c, bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+{
+    if (h->over) return fail(BDG_ERR_ARG, "a barcode was counted 2^32 times or more; the counts of a read map are uint32");
+    *n_valid = h->valid;
+    h->finished = true;
+    if (h->n == 0) return BDG_OK;                   // no valid row: no read map, as with a dedup call
+    cudaStream_t st = c.stream;
+    const uint32_t n = (uint32_t)h->n;
+    int end_bit = 1;                                // every first-sighting key is below the number of rows added
+    while (end_bit < 64 && (h->rows >> end_bit)) end_bit++;
+    // m_key := iota, m_fst := sorted keys, m_head := order (all hold >= n entries since the merge that made the set)
+    size_t tmp = 0;
+    CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp, (const unsigned long long*)h->fst[h->cur].p, (unsigned long long*)h->m_fst.p,
+                                           (const uint32_t*)h->m_key.p, (uint32_t*)h->m_head.p, (int)n, 0, end_bit, st));
+    if (int e = ensure_buf(h->scratch, tmp)) return e;
+    const int blocks = (int)std::min<size_t>((n + 255) / 256, (size_t)c.sms * 8);
+    bdg::iota_kernel<<<blocks, 256, 0, st>>>((uint32_t*)h->m_key.p, n);
+    CU_TRY(cub::DeviceRadixSort::SortPairs(h->scratch.p, tmp, (const unsigned long long*)h->fst[h->cur].p, (unsigned long long*)h->m_fst.p,
+                                           (const uint32_t*)h->m_key.p, (uint32_t*)h->m_head.p, (int)n, 0, end_bit, st));
+    // the read map of the token named last is about to be overwritten
+    c.map_token = 0;
+    c.cl_token = 0;
+    // growing a dd[] buffer frees its old memory: whatever is queued on the stream may still read it
+    CU_TRY(cudaStreamSynchronize(st));
+    for (int k : {0, 1, 2, 6}) if (int e = ensure_buf(c.dd[k], (size_t)n * 4)) return e;
+    bdg::tally_finish_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)h->m_head.p, (const uint32_t*)h->key[h->cur].p,
+                                                     (const unsigned long long*)h->cnt[h->cur].p, n, (uint32_t*)c.dd[2].p,
+                                                     (uint32_t*)c.dd[0].p, (uint32_t*)c.dd[1].p);
+    g_launches += 2;
+    CU_TRY(cudaGetLastError());
+    CU_TRY(cudaMemcpyAsync(c.dd[6].p, h->key[h->cur].p, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
+    c.map_rows = 0; c.map_reads = 0; c.map_masked = false;
+    c.map_distinct = n;
+    c.map_token = ++c.map_serial;
+    *n_distinct = n;
+    *token = c.map_token;
+    return BDG_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int bdg_tally_create(bdg_tally** out)
+{
+    if (!out) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    *out = nullptr;
+    if (int rc = need_ctx()) return rc;
+    bdg_tally* h = new (std::nothrow) bdg_tally();
+    if (!h) return fail(BDG_ERR_OOM, "host allocation failed");
+    h->dev = g_ctx[0].dev;
+    *out = h;
+    return BDG_OK;
+}
+
+void bdg_tally_free(bdg_tally* h)
+{
+    if (!h) return;
+    int prev = -1;
+    cudaGetDevice(&prev);
+    if (cudaSetDevice(h->dev) == cudaSuccess) {
+        for (int k = 0; k < 2; k++) { h->key[k].release(); h->cnt[k].release(); h->fst[k].release(); }
+        for (Buf* b : {&h->m_key, &h->m_cnt, &h->m_fst, &h->m_head, &h->m_scan, &h->scratch, &h->flag}) b->release();
+    }
+    if (prev >= 0) cudaSetDevice(prev);
+    delete h;
+}
+
+int bdg_tally_add(bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, size_t* n_valid)
+{
+    if (n_valid) *n_valid = 0;
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
+    if (R == 0) return BDG_OK;
+    if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    return tally_add_core(*c, h, ranks, valid, R, cudaMemcpyHostToDevice, n_valid);
+}
+
+int bdg_dev_tally_add(bdg_tally* h, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R, size_t* n_valid, void* stream)
+{
+    if (n_valid) *n_valid = 0;
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
+    if (R == 0) return BDG_OK;
+    if (!d_ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    if (int rc = check_on_first(d_ranks, "ranks")) return rc;
+    if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
+    CallerOrder order(*c, stream);
+    if (int rc = order.begin()) return rc;
+    return tally_add_core(*c, h, d_ranks, d_valid, R, cudaMemcpyDeviceToDevice, n_valid);
+}
+
+int bdg_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+{
+    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *n_valid = 0; *token = 0;
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    return tally_finish_core(*c, h, n_distinct, n_valid, token);
+}
+
+int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, void* stream)
+{
+    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *n_valid = 0; *token = 0;
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    CallerOrder order(*c, stream);
+    if (int rc = order.begin()) return rc;
+    return tally_finish_core(*c, h, n_distinct, n_valid, token);
+}
+
 // ---- a-6 / centre selection, barcode_graph.py:252-267, over the distinct barcodes a dedup call left on the device ----
 // cutoff = max(mean(counts of the first n_cells barcodes in first-seen order) / 5, 5) (:255-256); the barcodes with
 // count > cutoff in count-descending order, ties in first-seen order (the head of `bc_by_counts`, :253), with their counts and
@@ -1702,6 +1900,98 @@ int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx
         CU_TRY(cudaStreamSynchronize(c.stream));
         *n_assigned = (size_t)cnt;
     }
+    return BDG_OK;
+}
+
+// The per-read gather for rows outside any read map: every valid row's barcode is looked up among the token's nodes (the
+// ascending array dd[6]); d_ci as for assign_reads32_core.  Counters (assigned, missing) go to lk[0].
+static int assign_lookup32_core(DevCtx& c, const int32_t* d_ci, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R,
+                                uint32_t* d_out, uint8_t* d_oh)
+{
+    cudaStream_t st = c.stream;
+    if (int e = ensure_buf(c.lk[0], 16)) return e;
+    if (!d_ci) d_ci = (const int32_t*)c.cl[1].p;
+    CU_TRY(cudaMemsetAsync(c.lk[0].p, 0, 16, st));
+    const int rb = (int)std::min<size_t>((R + bdg::NT - 1) / bdg::NT, (size_t)c.sms * 8);
+    bdg::lookup_assign32_kernel<<<rb, bdg::NT, 0, st>>>((const uint32_t*)c.dd[6].p, (uint32_t)N, d_ci, d_ranks, d_valid, R, d_out, d_oh,
+                                                         (unsigned long long*)c.lk[0].p);
+    g_launches++;
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+static int check_lookup_args(DevCtx& c, unsigned long long token, bool resident, size_t N)
+{
+    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    if (N != c.map_distinct) return fail(BDG_ERR_ARG, "N does not match the read map the token names");
+    if (resident && c.cl_token != token) return fail(BDG_ERR_ARG, "no clustering result of this read map is resident on the device (bdg_cluster_resident)");
+    return BDG_OK;
+}
+
+static int read_lookup_counters(DevCtx& c, size_t* n_assigned, size_t* n_missing)
+{
+    unsigned long long cnt[2] = {0, 0};
+    CU_TRY(cudaMemcpyAsync(cnt, c.lk[0].p, 16, cudaMemcpyDeviceToHost, c.stream));
+    CU_TRY(cudaStreamSynchronize(c.stream));
+    if (n_assigned) *n_assigned = (size_t)cnt[0];
+    if (n_missing) *n_missing = (size_t)cnt[1];
+    return BDG_OK;
+}
+
+int bdg_assign_lookup32(unsigned long long token, const int32_t* centre_idx, size_t N, const uint32_t* ranks, const uint8_t* valid, size_t R,
+                        uint32_t* centre, uint8_t* has_centre, size_t* n_assigned, size_t* n_missing)
+{
+    if (n_assigned) *n_assigned = 0;
+    if (n_missing) *n_missing = 0;
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (int rc = check_lookup_args(c, token, !centre_idx, N)) return rc;
+    if (R == 0) return BDG_OK;
+    if (!ranks || !centre || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    CU_TRY(cudaSetDevice(c.dev));
+    cudaStream_t st = c.stream;
+    // lk[1] ranks, lk[2] valid bytes, lk[3] result (R x 5 bytes), lk[4] centre index per node
+    if (int e = ensure_buf(c.lk[1], R * 4)) return e;
+    if (int e = ensure_buf(c.lk[3], R * 5)) return e;
+    CU_TRY(cudaMemcpyAsync(c.lk[1].p, ranks, R * 4, cudaMemcpyHostToDevice, st));
+    if (valid) {
+        if (int e = ensure_buf(c.lk[2], R)) return e;
+        CU_TRY(cudaMemcpyAsync(c.lk[2].p, valid, R, cudaMemcpyHostToDevice, st));
+    }
+    const int32_t* d_ci = nullptr;
+    if (centre_idx) {
+        if (int e = ensure_buf(c.lk[4], N * 4)) return e;
+        CU_TRY(cudaMemcpyAsync(c.lk[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+        d_ci = (const int32_t*)c.lk[4].p;
+    }
+    uint32_t* d_out = (uint32_t*)c.lk[3].p;
+    uint8_t* d_oh = (uint8_t*)c.lk[3].p + R * 4;
+    if (int rc = assign_lookup32_core(c, d_ci, N, (const uint32_t*)c.lk[1].p, valid ? (const uint8_t*)c.lk[2].p : nullptr, R, d_out, d_oh)) return rc;
+    CU_TRY(cudaMemcpyAsync(centre, d_out, R * 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(has_centre, d_oh, R, cudaMemcpyDeviceToHost, st));
+    return read_lookup_counters(c, n_assigned, n_missing);
+}
+
+int bdg_dev_assign_lookup32(unsigned long long token, const int32_t* d_centre_idx, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid,
+                            size_t R, uint32_t* d_centre, uint8_t* d_has_centre, size_t* n_assigned, size_t* n_missing, void* stream)
+{
+    if (n_assigned) *n_assigned = 0;
+    if (n_missing) *n_missing = 0;
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (int rc = check_lookup_args(c, token, !d_centre_idx, N)) return rc;
+    if (R == 0) return BDG_OK;
+    if (!d_ranks || !d_centre || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    CU_TRY(cudaSetDevice(c.dev));
+    if (d_centre_idx) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
+    if (int rc = check_on_first(d_ranks, "ranks")) return rc;
+    if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
+    if (int rc = check_on_first(d_centre, "centre")) return rc;
+    if (int rc = check_on_first(d_has_centre, "has_centre")) return rc;
+    CallerOrder order(c, stream);
+    if (int rc = order.begin()) return rc;
+    if (int rc = assign_lookup32_core(c, d_centre_idx, N, d_ranks, d_valid, R, d_centre, d_has_centre)) return rc;
+    if (n_assigned || n_missing) return read_lookup_counters(c, n_assigned, n_missing);
     return BDG_OK;
 }
 

@@ -7,6 +7,8 @@
 //   kmer_unpack_kernel   packed position counts -> uint8[hits][11] (device form of a-5)        HBM bound
 //   member_kernel        sorted-whitelist membership (smem pivots + L2-resident search)       HBM/L2 bound
 //   pack16_kernel        16 ASCII bases -> 2-bit packed uint32 + validity                     HBM bound
+//   tally_merge_kernel   merge path of the running distinct set and a batch's distinct list   HBM bound
+//   lookup_assign32_kernel  per-read centre for rows outside a read map (smem pivots + search)  L2/HBM bound
 //   pipe_probe_kernel    LOP3 / IMAD / POPC issue-rate probe for the integer roofline
 //
 // No tensor cores on purpose: nothing here is a dense contraction (BASELINE.json north_star).
@@ -471,6 +473,178 @@ __global__ void merge_remap_kernel(uint32_t* __restrict__ read_to_distinct, uint
 {
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x)
         read_to_distinct[i] = __ldg(&global_pos[read_to_distinct[i]]);
+}
+
+// ---------------------------------------------------------------------------------------------------
+// Tally of reads that arrive in batches (bdg_tally_*): the running distinct set is ascending by barcode with a 64-bit count and a
+// 64-bit first-sighting key per barcode; every batch is deduplicated as above and its ascending list is merged into the set.
+//   tally_merge_kernel   merge path of the set A (na) and the batch B (nb): CTA k owns outputs [k*TALLY_TILE, (k+1)*TALLY_TILE),
+//                        finds where that stretch of the merged order starts and ends in A and B (two binary searches along the
+//                        cross diagonals), stages both key ranges in shared memory, and every thread merges TALLY_ITEMS outputs
+//                        from its own diagonal.  Ties take A first, so a barcode the set already holds is followed directly by
+//                        the batch's entry of it, which is flagged as no head.  The batch's entry of run r: key b_key[r], count
+//                        b_count[b_pos[r]], first-sighting key first_off + b_pos[r] (its first-seen position in the batch).
+//   (inclusive scan of the heads: the position of every run in the new set)
+//   tally_compact_kernel one entry per head, the count of a following non-head added in; counts of 2^32 or more are flagged
+//   (radix sort of the set by first-sighting key at tally_finish: the global first-seen order)
+//   tally_finish_kernel  distinct / counts (uint32) / first-seen -> ascending position, the read-map arrays of a dedup call
+// HBM bound: 20 B in and 24 B out per merged entry, then 24 B in and 20 B out per entry of the new set.
+// ---------------------------------------------------------------------------------------------------
+constexpr int TALLY_ITEMS = 8;
+constexpr int TALLY_TILE = NT * TALLY_ITEMS;
+
+// number of A entries among the first d outputs of the merge (ties: A first)
+template <typename GetA, typename GetB>
+__device__ __forceinline__ uint64_t merge_path_split(uint64_t d, uint64_t na, uint64_t nb, GetA a, GetB b)
+{
+    uint64_t lo = d > nb ? d - nb : 0, hi = d < na ? d : na;
+    while (lo < hi) {
+        const uint64_t mid = (lo + hi) >> 1;
+        if (a(mid) <= b(d - 1 - mid)) lo = mid + 1; else hi = mid;
+    }
+    return lo;
+}
+
+__global__ void __launch_bounds__(NT) tally_merge_kernel(const uint32_t* __restrict__ a_key, const unsigned long long* __restrict__ a_cnt,
+                                                         const unsigned long long* __restrict__ a_first, uint64_t na,
+                                                         const uint32_t* __restrict__ b_key, const uint32_t* __restrict__ b_count,
+                                                         const uint32_t* __restrict__ b_pos, uint64_t nb, unsigned long long first_off,
+                                                         uint32_t* __restrict__ m_key, unsigned long long* __restrict__ m_cnt,
+                                                         unsigned long long* __restrict__ m_first, uint32_t* __restrict__ m_head)
+{
+    __shared__ uint32_t s_key[TALLY_TILE];
+    __shared__ uint64_t s_split[2];
+    const uint64_t M = na + nb;
+    const uint64_t d0 = (uint64_t)blockIdx.x * TALLY_TILE, d1 = min(M, d0 + TALLY_TILE);
+    auto ga = [&](uint64_t i) { return __ldg(&a_key[i]); };
+    auto gb = [&](uint64_t j) { return __ldg(&b_key[j]); };
+    if (threadIdx.x < 2) s_split[threadIdx.x] = merge_path_split(threadIdx.x ? d1 : d0, na, nb, ga, gb);
+    __syncthreads();
+    const uint64_t a0 = s_split[0], a1 = s_split[1], b0 = d0 - a0, b1 = d1 - a1;
+    const uint32_t la = (uint32_t)(a1 - a0), lb = (uint32_t)(b1 - b0);     // la + lb = d1 - d0 <= TALLY_TILE
+    for (uint32_t k = threadIdx.x; k < la + lb; k += NT) s_key[k] = k < la ? ga(a0 + k) : gb(b0 + k - la);
+    __syncthreads();
+    const uint32_t* sa = s_key;
+    const uint32_t* sb = s_key + la;
+    const uint32_t dt = min((uint32_t)threadIdx.x * TALLY_ITEMS, la + lb);
+    uint32_t i = (uint32_t)merge_path_split(dt, la, lb, [&](uint64_t x) { return sa[x]; }, [&](uint64_t y) { return sb[y]; });
+    uint32_t j = dt - i;
+    // the A entry right before this thread's first output (the one a batch entry of the same barcode follows)
+    const bool have_prev = a0 + i > 0;
+    uint32_t prev_a = have_prev ? (i > 0 ? sa[i - 1] : ga(a0 - 1)) : 0u;
+    const uint32_t end = min(dt + TALLY_ITEMS, la + lb);
+    bool any_a = have_prev;
+    for (uint32_t o = dt; o < end; o++) {
+        const uint64_t g = d0 + o;
+        if (j >= lb || (i < la && sa[i] <= sb[j])) {
+            const uint64_t ai = a0 + i;
+            m_key[g] = sa[i];
+            m_cnt[g] = __ldg(&a_cnt[ai]);
+            m_first[g] = __ldg(&a_first[ai]);
+            m_head[g] = 1u;
+            prev_a = sa[i];
+            any_a = true;
+            i++;
+        } else {
+            const uint64_t bj = b0 + j;
+            const uint32_t k = sb[j], p = __ldg(&b_pos[bj]);
+            m_key[g] = k;
+            m_cnt[g] = __ldg(&b_count[p]);
+            m_first[g] = first_off + p;
+            m_head[g] = (any_a && prev_a == k) ? 0u : 1u;
+            j++;
+        }
+    }
+}
+
+// scan_incl[o] - 1 = position of head o in the new set; a non-head is always the entry right after its head
+__global__ void tally_compact_kernel(const uint32_t* __restrict__ m_key, const unsigned long long* __restrict__ m_cnt,
+                                     const unsigned long long* __restrict__ m_first, const uint32_t* __restrict__ m_head,
+                                     const uint32_t* __restrict__ scan_incl, uint64_t M, uint32_t* __restrict__ key,
+                                     unsigned long long* __restrict__ cnt, unsigned long long* __restrict__ first, unsigned int* __restrict__ over)
+{
+    for (uint64_t o = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; o < M; o += (uint64_t)gridDim.x * blockDim.x) {
+        if (!__ldg(&m_head[o])) continue;
+        const uint32_t r = __ldg(&scan_incl[o]) - 1u;
+        unsigned long long c = __ldg(&m_cnt[o]), f = __ldg(&m_first[o]);
+        if (o + 1 < M && !__ldg(&m_head[o + 1])) {
+            c += __ldg(&m_cnt[o + 1]);
+            f = min(f, __ldg(&m_first[o + 1]));
+        }
+        key[r] = __ldg(&m_key[o]);
+        cnt[r] = c;
+        first[r] = f;
+        if (c >> 32) *over = 1u;
+    }
+}
+
+// order[p] = ascending position of the barcode with the p-th smallest first-sighting key
+__global__ void tally_finish_kernel(const uint32_t* __restrict__ order, const uint32_t* __restrict__ key, const unsigned long long* __restrict__ cnt,
+                                    uint32_t n, uint32_t* __restrict__ distinct, uint32_t* __restrict__ counts, uint32_t* __restrict__ sorted_pos)
+{
+    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
+        const uint32_t r = __ldg(&order[p]);
+        distinct[p] = __ldg(&key[r]);
+        counts[p] = (uint32_t)__ldg(&cnt[r]);
+        sorted_pos[p] = r;
+    }
+}
+
+// ---------------------------------------------------------------------------------------------------
+// lookup_assign32_kernel: the per-read gather for rows outside any read map (bdg_assign_lookup32).  Every valid row's barcode is
+// searched in the ascending node array (MEM_PIV pivots in shared memory, then the window between two pivots, as member_kernel);
+// its node's centre index gives the centre node and that node's barcode.  A valid row whose barcode is no node counts as missing.
+// 4 + 1 B in and 5 B out per row, plus the search (L2-resident for the node arrays of a correction step).
+// ---------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(NT) lookup_assign32_kernel(const uint32_t* __restrict__ sorted, uint32_t N, const int32_t* __restrict__ centre_idx,
+                                                             const uint32_t* __restrict__ ranks, const uint8_t* __restrict__ valid, uint64_t R,
+                                                             uint32_t* __restrict__ out, uint8_t* __restrict__ out_has,
+                                                             unsigned long long* __restrict__ counters /* [0] assigned, [1] missing */)
+{
+    __shared__ uint32_t s_p[MEM_PIV];
+    const uint64_t step = ((uint64_t)N + MEM_PIV - 1) / MEM_PIV;
+    for (int p = threadIdx.x; p < MEM_PIV; p += NT) {
+        const uint64_t i = (uint64_t)p * step;
+        s_p[p] = __ldg(&sorted[i < N ? i : N - 1]);
+    }
+    __syncthreads();
+    unsigned long long assigned = 0, missing = 0;
+    for (uint64_t i = (uint64_t)blockIdx.x * NT + threadIdx.x; i < R; i += (uint64_t)gridDim.x * NT) {
+        uint32_t v = 0;
+        uint8_t h = 0;
+        if (!valid || __ldg(&valid[i])) {
+            const uint32_t q = __ldg(&ranks[i]);
+            int lo = 0, hi = MEM_PIV;
+#pragma unroll
+            for (int it = 0; it < 10; it++) {
+                const int mid = (lo + hi) >> 1;
+                if (s_p[mid] <= q) lo = mid; else hi = mid;
+            }
+            uint64_t l = (uint64_t)lo * step, u = min((uint64_t)N, l + step);
+            if (l >= N) { l = N - 1; u = N; }
+            while (l < u) {
+                const uint64_t mid = (l + u) >> 1;
+                if (__ldg(&sorted[mid]) < q) l = mid + 1; else u = mid;
+            }
+            if (l < N && __ldg(&sorted[l]) == q) {
+                const int32_t c = __ldg(&centre_idx[l]);
+                if (c >= 0 && (uint32_t)c < N) { v = __ldg(&sorted[c]); h = 1; }
+            } else {
+                missing++;
+            }
+        }
+        out[i] = v;
+        out_has[i] = h;
+        assigned += h;
+    }
+    for (int o = 16; o; o >>= 1) {
+        assigned += __shfl_down_sync(0xffffffffu, assigned, o);
+        missing += __shfl_down_sync(0xffffffffu, missing, o);
+    }
+    if ((threadIdx.x & 31) == 0) {
+        if (assigned) atomicAdd(&counters[0], assigned);
+        if (missing) atomicAdd(&counters[1], missing);
+    }
 }
 
 // ---------------------------------------------------------------------------------------------------

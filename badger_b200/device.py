@@ -258,6 +258,66 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
     return out, info
 
 
+class Tally(pipeline.Tally):
+    """pipeline.Tally on tensors: add(ranks, valid=None) and assign(ranks, valid=None) take tensors on the first device (checked
+    as dedup_reads checks them); assign returns (centre[R] in the dtype of its ranks, has_centre bool[R]).  Nothing of size R or
+    N crosses PCIe in add or assign; with high_sens the patched node -> centre array is uploaded once, by finish."""
+
+    _centres_above = staticmethod(centres_above)
+
+    def __init__(self):
+        _ready()
+        super().__init__()
+
+    def add(self, ranks: torch.Tensor, valid: torch.Tensor | None = None) -> int:
+        _check(ranks, "ranks", BARCODE_DTYPES)
+        R = ranks.numel()
+        _check_valid(valid, R)
+        nv = C.c_size_t(0)
+        check(lib().bdg_dev_tally_add(self._handle(), _ptr(ranks), _ptr(valid), R, C.byref(nv), _stream()))
+        self.rows += R
+        return int(nv.value)
+
+    def finish(self, *, true_barcodes=None, **kw) -> dict:
+        """pipeline.Tally.finish; whitelist_sorted is a tensor on the first device, true_barcodes an iterable or a tensor."""
+        if isinstance(true_barcodes, torch.Tensor):
+            true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+        return super().finish(true_barcodes=true_barcodes, **kw)
+
+    def _finish_call(self, n, nv, tok):
+        check(lib().bdg_dev_tally_finish(self._handle(), C.byref(n), C.byref(nv), C.byref(tok), _stream()))
+
+    def _upload(self, ci):
+        return torch.from_numpy(np.ascontiguousarray(ci, dtype=np.int32)).to(_device())
+
+    def assign(self, ranks: torch.Tensor, valid: torch.Tensor | None = None):
+        rm = self._ready_to_assign()
+        _check(ranks, "ranks", BARCODE_DTYPES)
+        R, dev = ranks.numel(), ranks.device
+        _check_valid(valid, R)
+        if rm is None:                                        # nothing was counted: only rows without a barcode can be assigned
+            n_valid = R if valid is None else int(torch.count_nonzero(valid))
+            if n_valid:
+                raise ValueError("%d valid rows have a barcode that was never added" % n_valid)
+            return torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)
+        centre = torch.empty(R, dtype=ranks.dtype, device=dev)
+        has = torch.empty(R, dtype=torch.bool, device=dev)
+        na, nm = C.c_size_t(0), C.c_size_t(0)
+        check(lib().bdg_dev_assign_lookup32(rm.token, _ptr(self._ci), rm.n_distinct, _ptr(ranks), _ptr(valid), R, _ptr(centre), _ptr(has),
+                                            C.byref(na), C.byref(nm), _stream()))
+        if nm.value:
+            raise ValueError("%d valid rows have a barcode that was never added" % nm.value)
+        self.info["assigned_reads"] += int(na.value)
+        return centre, has
+
+
+def _check_valid(valid, R):
+    if valid is not None:
+        _check(valid, "valid", MASK_DTYPES)
+        if valid.numel() != R:
+            raise ValueError("valid has %d rows, ranks %d" % (valid.numel(), R))
+
+
 # ---------------------------------------------------------------------------------------------- the whitelist operators
 def member_sorted(sorted_wl: torch.Tensor, q: torch.Tensor) -> torch.Tensor:
     """ops.member_sorted on tensors: bool[Q], hit[i] = q[i] is in sorted_wl.  sorted_wl must be ascending as uint32; it is

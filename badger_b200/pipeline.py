@@ -11,15 +11,19 @@ barcodes per read in, cluster-centre barcode per read out, every stage on the GP
       -> ops.assign_reads32              barcode_graph.py:322-329,395-404   centre of every row: gather kernel over the resident read map
 
 The string-based mirror (``BarcodeGraph`` + ``badger.py``) gives the same assignments; this module exists for callers
-that already hold packed barcodes and for the reads/s figure of ``bench.py``.
+that already hold packed barcodes and for the reads/s figure of ``bench.py``.  ``Tally`` is the same step for reads that
+arrive in batches: the dedup runs batch by batch into a running distinct set on the device, and the per-read gather looks
+every row's barcode up among the nodes.
 """
 from __future__ import annotations
 
+import ctypes as C
 import time
 
 import numpy as np
 
-from . import ops
+from . import _lib, ops
+from ._lib import check, lib, ptr
 from .barcode_graph import _unrank_many
 from .common import rank
 
@@ -98,6 +102,121 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
 
 def _tick(T, name, t0):
     T[name] = T.get(name, 0.0) + time.perf_counter() - t0
+
+
+class Tally:
+    """The correction step over reads that arrive in batches (include/badger_b200.h bdg_tally_*): `add` batches 0 ... B-1 in order,
+    `finish` once, then `assign` any rows.  The result of `assign` equals, element for element, what assign_packed(form="u32")
+    gives those rows when it runs on the concatenation of the added batches, and `finish` returns its `info` (with
+    "assigned_reads" summed over the assign calls).  Only the distinct barcodes, their counts and first sightings are kept
+    between batches, on the device; the device memory per read grows with the batch, not with the total, and the total may
+    exceed the 2^31 reads of one assign_packed call (each batch stays below 2^31 rows).
+
+    Every add and finish is a dedup call: it kills the read map of an outstanding ops.dedup_reads token, and a later dedup call
+    (another tally's add, assign_packed, ...) makes `assign` raise until `finish` runs again."""
+
+    _centres_above = staticmethod(ops.centres_above)
+
+    def __init__(self):
+        self._h = C.c_void_p()
+        check(lib().bdg_tally_create(C.byref(self._h)))
+        self.rows = 0
+        self.info = None              # finish's result: `info` of the one-call step
+        self._rm = None               # the read map finish installed (None: no valid read was added)
+        self._ci = None               # with high_sens, the patched node -> centre array; None: the clustering left on the device
+
+    def _handle(self):
+        if self._h is None or not self._h.value:
+            raise ValueError("the tally was freed")
+        return self._h
+
+    def add(self, ranks, valid=None) -> int:
+        """Count one batch (packed barcodes per row; valid: mask or None for all rows).  Returns its number of valid rows."""
+        r = np.ascontiguousarray(ranks, dtype=np.uint32)
+        v = _mask(valid, r.size)
+        nv = C.c_size_t(0)
+        check(lib().bdg_tally_add(self._handle(), ptr(r), ptr(v) if v is not None else None, r.size, C.byref(nv)))
+        self.rows += r.size
+        return int(nv.value)
+
+    def _finish_call(self, n, nv, tok):
+        check(lib().bdg_tally_finish(self._handle(), C.byref(n), C.byref(nv), C.byref(tok)))
+
+    def finish(self, *, threshold, n_cells, interval=25, whitelist_sorted=None, true_barcodes=None, high_sens=False, centre_order=None,
+               timings=None) -> dict:
+        """The stages after the dedup (run_stages, arguments as for assign_packed) over the counted batches.  The clustering
+        result stays for `assign`.  Returns `info`; no batch can be added afterwards."""
+        T = timings if timings is not None else {}
+        t0 = time.perf_counter()
+        n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
+        self._finish_call(n, nv, tok)
+        _tick(T, "tally_finish", t0)
+        self.info = info = {"reads": int(self.rows), "valid_reads": int(nv.value)}
+        self._rm, self._ci = None, None
+        if nv.value == 0:
+            return info
+        rm = ops.ReadMap(int(n.value), int(nv.value), 0, int(tok.value))
+
+        def keep(ci):
+            self._ci = None if ci is None else self._upload(ci)
+            return None, 0
+
+        run_stages(rm, info, T, keep, threshold=threshold, n_cells=n_cells, interval=interval, whitelist_sorted=whitelist_sorted,
+                   true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order, centres_above=self._centres_above)
+        self._rm = rm
+        return info
+
+    def _upload(self, ci):
+        return np.ascontiguousarray(ci, dtype=np.int32)
+
+    def _ready_to_assign(self):
+        if self.info is None:
+            raise ValueError("assign before finish")
+        return self._rm
+
+    def assign(self, ranks, valid=None):
+        """(centre uint32[R], has_centre uint8[R]) for the rows of `ranks`, any batching.  ValueError when a valid row's barcode
+        was never added.  With high_sens the patched node -> centre array is copied to the device with every call (the tensor
+        form, device.Tally, uploads it once)."""
+        rm = self._ready_to_assign()
+        r = np.ascontiguousarray(ranks, dtype=np.uint32)
+        v = _mask(valid, r.size)
+        R = r.size
+        if rm is None:                                        # nothing was counted: only rows without a barcode can be assigned
+            if R and (v is None or v.any()):
+                raise ValueError("%d valid rows have a barcode that was never added" % (R if v is None else int(np.count_nonzero(v))))
+            return np.zeros(R, np.uint32), np.zeros(R, np.uint8)
+        out = ops._pinned.array(R, np.uint32, eager=False)
+        has = ops._pinned.array(R, np.uint8, eager=False)
+        na, nm = C.c_size_t(0), C.c_size_t(0)
+        ci = self._ci
+        check(lib().bdg_assign_lookup32(rm.token, ptr(ci) if ci is not None else None, rm.n_distinct, ptr(r), ptr(v) if v is not None else None,
+                                        R, ptr(out), ptr(has), C.byref(na), C.byref(nm)))
+        if nm.value:
+            raise ValueError("%d valid rows have a barcode that was never added" % nm.value)
+        self.info["assigned_reads"] += int(na.value)
+        return out, has
+
+    def free(self):
+        if self._h is not None and self._h.value and _lib._lib is not None:
+            lib().bdg_tally_free(self._h)
+        self._h = None
+
+    def __del__(self):
+        try:
+            self.free()
+        except Exception:
+            pass
+
+
+def _mask(valid, n):
+    """A validity mask as uint8 for the C ABI (a bool mask is used in place), or None."""
+    if valid is None:
+        return None
+    v = np.ascontiguousarray(valid)
+    if v.size != n:
+        raise ValueError("valid has %d rows, ranks %d" % (v.size, n))
+    return v.view(np.uint8) if v.dtype == np.bool_ else (v != 0).view(np.uint8)
 
 
 def run_stages(rm, info, T, gather, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order,

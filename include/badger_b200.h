@@ -271,6 +271,45 @@ int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx
 int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first,
                         const size_t* starts, const size_t* sizes, int n_parts, int my_part, size_t* n_distinct,
                         unsigned long long* merged_token, void* stream);
+
+/* ---- the correction step over reads that arrive in batches (a tally) ----------------------------------------------------------
+ * add batches 0 .. B-1 in order, finish, then assign any rows: the per-read result equals what the one-call step
+ * (bdg_dedup_reads ... bdg_assign_reads32) gives for the concatenation of the batches.  Every batch holds fewer than 2^31 rows;
+ * the total may exceed 2^32.
+ *   tally_create  a handle on the first claimed device.  It keeps the running distinct set in its own buffers (not in the dedup
+ *                 workspace): every distinct barcode ascending, its 64-bit count and its 64-bit first sighting.  tally_free
+ *                 releases them.  A handle is refused (BDG_ERR_ARG) once its device is no longer the first claimed one.
+ *   tally_add     dedups the batch (the rows with valid[i] != 0; valid == NULL: all) with the dedup kernels and merges its
+ *                 ascending distinct list into the set (merge path; counts summed, the smaller first sighting kept).  *n_valid
+ *                 (may be NULL) = valid rows of the batch.  Like any dedup call, it kills the read map of an outstanding token.
+ *                 BDG_ERR_ARG after finish, for a batch of 2^31 rows or more, and for a batch that would take the set to 2^31
+ *                 distinct barcodes or more (the set keeps the batches before it).  Waits for the batch's sizes.
+ *   tally_finish  sorts the set by first sighting and installs it as the read map of a dedup call WITHOUT rows (*token; 0 when no
+ *                 valid row was added): distinct in first-seen order, counts, sorted_pos and sorted_distinct as bdg_dev_dedup_merge
+ *                 documents them, so bdg_edges_build_resident, bdg_[dev_]centres_above, bdg_centres_rest, bdg_cluster_resident and
+ *                 bdg_[dev_]dedup_fetch take the token unchanged.  *n_distinct = barcodes, *n_valid = valid rows added in all.  A
+ *                 barcode counted 2^32 times or more is refused with BDG_ERR_ARG (the read map's counts are uint32).  The tally
+ *                 takes no more batches afterwards; finish may be called again, to install the read map anew after a later
+ *                 dedup call killed the token.
+ *   assign_lookup32  the per-read gather for rows that are in no read map: every valid row's barcode is looked up among the nodes
+ *                 of the read map `token` names (its ascending array), node -> centre node (centre_idx[N] over those nodes; NULL:
+ *                 the result bdg_cluster_resident left for this read map) -> centre barcode.  centre / has_centre as for
+ *                 bdg_assign_reads32; *n_assigned = rows with a centre, *n_missing = valid rows whose barcode is no node (their
+ *                 has_centre is 0).  Any token works, a dedup call's too.  The device form waits only when n_assigned or
+ *                 n_missing is given.
+ * The bdg_dev_* forms take pointers on the first claimed device and order their work against `stream` as the correction-step
+ * device forms above do. */
+typedef struct bdg_tally bdg_tally;
+int bdg_tally_create(bdg_tally** out);
+void bdg_tally_free(bdg_tally* h);
+int bdg_tally_add(bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, size_t* n_valid);
+int bdg_dev_tally_add(bdg_tally* h, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R, size_t* n_valid, void* stream);
+int bdg_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token);
+int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, void* stream);
+int bdg_assign_lookup32(unsigned long long token, const int32_t* centre_idx, size_t N, const uint32_t* ranks, const uint8_t* valid, size_t R,
+                        uint32_t* centre, uint8_t* has_centre, size_t* n_assigned, size_t* n_missing);
+int bdg_dev_assign_lookup32(unsigned long long token, const int32_t* d_centre_idx, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid,
+                            size_t R, uint32_t* d_centre, uint8_t* d_has_centre, size_t* n_assigned, size_t* n_missing, void* stream);
 /* The phases of bdg_cluster_levels over node arrays the caller owns, on `stream` of the current (claimed) device and without a
  * synchronisation, so that processes can reduce the claims between the phases.  Nodes are positions in d_sorted[N]
  * (0 < N < 2^31); d_centre_idx / d_level as for bdg_cluster_levels, except that level 254 marks a node with an edge that no
