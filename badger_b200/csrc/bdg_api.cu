@@ -49,22 +49,31 @@ int fail(int code, const char* fmt, ...)
     } while (0)
 
 // grow-only device buffer: the host-buffer entry points reuse their workspaces from call to call
-// (cudaMalloc / cudaFree per call cost far more than the kernels at BASELINE config-2 sizes)
+// (cudaMalloc / cudaFree per call cost far more than the kernels at BASELINE config-2 sizes).  It owns its allocation: the
+// owner makes the buffer's device current before destroying it.
 struct Buf {
     void* p = nullptr;
     size_t cap = 0;
+    Buf() = default;
+    Buf(Buf&& o) noexcept : p(o.p), cap(o.cap) { o.p = nullptr; o.cap = 0; }
+    Buf& operator=(Buf&&) = delete;
+    ~Buf() { release(); }
+    // at least `bytes` bytes; growing frees the old contents.  BDG_ERR_OOM / BDG_ERR_CUDA with the message set on failure.
     int ensure(size_t bytes)
     {
         if (bytes <= cap) return BDG_OK;
-        if (p) cudaFree(p);
-        p = nullptr;
-        cap = 0;
+        release();
         const size_t want = bytes + bytes / 4 + 256;
-        cudaError_t e = cudaMalloc(&p, want);
-        if (e != cudaSuccess) { p = nullptr; return (int)e; }
+        if (cudaError_t e = cudaMalloc(&p, want)) {
+            p = nullptr;
+            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes,
+                        cudaGetErrorString(e));
+        }
         cap = want;
         return BDG_OK;
     }
+
+private:
     void release() { if (p) cudaFree(p); p = nullptr; cap = 0; }
 };
 
@@ -74,6 +83,48 @@ struct Plan {
     std::vector<uint32_t> item_start;
     uint32_t chunk_cols = 256;
     uint64_t pairs = 0;
+};
+
+// The read map a dedup call leaves on the first device, named by its token, and the clustering result that may belong to it.
+// Its arrays are the dedup workspaces after dedup_core, which reuses them within a call; merge and tally install theirs there.
+struct ReadMap {
+    Buf dd[10];                   // dedup_core's workspaces (see there); the map's arrays by name below
+    Buf valid, valid_scan;        // masked dedup: the rows' valid bytes and their exclusive scan (a valid row's index among the valid rows)
+    Buf centre, level;            // the last clustering on this device (cluster_on_device): centre index and level per node
+    unsigned long long token = 0, serial = 0;   // token of the live read map (0: none), last token issued
+    unsigned long long cl_token = 0;            // read-map token the clustering result belongs to (0: none)
+    size_t rows = 0, reads = 0, distinct = 0;   // rows of the dedup call, valid rows among them, distinct barcodes (the nodes)
+    bool masked = false;                        // the rows came with valid bytes
+
+    Buf& keys() { return dd[0]; }                                      // dedup_core's input: the key of every valid read
+    uint32_t* counts() const { return (uint32_t*)dd[0].p; }            // count of every distinct barcode, first-seen order
+    uint32_t* order() const { return (uint32_t*)dd[1].p; }             // first-seen position -> ascending position (node)
+    uint32_t* first_seen() const { return (uint32_t*)dd[2].p; }        // the distinct barcodes in first-seen order
+    uint32_t* run_pos() const { return (uint32_t*)dd[4].p; }           // node -> first-seen position (dedup calls only)
+    uint32_t* ascending() const { return (uint32_t*)dd[6].p; }         // the distinct barcodes ascending: the nodes
+    uint32_t* read_pos() const { return (uint32_t*)dd[7].p; }          // valid read -> first-seen position (`reads` entries)
+
+    void drop() { token = 0; cl_token = 0; }   // the workspaces are about to be reused: the live read map dies here
+
+    // Installs a distinct set of n barcodes as the live read map and issues its token: the four arrays counts, order, first-seen,
+    // ascending (as named above) hold n entries afterwards.  The sources (device arrays on this map's device) are copied in on
+    // st; NULL: the array is already in place, or the caller writes it on st right after the install.
+    int install(size_t n, const uint32_t* src_counts, const uint32_t* src_order, const uint32_t* src_first_seen,
+                const uint32_t* src_ascending, cudaStream_t st, unsigned long long* out_token)
+    {
+        drop();
+        CU_TRY(cudaStreamSynchronize(st));          // growing a buffer frees its old memory: queued work may still read it
+        const uint32_t* src[4] = {src_counts, src_order, src_first_seen, src_ascending};
+        const int slot[4] = {0, 1, 2, 6};
+        for (int k = 0; k < 4; k++) {
+            if (int e = dd[slot[k]].ensure(n * 4)) return e;
+            if (src[k]) CU_TRY(cudaMemcpyAsync(dd[slot[k]].p, src[k], n * 4, cudaMemcpyDeviceToDevice, st));
+        }
+        distinct = n;
+        token = ++serial;
+        *out_token = token;
+        return BDG_OK;
+    }
 };
 
 struct DevCtx {
@@ -88,19 +139,16 @@ struct DevCtx {
     cudaEvent_t ev_start = nullptr, ev_done[bdg::MAX_PASSES] = {nullptr, nullptr, nullptr};
     unsigned long long host_stats[bdg::MAX_PASSES][2] = {};   // interval tests done / tiles listed per pass of the last launch
     unsigned long long generation = 0;                        // bumped by every host-buffer edge build on this device
-    Buf dd[10];                                               // dedup: keys, idx, sorted keys/idx, heads, scan, run arrays, cub scratch
-    Buf cl[6];                                                // clustering: centres, centre index, level, claim min / max, flags
-    unsigned long long cl_token = 0;                          // read-map token the clustering result resident in cl[1] / cl[2] belongs to (0: none)
+    ReadMap map;                                              // the read map of the last dedup call (first device)
+    Buf cl[4];                                                // clustering: centres, claim min / max, flags + count (result: map.centre / map.level)
     Buf ce[9];                                                // centre selection: positions above the cutoff, sort keys / values, results, scratch
-    Buf as[8];                                                // masked dedup + per-read gather: all ranks, valid bytes, their scan, scratch, centre idx / value, result, counter
+    Buf as[6];                                                // masked dedup + per-read gather: all ranks, scan scratch, centre idx upload, centre values, result, counter
     Buf mg[12];                                               // merge of the parts' dedup results (bdg_dev_dedup_merge), see there
     Buf lk[5];                                                // per-read lookup (bdg_assign_lookup32): counters, and the host form's ranks, valid bytes, result, centre idx
-    unsigned long long map_token = 0, map_serial = 0;         // read map left on the device by bdg_dedup_reads (0: none)
-    size_t map_rows = 0, map_reads = 0, map_distinct = 0;
-    bool map_masked = false;
     Buf gather_a, gather_b;                                   // node indices of the edge ends: this device's own, and (first device) those of ALL devices, gathered for cluster()
     Buf top16;                                                // first node of every high half of the barcode (the node of an edge end is searched in that run)
-    Buf io[4];                                                // host-buffer calls of pack16 / membership: inputs, outputs, check flag
+    Buf io[4];                                                // host-buffer calls: pack16 letters / ranks / valid; membership whitelist / queries / hits;
+                                                              // nearest queries / targets / keys | argmin | distance; [3] check flag
     Buf nn[9];                                                // sparse nearest: rotated keys + payload (in/out) of queries and targets, scratch
     // join form of the t = 2 and t = 3 edge construction (bdg_join.cuh): barcodes in the key order of every condition's row side /
     // column side, first column of every key, bucket sizes and every barcode's place in its bucket, scan scratch, units per slab
@@ -116,7 +164,8 @@ struct DevCtx {
     unsigned long long* snap_dev = nullptr;
     cudaEvent_t ev_caller = nullptr;                          // bdg_dev_* correction-step calls: orders this device's stream against the caller's
 };
-std::vector<DevCtx> g_ctx;
+// Never deleted: the buffers are freed by bdg_shutdown, not by static destructors at process exit.
+std::vector<DevCtx>& g_ctx = *new std::vector<DevCtx>;
 
 int owner_of_tile(uint64_t I, int P)
 {
@@ -298,14 +347,9 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
 {
     if (int rc = scheme_ready<T>()) return rc;
     const auto& S = join_scheme<T>();
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     if constexpr (T == 2) {                                 // the table to constant memory, the hand-over table beside it
         if (ws->scheme_serial != g_scheme_serial) {
-            if (int e = ensure(ws->jn_lut, g_scheme_lut.size())) return e;
+            if (int e = ws->jn_lut.ensure(g_scheme_lut.size())) return e;
             CU_TRY(cudaMemcpyToSymbolAsync(bdg::c_scheme, &g_scheme, sizeof(g_scheme), 0, cudaMemcpyHostToDevice, caller));
             CU_TRY(cudaMemcpyAsync(ws->jn_lut.p, g_scheme_lut.data(), g_scheme_lut.size(), cudaMemcpyHostToDevice, caller));
             CU_TRY(cudaStreamSynchronize(caller));          // the host copies above are read asynchronously
@@ -313,7 +357,7 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
         }
     } else {                                                // too large for constant memory: a device copy
         if (ws->scheme3_serial != g_scheme3_serial) {
-            if (int e = ensure(ws->jn3_scheme, sizeof(g_scheme3))) return e;
+            if (int e = ws->jn3_scheme.ensure(sizeof(g_scheme3))) return e;
             CU_TRY(cudaMemcpyAsync(ws->jn3_scheme.p, &g_scheme3, sizeof(g_scheme3), cudaMemcpyHostToDevice, caller));
             CU_TRY(cudaStreamSynchronize(caller));          // the host copy above is read asynchronously
             ws->scheme3_serial = g_scheme3_serial;
@@ -342,7 +386,7 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
                 slots.col[c] = S.cond[c].self ? slots.row[c] : (uint8_t)slots.n++;
             }
             const size_t hist_bytes = (size_t)slots.n * maxtab * 4;
-            if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * bdg::SEED_MAX_CONDS)) return e;
+            if (int e = ws->jn_weigh.ensure(hist_bytes + 8 * bdg::SEED_MAX_CONDS)) return e;
             uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
             d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
             CU_TRY(cudaMemsetAsync(ws->jn_weigh.p, 0, hist_bytes + 8 * bdg::SEED_MAX_CONDS, caller));
@@ -355,7 +399,7 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
             for (int c = 0; c < S.nconds; c++) max_bits = std::max(max_bits, (int)S.ka[c].key_bits);
             const uint32_t tab = 1u << max_bits;
             const size_t hist_bytes = (size_t)max_set * tab * 4;
-            if (int e = ensure(ws->jn_weigh, hist_bytes + 8 * (size_t)bdg::SEED3_MAX_CONDS)) return e;
+            if (int e = ws->jn_weigh.ensure(hist_bytes + 8 * (size_t)bdg::SEED3_MAX_CONDS)) return e;
             uint32_t* d_hist = (uint32_t*)ws->jn_weigh.p;
             d_pairs = (unsigned long long*)((char*)ws->jn_weigh.p + hist_bytes);
             CU_TRY(cudaMemsetAsync(d_pairs, 0, 8 * (size_t)S.nconds, caller));
@@ -412,7 +456,7 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
         }
     }
     const size_t plan_bytes = PLAN_HDR * bdg::MAX_PASSES + 8 * (size_t)S.nconds;
-    if (int e = ensure(ws->plan, plan_bytes)) return e;
+    if (int e = ws->plan.ensure(plan_bytes)) return e;
     char* d_plan = (char*)ws->plan.p;
     CU_TRY(cudaMemsetAsync(d_plan, 0, plan_bytes, caller));
     for (int p = 0; p < bdg::MAX_PASSES; p++) ws->host_stats[p][0] = ws->host_stats[p][1] = 0;
@@ -425,15 +469,15 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
     CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp_b, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)(n_slabs + 1), caller));
     const size_t tmp_bytes = std::max(tmp_a, tmp_b);
     for (int k = 0; k < 2; k++) {                           // one scratch set per stream
-        if (int e = ensure(ws->jn_hist[k], (max_keys + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_tab[k], (max_keys + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_tabc[k], (max_keys + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_rows[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_cols[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_rank[k], N * 4)) return e;
-        if (int e = ensure(ws->jn_cub[k], tmp_bytes)) return e;
-        if (int e = ensure(ws->jn_counts[k], ((size_t)n_slabs + 1) * 4)) return e;
-        if (int e = ensure(ws->jn_offs[k], ((size_t)n_slabs + 1) * 4)) return e;
+        if (int e = ws->jn_hist[k].ensure((max_keys + 1) * 4)) return e;
+        if (int e = ws->jn_tab[k].ensure((max_keys + 1) * 4)) return e;
+        if (int e = ws->jn_tabc[k].ensure((max_keys + 1) * 4)) return e;
+        if (int e = ws->jn_rows[k].ensure(N * 4)) return e;
+        if (int e = ws->jn_cols[k].ensure(N * 4)) return e;
+        if (int e = ws->jn_rank[k].ensure(N * 4)) return e;
+        if (int e = ws->jn_cub[k].ensure(tmp_bytes)) return e;
+        if (int e = ws->jn_counts[k].ensure(((size_t)n_slabs + 1) * 4)) return e;
+        if (int e = ws->jn_offs[k].ensure(((size_t)n_slabs + 1) * 4)) return e;
     }
     const auto kern = rs == 8 ? bdg::join_kernel<T, 8> : bdg::join_kernel<T, 32>;
     int grid = 0;
@@ -597,8 +641,7 @@ int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts
     if (n_items == 0) return BDG_OK;
     const size_t nb_groups = plan.group_ids.size() * sizeof(uint32_t), nb_items = plan.item_start.size() * sizeof(uint32_t);
     const size_t hdr = PLAN_HDR * bdg::MAX_PASSES;
-    if (cudaError_t e = (cudaError_t)ws->plan.ensure(hdr + nb_groups + nb_items))
-        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "plan workspace: %s", cudaGetErrorString(e));
+    if (int e = ws->plan.ensure(hdr + nb_groups + nb_items)) return e;
     char* d_plan = (char*)ws->plan.p;   // [headers | group_ids | item_start]
     CU_TRY(cudaMemsetAsync(d_plan, 0, hdr, st));
     for (int p = 0; p < bdg::MAX_PASSES; p++) ws->host_stats[p][0] = ws->host_stats[p][1] = 0;
@@ -630,17 +673,12 @@ int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts
         w.pass = p;
         w.rot = sparse ? bdg::pass_rot(t, p) : 0;
         w.sorted = d_sorted;
-        auto ensure = [&](Buf& b, size_t bytes) -> int {
-            if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-                return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
-            return BDG_OK;
-        };
         if (w.rot != 0) {   // this pass scans the array in the order of rotl(key, rot): rotate, radix-sort
-            if (int e = ensure(ws->rot_in[p], N * 4)) return e;
-            if (int e = ensure(ws->rot_sorted[p], N * 4)) return e;
+            if (int e = ws->rot_in[p].ensure(N * 4)) return e;
+            if (int e = ws->rot_sorted[p].ensure(N * 4)) return e;
             size_t tmp_bytes = 0;
             CU_TRY(cub::DeviceRadixSort::SortKeys(nullptr, tmp_bytes, (const uint32_t*)ws->rot_in[p].p, (uint32_t*)ws->rot_sorted[p].p, (int)N, 0, 32, st));
-            if (int e = ensure(ws->sort_tmp[p], tmp_bytes)) return e;
+            if (int e = ws->sort_tmp[p].ensure(tmp_bytes)) return e;
             const int rb = (int)std::min<size_t>((N + 255) / 256, (size_t)ws->sms * 8);
             bdg::rotate_keys_kernel<<<rb, 256, 0, st>>>(d_sorted, (uint32_t*)ws->rot_in[p].p, (uint32_t)N, w.rot);
             g_launches++;
@@ -654,11 +692,11 @@ int launch_edges(const uint32_t* d_sorted, size_t N, int t, int part, int nparts
         } else {
             // level 1: interval scan of every (owned row group, sub-tile right of it) -> compact tile list
             const uint32_t NS = (uint32_t)((N + bdg::SSB - 1) / bdg::SSB);
-            if (int e = ensure(ws->tile_bnd[p], (size_t)NS * sizeof(uint2))) return e;
+            if (int e = ws->tile_bnd[p].ensure((size_t)NS * sizeof(uint2))) return e;
             if (ws->tile_list[p].cap == 0) {
                 size_t want = std::max<size_t>((size_t)1 << 22, 4 * N);
                 if (const char* e = getenv("BDG_TILE_LIST_CAP")) want = (size_t)std::max(1ll, atoll(e));   // tests: force the regrow path
-                if (int e = ensure(ws->tile_list[p], want * sizeof(uint2))) return e;
+                if (int e = ws->tile_list[p].ensure(want * sizeof(uint2))) return e;
             }
             bdg::tile_bounds_kernel<<<std::min<uint32_t>((NS + 255) / 256, (uint32_t)ws->sms * 8), 256, 0, st>>>(w.sorted, w.N, (uint2*)ws->tile_bnd[p].p, NS);
             g_launches++;
@@ -691,26 +729,21 @@ int launch_nearest_sparse(const uint32_t* d_q, size_t Q, const uint32_t* d_t, si
 {
     const int T_ = max_d <= 1 ? 1 : 2;
     const int passes = bdg::n_passes(T_);
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "workspace of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     // nn[0..3]: query keys in / payload in / keys sorted / payload sorted; nn[4..7]: the same for the targets; nn[8]: sort scratch
-    for (int k = 0; k < 4; k++) if (int e = ensure(ws->nn[k], Q * 4)) return e;
-    for (int k = 4; k < 8; k++) if (int e = ensure(ws->nn[k], W * 4)) return e;
+    for (int k = 0; k < 4; k++) if (int e = ws->nn[k].ensure(Q * 4)) return e;
+    for (int k = 4; k < 8; k++) if (int e = ws->nn[k].ensure(W * 4)) return e;
     uint32_t *qk = (uint32_t*)ws->nn[0].p, *qp = (uint32_t*)ws->nn[1].p, *qks = (uint32_t*)ws->nn[2].p, *qps = (uint32_t*)ws->nn[3].p;
     uint32_t *tk = (uint32_t*)ws->nn[4].p, *tp = (uint32_t*)ws->nn[5].p, *tks = (uint32_t*)ws->nn[6].p, *tps = (uint32_t*)ws->nn[7].p;
     size_t tmp_q = 0, tmp_t = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_q, qk, qks, qp, qps, (int)Q, 0, 32, st));
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_t, tk, tks, tp, tps, (int)W, 0, 32, st));
-    if (int e = ensure(ws->nn[8], std::max(tmp_q, tmp_t))) return e;
+    if (int e = ws->nn[8].ensure(std::max(tmp_q, tmp_t))) return e;
     const uint32_t NS = (uint32_t)((W + bdg::SSB - 1) / bdg::SSB);
     const uint32_t K = (uint32_t)((Q + bdg::GROUP - 1) / bdg::GROUP);
-    if (int e = ensure(ws->tile_bnd[0], (size_t)NS * sizeof(uint2))) return e;
+    if (int e = ws->tile_bnd[0].ensure((size_t)NS * sizeof(uint2))) return e;
     if (ws->tile_list[0].cap == 0)
-        if (int e = ensure(ws->tile_list[0], ((size_t)1 << 22) * sizeof(uint2))) return e;
-    if (int e = ensure(ws->plan, PLAN_HDR * bdg::MAX_PASSES)) return e;
+        if (int e = ws->tile_list[0].ensure(((size_t)1 << 22) * sizeof(uint2))) return e;
+    if (int e = ws->plan.ensure(PLAN_HDR * bdg::MAX_PASSES)) return e;
     char* d_plan = (char*)ws->plan.p;   // only the headers are used here; a cached edge plan behind them stays valid
     CU_TRY(cudaMemsetAsync(d_plan, 0, PLAN_HDR * bdg::MAX_PASSES, st));
     int grid = 0;
@@ -742,7 +775,7 @@ int launch_nearest_sparse(const uint32_t* d_q, size_t Q, const uint32_t* d_t, si
             CU_TRY(cudaStreamSynchronize(st));
             if (n_tiles <= l.cap) break;
             if (attempt == 1) return fail(BDG_ERR_CUDA, "tile list count changed between identical scans");
-            if (int e = ensure(ws->tile_list[0], (size_t)n_tiles * sizeof(uint2))) return e;
+            if (int e = ws->tile_list[0].ensure((size_t)n_tiles * sizeof(uint2))) return e;
         }
         if (n_tiles == 0) continue;
         bdg::TileList l{(uint2*)ws->tile_list[0].p, (unsigned long long*)(d_plan + PLAN_HDR * p + HDR_LIST), ws->tile_list[0].cap / sizeof(uint2)};
@@ -771,6 +804,40 @@ int need_ctx()
         int rc = bdg_init(nullptr, 0);
         if (rc) return rc;
     }
+    return BDG_OK;
+}
+
+// The first claimed context, its device made current, when `token` names the read map live there.
+int map_ctx(unsigned long long token, DevCtx** out)
+{
+    if (int rc = need_ctx()) return rc;
+    DevCtx& c = g_ctx[0];
+    if (token == 0 || token != c.map.token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    CU_TRY(cudaSetDevice(c.dev));
+    *out = &c;
+    return BDG_OK;
+}
+
+// The per-pass headers of the last edge launch on c (PLAN_HDR bytes each: work cursor, tile-list count, statistics), read back on st.
+constexpr size_t PLAN_WORDS = (PLAN_HDR / 8) * bdg::MAX_PASSES;
+int read_plan_headers(const DevCtx* c, cudaStream_t st, unsigned long long (&v)[PLAN_WORDS])
+{
+    if (!c || !c->plan.p) return fail(BDG_ERR_ARG, "no edge launch on this device yet");
+    CU_TRY(cudaMemcpyAsync(v, c->plan.p, sizeof(v), cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    return BDG_OK;
+}
+
+// After an edge count that came back with bit 63 set (a sparse pass listed more tiles than its list holds): every pass's tile
+// list grows to the longest list any pass asked for, so that the launch can run again.
+int grow_tile_lists(DevCtx& c)
+{
+    unsigned long long v[PLAN_WORDS];
+    if (int rc = read_plan_headers(&c, c.stream, v)) return rc;
+    unsigned long long need = 0;
+    for (int p = 0; p < bdg::MAX_PASSES; p++) need = std::max(need, v[(PLAN_HDR / 8) * p + HDR_LIST / 8]);
+    for (int p = 0; p < bdg::MAX_PASSES; p++)
+        if (int e = c.tile_list[p].ensure((size_t)need * sizeof(uint2))) return e;
     return BDG_OK;
 }
 
@@ -833,6 +900,7 @@ struct bdg_edges {
     std::vector<int> ctx;                 // indices into g_ctx
     std::vector<size_t> count;            // edges held by each of them
     std::vector<unsigned long long> gen;  // workspace generation at build time
+    unsigned long long read_map = 0;       // token of the read map whose ascending array the edges were built from (0: a caller's array)
 };
 
 // Known strings of a KmerIndexer / QGramIndex, resident on one device, plus grow-only query / result buffers.
@@ -884,12 +952,7 @@ int bdg_init(const int* device_ids, int n_devices)
             CU_TRY(cudaStreamCreateWithFlags(&c.aux[p], cudaStreamNonBlocking));
             CU_TRY(cudaEventCreateWithFlags(&c.ev_done[p], cudaEventDisableTiming));
         }
-        cudaMemPool_t pool;   // keep stream-ordered allocations cached instead of returning them at every sync
-        if (cudaDeviceGetDefaultMemPool(&pool, id) == cudaSuccess) {
-            unsigned long long keep = ~0ull;
-            cudaMemPoolSetAttribute(pool, cudaMemPoolAttrReleaseThreshold, &keep);
-        }
-        g_ctx.push_back(c);
+        g_ctx.push_back(std::move(c));
     }
     // direct NVLink copies into the first device (bdg_cluster_levels_from_edges gathers the other devices' edge lists there);
     // without peer access cudaMemcpyPeerAsync stages through host memory
@@ -911,35 +974,20 @@ int bdg_init(const int* device_ids, int n_devices)
 
 void bdg_shutdown(void)
 {
-    for (auto& c : g_ctx) {
-        if (c.stream) { cudaSetDevice(c.dev); cudaStreamSynchronize(c.stream); cudaStreamDestroy(c.stream); }
-        c.sorted.release(); c.ea.release(); c.eb.release(); c.ed.release(); c.count.release(); c.plan.release();
+    while (!g_ctx.empty()) {
+        DevCtx& c = g_ctx.back();
+        cudaSetDevice(c.dev);                              // the context's buffers are freed on its device
+        if (c.stream) { cudaStreamSynchronize(c.stream); cudaStreamDestroy(c.stream); }
         for (int p = 0; p < bdg::MAX_PASSES; p++) {
-            c.rot_in[p].release(); c.sort_tmp[p].release(); c.tile_bnd[p].release(); c.tile_list[p].release();
             if (c.aux[p]) cudaStreamDestroy(c.aux[p]);
             if (c.ev_done[p]) cudaEventDestroy(c.ev_done[p]);
         }
         if (c.ev_start) cudaEventDestroy(c.ev_start);
         if (c.ev_caller) cudaEventDestroy(c.ev_caller);
-        for (auto& b : c.dd) b.release();
-        for (auto& b : c.nn) b.release();
-        for (auto& b : c.io) b.release();
-        for (auto& b : c.cl) b.release();
-        c.gather_a.release(); c.gather_b.release(); c.top16.release();
-        for (auto& b : c.as) b.release();
-        for (auto& b : c.lk) b.release();
-        for (auto& b : c.ce) b.release();
-        for (auto& b : c.rot_sorted) b.release();
-        for (int k = 0; k < 2; k++) {
-            c.jn_rows[k].release(); c.jn_cols[k].release(); c.jn_tab[k].release(); c.jn_tabc[k].release(); c.jn_hist[k].release();
-            c.jn_cub[k].release(); c.jn_counts[k].release(); c.jn_offs[k].release();
-        }
-        c.jn_lut.release(); c.jn_weigh.release(); for (auto& b : c.jn_rank) b.release();
-        c.jn3_scheme.release();
         if (c.snap_host) { cudaFreeHost(c.snap_host); c.snap_host = nullptr; for (auto& e : c.ev_snap) if (e) cudaEventDestroy(e);
                            for (int q = 0; q < 2; q++) { if (c.ev_pre[q]) cudaEventDestroy(c.ev_pre[q]); if (c.ev_join[q]) cudaEventDestroy(c.ev_join[q]); } }
+        g_ctx.pop_back();
     }
-    g_ctx.clear();
 }
 
 unsigned long long bdg_part_pairs(size_t N, int part, int nparts)
@@ -985,11 +1033,10 @@ int bdg_set_edge_mode(int mode)
 
 int bdg_dev_edges_stats(unsigned long long* out5, void* stream)
 {
+    if (!out5) return fail(BDG_ERR_ARG, "NULL pointer argument");
     DevCtx* c = ctx_of_current_device();
-    if (!c || !c->plan.p || !out5) return fail(BDG_ERR_ARG, "no edge launch on this device yet");
-    unsigned long long v[(PLAN_HDR / 8) * bdg::MAX_PASSES];
-    CU_TRY(cudaMemcpyAsync(v, c->plan.p, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CU_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    unsigned long long v[PLAN_WORDS];
+    if (int rc = read_plan_headers(c, (cudaStream_t)stream, v)) return rc;
     for (int k = 0; k < 5; k++) {
         out5[k] = 0;
         const int slot = k < 4 ? k : 7;
@@ -1006,11 +1053,9 @@ int bdg_dev_edges_stats(unsigned long long* out5, void* stream)
 // [6] candidates with D <= 2, [7] pairs whose 6-mer score was computed; [4] / [5] sum / max of the warps' busy time in ns).
 int bdg_dev_edges_stats_raw(unsigned long long* out8, void* stream)
 {
-    DevCtx* c = ctx_of_current_device();
-    if (!c || !c->plan.p || !out8) return fail(BDG_ERR_ARG, "no edge launch on this device yet");
-    unsigned long long v[(PLAN_HDR / 8) * bdg::MAX_PASSES];
-    CU_TRY(cudaMemcpyAsync(v, c->plan.p, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CU_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    if (!out8) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    unsigned long long v[PLAN_WORDS];
+    if (int rc = read_plan_headers(ctx_of_current_device(), (cudaStream_t)stream, v)) return rc;
     for (int k = 0; k < 8; k++) {
         out8[k] = 0;
         for (int p = 0; p < bdg::MAX_PASSES; p++) {
@@ -1044,11 +1089,9 @@ int bdg_join_lane_stats(unsigned long long* out8, int reset)
 // measured from the first warp's start - the load-balance picture of the last edge launch.
 int bdg_dev_edges_balance(unsigned long long* out /* 2 * MAX_PASSES */, void* stream)
 {
-    DevCtx* c = ctx_of_current_device();
-    if (!c || !c->plan.p || !out) return fail(BDG_ERR_ARG, "no edge launch on this device yet");
-    unsigned long long v[(PLAN_HDR / 8) * bdg::MAX_PASSES];
-    CU_TRY(cudaMemcpyAsync(v, c->plan.p, sizeof(v), cudaMemcpyDeviceToHost, (cudaStream_t)stream));
-    CU_TRY(cudaStreamSynchronize((cudaStream_t)stream));
+    if (!out) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    unsigned long long v[PLAN_WORDS];
+    if (int rc = read_plan_headers(ctx_of_current_device(), (cudaStream_t)stream, v)) return rc;
     for (int p = 0; p < bdg::MAX_PASSES; p++) {
         out[2 * p] = v[(PLAN_HDR / 8) * p + HDR_STATS / 8 + 4];
         out[2 * p + 1] = v[(PLAN_HDR / 8) * p + HDR_STATS / 8 + 5];
@@ -1140,31 +1183,28 @@ int bdg_dev_pipe_probe(int kind, int blocks, int iters, uint32_t* d_sink, unsign
 
 // ---------------------------------------------------------------- host-buffer entry points
 // ---- a-2  dedup + count in first-seen order (barcode_graph.py:192-204) ------------------------------------
-// The keys of the n reads sit in dd[0] on entry (put there by the caller).  keep_map: compute the read -> first-seen
-// position map and leave it in dd[7] (download it too when read_to_distinct != NULL).
+// The keys of the n reads sit in dd[0] (ReadMap::keys) on entry (put there by the caller).  On return dd[] holds the arrays
+// ReadMap names; keep_map: compute the read -> first-seen position map and leave it in dd[7] (download it too when
+// read_to_distinct != NULL).
 static int dedup_core(DevCtx& c, uint32_t n, uint32_t* distinct, uint32_t* counts, uint32_t* read_to_distinct, uint32_t* sorted_pos,
                       bool keep_map, size_t* n_distinct, uint32_t* sorted_distinct = nullptr)
 {
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
+    Buf* dd = c.map.dd;
     const size_t R = n;
     // dd[0] keys, [1] idx, [2] sorted keys, [3] sorted idx, [4] heads, [5] inclusive scan, [6] run key, [7] run first, [8] run start, [9] scratch
-    for (int k = 1; k < 9; k++) if (int e = ensure(c.dd[k], R * 4)) return e;
-    uint32_t *d_k = (uint32_t*)c.dd[0].p, *d_i = (uint32_t*)c.dd[1].p, *d_sk = (uint32_t*)c.dd[2].p, *d_si = (uint32_t*)c.dd[3].p;
-    uint32_t *d_head = (uint32_t*)c.dd[4].p, *d_scan = (uint32_t*)c.dd[5].p, *d_rk = (uint32_t*)c.dd[6].p, *d_rf = (uint32_t*)c.dd[7].p, *d_rs = (uint32_t*)c.dd[8].p;
+    for (int k = 1; k < 9; k++) if (int e = dd[k].ensure(R * 4)) return e;
+    uint32_t *d_k = (uint32_t*)dd[0].p, *d_i = (uint32_t*)dd[1].p, *d_sk = (uint32_t*)dd[2].p, *d_si = (uint32_t*)dd[3].p;
+    uint32_t *d_head = (uint32_t*)dd[4].p, *d_scan = (uint32_t*)dd[5].p, *d_rk = (uint32_t*)dd[6].p, *d_rf = (uint32_t*)dd[7].p, *d_rs = (uint32_t*)dd[8].p;
     size_t tmp1 = 0, tmp2 = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp1, d_k, d_sk, d_i, d_si, (int)n, 0, 32, st));
     CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp2, d_head, d_scan, (int)n, st));
-    if (int e = ensure(c.dd[9], std::max(tmp1, tmp2))) return e;
+    if (int e = dd[9].ensure(std::max(tmp1, tmp2))) return e;
     const int blocks = (int)std::min<size_t>((R + 255) / 256, (size_t)c.sms * 8);
     bdg::iota_kernel<<<blocks, 256, 0, st>>>(d_i, n);
-    CU_TRY(cub::DeviceRadixSort::SortPairs(c.dd[9].p, tmp1, d_k, d_sk, d_i, d_si, (int)n, 0, 32, st));
+    CU_TRY(cub::DeviceRadixSort::SortPairs(dd[9].p, tmp1, d_k, d_sk, d_i, d_si, (int)n, 0, 32, st));
     bdg::dedup_heads_kernel<<<blocks, 256, 0, st>>>(d_sk, n, d_head);
-    CU_TRY(cub::DeviceScan::InclusiveSum(c.dd[9].p, tmp2, d_head, d_scan, (int)n, st));
+    CU_TRY(cub::DeviceScan::InclusiveSum(dd[9].p, tmp2, d_head, d_scan, (int)n, st));
     bdg::dedup_runs_kernel<<<blocks, 256, 0, st>>>(d_sk, d_si, d_head, d_scan, n, d_rk, d_rf, d_rs);
     uint32_t n_runs = 0;
     CU_TRY(cudaMemcpyAsync(&n_runs, d_scan + (n - 1), 4, cudaMemcpyDeviceToHost, st));
@@ -1172,7 +1212,7 @@ static int dedup_core(DevCtx& c, uint32_t n, uint32_t* distinct, uint32_t* count
     g_launches += 3;
     // order the runs by their first read index: reuse keys/idx buffers (d_k := sorted first indices, d_i := order), heads := iota
     bdg::iota_kernel<<<blocks, 256, 0, st>>>(d_head, n_runs);
-    CU_TRY(cub::DeviceRadixSort::SortPairs(c.dd[9].p, tmp1, d_rf, d_k, d_head, d_i, (int)n_runs, 0, 32, st));
+    CU_TRY(cub::DeviceRadixSort::SortPairs(dd[9].p, tmp1, d_rf, d_k, d_head, d_i, (int)n_runs, 0, 32, st));
     // d_sk is free again after dedup_runs: distinct / counts / pos_of_run live in d_sk, d_k, d_head
     uint32_t *d_distinct = d_sk, *d_counts = d_k, *d_pos = d_head;
     bdg::dedup_finish_kernel<<<blocks, 256, 0, st>>>(d_i, d_rk, d_rs, n_runs, n, d_distinct, d_counts, d_pos);
@@ -1203,10 +1243,9 @@ int bdg_dedup_first_seen(const uint32_t* ranks, size_t R, uint32_t* distinct, ui
     if (int rc = need_ctx()) return rc;
     DevCtx& c = g_ctx[0];
     CU_TRY(cudaSetDevice(c.dev));
-    c.map_token = 0;                                  // the workspaces are about to be reused: an older read map dies here
-    if (cudaError_t e = (cudaError_t)c.dd[0].ensure(R * 4))
-        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", R * 4, cudaGetErrorString(e));
-    CU_TRY(cudaMemcpyAsync(c.dd[0].p, ranks, R * 4, cudaMemcpyHostToDevice, c.stream));
+    c.map.drop();
+    if (int e = c.map.keys().ensure(R * 4)) return e;
+    CU_TRY(cudaMemcpyAsync(c.map.keys().p, ranks, R * 4, cudaMemcpyHostToDevice, c.stream));
     return dedup_core(c, (uint32_t)R, distinct, counts, read_to_distinct, sorted_pos, false, n_distinct);
 }
 
@@ -1218,36 +1257,31 @@ static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* val
                             unsigned long long* token)
 {
     cudaStream_t st = c.stream;
-    c.map_token = 0;
-    c.cl_token = 0;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    if (int e = ensure(c.dd[0], R_all * 4)) return e;
+    ReadMap& m = c.map;
+    m.drop();
+    if (int e = m.keys().ensure(R_all * 4)) return e;
     size_t n_reads = R_all;
-    c.map_masked = valid != nullptr;
+    m.masked = valid != nullptr;
     if (valid) {
-        // as[0] all ranks, as[1] valid bytes, as[2] exclusive scan of valid (the index of a valid row among the valid rows), as[3] scratch
-        if (int e = ensure(c.as[0], R_all * 4)) return e;
-        if (int e = ensure(c.as[1], R_all)) return e;
-        if (int e = ensure(c.as[2], (R_all + 1) * 4)) return e;
-        const uint8_t* d_valid = (const uint8_t*)c.as[1].p;
-        uint32_t* d_excl = (uint32_t*)c.as[2].p;
+        // as[0] all ranks (host input), as[1] scan scratch; the valid bytes and their scan stay with the read map
+        if (int e = c.as[0].ensure(R_all * 4)) return e;
+        if (int e = m.valid.ensure(R_all)) return e;
+        if (int e = m.valid_scan.ensure((R_all + 1) * 4)) return e;
+        const uint8_t* d_valid = (const uint8_t*)m.valid.p;
+        uint32_t* d_excl = (uint32_t*)m.valid_scan.p;
         auto flags = thrust::make_transform_iterator(d_valid, bdg::NonZero());
         size_t tmp = 0;
         CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, d_excl, (int)R_all, st));
-        if (int e = ensure(c.as[3], tmp)) return e;
+        if (int e = c.as[1].ensure(tmp)) return e;
         const uint32_t* d_ranks = ranks;
         if (kind == cudaMemcpyHostToDevice) {
             CU_TRY(cudaMemcpyAsync(c.as[0].p, ranks, R_all * 4, kind, st));
             d_ranks = (const uint32_t*)c.as[0].p;
         }
-        CU_TRY(cudaMemcpyAsync(c.as[1].p, valid, R_all, kind, st));
-        CU_TRY(cub::DeviceScan::ExclusiveSum(c.as[3].p, tmp, flags, d_excl, (int)R_all, st));
+        CU_TRY(cudaMemcpyAsync(m.valid.p, valid, R_all, kind, st));
+        CU_TRY(cub::DeviceScan::ExclusiveSum(c.as[1].p, tmp, flags, d_excl, (int)R_all, st));
         const int blocks = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
-        bdg::compact_valid_kernel<<<blocks, 256, 0, st>>>(d_ranks, d_valid, d_excl, (uint32_t)R_all, (uint32_t*)c.dd[0].p);
+        bdg::compact_valid_kernel<<<blocks, 256, 0, st>>>(d_ranks, d_valid, d_excl, (uint32_t)R_all, (uint32_t*)m.keys().p);
         g_launches++;
         uint32_t last_excl = 0;
         uint8_t last_valid = 0;
@@ -1256,16 +1290,13 @@ static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* val
         CU_TRY(cudaStreamSynchronize(st));
         n_reads = (size_t)last_excl + (last_valid ? 1 : 0);
     } else {
-        CU_TRY(cudaMemcpyAsync(c.dd[0].p, ranks, R_all * 4, kind, st));
+        CU_TRY(cudaMemcpyAsync(m.keys().p, ranks, R_all * 4, kind, st));
     }
     *n_valid = n_reads;
-    c.map_rows = R_all; c.map_reads = n_reads; c.map_distinct = 0;
+    m.rows = R_all; m.reads = n_reads; m.distinct = 0;
     if (n_reads == 0) return BDG_OK;
     if (int rc = dedup_core(c, (uint32_t)n_reads, distinct, counts, nullptr, sorted_pos, true, n_distinct, sorted_distinct)) return rc;
-    c.map_distinct = *n_distinct;
-    c.map_token = ++c.map_serial;
-    *token = c.map_token;
-    return BDG_OK;
+    return m.install(*n_distinct, nullptr, nullptr, nullptr, nullptr, st, token);       // dedup_core left the arrays in place
 }
 
 int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos,
@@ -1304,45 +1335,40 @@ int bdg_dev_dedup_reads(const uint32_t* d_ranks, const uint8_t* d_valid, size_t 
 // (kind = cudaMemcpyDeviceToHost, the call waits for the copies) or to device memory on c.dev (stream-ordered, no wait).
 static int dedup_fetch_core(DevCtx& c, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, cudaMemcpyKind kind)
 {
-    const size_t n = c.map_distinct;
-    if (distinct) CU_TRY(cudaMemcpyAsync(distinct, c.dd[2].p, n * 4, kind, c.stream));
-    if (counts) CU_TRY(cudaMemcpyAsync(counts, c.dd[0].p, n * 4, kind, c.stream));
-    if (sorted_pos) CU_TRY(cudaMemcpyAsync(sorted_pos, c.dd[1].p, n * 4, kind, c.stream));
-    if (sorted_distinct) CU_TRY(cudaMemcpyAsync(sorted_distinct, c.dd[6].p, n * 4, kind, c.stream));
+    const ReadMap& m = c.map;
+    const size_t n = m.distinct;
+    if (distinct) CU_TRY(cudaMemcpyAsync(distinct, m.first_seen(), n * 4, kind, c.stream));
+    if (counts) CU_TRY(cudaMemcpyAsync(counts, m.counts(), n * 4, kind, c.stream));
+    if (sorted_pos) CU_TRY(cudaMemcpyAsync(sorted_pos, m.order(), n * 4, kind, c.stream));
+    if (sorted_distinct) CU_TRY(cudaMemcpyAsync(sorted_distinct, m.ascending(), n * 4, kind, c.stream));
     if (kind == cudaMemcpyDeviceToHost) CU_TRY(cudaStreamSynchronize(c.stream));
     return BDG_OK;
 }
 
 int bdg_dedup_fetch(unsigned long long token, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct)
 {
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    CU_TRY(cudaSetDevice(c.dev));
-    return dedup_fetch_core(c, distinct, counts, sorted_pos, sorted_distinct, cudaMemcpyDeviceToHost);
+    DevCtx* c = nullptr;
+    if (int rc = map_ctx(token, &c)) return rc;
+    return dedup_fetch_core(*c, distinct, counts, sorted_pos, sorted_distinct, cudaMemcpyDeviceToHost);
 }
 
 int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t* d_counts, uint32_t* d_sorted_pos, uint32_t* d_sorted_distinct,
                         void* stream)
 {
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = map_ctx(token, &c)) return rc;
     uint32_t* outs[4] = {d_distinct, d_counts, d_sorted_pos, d_sorted_distinct};
     for (uint32_t* p : outs)
-        if (p && c.map_distinct) if (int rc = check_on_first(p, "output")) return rc;
-    CallerOrder order(c, stream);
+        if (p && c->map.distinct) if (int rc = check_on_first(p, "output")) return rc;
+    CallerOrder order(*c, stream);
     if (int rc = order.begin()) return rc;
-    return dedup_fetch_core(c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice);
+    return dedup_fetch_core(*c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice);
 }
 
-static int ensure_buf(Buf& b, size_t bytes);
-
 // ---- the dedup results of P parts (one process per GPU) reduced to the global distinct set (bdg_kernels.cuh, merge_*) ----
-// The work arrays live in mg[] until the end, so that a failed check leaves the token's read map as it was; only then do the
-// global arrays move to where the token's consumers read them (dd[0] counts, dd[1] first-seen -> ascending, dd[2] distinct,
-// dd[6] ascending) and the read map dd[7] is rewritten in place.  as[1] / as[2] (the valid rows) are not touched.
+// The work arrays live in mg[] until the end, so that a failed check leaves the token's read map as it was; only then are the
+// global arrays installed as the read map (counts, order, first-seen, ascending) and its read_pos rewritten in place.  The valid
+// rows are not touched.
 static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first, const size_t* starts,
                             const size_t* sizes, int n_parts, int my_part, size_t* n_distinct, unsigned long long* merged_token)
 {
@@ -1361,10 +1387,10 @@ static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d
     const uint32_t T = (uint32_t)total, n_mine = (uint32_t)sizes[my_part], off_mine = h_offs[my_part];
     // mg[0] part starts, [1] part offsets, [2] keys, [3] entry index, [4] sorted keys, [5] sorted index, [6] counts, [7] first keys,
     // [8] heads / run order, [9] scan / sorted first keys, [10] run key | count | first | own run | position of run | local -> global, [11] scratch
-    if (int e = ensure_buf(c.mg[0], (size_t)n_parts * 8)) return e;
-    if (int e = ensure_buf(c.mg[1], ((size_t)n_parts + 1) * 4 + 4)) return e;
-    for (int k = 2; k < 10; k++) if (int e = ensure_buf(c.mg[k], total * 4)) return e;
-    if (int e = ensure_buf(c.mg[10], (5 * total + std::max<size_t>(n_mine, 1)) * 4)) return e;
+    if (int e = c.mg[0].ensure((size_t)n_parts * 8)) return e;
+    if (int e = c.mg[1].ensure(((size_t)n_parts + 1) * 4 + 4)) return e;
+    for (int k = 2; k < 10; k++) if (int e = c.mg[k].ensure(total * 4)) return e;
+    if (int e = c.mg[10].ensure((5 * total + std::max<size_t>(n_mine, 1)) * 4)) return e;
     uint32_t *d_key = (uint32_t*)c.mg[2].p, *d_idx = (uint32_t*)c.mg[3].p, *d_sk = (uint32_t*)c.mg[4].p, *d_si = (uint32_t*)c.mg[5].p;
     uint32_t *d_cnt = (uint32_t*)c.mg[6].p, *d_fst = (uint32_t*)c.mg[7].p, *d_head = (uint32_t*)c.mg[8].p, *d_scan = (uint32_t*)c.mg[9].p;
     uint32_t *d_rk = (uint32_t*)c.mg[10].p, *d_rc = d_rk + total, *d_rf = d_rc + total, *d_mrun = d_rf + total, *d_prun = d_mrun + total,
@@ -1373,13 +1399,13 @@ static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d
     size_t tmp1 = 0, tmp2 = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
     CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp2, d_head, d_scan, (int)T, st));
-    if (int e = ensure_buf(c.mg[11], std::max(tmp1, tmp2))) return e;
+    if (int e = c.mg[11].ensure(std::max(tmp1, tmp2))) return e;
     CU_TRY(cudaMemcpyAsync(c.mg[0].p, h_starts.data(), (size_t)n_parts * 8, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemcpyAsync(c.mg[1].p, h_offs.data(), ((size_t)n_parts + 1) * 4, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemsetAsync(d_bad, 0, 4, st));
     const int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)c.sms * 8);
     bdg::merge_gather_kernel<<<blocks, 256, 0, st>>>(d_keys, d_counts, d_first, (const uint64_t*)c.mg[0].p, (const uint32_t*)c.mg[1].p, (uint32_t)n_parts,
-                                                     T, (uint32_t)my_part, (const uint32_t*)c.dd[6].p, d_key, d_idx, d_cnt, d_fst, d_bad);
+                                                     T, (uint32_t)my_part, c.map.ascending(), d_key, d_idx, d_cnt, d_fst, d_bad);
     CU_TRY(cub::DeviceRadixSort::SortPairs(c.mg[11].p, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
     bdg::dedup_heads_kernel<<<blocks, 256, 0, st>>>(d_sk, T, d_head);
     CU_TRY(cub::DeviceScan::InclusiveSum(c.mg[11].p, tmp2, d_head, d_scan, (int)T, st));
@@ -1400,24 +1426,15 @@ static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d
     g_launches += 2;
     if (n_mine) {
         const int lb = (int)std::min<size_t>((n_mine + 255) / 256, (size_t)c.sms * 8);
-        const int rb = (int)std::min<size_t>((c.map_reads + 255) / 256, (size_t)c.sms * 8);
-        bdg::merge_local_kernel<<<lb, 256, 0, st>>>((const uint32_t*)c.dd[1].p, d_mrun, d_prun, n_mine, d_loc);
-        bdg::merge_remap_kernel<<<rb, 256, 0, st>>>((uint32_t*)c.dd[7].p, (uint32_t)c.map_reads, d_loc);
+        const int rb = (int)std::min<size_t>((c.map.reads + 255) / 256, (size_t)c.sms * 8);
+        bdg::merge_local_kernel<<<lb, 256, 0, st>>>(c.map.order(), d_mrun, d_prun, n_mine, d_loc);
+        bdg::merge_remap_kernel<<<rb, 256, 0, st>>>(c.map.read_pos(), (uint32_t)c.map.reads, d_loc);
         g_launches += 2;
     }
     CU_TRY(cudaGetLastError());
-    // growing a dd[] buffer frees its old memory: the kernels above that read dd[1] / dd[6] must have finished
-    CU_TRY(cudaStreamSynchronize(st));
-    for (int k : {0, 1, 2, 6}) if (int e = ensure_buf(c.dd[k], (size_t)n_runs * 4)) return e;
-    CU_TRY(cudaMemcpyAsync(c.dd[0].p, d_cnt, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(c.dd[1].p, d_head, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));   // order[pos] = run = ascending position
-    CU_TRY(cudaMemcpyAsync(c.dd[2].p, d_key, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));
-    CU_TRY(cudaMemcpyAsync(c.dd[6].p, d_rk, (size_t)n_runs * 4, cudaMemcpyDeviceToDevice, st));    // runs are numbered in key order
-    c.map_distinct = n_runs;
-    c.cl_token = 0;
-    c.map_token = ++c.map_serial;
+    // order[pos] = run = ascending position; runs are numbered in key order
+    if (int rc = c.map.install(n_runs, d_cnt, d_head, d_key, d_rk, st, merged_token)) return rc;
     *n_distinct = n_runs;
-    *merged_token = c.map_token;
     return BDG_OK;
 }
 
@@ -1428,15 +1445,20 @@ int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const 
     *n_distinct = 0; *merged_token = 0;
     if (n_parts < 1 || my_part < 0 || my_part >= n_parts || !starts || !sizes) return fail(BDG_ERR_ARG, "need 0 <= my_part < n_parts and the parts' starts / sizes");
     if (!d_keys || !d_counts || !d_first) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
     // token 0: this part has no valid read (the dedup call issued no token); its list must then be empty
-    if (token != 0 && token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    if (sizes[my_part] != (token ? c.map_distinct : 0))
-        return fail(BDG_ERR_ARG, "part %d has %zu barcodes, the read map of the token %zu", my_part, sizes[my_part], token ? c.map_distinct : (size_t)0);
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* cp = nullptr;
+    if (token != 0) {
+        if (int rc = map_ctx(token, &cp)) return rc;
+    } else {
+        if (int rc = need_ctx()) return rc;
+        cp = &g_ctx[0];
+        CU_TRY(cudaSetDevice(cp->dev));
+    }
+    DevCtx& c = *cp;
+    if (sizes[my_part] != (token ? c.map.distinct : 0))
+        return fail(BDG_ERR_ARG, "part %d has %zu barcodes, the read map of the token %zu", my_part, sizes[my_part], token ? c.map.distinct : (size_t)0);
     for (const uint32_t* p : {d_keys, d_counts, d_first}) if (int rc = check_on_first(p, "merge input")) return rc;
-    if (token == 0) { c.map_token = 0; c.map_rows = 0; c.map_reads = 0; c.map_masked = false; }
+    if (token == 0) { c.map.drop(); c.map.rows = 0; c.map.reads = 0; c.map.masked = false; }
     CallerOrder order(c, stream);
     if (int rc = order.begin()) return rc;
     return dedup_merge_core(c, d_keys, d_counts, d_first, starts, sizes, n_parts, my_part, n_distinct, merged_token);
@@ -1449,7 +1471,7 @@ int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const 
 // barcode: the rows added before the batch + the barcode's first-seen position in the batch, so that the keys sort in the
 // first-seen order of the concatenated batches.  add merges a batch into the other half of the double buffer and swaps; a
 // refused batch leaves the set as it was.  finish sorts the set by first-sighting key and installs the read-map arrays of a
-// dedup call without rows (dd[0] counts, dd[1] first-seen -> ascending, dd[2] distinct, dd[6] ascending).
+// dedup call without rows (counts, first-seen -> ascending, distinct in first-seen order, ascending).
 struct bdg_tally {
     int dev = -1;                                   // the first claimed device when the tally was created
     Buf key[2], cnt[2], fst[2];                     // the running set and the half the next batch is merged into
@@ -1481,25 +1503,25 @@ int tally_add_core(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t
     size_t nb = 0, nv = 0;
     unsigned long long tok = 0;
     const int rc = dedup_reads_core(c, ranks, valid, R, kind, nullptr, nullptr, nullptr, nullptr, &nb, &nv, &tok);
-    c.map_token = 0;                                // the batch's read map is not handed out
+    c.map.drop();                                   // the batch's read map is not handed out
     if (rc) return rc;
     if (n_valid) *n_valid = nv;
     if (nv == 0) { h->rows += R; return BDG_OK; }
     cudaStream_t st = c.stream;
     const int nx = h->cur ^ 1;
     const size_t na = h->n, M = na + nb;            // na < 2^31 and nb < 2^31: M < 2^32
-    for (Buf* b : {&h->m_key, &h->m_head, &h->m_scan, &h->key[nx]}) if (int e = ensure_buf(*b, M * 4)) return e;
-    for (Buf* b : {&h->m_cnt, &h->m_fst, &h->cnt[nx], &h->fst[nx]}) if (int e = ensure_buf(*b, M * 8)) return e;
-    if (int e = ensure_buf(h->flag, 16)) return e;
+    for (Buf* b : {&h->m_key, &h->m_head, &h->m_scan, &h->key[nx]}) if (int e = b->ensure(M * 4)) return e;
+    for (Buf* b : {&h->m_cnt, &h->m_fst, &h->cnt[nx], &h->fst[nx]}) if (int e = b->ensure(M * 8)) return e;
+    if (int e = h->flag.ensure(16)) return e;
     size_t tmp = 0;
     CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
-    if (int e = ensure_buf(h->scratch, tmp)) return e;
+    if (int e = h->scratch.ensure(tmp)) return e;
     unsigned int* d_flag = (unsigned int*)h->flag.p;
     CU_TRY(cudaMemsetAsync(d_flag, 0, 4, st));
     bdg::tally_merge_kernel<<<(unsigned)((M + bdg::TALLY_TILE - 1) / bdg::TALLY_TILE), bdg::NT, 0, st>>>(
         (const uint32_t*)h->key[h->cur].p, (const unsigned long long*)h->cnt[h->cur].p, (const unsigned long long*)h->fst[h->cur].p, na,
-        (const uint32_t*)c.dd[6].p /* batch runs ascending */, (const uint32_t*)c.dd[0].p /* counts, first-seen order */,
-        (const uint32_t*)c.dd[4].p /* run -> first-seen position */, nb, h->rows, (uint32_t*)h->m_key.p, (unsigned long long*)h->m_cnt.p,
+        c.map.ascending() /* batch runs ascending */, c.map.counts() /* counts, first-seen order */,
+        c.map.run_pos() /* run -> first-seen position */, nb, h->rows, (uint32_t*)h->m_key.p, (unsigned long long*)h->m_cnt.p,
         (unsigned long long*)h->m_fst.p, (uint32_t*)h->m_head.p);
     CU_TRY(cub::DeviceScan::InclusiveSum(h->scratch.p, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
     const int blocks = (int)std::min<size_t>((M + 255) / 256, (size_t)c.sms * 8);
@@ -1537,28 +1559,26 @@ int tally_finish_core(DevCtx& c, bdg_tally* h, size_t* n_distinct, size_t* n_val
     size_t tmp = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp, (const unsigned long long*)h->fst[h->cur].p, (unsigned long long*)h->m_fst.p,
                                            (const uint32_t*)h->m_key.p, (uint32_t*)h->m_head.p, (int)n, 0, end_bit, st));
-    if (int e = ensure_buf(h->scratch, tmp)) return e;
+    if (int e = h->scratch.ensure(tmp)) return e;
     const int blocks = (int)std::min<size_t>((n + 255) / 256, (size_t)c.sms * 8);
     bdg::iota_kernel<<<blocks, 256, 0, st>>>((uint32_t*)h->m_key.p, n);
     CU_TRY(cub::DeviceRadixSort::SortPairs(h->scratch.p, tmp, (const unsigned long long*)h->fst[h->cur].p, (unsigned long long*)h->m_fst.p,
                                            (const uint32_t*)h->m_key.p, (uint32_t*)h->m_head.p, (int)n, 0, end_bit, st));
-    // the read map of the token named last is about to be overwritten
-    c.map_token = 0;
-    c.cl_token = 0;
-    // growing a dd[] buffer frees its old memory: whatever is queued on the stream may still read it
-    CU_TRY(cudaStreamSynchronize(st));
-    for (int k : {0, 1, 2, 6}) if (int e = ensure_buf(c.dd[k], (size_t)n * 4)) return e;
+    g_launches++;
+    // the ascending array is the set itself; first-seen, counts and order are written in place by the kernel below
+    c.map.rows = 0; c.map.reads = 0; c.map.masked = false;
+    unsigned long long tok = 0;
+    if (int rc = c.map.install(n, nullptr, nullptr, nullptr, (const uint32_t*)h->key[h->cur].p, st, &tok)) return rc;
     bdg::tally_finish_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)h->m_head.p, (const uint32_t*)h->key[h->cur].p,
-                                                     (const unsigned long long*)h->cnt[h->cur].p, n, (uint32_t*)c.dd[2].p,
-                                                     (uint32_t*)c.dd[0].p, (uint32_t*)c.dd[1].p);
-    g_launches += 2;
-    CU_TRY(cudaGetLastError());
-    CU_TRY(cudaMemcpyAsync(c.dd[6].p, h->key[h->cur].p, (size_t)n * 4, cudaMemcpyDeviceToDevice, st));
-    c.map_rows = 0; c.map_reads = 0; c.map_masked = false;
-    c.map_distinct = n;
-    c.map_token = ++c.map_serial;
+                                                     (const unsigned long long*)h->cnt[h->cur].p, n, c.map.first_seen(), c.map.counts(),
+                                                     c.map.order());
+    g_launches++;
+    if (cudaError_t e = cudaGetLastError()) {
+        c.map.drop();
+        return fail(BDG_ERR_CUDA, "tally finish launch failed: %s", cudaGetErrorString(e));
+    }
     *n_distinct = n;
-    *token = c.map_token;
+    *token = tok;
     return BDG_OK;
 }
 
@@ -1583,12 +1603,9 @@ void bdg_tally_free(bdg_tally* h)
     if (!h) return;
     int prev = -1;
     cudaGetDevice(&prev);
-    if (cudaSetDevice(h->dev) == cudaSuccess) {
-        for (int k = 0; k < 2; k++) { h->key[k].release(); h->cnt[k].release(); h->fst[k].release(); }
-        for (Buf* b : {&h->m_key, &h->m_cnt, &h->m_fst, &h->m_head, &h->m_scan, &h->scratch, &h->flag}) b->release();
-    }
-    if (prev >= 0) cudaSetDevice(prev);
+    cudaSetDevice(h->dev);                          // the buffers are freed on their device
     delete h;
+    if (prev >= 0) cudaSetDevice(prev);
 }
 
 int bdg_tally_add(bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, size_t* n_valid)
@@ -1646,19 +1663,14 @@ int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsi
 static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_wl, bool wl_on_device, size_t W, uint32_t* top_ranks,
                               uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
 {
-    const size_t N = c.map_distinct;
+    const size_t N = c.map.distinct;
     const size_t first = std::min(n_cells, N);
     if (first == 0) return fail(BDG_ERR_ARG, "mean requires at least one data point");
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    const uint32_t* d_distinct = (const uint32_t*)c.dd[2].p;
-    const uint32_t* d_counts = (const uint32_t*)c.dd[0].p;
+    const uint32_t* d_distinct = c.map.first_seen();
+    const uint32_t* d_counts = c.map.counts();
     // ce[0] selected positions, [1] keys, [2] sorted keys, [3] sorted positions, [4] top ranks, [5] top counts, [6] hits, [7] scalars + cub scratch
-    if (int e = ensure(c.ce[7], 64)) return e;
+    if (int e = c.ce[7].ensure(64)) return e;
     unsigned long long* d_sum = (unsigned long long*)c.ce[7].p;
     uint32_t* d_nsel = (uint32_t*)((char*)c.ce[7].p + 8);
     CU_TRY(cudaMemsetAsync(d_sum, 0, 16, st));
@@ -1670,12 +1682,12 @@ static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_
     const double cut = std::max(((double)sum / (double)first) / 5.0, 5.0);
     *cutoff = cut;
     const uint32_t thr = (uint32_t)std::floor(cut);          // counts are integers: count > cutoff <=> count > floor(cutoff)
-    if (int e = ensure(c.ce[0], N * 4)) return e;
+    if (int e = c.ce[0].ensure(N * 4)) return e;
     thrust::counting_iterator<uint32_t> all(0);
     bdg::CountAbove pred{d_counts, thr};
     size_t tmp = 0;
     CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, pred, st));
-    if (int e = ensure(c.ce[8], tmp)) return e;
+    if (int e = c.ce[8].ensure(tmp)) return e;
     CU_TRY(cub::DeviceSelect::If(c.ce[8].p, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, pred, st));
     uint32_t nsel = 0;
     CU_TRY(cudaMemcpyAsync(&nsel, d_nsel, 4, cudaMemcpyDeviceToHost, st));
@@ -1684,13 +1696,13 @@ static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_
     if (nsel == 0) return BDG_OK;
     if (nsel > cap) return fail(BDG_ERR_CAPACITY, "%u barcodes above the cutoff but room for %zu", nsel, cap);
     if (!top_ranks || !top_counts) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    for (int k = 1; k <= 5; k++) if (int e = ensure(c.ce[k], (size_t)nsel * 4)) return e;
-    if (int e = ensure(c.ce[6], nsel)) return e;
+    for (int k = 1; k <= 5; k++) if (int e = c.ce[k].ensure((size_t)nsel * 4)) return e;
+    if (int e = c.ce[6].ensure(nsel)) return e;
     const int nb = (int)std::min<size_t>(((size_t)nsel + 255) / 256, (size_t)c.sms * 4);
     bdg::centres_keys_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.ce[0].p, d_counts, nsel, (uint32_t*)c.ce[1].p);
     size_t tmp2 = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp2, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[3].p, (int)nsel, 0, 32, st));
-    if (int e = ensure(c.ce[8], tmp2)) return e;
+    if (int e = c.ce[8].ensure(tmp2)) return e;
     CU_TRY(cub::DeviceRadixSort::SortPairs(c.ce[8].p, tmp2, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[3].p, (int)nsel, 0, 32, st));
     bdg::centres_gather_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.ce[3].p, d_distinct, d_counts, nsel, (uint32_t*)c.ce[4].p, (uint32_t*)c.ce[5].p);
     g_launches += 2;
@@ -1698,11 +1710,11 @@ static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_
     if (top_hits) {
         if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
         if (W && !sorted_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
-        if (int e = ensure(c.io[3], 8)) return e;
+        if (int e = c.io[3].ensure(8)) return e;
         unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
         const uint32_t* d_wl = sorted_wl;
         if (!wl_on_device) {
-            if (int e = ensure(c.io[0], std::max<size_t>(W, 1) * 4)) return e;
+            if (int e = c.io[0].ensure(std::max<size_t>(W, 1) * 4)) return e;
             CU_TRY(cudaMemcpyAsync(c.io[0].p, sorted_wl, W * 4, cudaMemcpyHostToDevice, st));
             d_wl = (const uint32_t*)c.io[0].p;
         }
@@ -1732,11 +1744,9 @@ int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* 
 {
     if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
     *n_above = 0; *cutoff = 0.0;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    CU_TRY(cudaSetDevice(c.dev));
-    return centres_above_core(c, n_cells, sorted_wl, false, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
+    DevCtx* c = nullptr;
+    if (int rc = map_ctx(token, &c)) return rc;
+    return centres_above_core(*c, n_cells, sorted_wl, false, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
 }
 
 int bdg_dev_centres_above(unsigned long long token, size_t n_cells, const uint32_t* d_sorted_wl, size_t W, uint32_t* top_ranks,
@@ -1744,14 +1754,12 @@ int bdg_dev_centres_above(unsigned long long token, size_t n_cells, const uint32
 {
     if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
     *n_above = 0; *cutoff = 0.0;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = map_ctx(token, &c)) return rc;
     if (top_hits && W) if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
-    CallerOrder order(c, stream);
+    CallerOrder order(*c, stream);
     if (int rc = order.begin()) return rc;
-    return centres_above_core(c, n_cells, d_sorted_wl, true, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
+    return centres_above_core(*c, n_cells, d_sorted_wl, true, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
 }
 
 // The stretch of `bc_by_counts` right behind the head bdg_centres_above returns (barcode_graph.py:273-276 runs into it when too few
@@ -1763,28 +1771,22 @@ int bdg_centres_rest(unsigned long long token, double cutoff, size_t need, uint3
     *n_out = 0;
     if (need == 0) return BDG_OK;
     if (!out_ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    const size_t N = c.map_distinct;
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    const size_t N = c.map.distinct;
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    const uint32_t* d_distinct = (const uint32_t*)c.dd[2].p;
-    const uint32_t* d_counts = (const uint32_t*)c.dd[0].p;
-    if (int e = ensure(c.ce[0], N * 4)) return e;
-    if (int e = ensure(c.ce[4], std::min(need, N) * 4)) return e;
-    if (int e = ensure(c.ce[5], std::min(need, N) * 4)) return e;
-    if (int e = ensure(c.ce[7], 64)) return e;
+    const uint32_t* d_distinct = c.map.first_seen();
+    const uint32_t* d_counts = c.map.counts();
+    if (int e = c.ce[0].ensure(N * 4)) return e;
+    if (int e = c.ce[4].ensure(std::min(need, N) * 4)) return e;
+    if (int e = c.ce[5].ensure(std::min(need, N) * 4)) return e;
+    if (int e = c.ce[7].ensure(64)) return e;
     uint32_t* d_nsel = (uint32_t*)((char*)c.ce[7].p + 8);
     thrust::counting_iterator<uint32_t> all(0);
     size_t tmp = 0;
     CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, bdg::CountIs{d_counts, 0u}, st));
-    if (int e = ensure(c.ce[8], tmp)) return e;
+    if (int e = c.ce[8].ensure(tmp)) return e;
     size_t got = 0;
     for (long long v = (long long)std::floor(cutoff); v >= 1 && got < need; v--) {
         CU_TRY(cub::DeviceSelect::If(c.ce[8].p, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, bdg::CountIs{d_counts, (uint32_t)v}, st));
@@ -1804,42 +1806,36 @@ int bdg_centres_rest(unsigned long long token, double cutoff, size_t need, uint3
     return BDG_OK;
 }
 
-static int ensure_buf(Buf& b, size_t bytes)
+// c: the context map_ctx returned for the token
+static int check_assign_args(const DevCtx& c, bool resident, size_t N, size_t R_all)
 {
-    if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-    return BDG_OK;
-}
-
-static int check_assign_args(DevCtx& c, unsigned long long token, bool resident, size_t N, size_t R_all)
-{
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    if (N != c.map_distinct || R_all != c.map_rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
-    if (resident && N && c.cl_token != token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
+    if (N != c.map.distinct || R_all != c.map.rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
+    if (resident && N && c.map.cl_token != c.map.token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
     return BDG_OK;
 }
 
 // The per-read gather on c.stream: d_ci (device, on c.dev) is the centre index per node, NULL for the resident clustering result;
-// the 5-byte result goes to d_out / d_oh (device, R_all rows) and the number of rows with a centre to the counter in as[7].
+// the 5-byte result goes to d_out / d_oh (device, R_all rows) and the number of rows with a centre to the counter in as[5].
 static int assign_reads32_core(DevCtx& c, const int32_t* d_ci, size_t N, uint32_t* d_out, uint8_t* d_oh, size_t R_all)
 {
     cudaStream_t st = c.stream;
-    // as[5] centre value + has byte per distinct barcode, as[7] counter
-    if (int e = ensure_buf(c.as[5], std::max<size_t>(N, 1) * 5)) return e;
-    if (int e = ensure_buf(c.as[7], 8)) return e;
-    if (!d_ci) d_ci = (const int32_t*)c.cl[1].p;
-    CU_TRY(cudaMemsetAsync(c.as[7].p, 0, 8, st));
-    uint32_t* d_cv = (uint32_t*)c.as[5].p;
-    uint8_t* d_ch = (uint8_t*)c.as[5].p + std::max<size_t>(N, 1) * 4;
+    const ReadMap& m = c.map;
+    // as[3] centre value + has byte per distinct barcode, as[5] counter
+    if (int e = c.as[3].ensure(std::max<size_t>(N, 1) * 5)) return e;
+    if (int e = c.as[5].ensure(8)) return e;
+    if (!d_ci) d_ci = (const int32_t*)m.centre.p;
+    CU_TRY(cudaMemsetAsync(c.as[5].p, 0, 8, st));
+    uint32_t* d_cv = (uint32_t*)c.as[3].p;
+    uint8_t* d_ch = (uint8_t*)c.as[3].p + std::max<size_t>(N, 1) * 4;
     if (N) {
         const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
-        bdg::centre_of_distinct32_kernel<<<nb, 256, 0, st>>>(d_ci, (const uint32_t*)c.dd[1].p /* first-seen -> node */,
-                                                             (const uint32_t*)c.dd[6].p /* node -> barcode */, (uint32_t)N, d_cv, d_ch);
+        bdg::centre_of_distinct32_kernel<<<nb, 256, 0, st>>>(d_ci, m.order() /* first-seen -> node */, m.ascending() /* node -> barcode */,
+                                                             (uint32_t)N, d_cv, d_ch);
     }
     const int rb = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
-    bdg::assign_reads32_kernel<<<rb, 256, 0, st>>>(d_cv, d_ch, (const uint32_t*)c.dd[7].p, c.map_masked ? (const uint8_t*)c.as[1].p : nullptr,
-                                                   c.map_masked ? (const uint32_t*)c.as[2].p : nullptr, (uint32_t)R_all, d_out, d_oh,
-                                                   (unsigned long long*)c.as[7].p);
+    bdg::assign_reads32_kernel<<<rb, 256, 0, st>>>(d_cv, d_ch, m.read_pos(), m.masked ? (const uint8_t*)m.valid.p : nullptr,
+                                                   m.masked ? (const uint32_t*)m.valid_scan.p : nullptr, (uint32_t)R_all, d_out, d_oh,
+                                                   (unsigned long long*)c.as[5].p);
     g_launches += 2;
     CU_TRY(cudaGetLastError());
     return BDG_OK;
@@ -1853,26 +1849,26 @@ int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size
     if (n_assigned) *n_assigned = 0;
     if (R_all == 0) return BDG_OK;
     if (!centre_per_row || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (int rc = check_assign_args(c, token, !centre_idx, N, R_all)) return rc;
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    if (int rc = check_assign_args(c, !centre_idx, N, R_all)) return rc;
     cudaStream_t st = c.stream;
-    // as[4] centre index per node (upload), as[6] result per row
-    if (int e = ensure_buf(c.as[6], R_all * 5)) return e;
+    // as[2] centre index per node (upload), as[4] result per row
+    if (int e = c.as[4].ensure(R_all * 5)) return e;
     const int32_t* d_ci = nullptr;
     if (centre_idx) {
-        if (int e = ensure_buf(c.as[4], std::max<size_t>(N, 1) * 4)) return e;
-        CU_TRY(cudaMemcpyAsync(c.as[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-        d_ci = (const int32_t*)c.as[4].p;
+        if (int e = c.as[2].ensure(std::max<size_t>(N, 1) * 4)) return e;
+        CU_TRY(cudaMemcpyAsync(c.as[2].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+        d_ci = (const int32_t*)c.as[2].p;
     }
-    uint32_t* d_out = (uint32_t*)c.as[6].p;
-    uint8_t* d_oh = (uint8_t*)c.as[6].p + R_all * 4;
+    uint32_t* d_out = (uint32_t*)c.as[4].p;
+    uint8_t* d_oh = (uint8_t*)c.as[4].p + R_all * 4;
     if (int rc = assign_reads32_core(c, d_ci, N, d_out, d_oh, R_all)) return rc;
     unsigned long long cnt = 0;
     CU_TRY(cudaMemcpyAsync(centre_per_row, d_out, R_all * 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(has_centre, d_oh, R_all, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(&cnt, c.as[7].p, 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     if (n_assigned) *n_assigned = (size_t)cnt;
     return BDG_OK;
@@ -1884,10 +1880,10 @@ int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx
     if (n_assigned) *n_assigned = 0;
     if (R_all == 0) return BDG_OK;
     if (!d_centre_per_row || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (int rc = check_assign_args(c, token, !d_centre_idx, N, R_all)) return rc;
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    if (int rc = check_assign_args(c, !d_centre_idx, N, R_all)) return rc;
     if (d_centre_idx && N) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
     if (int rc = check_on_first(d_centre_per_row, "centre_per_row")) return rc;
     if (int rc = check_on_first(d_has_centre, "has_centre")) return rc;
@@ -1896,7 +1892,7 @@ int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx
     if (int rc = assign_reads32_core(c, N ? d_centre_idx : nullptr, N, d_centre_per_row, d_has_centre, R_all)) return rc;
     if (n_assigned) {
         unsigned long long cnt = 0;
-        CU_TRY(cudaMemcpyAsync(&cnt, c.as[7].p, 8, cudaMemcpyDeviceToHost, c.stream));
+        CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, c.stream));
         CU_TRY(cudaStreamSynchronize(c.stream));
         *n_assigned = (size_t)cnt;
     }
@@ -1904,27 +1900,27 @@ int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx
 }
 
 // The per-read gather for rows outside any read map: every valid row's barcode is looked up among the token's nodes (the
-// ascending array dd[6]); d_ci as for assign_reads32_core.  Counters (assigned, missing) go to lk[0].
+// ascending array); d_ci as for assign_reads32_core.  Counters (assigned, missing) go to lk[0].
 static int assign_lookup32_core(DevCtx& c, const int32_t* d_ci, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R,
                                 uint32_t* d_out, uint8_t* d_oh)
 {
     cudaStream_t st = c.stream;
-    if (int e = ensure_buf(c.lk[0], 16)) return e;
-    if (!d_ci) d_ci = (const int32_t*)c.cl[1].p;
+    if (int e = c.lk[0].ensure(16)) return e;
+    if (!d_ci) d_ci = (const int32_t*)c.map.centre.p;
     CU_TRY(cudaMemsetAsync(c.lk[0].p, 0, 16, st));
     const int rb = (int)std::min<size_t>((R + bdg::NT - 1) / bdg::NT, (size_t)c.sms * 8);
-    bdg::lookup_assign32_kernel<<<rb, bdg::NT, 0, st>>>((const uint32_t*)c.dd[6].p, (uint32_t)N, d_ci, d_ranks, d_valid, R, d_out, d_oh,
+    bdg::lookup_assign32_kernel<<<rb, bdg::NT, 0, st>>>(c.map.ascending(), (uint32_t)N, d_ci, d_ranks, d_valid, R, d_out, d_oh,
                                                          (unsigned long long*)c.lk[0].p);
     g_launches++;
     CU_TRY(cudaGetLastError());
     return BDG_OK;
 }
 
-static int check_lookup_args(DevCtx& c, unsigned long long token, bool resident, size_t N)
+// c: the context map_ctx returned for the token
+static int check_lookup_args(const DevCtx& c, bool resident, size_t N)
 {
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    if (N != c.map_distinct) return fail(BDG_ERR_ARG, "N does not match the read map the token names");
-    if (resident && c.cl_token != token) return fail(BDG_ERR_ARG, "no clustering result of this read map is resident on the device (bdg_cluster_resident)");
+    if (N != c.map.distinct) return fail(BDG_ERR_ARG, "N does not match the read map the token names");
+    if (resident && c.map.cl_token != c.map.token) return fail(BDG_ERR_ARG, "no clustering result of this read map is resident on the device (bdg_cluster_resident)");
     return BDG_OK;
 }
 
@@ -1943,24 +1939,24 @@ int bdg_assign_lookup32(unsigned long long token, const int32_t* centre_idx, siz
 {
     if (n_assigned) *n_assigned = 0;
     if (n_missing) *n_missing = 0;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (int rc = check_lookup_args(c, token, !centre_idx, N)) return rc;
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    if (int rc = check_lookup_args(c, !centre_idx, N)) return rc;
     if (R == 0) return BDG_OK;
     if (!ranks || !centre || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    CU_TRY(cudaSetDevice(c.dev));
     cudaStream_t st = c.stream;
     // lk[1] ranks, lk[2] valid bytes, lk[3] result (R x 5 bytes), lk[4] centre index per node
-    if (int e = ensure_buf(c.lk[1], R * 4)) return e;
-    if (int e = ensure_buf(c.lk[3], R * 5)) return e;
+    if (int e = c.lk[1].ensure(R * 4)) return e;
+    if (int e = c.lk[3].ensure(R * 5)) return e;
     CU_TRY(cudaMemcpyAsync(c.lk[1].p, ranks, R * 4, cudaMemcpyHostToDevice, st));
     if (valid) {
-        if (int e = ensure_buf(c.lk[2], R)) return e;
+        if (int e = c.lk[2].ensure(R)) return e;
         CU_TRY(cudaMemcpyAsync(c.lk[2].p, valid, R, cudaMemcpyHostToDevice, st));
     }
     const int32_t* d_ci = nullptr;
     if (centre_idx) {
-        if (int e = ensure_buf(c.lk[4], N * 4)) return e;
+        if (int e = c.lk[4].ensure(N * 4)) return e;
         CU_TRY(cudaMemcpyAsync(c.lk[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
         d_ci = (const int32_t*)c.lk[4].p;
     }
@@ -1977,12 +1973,12 @@ int bdg_dev_assign_lookup32(unsigned long long token, const int32_t* d_centre_id
 {
     if (n_assigned) *n_assigned = 0;
     if (n_missing) *n_missing = 0;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (int rc = check_lookup_args(c, token, !d_centre_idx, N)) return rc;
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    if (int rc = check_lookup_args(c, !d_centre_idx, N)) return rc;
     if (R == 0) return BDG_OK;
     if (!d_ranks || !d_centre || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    CU_TRY(cudaSetDevice(c.dev));
     if (d_centre_idx) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
     if (int rc = check_on_first(d_ranks, "ranks")) return rc;
     if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
@@ -2000,38 +1996,33 @@ int bdg_assign_reads(unsigned long long token, const int32_t* centre_idx, size_t
     if (n_assigned) *n_assigned = 0;
     if (R_all == 0) return BDG_OK;
     if (!centre_per_row || (N && !centre_idx)) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    if (token == 0 || token != c.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
-    if (N != c.map_distinct || R_all != c.map_rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* cp = nullptr;
+    if (int rc = map_ctx(token, &cp)) return rc;
+    DevCtx& c = *cp;
+    if (int rc = check_assign_args(c, false, N, R_all)) return rc;
+    const ReadMap& m = c.map;
     cudaStream_t st = c.stream;
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
-    // as[4] centre index per node (upload), as[5] centre value per distinct barcode in first-seen order, as[6] result per row, as[7] counter
-    if (int e = ensure(c.as[4], std::max<size_t>(N, 1) * 4)) return e;
-    if (int e = ensure(c.as[5], std::max<size_t>(N, 1) * 8)) return e;
-    if (int e = ensure(c.as[6], R_all * 8)) return e;
-    if (int e = ensure(c.as[7], 8)) return e;
-    CU_TRY(cudaMemcpyAsync(c.as[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemsetAsync(c.as[7].p, 0, 8, st));
+    // as[2] centre index per node (upload), as[3] centre value per distinct barcode in first-seen order, as[4] result per row, as[5] counter
+    if (int e = c.as[2].ensure(std::max<size_t>(N, 1) * 4)) return e;
+    if (int e = c.as[3].ensure(std::max<size_t>(N, 1) * 8)) return e;
+    if (int e = c.as[4].ensure(R_all * 8)) return e;
+    if (int e = c.as[5].ensure(8)) return e;
+    CU_TRY(cudaMemcpyAsync(c.as[2].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemsetAsync(c.as[5].p, 0, 8, st));
     if (N) {
         const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
-        bdg::centre_of_distinct_kernel<<<nb, 256, 0, st>>>((const int32_t*)c.as[4].p, (const uint32_t*)c.dd[1].p /* first-seen -> node */,
-                                                           (const uint32_t*)c.dd[6].p /* node -> barcode */, (uint32_t)N, (uint64_t*)c.as[5].p);
+        bdg::centre_of_distinct_kernel<<<nb, 256, 0, st>>>((const int32_t*)c.as[2].p, m.order() /* first-seen -> node */,
+                                                           m.ascending() /* node -> barcode */, (uint32_t)N, (uint64_t*)c.as[3].p);
     }
     const int rb = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
-    bdg::assign_reads_kernel<<<rb, 256, 0, st>>>((const uint64_t*)c.as[5].p, (const uint32_t*)c.dd[7].p, c.map_masked ? (const uint8_t*)c.as[1].p : nullptr,
-                                                 c.map_masked ? (const uint32_t*)c.as[2].p : nullptr, (uint32_t)R_all, (uint64_t*)c.as[6].p,
-                                                 (unsigned long long*)c.as[7].p);
+    bdg::assign_reads_kernel<<<rb, 256, 0, st>>>((const uint64_t*)c.as[3].p, m.read_pos(), m.masked ? (const uint8_t*)m.valid.p : nullptr,
+                                                 m.masked ? (const uint32_t*)m.valid_scan.p : nullptr, (uint32_t)R_all, (uint64_t*)c.as[4].p,
+                                                 (unsigned long long*)c.as[5].p);
     g_launches += 2;
     CU_TRY(cudaGetLastError());
     unsigned long long cnt = 0;
-    CU_TRY(cudaMemcpyAsync(centre_per_row, c.as[6].p, R_all * 8, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(&cnt, c.as[7].p, 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(centre_per_row, c.as[4].p, R_all * 8, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     if (n_assigned) *n_assigned = (size_t)cnt;
     return BDG_OK;
@@ -2046,8 +2037,7 @@ int bdg_pack16(const char* seqs, size_t R, uint32_t* out, uint8_t* valid)
     CU_TRY(cudaSetDevice(c.dev));
     const size_t sizes[3] = {R * 16, R * 4, R};               // grow-only workspaces: letters, ranks, validity
     for (int k = 0; k < 3; k++)
-        if (cudaError_t e = (cudaError_t)c.io[k].ensure(sizes[k]))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", sizes[k], cudaGetErrorString(e));
+        if (int e = c.io[k].ensure(sizes[k])) return e;
     CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, c.stream));
     if (int rc = bdg_dev_pack16((const char*)c.io[0].p, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, c.stream)) return rc;
     CU_TRY(cudaMemcpyAsync(out, c.io[1].p, R * 4, cudaMemcpyDeviceToHost, c.stream));
@@ -2063,19 +2053,18 @@ int bdg_pack16(const char* seqs, size_t R, uint32_t* out, uint8_t* valid)
 static int pack16_sorted_core(DevCtx& c, const char* d_seqs, size_t R, size_t* n)
 {
     cudaStream_t st = c.stream;
-    auto ensure = ensure_buf;
     // io[1] ranks, io[2] validity; ce[0] kept ranks, ce[1] sorted, ce[2] distinct, ce[7] count, ce[8] cub scratch
-    if (int e = ensure(c.io[1], R * 4)) return e;
-    if (int e = ensure(c.io[2], R)) return e;
-    for (int k = 0; k < 3; k++) if (int e = ensure(c.ce[k], R * 4)) return e;
-    if (int e = ensure(c.ce[7], 64)) return e;
+    if (int e = c.io[1].ensure(R * 4)) return e;
+    if (int e = c.io[2].ensure(R)) return e;
+    for (int k = 0; k < 3; k++) if (int e = c.ce[k].ensure(R * 4)) return e;
+    if (int e = c.ce[7].ensure(64)) return e;
     uint32_t* d_n = (uint32_t*)c.ce[7].p;
     if (int rc = bdg_dev_pack16(d_seqs, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, st)) return rc;
     size_t t1 = 0, t2 = 0, t3 = 0;
     CU_TRY(cub::DeviceSelect::Flagged(nullptr, t1, (const uint32_t*)c.io[1].p, (const uint8_t*)c.io[2].p, (uint32_t*)c.ce[0].p, d_n, (int)R, st));
     CU_TRY(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[1].p, (int)R, 0, 32, st));
     CU_TRY(cub::DeviceSelect::Unique(nullptr, t3, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, d_n, (int)R, st));
-    if (int e = ensure(c.ce[8], std::max(t1, std::max(t2, t3)))) return e;
+    if (int e = c.ce[8].ensure(std::max(t1, std::max(t2, t3)))) return e;
     CU_TRY(cub::DeviceSelect::Flagged(c.ce[8].p, t1, (const uint32_t*)c.io[1].p, (const uint8_t*)c.io[2].p, (uint32_t*)c.ce[0].p, d_n, (int)R, st));
     uint32_t kept = 0;
     CU_TRY(cudaMemcpyAsync(&kept, d_n, 4, cudaMemcpyDeviceToHost, st));
@@ -2100,7 +2089,7 @@ int bdg_pack16_sorted(const char* seqs, size_t R, uint32_t* out_sorted, size_t* 
     if (int rc = need_ctx()) return rc;
     DevCtx& c = g_ctx[0];
     CU_TRY(cudaSetDevice(c.dev));
-    if (int e = ensure_buf(c.io[0], R * 16)) return e;     // io[0] letters
+    if (int e = c.io[0].ensure(R * 16)) return e;     // io[0] letters
     CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, c.stream));
     size_t kept = 0;
     if (int rc = pack16_sorted_core(c, (const char*)c.io[0].p, R, &kept)) return rc;
@@ -2138,14 +2127,9 @@ int bdg_dev_pack16_sorted(const char* d_seqs, size_t R, uint32_t* d_out_sorted, 
 // when that is this device's own workspace).
 static int edges_on_device(DevCtx& c, const uint32_t* sorted, size_t N, int t, int part, int nparts, size_t* n_out, int src_dev = -1)
 {
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     CU_TRY(cudaSetDevice(c.dev));
-    if (int e = ensure(c.sorted, std::max<size_t>(N, 1) * 4)) return e;
-    if (int e = ensure(c.count, 2 * sizeof(unsigned long long))) return e;      // [edge count | first unsorted index]
+    if (int e = c.sorted.ensure(std::max<size_t>(N, 1) * 4)) return e;
+    if (int e = c.count.ensure(2 * sizeof(unsigned long long))) return e;      // [edge count | first unsorted index]
     if (src_dev < 0) CU_TRY(cudaMemcpyAsync(c.sorted.p, sorted, N * 4, cudaMemcpyHostToDevice, c.stream));
     else if (src_dev == c.dev) CU_TRY(cudaMemcpyAsync(c.sorted.p, sorted, N * 4, cudaMemcpyDeviceToDevice, c.stream));
     else CU_TRY(cudaMemcpyPeerAsync(c.sorted.p, c.dev, sorted, src_dev, N * 4, c.stream));
@@ -2161,9 +2145,9 @@ static int edges_on_device(DevCtx& c, const uint32_t* sorted, size_t N, int t, i
     unsigned long long count = 0;
     bool done = false;
     for (int attempt = 0; attempt < 4 && !done; attempt++) {
-        if (int e = ensure(c.ea, cap * 4)) return e;
-        if (int e = ensure(c.eb, cap * 4)) return e;
-        if (int e = ensure(c.ed, cap)) return e;
+        if (int e = c.ea.ensure(cap * 4)) return e;
+        if (int e = c.eb.ensure(cap * 4)) return e;
+        if (int e = c.ed.ensure(cap)) return e;
         if (int e = launch_edges((const uint32_t*)c.sorted.p, N, t, part, nparts, (uint32_t*)c.ea.p, (uint32_t*)c.eb.p, (uint8_t*)c.ed.p, cap,
                                  (unsigned long long*)c.count.p, c.stream, &c)) return e;
         unsigned long long both[2] = {0, 0};
@@ -2173,12 +2157,7 @@ static int edges_on_device(DevCtx& c, const uint32_t* sorted, size_t N, int t, i
         first_bad = both[1];
         if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "input not strictly increasing at index %llu", first_bad);
         if (count >> 63) {                     // rare: a sparse pass listed more tiles than the list holds; grow it and run again
-            unsigned long long hdr[(PLAN_HDR / 8) * bdg::MAX_PASSES];
-            CU_TRY(cudaMemcpy(hdr, c.plan.p, sizeof(hdr), cudaMemcpyDeviceToHost));
-            unsigned long long need = 0;
-            for (int p = 0; p < bdg::MAX_PASSES; p++) need = std::max(need, hdr[(PLAN_HDR / 8) * p + HDR_LIST / 8]);
-            for (int p = 0; p < bdg::MAX_PASSES; p++)
-                if (int e = ensure(c.tile_list[p], (size_t)need * sizeof(uint2))) return e;
+            if (int e = grow_tile_lists(c)) return e;
         } else if (count > cap) {              // rare: the capacity guess was too small; the edge set is deterministic, so run again
             cap = (size_t)count;
         } else {
@@ -2255,16 +2234,16 @@ int bdg_edges_build_resident(unsigned long long token, int t, bdg_edges** out)
 {
     if (!out) return fail(BDG_ERR_ARG, "NULL pointer argument");
     *out = nullptr;
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c0 = g_ctx[0];
-    if (token == 0 || token != c0.map_token) return fail(BDG_ERR_ARG, "stale read-map token: a later dedup call has reused the workspaces");
+    DevCtx* c0 = nullptr;
+    if (int rc = map_ctx(token, &c0)) return rc;
     bdg_edges* res = new (std::nothrow) bdg_edges();
     if (!res) return fail(BDG_ERR_OOM, "host allocation failed");
+    res->read_map = token;
     std::vector<int> idx, parts;
     const int G = (int)g_ctx.size();
     for (int g = 0; g < G; g++) { idx.push_back(g); parts.push_back(g); }
     int rc = BDG_OK;
-    try { rc = edges_on_devices((const uint32_t*)c0.dd[6].p, c0.map_distinct, t, idx, parts, G, res, c0.dev); }
+    try { rc = edges_on_devices(c0->map.ascending(), c0->map.distinct, t, idx, parts, G, res, c0->dev); }
     catch (const std::bad_alloc&) { rc = fail(BDG_ERR_OOM, "host allocation failed"); }
     catch (const std::exception& e) { rc = fail(BDG_ERR_CUDA, "host thread failure: %s", e.what()); }
     if (rc) { delete res; return rc; }
@@ -2283,18 +2262,13 @@ int bdg_edges_build_into(const uint32_t* sorted_unique, size_t N, int t, int par
     if (nparts < 1 || part < 0 || part >= nparts) return fail(BDG_ERR_ARG, "part %d of %d is not a valid part", part, nparts);
     if (int rc = need_ctx()) return rc;
     DevCtx& c = g_ctx[0];
-    auto ensure = [&](Buf& bf, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)bf.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     CU_TRY(cudaSetDevice(c.dev));
     const size_t dcap = std::max<size_t>(cap, 1);
-    if (int e = ensure(c.sorted, std::max<size_t>(N, 1) * 4)) return e;
-    if (int e = ensure(c.count, 2 * sizeof(unsigned long long))) return e;
-    if (int e = ensure(c.ea, dcap * 4)) return e;
-    if (int e = ensure(c.eb, dcap * 4)) return e;
-    if (int e = ensure(c.ed, dcap)) return e;
+    if (int e = c.sorted.ensure(std::max<size_t>(N, 1) * 4)) return e;
+    if (int e = c.count.ensure(2 * sizeof(unsigned long long))) return e;
+    if (int e = c.ea.ensure(dcap * 4)) return e;
+    if (int e = c.eb.ensure(dcap * 4)) return e;
+    if (int e = c.ed.ensure(dcap)) return e;
     c.generation++;                                         // older handles on this device lose their edges
     CU_TRY(cudaMemcpyAsync(c.sorted.p, sorted_unique, N * 4, cudaMemcpyHostToDevice, c.stream));
     unsigned long long* d_bad = (unsigned long long*)c.count.p + 1;
@@ -2313,12 +2287,7 @@ int bdg_edges_build_into(const uint32_t* sorted_unique, size_t N, int t, int par
         CU_TRY(cudaStreamSynchronize(c.stream));
         if (both[1] != ~0ull) return fail(BDG_ERR_ARG, "input not strictly increasing at index %llu", both[1]);
         if (both[0] >> 63) {                                // a sparse pass listed more tiles than its list holds: grow it and run again
-            unsigned long long hdr[(PLAN_HDR / 8) * bdg::MAX_PASSES];
-            CU_TRY(cudaMemcpy(hdr, c.plan.p, sizeof(hdr), cudaMemcpyDeviceToHost));
-            unsigned long long need = 0;
-            for (int p = 0; p < bdg::MAX_PASSES; p++) need = std::max(need, hdr[(PLAN_HDR / 8) * p + HDR_LIST / 8]);
-            for (int p = 0; p < bdg::MAX_PASSES; p++)
-                if (int e = ensure(c.tile_list[p], (size_t)need * sizeof(uint2))) return e;
+            if (int e = grow_tile_lists(c)) return e;
             continue;
         }
         *count = (size_t)both[0];
@@ -2434,15 +2403,14 @@ void bdg_edges_free(bdg_edges* e) { delete e; }
 
 // ---- f-3  cluster(): barcode_graph.py:279-301 -------------------------------------------------------------
 // d_ea / d_eb hold barcode VALUES on entry and node indices on return (converted in place).
-// centre_idx / level may be NULL: the result then only stays on the device (cl[1] / cl[2]) for bdg_assign_reads*.
+// centre_idx / level may be NULL: the result then only stays on the device (map.centre / map.level) for bdg_assign_reads*.
 // The phases of cluster() over node arrays the caller owns, each on the stream it is given: cluster_on_device runs them on one
 // device; the bdg_dev_cluster_* entry points expose them to one process per GPU, which reduces the claims between the ranks.
 // values -> node indices of the E edges (ea, eb) against d_sorted[N] on device c (top16: its search table), written to (oa, ob)
 static int index_edges(DevCtx& c, const uint32_t* d_sorted, size_t N, const uint32_t* d_ea, const uint32_t* d_eb, size_t E, uint32_t* d_oa,
                        uint32_t* d_ob, cudaStream_t st)
 {
-    if (cudaError_t e = (cudaError_t)c.top16.ensure(65537 * 4))
-        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation: %s", cudaGetErrorString(e));
+    if (int e = c.top16.ensure(65537 * 4)) return e;
     const int nb = (int)std::min<size_t>((N + 256) / 256, (size_t)c.sms * 8);
     bdg::top_start_kernel<<<nb, 256, 0, st>>>(d_sorted, (uint32_t)N, (uint32_t*)c.top16.p);
     if (E) {
@@ -2496,29 +2464,24 @@ static int cluster_resolve(int32_t* d_ci, uint8_t* d_lv, int32_t* d_min, int32_t
 }
 
 // d_ea / d_eb hold barcode VALUES on entry and node indices on return (converted in place) unless `indexed`.
-// centre_idx / level may be NULL: the result then only stays on the device (cl[1] / cl[2]) for bdg_assign_reads*.
+// centre_idx / level may be NULL: the result then only stays on the device (map.centre / map.level) for bdg_assign_reads*.
 static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint32_t* d_ea, uint32_t* d_eb, size_t E,
                              const uint32_t* centres, size_t C, int rounds, int32_t* centre_idx, uint8_t* level, size_t* n_has_edge = nullptr,
                              bool indexed = false)
 {
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     cudaStream_t st = c.stream;
-    if (int e = ensure(c.cl[0], std::max<size_t>(C, 1) * 4)) return e;
-    if (int e = ensure(c.cl[1], N * 4)) return e;
-    if (int e = ensure(c.cl[2], N)) return e;
-    if (int e = ensure(c.cl[3], N * 4)) return e;
-    if (int e = ensure(c.cl[4], N * 4)) return e;
-    if (int e = ensure(c.cl[5], 16)) return e;
-    c.cl_token = 0;                                        // the resident result is about to be overwritten
-    unsigned int* d_bad = (unsigned int*)c.cl[5].p;
+    c.map.cl_token = 0;                                    // the resident result is about to be overwritten
+    if (int e = c.cl[0].ensure(std::max<size_t>(C, 1) * 4)) return e;
+    if (int e = c.map.centre.ensure(N * 4)) return e;
+    if (int e = c.map.level.ensure(N)) return e;
+    if (int e = c.cl[1].ensure(N * 4)) return e;
+    if (int e = c.cl[2].ensure(N * 4)) return e;
+    if (int e = c.cl[3].ensure(16)) return e;
+    unsigned int* d_bad = (unsigned int*)c.cl[3].p;
     CU_TRY(cudaMemsetAsync(d_bad, 0, 4, c.stream));
     uint32_t* d_cen = (uint32_t*)c.cl[0].p;
-    int32_t *d_ci = (int32_t*)c.cl[1].p, *d_min = (int32_t*)c.cl[3].p, *d_max = (int32_t*)c.cl[4].p;
-    uint8_t* d_lv = (uint8_t*)c.cl[2].p;
+    int32_t *d_ci = (int32_t*)c.map.centre.p, *d_min = (int32_t*)c.cl[1].p, *d_max = (int32_t*)c.cl[2].p;
+    uint8_t* d_lv = (uint8_t*)c.map.level.p;
     const int nb = node_blocks(N, c.sms);
     const bool trace = getenv("BDG_TRACE") != nullptr;
     double tr0 = 0, tr1 = 0, tr2 = 0;
@@ -2541,7 +2504,7 @@ static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint
     if (level) CU_TRY(cudaMemcpyAsync(level, d_lv, N, cudaMemcpyDeviceToHost, st));
     unsigned long long has_edge = 0;
     if (n_has_edge) {
-        unsigned long long* d_cnt = (unsigned long long*)((char*)c.cl[5].p + 8);
+        unsigned long long* d_cnt = (unsigned long long*)((char*)c.cl[3].p + 8);
         CU_TRY(cudaMemsetAsync(d_cnt, 0, 8, st));
         bdg::count_has_edge_kernel<<<nb, 256, 0, st>>>(d_lv, (uint32_t)N, d_cnt);
         g_launches++;
@@ -2568,15 +2531,10 @@ int bdg_cluster_levels(const uint32_t* sorted_unique, size_t N, const uint32_t* 
     if (int rc = need_ctx()) return rc;
     DevCtx& c = g_ctx[0];
     CU_TRY(cudaSetDevice(c.dev));
-    auto ensure = [&](Buf& b, size_t bytes) -> int {
-        if (cudaError_t e = (cudaError_t)b.ensure(bytes))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", bytes, cudaGetErrorString(e));
-        return BDG_OK;
-    };
     // the edge workspaces of an earlier build are reused for the index arrays: older handles become stale
-    if (int e = ensure(c.sorted, N * 4)) return e;
-    if (int e = ensure(c.ea, std::max<size_t>(E, 1) * 4)) return e;
-    if (int e = ensure(c.eb, std::max<size_t>(E, 1) * 4)) return e;
+    if (int e = c.sorted.ensure(N * 4)) return e;
+    if (int e = c.ea.ensure(std::max<size_t>(E, 1) * 4)) return e;
+    if (int e = c.eb.ensure(std::max<size_t>(E, 1) * 4)) return e;
     c.generation++;
     CU_TRY(cudaMemcpyAsync(c.sorted.p, sorted_unique, N * 4, cudaMemcpyHostToDevice, c.stream));
     CU_TRY(cudaMemcpyAsync(c.ea.p, ea, E * 4, cudaMemcpyHostToDevice, c.stream));
@@ -2597,7 +2555,8 @@ int bdg_cluster_resident(bdg_edges* e, size_t N, const uint32_t* centres, size_t
 {
     if (n_has_edge) *n_has_edge = 0;
     if (int rc = cluster_from_edges(e, N, centres, C, rounds, nullptr, nullptr, n_has_edge)) return rc;
-    if (e && !e->ctx.empty() && e->ctx[0] == 0 && N == g_ctx[0].map_distinct) g_ctx[0].cl_token = g_ctx[0].map_token;   // the result of THIS dedup's graph
+    ReadMap& m = g_ctx[0].map;
+    if (e->read_map && e->read_map == m.token && N == m.distinct) m.cl_token = m.token;   // the graph of the live read map
     return BDG_OK;
 }
 
@@ -2620,10 +2579,8 @@ static int cluster_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, s
         // by the build), into buffers of its own - the handle's edges stay intact on their devices.
         size_t total = 0;
         for (size_t k : e->count) total += k;
-        if (cudaError_t err = (cudaError_t)c.gather_a.ensure(std::max<size_t>(total, 1) * 4))
-            return fail(err == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "gather buffer of %zu edges: %s", total, cudaGetErrorString(err));
-        if (cudaError_t err = (cudaError_t)c.gather_b.ensure(std::max<size_t>(total, 1) * 4))
-            return fail(err == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "gather buffer of %zu edges: %s", total, cudaGetErrorString(err));
+        if (int rc = c.gather_a.ensure(std::max<size_t>(total, 1) * 4)) return rc;
+        if (int rc = c.gather_b.ensure(std::max<size_t>(total, 1) * 4)) return rc;
         // every device turns its own edges into node indices (its copy of the array, its SMs), then the indices travel
         size_t off = 0;
         for (size_t g = 0; g < e->ctx.size(); g++) {
@@ -2635,8 +2592,8 @@ static int cluster_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, s
                 if (int rc = index_edges(c, (const uint32_t*)c.sorted.p, N, (const uint32_t*)c.ea.p, (const uint32_t*)c.eb.p, k, (uint32_t*)c.gather_a.p + off, (uint32_t*)c.gather_b.p + off, c.stream)) return rc;
             } else {
                 CU_TRY(cudaSetDevice(src.dev));
-                if (cudaError_t err = (cudaError_t)src.gather_a.ensure(k * 4)) return fail(BDG_ERR_OOM, "index buffer: %s", cudaGetErrorString(err));
-                if (cudaError_t err = (cudaError_t)src.gather_b.ensure(k * 4)) return fail(BDG_ERR_OOM, "index buffer: %s", cudaGetErrorString(err));
+                if (int rc = src.gather_a.ensure(k * 4)) return rc;
+                if (int rc = src.gather_b.ensure(k * 4)) return rc;
                 if (int rc = index_edges(src, (const uint32_t*)src.sorted.p, N, (const uint32_t*)src.ea.p, (const uint32_t*)src.eb.p, k, (uint32_t*)src.gather_a.p, (uint32_t*)src.gather_b.p, src.stream)) return rc;
                 CU_TRY(cudaMemcpyPeerAsync((uint32_t*)c.gather_a.p + off, c.dev, src.gather_a.p, src.dev, k * 4, src.stream));
                 CU_TRY(cudaMemcpyPeerAsync((uint32_t*)c.gather_b.p + off, c.dev, src.gather_b.p, src.dev, k * 4, src.stream));
@@ -2727,8 +2684,7 @@ int bdg_member_sorted(const uint32_t* sorted_wl, size_t W, const uint32_t* q, si
     CU_TRY(cudaSetDevice(c.dev));
     const size_t sizes[4] = {std::max<size_t>(W, 1) * 4, Q * 4, Q, 8};       // grow-only workspaces: whitelist, queries, hits, check flag
     for (int k = 0; k < 4; k++)
-        if (cudaError_t e = (cudaError_t)c.io[k].ensure(sizes[k]))
-            return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", sizes[k], cudaGetErrorString(e));
+        if (int e = c.io[k].ensure(sizes[k])) return e;
     uint32_t *d_wl = (uint32_t*)c.io[0].p, *d_q = (uint32_t*)c.io[1].p;
     uint8_t* d_hit = (uint8_t*)c.io[2].p;
     unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
@@ -2758,7 +2714,7 @@ int bdg_dev_whitelist_check(const uint32_t* d_sorted_wl, size_t W, void* stream)
     DevCtx& c = g_ctx[0];
     CU_TRY(cudaSetDevice(c.dev));
     if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
-    if (int e = ensure_buf(c.io[3], 8)) return e;
+    if (int e = c.io[3].ensure(8)) return e;
     unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
     CallerOrder order(c, stream);
     if (int rc = order.begin()) return rc;
@@ -2780,38 +2736,33 @@ int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, si
     if (int rc = need_ctx()) return rc;
     // queries are independent: deal contiguous slices to the devices, targets replicated (SURVEY.md §8e)
     const int G = (int)g_ctx.size();
-    struct Run { uint32_t *d_q = nullptr, *d_t = nullptr, *d_keys = nullptr; int32_t* d_arg = nullptr; uint8_t* d_dist = nullptr; size_t lo = 0, n = 0; };
-    std::vector<Run> runs(G);
     int rc = BDG_OK;
     const size_t per = (Q + G - 1) / G;
     for (int g = 0; g < G && rc == BDG_OK; g++) {
-        Run& r = runs[g];
-        r.lo = std::min(Q, per * g);
-        r.n = std::min(Q, per * (g + 1)) - r.lo;
-        if (r.n == 0) continue;
+        const size_t lo = std::min(Q, per * g), n = std::min(Q, per * (g + 1)) - lo;
+        if (n == 0) continue;
         DevCtx& c = g_ctx[g];
         rc = [&]() -> int {
             CU_TRY(cudaSetDevice(c.dev));
-            CU_TRY(cudaMallocAsync((void**)&r.d_q, r.n * 4, c.stream));
-            CU_TRY(cudaMallocAsync((void**)&r.d_t, std::max<size_t>(W, 1) * 4, c.stream));
-            CU_TRY(cudaMallocAsync((void**)&r.d_keys, r.n * 4, c.stream));
-            CU_TRY(cudaMallocAsync((void**)&r.d_arg, r.n * 4, c.stream));
-            CU_TRY(cudaMallocAsync((void**)&r.d_dist, r.n, c.stream));
-            CU_TRY(cudaMemcpyAsync(r.d_q, q + r.lo, r.n * 4, cudaMemcpyHostToDevice, c.stream));
-            CU_TRY(cudaMemcpyAsync(r.d_t, targets, W * 4, cudaMemcpyHostToDevice, c.stream));
-            if (int e = bdg_dev_nearest_bounded(r.d_q, r.n, r.d_t, W, max_d, r.d_keys, r.d_arg, r.d_dist, c.stream)) return e;
-            CU_TRY(cudaMemcpyAsync(argmin + r.lo, r.d_arg, r.n * 4, cudaMemcpyDeviceToHost, c.stream));
-            CU_TRY(cudaMemcpyAsync(dist + r.lo, r.d_dist, r.n, cudaMemcpyDeviceToHost, c.stream));
+            // io[0] queries, io[1] targets, io[2] keys | argmin | distance
+            if (int e = c.io[0].ensure(n * 4)) return e;
+            if (int e = c.io[1].ensure(std::max<size_t>(W, 1) * 4)) return e;
+            if (int e = c.io[2].ensure(n * 9)) return e;
+            uint32_t *d_q = (uint32_t*)c.io[0].p, *d_t = (uint32_t*)c.io[1].p, *d_keys = (uint32_t*)c.io[2].p;
+            int32_t* d_arg = (int32_t*)(d_keys + n);
+            uint8_t* d_dist = (uint8_t*)(d_arg + n);
+            CU_TRY(cudaMemcpyAsync(d_q, q + lo, n * 4, cudaMemcpyHostToDevice, c.stream));
+            CU_TRY(cudaMemcpyAsync(d_t, targets, W * 4, cudaMemcpyHostToDevice, c.stream));
+            if (int e = bdg_dev_nearest_bounded(d_q, n, d_t, W, max_d, d_keys, d_arg, d_dist, c.stream)) return e;
+            CU_TRY(cudaMemcpyAsync(argmin + lo, d_arg, n * 4, cudaMemcpyDeviceToHost, c.stream));
+            CU_TRY(cudaMemcpyAsync(dist + lo, d_dist, n, cudaMemcpyDeviceToHost, c.stream));
             return BDG_OK;
         }();
     }
     for (int g = 0; g < G; g++) {
-        Run& r = runs[g];
-        if (r.n == 0) continue;
+        if (per * g >= Q) continue;
         DevCtx& c = g_ctx[g];
         cudaSetDevice(c.dev);
-        cudaFreeAsync(r.d_q, c.stream); cudaFreeAsync(r.d_t, c.stream); cudaFreeAsync(r.d_keys, c.stream);
-        cudaFreeAsync(r.d_arg, c.stream); cudaFreeAsync(r.d_dist, c.stream);
         cudaError_t e = cudaStreamSynchronize(c.stream);
         if (e != cudaSuccess && rc == BDG_OK) rc = fail(BDG_ERR_CUDA, "stream sync failed: %s", cudaGetErrorString(e));
     }
@@ -2833,9 +2784,9 @@ static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, cudaMe
     ix->dev = g_ctx[0].dev;
     ix->W = W;
     CU_TRY(cudaSetDevice(ix->dev));
-    if (cudaError_t e = (cudaError_t)ix->wl.ensure(std::max<size_t>(W, 1) * 4)) {
+    if (int e = ix->wl.ensure(std::max<size_t>(W, 1) * 4)) {
         delete ix;
-        return fail(e == cudaErrorMemoryAllocation ? BDG_ERR_OOM : BDG_ERR_CUDA, "device allocation of %zu bytes: %s", W * 4, cudaGetErrorString(e));
+        return e;
     }
     cudaError_t e = cudaMemcpyAsync(ix->wl.p, wl, W * 4, kind, g_ctx[0].stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(g_ctx[0].stream);
@@ -2868,7 +2819,6 @@ static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, cudaMe
                 ok = cudaStreamSynchronize(st) == cudaSuccess && cudaGetLastError() == cudaSuccess;
             }
         }
-        cubtmp.release();
         if (!ok) { bdg_kmer_index_free(ix); return fail(BDG_ERR_CUDA, "building the 6-mer posting lists failed: %s", cudaGetErrorString(cudaGetLastError())); }
         ix->posted = true;
     }
@@ -2914,9 +2864,7 @@ int bdg_kmer_index_info(const bdg_kmer_index* ix, int* posted, double* kernel_ms
 void bdg_kmer_index_free(bdg_kmer_index* ix)
 {
     if (!ix) return;
-    cudaSetDevice(ix->dev);
-    ix->wl.release(); ix->kstart.release(); ix->post.release(); ix->scratch.release();
-    for (auto& b : ix->outb) b.release();
+    cudaSetDevice(ix->dev);                         // the buffers are freed on their device
     for (auto& e : ix->ev) if (e) cudaEventDestroy(e);
     delete ix;
 }
@@ -2927,7 +2875,7 @@ static int kmer_query_core(bdg_kmer_index* ix, DevCtx& c, const uint32_t* d_q, s
                            uint32_t* d_hw, uint8_t* d_cnt, unsigned long long* d_mult, unsigned long long* tot)
 {
     const size_t W = ix->W;
-    if (int e = ensure_buf(ix->outb[5], 8)) return e;
+    if (int e = ix->outb[5].ensure(8)) return e;
     unsigned long long* d_total = (unsigned long long*)ix->outb[5].p;
     CU_TRY(cudaMemsetAsync(d_total, 0, 8, c.stream));
     CU_TRY(cudaEventRecord(ix->ev[0], c.stream));
@@ -2969,7 +2917,7 @@ int bdg_kmer_index_query(bdg_kmer_index* ix, const uint32_t* q, size_t Q, int mi
     const size_t capa = std::max<size_t>(cap, 1);
     const size_t sizes[5] = {Q * 4, capa * 4, capa * 4, capa, capa * 8};     // queries, hit_q, hit_w, cnt, mult
     for (int k = 0; k < 5; k++)
-        if (int e = ensure_buf(ix->outb[k], sizes[k])) return e;
+        if (int e = ix->outb[k].ensure(sizes[k])) return e;
     uint32_t *d_q = (uint32_t*)ix->outb[0].p, *d_hq = (uint32_t*)ix->outb[1].p, *d_hw = (uint32_t*)ix->outb[2].p;
     uint8_t* d_cnt = (uint8_t*)ix->outb[3].p;
     unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
@@ -3008,7 +2956,7 @@ int bdg_dev_kmer_index_query(bdg_kmer_index* ix, const uint32_t* d_q, size_t Q, 
         for (const void* p : outs) if (int rc = check_on_first(p, "output")) return rc;
     }
     // the position counts are unpacked from library scratch into d_pos; the other outputs are written by the kernels in place
-    if (int e = ensure_buf(ix->outb[4], std::max<size_t>(cap, 1) * 8)) return e;
+    if (int e = ix->outb[4].ensure(std::max<size_t>(cap, 1) * 8)) return e;
     unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
     CallerOrder order(c, stream);
     if (int rc = order.begin()) return rc;

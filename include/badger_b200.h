@@ -154,7 +154,8 @@ int bdg_cluster_levels(const uint32_t* sorted_unique, size_t N, const uint32_t* 
 int bdg_cluster_levels_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, size_t C, int rounds, int32_t* centre_idx,
                                   uint8_t* level);
 /* The same with the result left on the first device for bdg_assign_reads32(token, NULL, ...).  *n_has_edge = nodes that are no
- * centre and have at least one edge (what `len(graph.edges.keys())`, badger.py:131, counts beside the centres). */
+ * centre and have at least one edge (what `len(graph.edges.keys())`, badger.py:131, counts beside the centres).  The result
+ * belongs to the read map the handle was built from (bdg_edges_build_resident), and only while that read map's token is live. */
 int bdg_cluster_resident(bdg_edges* e, size_t N, const uint32_t* centres, size_t C, int rounds, size_t* n_has_edge);
 
 /* ---- a-6  whitelist membership: `unrank(r) in barcode_list`, barcode_graph.py:262-267 -------------- */
