@@ -280,8 +280,8 @@ int scheme_ready()
     }
     if constexpr (T == 2) {
         if (!bdg::seed_scheme_build(g_scheme, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN_BLOCKS is not a usable block layout (3..6 blocks, 15 bases in all)");
-        g_scheme_lut.assign((size_t)1 << g_scheme.nflags, 0);
-        bdg::seed_lut_build(g_scheme, g_scheme_lut.data());
+        g_scheme_lut.assign((size_t)1 << (g_scheme.nflags + 2), 0);          // block-match flags and the two side bits
+        bdg::seed_lut_build_sides(g_scheme, g_scheme_lut.data());
     } else {
         if (!bdg::seed3_scheme_build(g_scheme3, bases, nb)) return fail(BDG_ERR_ARG, "BDG_JOIN3_BLOCKS is not a usable block layout (4..7 blocks of >= 2 bases, 15 bases in all)");
     }
@@ -479,7 +479,10 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
         if (int e = ws->jn_counts[k].ensure(((size_t)n_slabs + 1) * 4)) return e;
         if (int e = ws->jn_offs[k].ensure(((size_t)n_slabs + 1) * 4)) return e;
     }
+    // t = 2: the shifted conditions have a kernel of their own (the one-sided test is compiled in; at t = 3 it is the same kernel);
+    // both are built for the same residency, so one grid serves both
     const auto kern = rs == 8 ? bdg::join_kernel<T, 8> : bdg::join_kernel<T, 32>;
+    const auto kern_shf = rs == 8 ? bdg::join_kernel<T, 8, T == 2> : bdg::join_kernel<T, 32, T == 2>;
     int grid = 0;
     if (int rc = grid_for((const void*)kern, &grid, bdg::ENT)) return rc;
     if (const char* e = getenv("BDG_JOIN_CTAS")) grid = std::min(grid, ws->sms * std::max(1, atoi(e)));   // CTAs per SM of a join launch
@@ -573,7 +576,7 @@ int launch_edges_join(const uint32_t* d_sorted, size_t N, int part, int nparts, 
             CU_TRY(cudaEventRecord(ws->ev_pre[k], sp));
             CU_TRY(cudaStreamWaitEvent(st, ws->ev_pre[k], 0));
         }
-        kern<<<grid, bdg::ENT, 0, st>>>(A, o);
+        (S.cond[c].self ? kern : kern_shf)<<<grid, bdg::ENT, 0, st>>>(A, o);
         g_launches += 3;
         CU_TRY(cudaGetLastError());
         if (ahead) { CU_TRY(cudaEventRecord(ws->ev_join[k], st)); set_joined[k] = true; }

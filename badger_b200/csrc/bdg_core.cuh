@@ -200,6 +200,23 @@ BDG_HD uint32_t quick_marks(uint32_t a, uint32_t b0, uint32_t bP, uint32_t bM)
     const uint32_t x0 = a ^ b0, xp = a ^ bP, xm = a ^ bM;
     return (x0 | (x0 << 1)) & (xp | (xp << 1)) & (xm | (xm << 1)) & QUICK_VALID;
 }
+// One diagonal side of the same test: marks of the columns 0..14 of x that match y neither on diagonal 0 (yd = y) nor on the
+// one shifted word ys (y >> 2: x[i] vs y[i + 1]).  Column 15 is left out and column 14 meets the zero shifted in at the top,
+// exactly as in quick_marks.  A script of <= 2 operations keeps its columns on {0, +1} or on {0, -1} (bdg_seed.cuh), so under
+// one labelling of a pair with D <= 2 at most two marks of side_marks(p, q, q >> 2) are set.
+BDG_HD uint32_t side_marks(uint32_t x, uint32_t yd, uint32_t ys)
+{
+    const uint32_t x0 = x ^ yd, xs = x ^ ys;
+    return (x0 | (x0 << 1)) & (xs | (xs << 1)) & QUICK_VALID;
+}
+// at most two marks: drop the two lowest, test for zero.  one / mone are 1 / -1 (the kernels pass them at run time, so that
+// w * one + mone is an IMAD on the FMA pipe instead of an add on the ALU pipe)
+BDG_HD bool marks_le2(uint32_t w, uint32_t one, uint32_t mone)
+{
+    w &= w * one + mone;
+    w &= w * one + mone;
+    return w == 0;
+}
 BDG_HD bool quick_pass(uint32_t a, uint32_t b, int t)
 {
     uint32_t u = quick_marks(a, b, b >> 2, b << 2);

@@ -10,16 +10,17 @@
 //                          pass keeps the place its atomic returned.
 //   join_band_kernel<T>    per slab of 32 consecutive rows: number of work units (runs of <= JUNIT columns) it needs
 //   (cub::DeviceScan::ExclusiveSum: unit index -> slab)
-//   join_kernel<T, RS>     one persistent launch per condition: warps pull batches of units from an atomic cursor, stage the
+//   join_kernel<T, RS, SHF> one persistent launch per condition: warps pull batches of units from an atomic cursor, stage the
 //                          unit's columns in their own slice of shared memory (y, y >> 2, y << 2, key) and test
 //                          (row, column) pairs: quick test of bdg_core.cuh + key equality, one hit bit per pair; hits go
 //                          through the warp's queue to the exact stage on full warps, edges are appended with one atomic per warp.
 // A unit's 32 rows are worked through as 32/RS sub-slabs of RS rows x 32/RS column phases, each against its own column run:
 // RS = 32 when the key buckets are long, RS = 8 when they are short (fewer rows span fewer foreign buckets).
 // What differs between the thresholds T is the per-pair stage:
-//   T = 2  quick test on the diagonals -1..1 (quick_marks), two marks dropped; exact stage join_process: dist_small, the
-//          hand-over table over seed_flags on full batches of close pairs, then the 6-mer score in two queues (the middle
-//          diagonals, then the other eighteen).
+//   T = 2  quick test on ONE diagonal side (join2_quick, bdg_seed.cuh), two marks dropped: a shifted condition (SHF) tests the
+//          row's side {0, +1} and stages no y << 2, a symmetric one passes a pair on {0, +1} or on {0, -1}; exact stage
+//          join_process: dist_small, the hand-over table over seed_flags and the two side bits (seed_side_bits) on full batches
+//          of close pairs, then the 6-mer score in two queues (the middle diagonals, then the other eighteen).
 //   T = 3  quick test on the diagonals -2..2 (quick3_marks; the +-2 words are derived from the staged +-1 ones), three marks
 //          dropped; exact stage join3_process: dist3_min (Myers' bit-vector pass; D <= 3 has no case analysis), the hand-over
 //          walk seed3_first, then the 6-mer score through one queue.  The t = 3 scheme is too large for constant memory next to
@@ -295,7 +296,8 @@ __device__ __noinline__ uint32_t join_process(uint2* q2, uint8_t* q2d, const uin
         if (lane < take) {
             v = q2[JQ_CLOSE + nc + lane];
             vd = q2d[JQ_CLOSE + nc + lane];
-            own = __ldg(&lut[seed_flags(c_scheme, v.x, v.y)]) == (uint8_t)((vd & 4) ? want1 : want0);   // emitted by the first (condition, orientation) the pair meets
+            const uint32_t idx = seed_flags(c_scheme, v.x, v.y) | seed_side_bits(v.x, v.y) << c_scheme.nflags;
+            own = __ldg(&lut[idx]) == (uint8_t)((vd & 4) ? want1 : want0);   // emitted by the first (condition, orientation) that meets and passes the pair
         }
         const unsigned m = __ballot_sync(FULL, own);
         n_own = (uint32_t)__popc(m);
@@ -435,13 +437,17 @@ __device__ __forceinline__ void join_push(uint32_t h, uint32_t x, const uint32_t
 }
 
 // T = 2 is compiled for 5 resident CTAs per SM (48 registers; its three exact-stage queues take 41 KB of shared memory per CTA),
-// T = 3 for 4: its exact stage needs the registers
-template <int T, int RS>
+// T = 3 for 4: its exact stage needs the registers.
+// SHF (T = 2 only): a launch of a shifted condition, whose pairs are tested on the one diagonal side {0, +1} of the row
+// (join2_quick<true>; the y << 2 words are neither staged nor read); the symmetric conditions test either side.  T = 3 keeps
+// the test on -2..2 and the symmetric / shifted split at run time.
+template <int T, int RS, bool SHF = false>
 __global__ void __launch_bounds__(ENT, T == 2 ? 5 : 4) join_kernel(const JoinArgsT<T> A, const EdgeOut out)
 {
+    static_assert(T == 2 || !SHF, "the one-sided test is the t = 2 one");
     constexpr int PH = 32 / RS;                          // column phases of a warp
     constexpr int STEP = 4 * PH;                         // columns per inner step
-    __shared__ __align__(16) uint32_t s_b[EW][4][JCH + JPAD];   // y, y >> 2, y << 2, key of the staged columns
+    __shared__ __align__(16) uint32_t s_b[EW][4][JCH + JPAD];   // y, y >> 2, y << 2 (not for SHF), key of the staged columns
     __shared__ uint2 s_q[EW][JQCAP];
     __shared__ uint2 s_q2[EW][T == 2 ? 3 * JQ2CAP : JQ2CAP];   // pairs that need their score | (t = 2) pairs that need the far diagonals | close pairs
     __shared__ uint8_t s_q2d[EW][T == 2 ? 3 * JQ2CAP : JQ2CAP];
@@ -461,7 +467,7 @@ __global__ void __launch_bounds__(ENT, T == 2 ? 5 : 4) join_kernel(const JoinArg
     unsigned long long n_units = 0, n_pairs = 0, n_cand = 0;
     const SeedKey& ka = join_ka<T>(A);
     const SeedKey& kb = join_kb<T>(A);
-    const bool self = A.self != 0;
+    const bool self = !SHF && A.self != 0;               // (a run-time flag otherwise: the compiler versions the loops on it)
     const uint32_t total_units = __ldg(&A.offs[A.n_slabs]);
     const uint32_t n_batches = (total_units + JBATCH - 1) / JBATCH;
     const uint32_t r0 = join_cut(A.rowstart, A.nkeys, A.N, A.f0, A.fden), r1 = join_cut(A.rowstart, A.nkeys, A.N, A.f1, A.fden);   // this part's rows
@@ -512,7 +518,7 @@ __global__ void __launch_bounds__(ENT, T == 2 ? 5 : 4) join_kernel(const JoinArg
                     const uint32_t y = real ? __ldg(&A.cols[j]) : 0u;
                     sb0[t * 32 + lane] = y;
                     sbP[t * 32 + lane] = y >> 2;
-                    sbM[t * 32 + lane] = y << 2;
+                    if constexpr (!SHF) sbM[t * 32 + lane] = y << 2;
                     sbK[t * 32 + lane] = real ? seed_key(y, kb) : 0xFFFFFFFEu;   // a pad column matches no row
                 }
                 __syncwarp();
@@ -537,16 +543,21 @@ __global__ void __launch_bounds__(ENT, T == 2 ? 5 : 4) join_kernel(const JoinArg
                                 const int off = g0 + st * STEP + 4 * ph;
                                 const uint4 B0 = *reinterpret_cast<const uint4*>(&sb0[off]);
                                 const uint4 BP = *reinterpret_cast<const uint4*>(&sbP[off]);
-                                const uint4 BM = *reinterpret_cast<const uint4*>(&sbM[off]);
+                                const uint4 BM = SHF ? make_uint4(0u, 0u, 0u, 0u) : *reinterpret_cast<const uint4*>(&sbM[off]);
                                 const uint4 BK = *reinterpret_cast<const uint4*>(&sbK[off]);
 #pragma unroll
                                 for (int kk = 0; kk < 4; kk++) {
-                                    uint32_t w = T == 2 ? quick_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk))
-                                                        : quick3_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk));
-                                    w &= w * A.one + mone;   // drop the t lowest marks (IMAD keeps the -1 off the ALU pipe)
-                                    w &= w * A.one + mone;
-                                    if constexpr (T == 3) w &= w * A.one + mone;
-                                    bool hit = w == 0 && pick4(BK, kk) == kq;
+                                    bool pass;
+                                    if constexpr (T == 2) {
+                                        pass = join2_quick<SHF>(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk), A.one, mone);
+                                    } else {
+                                        uint32_t w = quick3_marks(xq, pick4(B0, kk), pick4(BP, kk), pick4(BM, kk));
+                                        w &= w * A.one + mone;   // drop the t lowest marks (IMAD keeps the -1 off the ALU pipe)
+                                        w &= w * A.one + mone;
+                                        w &= w * A.one + mone;
+                                        pass = w == 0;
+                                    }
+                                    bool hit = pass && pick4(BK, kk) == kq;
                                     if (self) hit = hit && base + (uint32_t)(off + kk) > iq;
                                     h |= (hit ? 1u : 0u) << (st * 4 + kk);
                                 }

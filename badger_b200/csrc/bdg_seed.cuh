@@ -16,10 +16,14 @@
 // are all 0 are symmetric ("self": one sort, each unordered couple once); the others pair (x, y) in both value orders.
 //   B = 4 (4,4,4,3 bases): 13 conditions on 14/16 key bits;  B = 5 (3 bases each): 25 conditions on 18 key bits.
 // A pair that meets several conditions is emitted by the FIRST (condition, orientation) in table order; that index is
-// looked up in a table over the pair's block-match flags (seed_flags / first_lut), built here on the host.
+// looked up in a table over the pair's block-match flags (seed_flags / seed_lut_build), built here on the host.  The join
+// kernel tests a shifted condition's pairs on one diagonal side only (join2_quick), so its hand-over table also takes the
+// pair's two side bits and names the first (condition, orientation) that meets the pair AND lets it through its filter
+// (seed_side_bits, seed_first_sides_slow, seed_lut_build_sides).
 //
 // Everything is __host__ __device__: tests/test_core_host.py compiles this header with g++ and checks, against the oracle's
-// distances, that the conditions are necessary for D <= 2, and that the emulated passes give the oracle's edge set.
+// distances, that the conditions are necessary for D <= 2, and that the emulated passes give the oracle's edge set;
+// tests/test_join_sides_host.py does the same for the one-sided filter and the side-aware table.
 #pragma once
 #include "bdg_core.cuh"
 
@@ -115,6 +119,42 @@ BDG_HD uint32_t seed_flags(const SeedScheme& s, uint32_t a, uint32_t b)
     return f;
 }
 
+// ---- the per-pair filter of the t = 2 join and the hand-over that knows it --------------------------------------------
+// join_kernel<2, RS, SHF> tests a (row x, column y) pair of equal keys with
+//   SHF (a shifted condition): at most two columns of x[0:15] mismatch y on both diagonals 0 and +1 - the frame of the
+//                              condition's own diagonals (x[block] == y[block + d], d in {0, 1});
+//   symmetric condition:       the same on {0, +1} OR on {0, -1}: either side, since the buckets hold the pair in no fixed order.
+// yP = y >> 2, yM = y << 2 (yM unused by SHF).  A pair with D <= 2 always passes the symmetric test; it passes the shifted one
+// under the labelling whose diagonals are >= 0, which is the labelling in which it meets a shifted condition.
+template <bool SHF>
+BDG_HD bool join2_quick(uint32_t x, uint32_t y, uint32_t yP, uint32_t yM, uint32_t one, uint32_t mone)
+{
+    if constexpr (SHF) return marks_le2(side_marks(x, y, yP), one, mone);
+    else return marks_le2(side_marks(x, y, yP), one, mone) | marks_le2(side_marks(x, y, yM), one, mone);
+}
+
+// The two side bits of a pair a < b: bit 0 = the row test of a shifted condition with (row, column) = (a, b) passes, bit 1 = the
+// same with (b, a).  The very function of the kernel's filter, so that the hand-over never names a pass whose filter dropped the pair.
+BDG_HD uint32_t seed_side_bits(uint32_t a, uint32_t b)
+{
+    return (join2_quick<true>(a, b, b >> 2, 0u, 1u, 0xFFFFFFFFu) ? 1u : 0u) | (join2_quick<true>(b, a, a >> 2, 0u, 1u, 0xFFFFFFFFu) ? 2u : 0u);
+}
+
+// The hand-over of the t = 2 join: the first (condition, orientation) in table order that the pair meets AND whose kernel filter
+// passes it - symmetric: always (the table is read for pairs with D <= 2 only, and they all pass); shifted, o = 0: side bit 0;
+// shifted, o = 1: side bit 1.  Every pair with D <= 2 has exactly one owner: its labelling with diagonals >= 0 meets some
+// condition, and the one-sided test passes in that labelling.  The definition; the kernels read the table below at
+// seed_flags | seed_side_bits << nflags.
+BDG_HD int seed_first_sides_slow(const SeedScheme& s, uint32_t a, uint32_t b)
+{
+    const uint32_t sides = seed_side_bits(a, b);
+    for (int c = 0; c < s.nconds; c++) {
+        if (seed_pred(s, c, a, b) && (s.cond[c].self || (sides & 1u))) return 2 * c;
+        if (!s.cond[c].self && seed_pred(s, c, b, a) && (sides & 2u)) return 2 * c + 1;
+    }
+    return SEED_NONE;
+}
+
 // ---- host side: table of conditions, sort forms, hand-over table -------------------------------------------------
 // blocks: number of bases of every block (sum 15).  Returns false if the layout does not fit the limits.
 inline bool seed_scheme_build(SeedScheme& s, const int* bases, int nblocks)
@@ -196,6 +236,31 @@ inline void seed_lut_build(const SeedScheme& s, uint8_t* lut)
             }
         }
         lut[f] = first;
+    }
+}
+
+// lut: 1 << (s.nflags + 2) entries, lut[flags | sides << nflags] = seed_first_sides_slow.  One walk of the conditions per flag
+// word fills its four side combinations.
+inline void seed_lut_build_sides(const SeedScheme& s, uint8_t* lut)
+{
+    const uint32_t nf = 1u << s.nflags;
+    for (uint32_t f = 0; f < nf; f++) {
+        uint8_t first[4] = {SEED_NONE, SEED_NONE, SEED_NONE, SEED_NONE};
+        int open = 4;
+        for (int c = 0; c < s.nconds && open; c++) {
+            for (int o = 0; o < (s.cond[c].self ? 1 : 2); o++) {
+                bool all = true;
+                for (int k = 0; k < s.cond[c].nf; k++) {
+                    const int b = s.cond[c].blk[k];
+                    const int bit = 3 * b + (s.cond[c].d[k] == 0 ? 0 : (o == 0 ? 1 : 2));
+                    all = all && ((f >> bit) & 1u);
+                }
+                if (!all) continue;
+                for (uint32_t sd = 0; sd < 4; sd++)
+                    if (first[sd] == SEED_NONE && (s.cond[c].self || ((sd >> o) & 1u))) { first[sd] = (uint8_t)(2 * c + o); open--; }
+            }
+        }
+        for (uint32_t sd = 0; sd < 4; sd++) lut[f | sd << s.nflags] = first[sd];
     }
 }
 
