@@ -106,6 +106,9 @@ def lib():
     L.bdg_dev_tally_add.argtypes = [_vp, _vp, _vp, _sz, C.POINTER(_sz), _vp]
     L.bdg_tally_finish.argtypes = [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong)]
     L.bdg_dev_tally_finish.argtypes = [_vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong), _vp]
+    L.bdg_tally_info.argtypes = [_vp, C.POINTER(_sz), C.POINTER(C.c_ulonglong), C.POINTER(C.c_ulonglong)]
+    L.bdg_dev_tally_copy.argtypes = [_vp, _vp, _vp, _vp, _vp]
+    L.bdg_dev_tally_merge_parts.argtypes = [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _i, _i, C.c_ulonglong, C.c_ulonglong, _vp]
     L.bdg_assign_lookup32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, _vp, _vp, C.POINTER(_sz), C.POINTER(_sz)]
     L.bdg_dev_assign_lookup32.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _vp, _sz, _vp, _vp, C.POINTER(_sz), C.POINTER(_sz), _vp]
     L.bdg_part_pairs.argtypes = [_sz, _i, _i]
@@ -132,7 +135,8 @@ def lib():
                  "bdg_dev_edges_copy", "bdg_dev_assign_reads32", "bdg_dev_dedup_merge", "bdg_dev_index_edges", "bdg_dev_cluster_init",
                  "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve", "bdg_dev_whitelist_check",
                  "bdg_dev_kmer_index_create", "bdg_dev_kmer_index_query", "bdg_dev_kmer_score", "bdg_tally_create", "bdg_tally_add",
-                 "bdg_dev_tally_add", "bdg_tally_finish", "bdg_dev_tally_finish", "bdg_assign_lookup32", "bdg_dev_assign_lookup32"):
+                 "bdg_dev_tally_add", "bdg_tally_finish", "bdg_dev_tally_finish", "bdg_tally_info", "bdg_dev_tally_copy",
+                 "bdg_dev_tally_merge_parts", "bdg_assign_lookup32", "bdg_dev_assign_lookup32"):
         getattr(L, name).restype = _i
     _lib = L
     return L

@@ -1499,6 +1499,40 @@ int tally_ready(bdg_tally* h, DevCtx** out)
     return BDG_OK;
 }
 
+// One merge of the B side into the set of src_n entries in key[src] (merge path, scan of the heads, compaction into key[dst]):
+// *n_out = entries of the new set, *over = some count reached 2^32.  Waits for both.
+template <typename BSide>
+int tally_merge_step(DevCtx& c, bdg_tally* h, int src, size_t src_n, int dst, const BSide& b, uint32_t* n_out, bool* over)
+{
+    cudaStream_t st = c.stream;
+    const size_t na = src_n, M = na + b.n;          // na < 2^31 and nb < 2^31: M < 2^32
+    for (Buf* x : {&h->m_key, &h->m_head, &h->m_scan, &h->key[dst]}) if (int e = x->ensure(M * 4)) return e;
+    for (Buf* x : {&h->m_cnt, &h->m_fst, &h->cnt[dst], &h->fst[dst]}) if (int e = x->ensure(M * 8)) return e;
+    if (int e = h->flag.ensure(16)) return e;
+    size_t tmp = 0;
+    CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
+    if (int e = h->scratch.ensure(tmp)) return e;
+    unsigned int* d_flag = (unsigned int*)h->flag.p;
+    CU_TRY(cudaMemsetAsync(d_flag, 0, 4, st));
+    bdg::tally_merge_kernel<BSide><<<(unsigned)((M + bdg::TALLY_TILE - 1) / bdg::TALLY_TILE), bdg::NT, 0, st>>>(
+        (const uint32_t*)h->key[src].p, (const unsigned long long*)h->cnt[src].p, (const unsigned long long*)h->fst[src].p, na, b.key, b.x,
+        b.y, b.n, b.first_off, (uint32_t*)h->m_key.p, (unsigned long long*)h->m_cnt.p, (unsigned long long*)h->m_fst.p, (uint32_t*)h->m_head.p);
+    CU_TRY(cub::DeviceScan::InclusiveSum(h->scratch.p, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
+    const int blocks = (int)std::min<size_t>((M + 255) / 256, (size_t)c.sms * 8);
+    bdg::tally_compact_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)h->m_key.p, (const unsigned long long*)h->m_cnt.p,
+                                                      (const unsigned long long*)h->m_fst.p, (const uint32_t*)h->m_head.p,
+                                                      (const uint32_t*)h->m_scan.p, M, (uint32_t*)h->key[dst].p,
+                                                      (unsigned long long*)h->cnt[dst].p, (unsigned long long*)h->fst[dst].p, d_flag);
+    g_launches += 2;
+    CU_TRY(cudaGetLastError());
+    uint32_t over_flag = 0;
+    CU_TRY(cudaMemcpyAsync(n_out, (const uint32_t*)h->m_scan.p + (M - 1), 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(&over_flag, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    *over = over_flag != 0;
+    return BDG_OK;
+}
+
 int tally_add_core(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, cudaMemcpyKind kind, size_t* n_valid)
 {
     if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
@@ -1510,41 +1544,86 @@ int tally_add_core(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t
     if (rc) return rc;
     if (n_valid) *n_valid = nv;
     if (nv == 0) { h->rows += R; return BDG_OK; }
-    cudaStream_t st = c.stream;
     const int nx = h->cur ^ 1;
-    const size_t na = h->n, M = na + nb;            // na < 2^31 and nb < 2^31: M < 2^32
-    for (Buf* b : {&h->m_key, &h->m_head, &h->m_scan, &h->key[nx]}) if (int e = b->ensure(M * 4)) return e;
-    for (Buf* b : {&h->m_cnt, &h->m_fst, &h->cnt[nx], &h->fst[nx]}) if (int e = b->ensure(M * 8)) return e;
-    if (int e = h->flag.ensure(16)) return e;
-    size_t tmp = 0;
-    CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
-    if (int e = h->scratch.ensure(tmp)) return e;
-    unsigned int* d_flag = (unsigned int*)h->flag.p;
-    CU_TRY(cudaMemsetAsync(d_flag, 0, 4, st));
-    bdg::tally_merge_kernel<<<(unsigned)((M + bdg::TALLY_TILE - 1) / bdg::TALLY_TILE), bdg::NT, 0, st>>>(
-        (const uint32_t*)h->key[h->cur].p, (const unsigned long long*)h->cnt[h->cur].p, (const unsigned long long*)h->fst[h->cur].p, na,
-        c.map.ascending() /* batch runs ascending */, c.map.counts() /* counts, first-seen order */,
-        c.map.run_pos() /* run -> first-seen position */, nb, h->rows, (uint32_t*)h->m_key.p, (unsigned long long*)h->m_cnt.p,
-        (unsigned long long*)h->m_fst.p, (uint32_t*)h->m_head.p);
-    CU_TRY(cub::DeviceScan::InclusiveSum(h->scratch.p, tmp, (const uint32_t*)h->m_head.p, (uint32_t*)h->m_scan.p, (int64_t)M, st));
-    const int blocks = (int)std::min<size_t>((M + 255) / 256, (size_t)c.sms * 8);
-    bdg::tally_compact_kernel<<<blocks, 256, 0, st>>>((const uint32_t*)h->m_key.p, (const unsigned long long*)h->m_cnt.p,
-                                                      (const unsigned long long*)h->m_fst.p, (const uint32_t*)h->m_head.p,
-                                                      (const uint32_t*)h->m_scan.p, M, (uint32_t*)h->key[nx].p,
-                                                      (unsigned long long*)h->cnt[nx].p, (unsigned long long*)h->fst[nx].p, d_flag);
-    g_launches += 2;
-    CU_TRY(cudaGetLastError());
-    uint32_t n_out = 0, over = 0;
-    CU_TRY(cudaMemcpyAsync(&n_out, (const uint32_t*)h->m_scan.p + (M - 1), 4, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(&over, d_flag, 4, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
+    const bdg::TallyBatchSide batch{c.map.ascending() /* batch runs ascending */, c.map.counts() /* counts, first-seen order */,
+                                    c.map.run_pos() /* run -> first-seen position */, nb, h->rows};
+    uint32_t n_out = 0;
+    bool over = false;
+    if (int e = tally_merge_step(c, h, h->cur, h->n, nx, batch, &n_out, &over)) return e;
     if (n_out > 0x7FFFFFFFu)
         return fail(BDG_ERR_ARG, "the batch would take the tally to %u distinct barcodes; fewer than 2^31 are allowed (the set keeps the batches before it)", n_out);
     h->cur = nx;
     h->n = n_out;
     h->rows += R;
     h->valid += nv;
-    h->over = h->over || over != 0;
+    h->over = h->over || over;
+    return BDG_OK;
+}
+
+// The P parts' sets folded into one, part 0 first: every step merges the next part into the running union, alternating between the
+// handle's two halves.  The checks run first; a refusal after the fold began restores the handle's set from the caller's own
+// part, which the checks found equal to it entry for entry.
+int tally_merge_parts_core(DevCtx& c, bdg_tally* h, const uint32_t* d_keys, const unsigned long long* d_cnts, const unsigned long long* d_firsts,
+                           const size_t* starts, const size_t* sizes, const unsigned long long* row_offsets, int n_parts, int my_part,
+                           unsigned long long total_rows, unsigned long long total_valid)
+{
+    cudaStream_t st = c.stream;
+    auto part = [&](int p) {
+        return bdg::TallySetSide{d_keys + starts[p], d_cnts + starts[p], d_firsts + starts[p], (uint64_t)sizes[p], row_offsets[p]};
+    };
+    if (int e = h->flag.ensure(16)) return e;
+    unsigned int* d_flag = (unsigned int*)h->flag.p;
+    CU_TRY(cudaMemsetAsync(d_flag, 0, 4, st));
+    for (int p = 0; p < n_parts; p++) {
+        if (!sizes[p]) continue;
+        const bool mine = p == my_part;
+        const int blocks = (int)std::min<size_t>((sizes[p] + 255) / 256, (size_t)c.sms * 8);
+        bdg::tally_part_check_kernel<<<blocks, 256, 0, st>>>(part(p), total_rows, mine ? (const uint32_t*)h->key[h->cur].p : nullptr,
+                                                             mine ? (const unsigned long long*)h->cnt[h->cur].p : nullptr,
+                                                             mine ? (const unsigned long long*)h->fst[h->cur].p : nullptr, d_flag);
+        g_launches++;
+    }
+    CU_TRY(cudaGetLastError());
+    unsigned int bad = 0;
+    CU_TRY(cudaMemcpyAsync(&bad, d_flag, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaStreamSynchronize(st));
+    if (bad & 1u) return fail(BDG_ERR_ARG, "the barcodes of a part are not strictly ascending");
+    if (bad & 2u) return fail(BDG_ERR_ARG, "part %d is not the tally's own set", my_part);
+    if (bad & 4u) return fail(BDG_ERR_ARG, "a shifted first sighting is not below the %llu rows of all parts", total_rows);
+
+    auto restore = [&]() {
+        const size_t n = h->n, s = starts[my_part];   // key[cur] still has room for n entries: buffers only grow
+        if (n == 0) return;
+        cudaMemcpyAsync(h->key[h->cur].p, d_keys + s, n * 4, cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(h->cnt[h->cur].p, d_cnts + s, n * 8, cudaMemcpyDeviceToDevice, st);
+        cudaMemcpyAsync(h->fst[h->cur].p, d_firsts + s, n * 8, cudaMemcpyDeviceToDevice, st);
+        cudaStreamSynchronize(st);
+    };
+    int cur = h->cur;
+    size_t n = 0;
+    bool over = false;
+    for (int p = 0; p < n_parts; p++) {
+        if (!sizes[p]) continue;
+        uint32_t n_out = 0;
+        bool o = false;
+        if (int e = tally_merge_step(c, h, cur, n, cur ^ 1, part(p), &n_out, &o)) {
+            restore();
+            return e;
+        }
+        if (n_out > 0x7FFFFFFFu) {
+            restore();
+            return fail(BDG_ERR_ARG, "the parts hold %u or more distinct barcodes in all; fewer than 2^31 are allowed", n_out);
+        }
+        cur ^= 1;
+        n = n_out;
+        over = over || o;
+    }
+    h->cur = cur;
+    h->n = n;
+    h->rows = total_rows;
+    h->valid = total_valid;
+    h->over = over;                                 // from the merged counts alone: the same on every part
+    h->finished = true;                             // the set holds the other parts' batches: no batch can follow them
     return BDG_OK;
 }
 
@@ -1656,6 +1735,63 @@ int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsi
     CallerOrder order(*c, stream);
     if (int rc = order.begin()) return rc;
     return tally_finish_core(*c, h, n_distinct, n_valid, token);
+}
+
+int bdg_tally_info(bdg_tally* h, size_t* n_distinct, unsigned long long* rows, unsigned long long* valid)
+{
+    if (!n_distinct || !rows || !valid) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *rows = 0; *valid = 0;
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    *n_distinct = h->n;
+    *rows = h->rows;
+    *valid = h->valid;
+    return BDG_OK;
+}
+
+int bdg_dev_tally_copy(bdg_tally* h, uint32_t* d_key, unsigned long long* d_cnt, unsigned long long* d_first, void* stream)
+{
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    if (h->n == 0) return BDG_OK;
+    if (!d_key || !d_cnt || !d_first) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    for (const void* p : {(const void*)d_key, (const void*)d_cnt, (const void*)d_first})
+        if (int rc = check_on_first(p, "output")) return rc;
+    CallerOrder order(*c, stream);
+    if (int rc = order.begin()) return rc;
+    cudaStream_t st = c->stream;
+    CU_TRY(cudaMemcpyAsync(d_key, h->key[h->cur].p, h->n * 4, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(d_cnt, h->cnt[h->cur].p, h->n * 8, cudaMemcpyDeviceToDevice, st));
+    CU_TRY(cudaMemcpyAsync(d_first, h->fst[h->cur].p, h->n * 8, cudaMemcpyDeviceToDevice, st));
+    return BDG_OK;
+}
+
+int bdg_dev_tally_merge_parts(bdg_tally* h, const uint32_t* d_keys, const unsigned long long* d_cnts, const unsigned long long* d_firsts,
+                              const size_t* starts, const size_t* sizes, const unsigned long long* row_offsets, int n_parts, int my_part,
+                              unsigned long long total_rows, unsigned long long total_valid, void* stream)
+{
+    DevCtx* c = nullptr;
+    if (int rc = tally_ready(h, &c)) return rc;
+    if (h->finished) return fail(BDG_ERR_ARG, "merge after finish: the tally is closed");
+    if (n_parts < 1 || my_part < 0 || my_part >= n_parts || !starts || !sizes || !row_offsets)
+        return fail(BDG_ERR_ARG, "need 0 <= my_part < n_parts and the parts' starts / sizes / row offsets");
+    if (sizes[my_part] != h->n) return fail(BDG_ERR_ARG, "part %d has %zu barcodes, the tally's set %zu", my_part, sizes[my_part], h->n);
+    if (total_rows < h->rows || total_valid < h->valid || total_valid > total_rows)
+        return fail(BDG_ERR_ARG, "%llu rows / %llu valid rows in all, but the tally alone added %llu / %llu", total_rows, total_valid,
+                    h->rows, h->valid);
+    size_t total = 0;
+    for (int p = 0; p < n_parts; p++) {
+        if (sizes[p] > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "part %d has %zu barcodes; fewer than 2^31 are allowed", p, sizes[p]);
+        total += sizes[p];
+    }
+    if (total) {
+        if (!d_keys || !d_cnts || !d_firsts) return fail(BDG_ERR_ARG, "NULL pointer argument");
+        for (const void* p : {(const void*)d_keys, (const void*)d_cnts, (const void*)d_firsts})
+            if (int rc = check_on_first(p, "merge input")) return rc;
+    }
+    CallerOrder order(*c, stream);
+    if (int rc = order.begin()) return rc;
+    return tally_merge_parts_core(*c, h, d_keys, d_cnts, d_firsts, starts, sizes, row_offsets, n_parts, my_part, total_rows, total_valid);
 }
 
 // ---- a-6 / centre selection, barcode_graph.py:252-267, over the distinct barcodes a dedup call left on the device ----

@@ -7,7 +7,7 @@
 //   kmer_unpack_kernel   packed position counts -> uint8[hits][11] (device form of a-5)        HBM bound
 //   member_kernel        sorted-whitelist membership (smem pivots + L2-resident search)       HBM/L2 bound
 //   pack16_kernel        16 ASCII bases -> 2-bit packed uint32 + validity                     HBM bound
-//   tally_merge_kernel   merge path of the running distinct set and a batch's distinct list   HBM bound
+//   tally_merge_kernel<B> merge path of the running distinct set and a batch's list / another set  HBM bound
 //   lookup_assign32_kernel  per-read centre for rows outside a read map (smem pivots + search)  L2/HBM bound
 //   pipe_probe_kernel    LOP3 / IMAD / POPC issue-rate probe for the integer roofline
 //
@@ -482,16 +482,52 @@ __global__ void merge_remap_kernel(uint32_t* __restrict__ read_to_distinct, uint
 //                        finds where that stretch of the merged order starts and ends in A and B (two binary searches along the
 //                        cross diagonals), stages both key ranges in shared memory, and every thread merges TALLY_ITEMS outputs
 //                        from its own diagonal.  Ties take A first, so a barcode the set already holds is followed directly by
-//                        the batch's entry of it, which is flagged as no head.  The batch's entry of run r: key b_key[r], count
-//                        b_count[b_pos[r]], first-sighting key first_off + b_pos[r] (its first-seen position in the batch).
+//                        the batch's entry of it, which is flagged as no head.  B is read through an accessor (template
+//                        parameter): TallyBatchSide, a batch's dedup output, or TallySetSide, the set of another tally
+//                        (bdg_dev_tally_merge_parts folds the sets of P ranks one by one; each set is distinct, so a head is still
+//                        followed by at most one non-head).
 //   (inclusive scan of the heads: the position of every run in the new set)
 //   tally_compact_kernel one entry per head, the count of a following non-head added in; counts of 2^32 or more are flagged
 //   (radix sort of the set by first-sighting key at tally_finish: the global first-seen order)
 //   tally_finish_kernel  distinct / counts (uint32) / first-seen -> ascending position, the read-map arrays of a dedup call
+//   tally_part_check_kernel  the checks of bdg_dev_tally_merge_parts on one part before the fold
 // HBM bound: 20 B in and 24 B out per merged entry, then 24 B in and 20 B out per entry of the new set.
 // ---------------------------------------------------------------------------------------------------
 constexpr int TALLY_ITEMS = 8;
 constexpr int TALLY_TILE = NT * TALLY_ITEMS;
+
+// B of the merge: n entries, key[j] the j-th smallest barcode; at(j) locates entry j in the arrays x and y, count(at(j)) and
+// first(at(j)) are its count and first-sighting key.  The kernel takes key, x, y, n and first_off as separate parameters, in the
+// batch form's former order and types, so the batch form compiles as before.
+// A batch's dedup output: y[j] is run j's first-seen position in the batch, x the counts in first-seen order, first_off the rows
+// added before the batch.
+struct TallyBatchSide {
+    using X = uint32_t;
+    using Y = uint32_t;
+    const uint32_t* key;
+    const X* x;
+    const Y* y;
+    uint64_t n;
+    unsigned long long first_off;
+    __device__ __forceinline__ uint32_t at(uint64_t j) const { return __ldg(&y[j]); }
+    __device__ __forceinline__ unsigned long long count(uint32_t p) const { return __ldg(&x[p]); }
+    __device__ __forceinline__ unsigned long long first(uint32_t p) const { return first_off + p; }
+};
+
+// The running set of another tally: 64-bit counts x, 64-bit first-sighting keys y, shifted by first_off (the rows of the parts
+// before it).
+struct TallySetSide {
+    using X = unsigned long long;
+    using Y = unsigned long long;
+    const uint32_t* key;
+    const X* x;
+    const Y* y;
+    uint64_t n;
+    unsigned long long first_off;
+    __device__ __forceinline__ uint64_t at(uint64_t j) const { return j; }
+    __device__ __forceinline__ unsigned long long count(uint64_t j) const { return __ldg(&x[j]); }
+    __device__ __forceinline__ unsigned long long first(uint64_t j) const { return first_off + __ldg(&y[j]); }
+};
 
 // number of A entries among the first d outputs of the merge (ties: A first)
 template <typename GetA, typename GetB>
@@ -505,15 +541,17 @@ __device__ __forceinline__ uint64_t merge_path_split(uint64_t d, uint64_t na, ui
     return lo;
 }
 
+template <typename BSide>
 __global__ void __launch_bounds__(NT) tally_merge_kernel(const uint32_t* __restrict__ a_key, const unsigned long long* __restrict__ a_cnt,
                                                          const unsigned long long* __restrict__ a_first, uint64_t na,
-                                                         const uint32_t* __restrict__ b_key, const uint32_t* __restrict__ b_count,
-                                                         const uint32_t* __restrict__ b_pos, uint64_t nb, unsigned long long first_off,
+                                                         const uint32_t* __restrict__ b_key, const typename BSide::X* __restrict__ b_x,
+                                                         const typename BSide::Y* __restrict__ b_y, uint64_t nb, unsigned long long first_off,
                                                          uint32_t* __restrict__ m_key, unsigned long long* __restrict__ m_cnt,
                                                          unsigned long long* __restrict__ m_first, uint32_t* __restrict__ m_head)
 {
     __shared__ uint32_t s_key[TALLY_TILE];
     __shared__ uint64_t s_split[2];
+    const BSide b{b_key, b_x, b_y, nb, first_off};
     const uint64_t M = na + nb;
     const uint64_t d0 = (uint64_t)blockIdx.x * TALLY_TILE, d1 = min(M, d0 + TALLY_TILE);
     auto ga = [&](uint64_t i) { return __ldg(&a_key[i]); };
@@ -546,11 +584,11 @@ __global__ void __launch_bounds__(NT) tally_merge_kernel(const uint32_t* __restr
             any_a = true;
             i++;
         } else {
-            const uint64_t bj = b0 + j;
-            const uint32_t k = sb[j], p = __ldg(&b_pos[bj]);
+            const uint32_t k = sb[j];
+            const auto p = b.at(b0 + j);
             m_key[g] = k;
-            m_cnt[g] = __ldg(&b_count[p]);
-            m_first[g] = first_off + p;
+            m_cnt[g] = b.count(p);
+            m_first[g] = b.first(p);
             m_head[g] = (any_a && prev_a == k) ? 0u : 1u;
             j++;
         }
@@ -576,6 +614,23 @@ __global__ void tally_compact_kernel(const uint32_t* __restrict__ m_key, const u
         first[r] = f;
         if (c >> 32) *over = 1u;
     }
+}
+
+// One part of bdg_dev_tally_merge_parts: bit 1 of *bad when its keys are not strictly ascending, bit 4 when a shifted first key is
+// not below the total rows; when own_key is given (the caller's own part), bit 2 when an entry differs from the handle's set.
+__global__ void tally_part_check_kernel(const TallySetSide b, unsigned long long rows, const uint32_t* __restrict__ own_key,
+                                        const unsigned long long* __restrict__ own_cnt, const unsigned long long* __restrict__ own_first,
+                                        unsigned int* __restrict__ bad)
+{
+    unsigned int f = 0;
+    for (uint64_t j = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; j < b.n; j += (uint64_t)gridDim.x * blockDim.x) {
+        const uint32_t k = __ldg(&b.key[j]);
+        const unsigned long long c = b.count(j), first = b.first(j);
+        if (j > 0 && __ldg(&b.key[j - 1]) >= k) f |= 1u;
+        if (first >= rows || first < b.first_off) f |= 4u;
+        if (own_key && (__ldg(&own_key[j]) != k || __ldg(&own_cnt[j]) != c || __ldg(&own_first[j]) + b.first_off != first)) f |= 2u;
+    }
+    if (f) atomicOr(bad, f);
 }
 
 // order[p] = ascending position of the barcode with the p-th smallest first-sighting key

@@ -14,9 +14,19 @@
 Nothing per read is exchanged.  Concatenated in rank order, the results equal those of device.assign_packed (and
 pipeline.assign_packed(form="u32")) run in one process on the concatenation of the ranks' inputs in rank order.
 
-Every call is collective: all ranks of the group make it, with the same scalar arguments.  Which collectives run depends only on
-those arguments and on values reduced over the group, never on a rank's own reads, so a rank with no rows, or with no valid row,
-takes part like any other.  Collectives run on CUDA tensors in the order of torch.cuda.current_stream() (NCCL or gloo).
+`Tally` is the same step for reads that every rank adds in batches (device.Tally on each rank):
+
+    every rank                                   what crosses between the ranks
+      add: bdg_dev_tally_add of its own batches    -   (rank-local, any number of batches)
+      finish: bdg_tally_info                       all-gather of the status, set size, rows, valid rows and scalar arguments
+      bdg_dev_tally_copy of its running set        all-gather of the sets padded to the longest (20 B per entry per rank)
+      bdg_dev_tally_merge_parts, bdg_dev_tally_finish   -   (the union in rank-major order, the same on every rank)
+      run_stages: edges, centres, rounds, --high_sens   as for assign_packed above
+      assign: bdg_dev_assign_lookup32 of any rows  -   (rank-local)
+
+Every call of assign_packed, and Tally.finish, is collective: all ranks of the group make it, with the same scalar arguments.
+Which collectives run depends only on those arguments and on values reduced over the group, never on a rank's own reads, so a rank
+with no rows, or with no valid row, takes part like any other.  Collectives run on CUDA tensors in the order of torch.cuda.current_stream() (NCCL or gloo).
 """
 from __future__ import annotations
 
@@ -148,43 +158,24 @@ def cluster_levels(sorted_distinct: torch.Tensor, ea: torch.Tensor, eb: torch.Te
     return ci, lv
 
 
-def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, threshold, n_cells, interval=25, whitelist_sorted=None,
-                  true_barcodes=None, high_sens=False, centre_order=None, group=None, timings=None):
-    """device.assign_packed over the ranks of `group` (None: the default group; no initialised process group: a world of one).
-    Called on every rank with that rank's reads (ranks / valid: CUDA tensors on the first device given to badger_b200.init, as
-    for device.assign_packed) and the same scalar arguments; whitelist_sorted and true_barcodes are the same on every rank.
-    Returns ((centre, has_centre), info) for the rank's own rows.  Concatenated in rank order, the results of all ranks equal
-    device.assign_packed run in one process on the concatenation of their inputs in rank order (first-seen order therefore
-    starts with rank 0's reads), and `info` - the same on every rank - equals its `info`.
-
-    With high_sens, rank 0 runs the per-barcode --high_sens work of pipeline.assign_packed on the host and broadcasts the result;
-    centre_order="set" is the set order of rank 0's process.  timings: a dict that receives the host time of every stage, each
-    stage ended by a device synchronise, and under "collective_bytes" the bytes each kind of collective delivered to this rank."""
-    bd._ready()
-    bd._check(ranks, "ranks", bd.BARCODE_DTYPES)
-    if whitelist_sorted is not None:
-        bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
-    if isinstance(true_barcodes, torch.Tensor):
-        true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+def _ticker(timings):
+    """tick(name, t0): adds the host time since t0 to timings[name], after a device synchronise (nothing without timings)."""
     T = timings if timings is not None else {}
-    g = _Group(group, T.setdefault("collective_bytes", {}) if timings is not None else None)
-    R, dev = ranks.numel(), ranks.device
 
     def tick(name, t0):
         if timings is not None:
-            torch.cuda.synchronize(dev)
+            torch.cuda.synchronize(bd._device())
         pipeline._tick(T, name, t0)
+    return tick
 
-    t0 = time.perf_counter()
-    rm = bd.dedup_reads(ranks, valid)
-    tick("dedup_first_seen", t0)
 
-    t0 = time.perf_counter()
-    merged, total_valid, total_rows = dedup_merge(rm, _g=g)
-    tick("exchange_merge", t0)
-    info = {"reads": total_rows, "valid_reads": total_valid}
-    if merged is None:
-        return (torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)), info
+def run_stages(merged, g, info, timings, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order):
+    """The stages after the merge of the ranks' barcodes, over the global read map `merged` (a DeviceReadMap with at least one
+    valid read, the same on every rank): edges (part `rank` of `world`), centres, the clustering rounds and --high_sens on rank 0.
+    Collective over `g` (a _Group).  Fills `info` and the timings; returns (centre_idx int32[N] tensor, info), centre_idx the same
+    on every rank."""
+    tick = _ticker(timings)
+    dev = bd._device()
     N = merged.n_distinct
 
     t0 = time.perf_counter()
@@ -215,6 +206,46 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
             ci.copy_(torch.from_numpy(patched))
         g.broadcast_from_first(ci, "high_sens")
         tick("high_sens", t0)
+    return ci, info
+
+
+def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, threshold, n_cells, interval=25, whitelist_sorted=None,
+                  true_barcodes=None, high_sens=False, centre_order=None, group=None, timings=None):
+    """device.assign_packed over the ranks of `group` (None: the default group; no initialised process group: a world of one).
+    Called on every rank with that rank's reads (ranks / valid: CUDA tensors on the first device given to badger_b200.init, as
+    for device.assign_packed) and the same scalar arguments; whitelist_sorted and true_barcodes are the same on every rank.
+    Returns ((centre, has_centre), info) for the rank's own rows.  Concatenated in rank order, the results of all ranks equal
+    device.assign_packed run in one process on the concatenation of their inputs in rank order (first-seen order therefore
+    starts with rank 0's reads), and `info` - the same on every rank - equals its `info`.
+
+    With high_sens, rank 0 runs the per-barcode --high_sens work of pipeline.assign_packed on the host and broadcasts the result;
+    centre_order="set" is the set order of rank 0's process.  timings: a dict that receives the host time of every stage, each
+    stage ended by a device synchronise, and under "collective_bytes" the bytes each kind of collective delivered to this rank."""
+    bd._ready()
+    bd._check(ranks, "ranks", bd.BARCODE_DTYPES)
+    if whitelist_sorted is not None:
+        bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
+    if isinstance(true_barcodes, torch.Tensor):
+        true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+    T = timings if timings is not None else {}
+    g = _Group(group, T.setdefault("collective_bytes", {}) if timings is not None else None)
+    R, dev = ranks.numel(), ranks.device
+    tick = _ticker(timings)
+
+    t0 = time.perf_counter()
+    rm = bd.dedup_reads(ranks, valid)
+    tick("dedup_first_seen", t0)
+
+    t0 = time.perf_counter()
+    merged, total_valid, total_rows = dedup_merge(rm, _g=g)
+    tick("exchange_merge", t0)
+    info = {"reads": total_rows, "valid_reads": total_valid}
+    if merged is None:
+        return (torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)), info
+    N = merged.n_distinct
+
+    ci, info = run_stages(merged, g, info, timings, threshold=threshold, n_cells=n_cells, interval=interval,
+                          whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order)
 
     t0 = time.perf_counter()
     centre = torch.zeros(R, dtype=ranks.dtype, device=dev)
@@ -226,3 +257,104 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
     info["assigned_reads"] = int(n_assigned.item())
     tick("gather", t0)
     return (centre, has), info
+
+
+class Tally(bd.Tally):
+    """device.Tally over the ranks of `group` (None: the default group; no initialised process group: a world of one, which
+    equals device.Tally).  Every rank adds its own batches; finish merges the ranks' running sets on the device.
+
+    add(ranks, valid=None) and assign(ranks, valid=None) are rank-local, as in device.Tally: a rank may add any number of batches
+    (none too), and assign any rows, another rank's included.  finish(...) is collective: every rank of the group calls it with the
+    same scalar arguments, the same whitelist and the same true barcodes.  The result equals pipeline.assign_packed(form="u32")
+    run in one process on the rank-major concatenation of the batches: rank 0's batches in add order, then rank 1's, ...  So
+    first-seen order, count ties and the n_cells cutoff start with rank 0's first batch; with high_sens, rank 0 patches and
+    broadcasts, and centre_order="set" is the set order of rank 0's process.  `info` is that process's info on every rank, except
+    "assigned_reads": 0 after finish, then the rows with a centre of this rank's assign calls (summed over the ranks: the
+    one-process figure).
+
+    A refusal is decided from data that is the same on every rank: a rank-local problem (a freed tally, a bad argument, a finish
+    on some ranks only) travels in the first all-gather of finish, and every rank raises."""
+
+    def __init__(self, group=None):
+        super().__init__()
+        self._group = group
+        self._totals = None           # (rows, valid rows) of all ranks once finish merged the sets
+
+    def finish(self, *, threshold, n_cells, interval=25, whitelist_sorted=None, true_barcodes=None, high_sens=False, centre_order=None,
+               timings=None) -> dict:
+        """Steps: (1) all-gather of every rank's status, set size, rows and scalar arguments; (2) all-gather of the sets
+        (bdg_dev_tally_copy, padded to the longest); (3) bdg_dev_tally_merge_parts; (4) bdg_dev_tally_finish; (5) run_stages.  The
+        node -> centre array stays on the device for assign.  timings: as for assign_packed, with "exchange_merge",
+        "tally_finish", "edges", "centres", "cluster", "high_sens" and "collective_bytes"."""
+        T = timings if timings is not None else {}
+        g = _Group(self._group, T.setdefault("collective_bytes", {}) if timings is not None else None)
+        dev, tick, L = bd._device(), _ticker(timings), lib()
+
+        t0 = time.perf_counter()
+        err, status, own = None, 0, [0, 0, 0]
+        scalars = [0, 0, 0, 0]
+        try:
+            h = self._handle()
+            scalars = [int(threshold), int(n_cells), int(interval), int(bool(high_sens))]
+            if whitelist_sorted is not None:
+                bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
+            if isinstance(true_barcodes, torch.Tensor):
+                true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+            n, rows, valid = C.c_size_t(0), C.c_ulonglong(0), C.c_ulonglong(0)
+            check(L.bdg_tally_info(h, C.byref(n), C.byref(rows), C.byref(valid)))
+            own = [int(n.value), int(rows.value), int(valid.value)] if self._totals is None else [0, *self._totals]
+        except _lib.BadgerB200Error as e:
+            err, status = e, 2
+        except (TypeError, ValueError) as e:
+            err, status = e, 1
+        meta = torch.tensor([status, int(self._totals is not None)] + own + scalars, dtype=torch.int64, device=dev)
+        metas = g.all_gather(meta, "sizes").cpu()                     # host wait: the sizes decide the shapes below
+        refused = [r for r in range(g.world) if metas[r, 0]]
+        if refused:
+            if err is not None:
+                raise err
+            msg = "finish was refused on rank(s) %s" % refused
+            if int(metas[refused[0], 0]) == 2:
+                raise _lib.BadgerB200Error(_lib.BDG_ERR_ARG, msg)
+            raise ValueError(msg)
+        if not bool((metas[:, 5:] == metas[0, 5:]).all()):
+            raise ValueError("the ranks called finish with different threshold / n_cells / interval / high_sens")
+        if not bool((metas[:, 1] == metas[0, 1]).all()):
+            raise ValueError("finish ran before on some ranks only")
+        if self._totals is not None:                                  # a second finish: the handle holds the union already
+            total_rows, total_valid = int(metas[0, 3]), int(metas[0, 4])
+        else:
+            sizes = [int(x) for x in metas[:, 2]]
+            rows = [int(x) for x in metas[:, 3]]
+            total_rows, total_valid = sum(rows), int(metas[:, 4].sum())
+            if total_valid:
+                width = max(sizes)
+                key = torch.empty(width, dtype=torch.int32, device=dev)
+                cnt = torch.empty(width, dtype=torch.int64, device=dev)
+                first = torch.empty(width, dtype=torch.int64, device=dev)
+                with torch.cuda.device(dev):
+                    check(L.bdg_dev_tally_copy(h, key.data_ptr(), cnt.data_ptr(), first.data_ptr(), bd._stream()))
+                keys, cnts, firsts = (g.all_gather(x, "sets") for x in (key, cnt, first))     # [world, width] each
+                offsets = np.concatenate([[0], np.cumsum(rows)[:-1]]).tolist()
+                with torch.cuda.device(dev):
+                    check(L.bdg_dev_tally_merge_parts(h, keys.data_ptr(), cnts.data_ptr(), firsts.data_ptr(),
+                                                      (C.c_size_t * g.world)(*[width * p for p in range(g.world)]),
+                                                      (C.c_size_t * g.world)(*sizes), (C.c_ulonglong * g.world)(*offsets), g.world,
+                                                      g.rank, total_rows, total_valid, bd._stream()))
+            self._totals = (total_rows, total_valid)
+        tick("exchange_merge", t0)
+
+        t0 = time.perf_counter()
+        n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
+        self._finish_call(n, nv, tok)                                 # a merged count of 2^32 or more: refused on every rank
+        tick("tally_finish", t0)
+        self.info = info = {"reads": total_rows, "valid_reads": total_valid}
+        self._rm, self._ci = None, None
+        if total_valid == 0:
+            return info
+        rm = bd.DeviceReadMap(int(n.value), int(nv.value), 0, int(tok.value), torch.int32)
+        ci, info = run_stages(rm, g, info, timings, threshold=threshold, n_cells=n_cells, interval=interval,
+                              whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order)
+        info["assigned_reads"] = 0
+        self._rm, self._ci = rm, ci
+        return info

@@ -298,6 +298,23 @@ int bdg_dev_dedup_merge(unsigned long long token, const uint32_t* d_keys, const 
  *                 bdg_assign_reads32; *n_assigned = rows with a centre, *n_missing = valid rows whose barcode is no node (their
  *                 has_centre is 0).  Any token works, a dedup call's too.  The device form waits only when n_assigned or
  *                 n_missing is given.
+ *   tally_info    *n_distinct = barcodes in the running set, *rows / *valid = rows and valid rows added so far.
+ * Over P processes (badger_b200.distributed.Tally), every process adds its own batches to its own tally; then the P sets become
+ * one.  The merge order is RANK-MAJOR: part 0's batches in add order, then part 1's, ...  The result equals one tally that added
+ * that concatenation of batches.
+ *   dev_tally_copy  the running set, ascending, into device buffers of tally_info's *n_distinct entries: barcodes, counts and
+ *                 first sightings (the rows added before the batch of the first sighting + the barcode's first-seen position in it).
+ *   dev_tally_merge_parts  replaces the set with the union of the P parts' sets.  d_keys / d_cnts / d_firsts: device memory on the
+ *                 first claimed device; part p's set has sizes[p] entries at index starts[p] of each array (host arrays of n_parts,
+ *                 as bdg_dev_tally_copy wrote them), and its first sightings are shifted by row_offsets[p], the rows of the parts
+ *                 before it.  Counts are summed, and the smallest shifted first sighting is kept.  *rows / *valid of the handle become
+ *                 total_rows / total_valid, so that finish sorts the first sightings of all parts.  The parts are folded into the
+ *                 set one by one, part 0 first (a merge path over every entry of the running union per part).  BDG_ERR_ARG, with
+ *                 the set as it was, for a part whose barcodes are not strictly ascending or whose shifted first sightings are not
+ *                 below total_rows, a part my_part that is not this handle's set (size, and every entry on the device), a union of
+ *                 2^31 barcodes or more, a finished handle, and pointers off the first claimed device.  A merged count of 2^32 or
+ *                 more is not refused here: tally_finish refuses it, on every part alike.  After the merge the tally takes no
+ *                 more batches and no second merge; tally_finish follows.  Waits for the size of every step.
  * The bdg_dev_* forms take pointers on the first claimed device and order their work against `stream` as the correction-step
  * device forms above do. */
 typedef struct bdg_tally bdg_tally;
@@ -307,6 +324,11 @@ int bdg_tally_add(bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, siz
 int bdg_dev_tally_add(bdg_tally* h, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R, size_t* n_valid, void* stream);
 int bdg_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token);
 int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, void* stream);
+int bdg_tally_info(bdg_tally* h, size_t* n_distinct, unsigned long long* rows, unsigned long long* valid);
+int bdg_dev_tally_copy(bdg_tally* h, uint32_t* d_key, unsigned long long* d_cnt, unsigned long long* d_first, void* stream);
+int bdg_dev_tally_merge_parts(bdg_tally* h, const uint32_t* d_keys, const unsigned long long* d_cnts, const unsigned long long* d_firsts,
+                              const size_t* starts, const size_t* sizes, const unsigned long long* row_offsets, int n_parts, int my_part,
+                              unsigned long long total_rows, unsigned long long total_valid, void* stream);
 int bdg_assign_lookup32(unsigned long long token, const int32_t* centre_idx, size_t N, const uint32_t* ranks, const uint8_t* valid, size_t R,
                         uint32_t* centre, uint8_t* has_centre, size_t* n_assigned, size_t* n_missing);
 int bdg_dev_assign_lookup32(unsigned long long token, const int32_t* d_centre_idx, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid,
