@@ -64,6 +64,35 @@ def _check_records(seqs, name):
         raise ValueError("%s must start on a 16-byte boundary" % name)
 
 
+def _rows(ranks, valid):
+    """Reject barcodes per row, or their validity mask (None: all rows valid), that the library cannot take; returns them."""
+    _check(ranks, "ranks", BARCODE_DTYPES)
+    if valid is not None:
+        _check(valid, "valid", MASK_DTYPES)
+        if valid.numel() != ranks.numel():
+            raise ValueError("valid has %d rows, ranks %d" % (valid.numel(), ranks.numel()))
+    return ranks, valid
+
+
+def _check_whitelist(whitelist_sorted):
+    if whitelist_sorted is not None:
+        _check(whitelist_sorted, "whitelist_sorted", BARCODE_DTYPES)
+    return whitelist_sorted
+
+
+def _true_barcodes(true_barcodes):
+    """--true_barcodes as pipeline.select_centres takes them: a tensor becomes the list of its uint32 values."""
+    if isinstance(true_barcodes, torch.Tensor):
+        return (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+    return true_barcodes
+
+
+def _zeros(ranks):
+    """The result of rows none of which has a centre: (centre[R] in the dtype of ranks, has_centre bool[R]), all zero."""
+    R, dev = ranks.numel(), ranks.device
+    return torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)
+
+
 def _ready():
     """The library's contexts, claimed the way the host operators claim them when nobody called init()."""
     if lib().bdg_device_count() == 0:
@@ -182,12 +211,8 @@ def dedup_reads(ranks: torch.Tensor, valid: torch.Tensor | None = None) -> Devic
     """barcode_graph.py:192-204 over the rows with valid[i] (None: all), as ops.dedup_reads: everything it produces stays on the
     device under the token until the next dedup call; the caller's tensors are free again when it returns."""
     _ready()
-    _check(ranks, "ranks", BARCODE_DTYPES)
+    _rows(ranks, valid)
     R = ranks.numel()
-    if valid is not None:
-        _check(valid, "valid", MASK_DTYPES)
-        if valid.numel() != R:
-            raise ValueError("valid has %d rows, ranks %d" % (valid.numel(), R))
     n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
     if R:
         check(lib().bdg_dev_dedup_reads(ranks.data_ptr(), _ptr(valid), R, C.byref(n), C.byref(nv), C.byref(tok), _stream()))
@@ -197,9 +222,7 @@ def dedup_reads(ranks: torch.Tensor, valid: torch.Tensor | None = None) -> Devic
 def centres_above(rmap, n_cells: int, whitelist_sorted: torch.Tensor | None = None):
     """ops.centres_above with the sorted whitelist in a tensor on the first device; the result (a few thousand barcodes) is on
     the host, where walk_centres runs."""
-    wl = whitelist_sorted
-    if wl is not None:
-        _check(wl, "whitelist_sorted", BARCODE_DTYPES)
+    wl = _check_whitelist(whitelist_sorted)
     cap = 1 << 16
     while True:
         top = np.empty(cap, np.uint32); cnt = np.empty(cap, np.uint32)
@@ -228,10 +251,8 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
     pipeline.assign_packed."""
     _ready()
     _check(ranks, "ranks", BARCODE_DTYPES)
-    if whitelist_sorted is not None:
-        _check(whitelist_sorted, "whitelist_sorted", BARCODE_DTYPES)
-    if isinstance(true_barcodes, torch.Tensor):
-        true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+    _check_whitelist(whitelist_sorted)
+    true_barcodes = _true_barcodes(true_barcodes)
     T = timings if timings is not None else {}
     R, dev = ranks.numel(), ranks.device
     info = {"reads": int(R)}
@@ -240,7 +261,7 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
     pipeline._tick(T, "dedup_first_seen", t0)
     info["valid_reads"] = int(rm.n_valid)
     if rm.n_valid == 0:
-        return (torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)), info
+        return _zeros(ranks), info
 
     def gather(ci):
         # ci: None (the clustering result on the device) or, with high_sens, the patched centre index per node from the host
@@ -252,7 +273,7 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
                                            _stream()))
         return (centre, has), int(n.value)
 
-    out = pipeline.run_stages(rm.host, info, T, gather, threshold=threshold, n_cells=n_cells, interval=interval,
+    out = pipeline.run_stages(rm.host, info, T, pipeline._OneProcess(), gather, threshold=threshold, n_cells=n_cells, interval=interval,
                               whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens,
                               centre_order=centre_order, centres_above=centres_above)
     return out, info
@@ -260,62 +281,44 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
 
 class Tally(pipeline.Tally):
     """pipeline.Tally on tensors: add(ranks, valid=None) and assign(ranks, valid=None) take tensors on the first device (checked
-    as dedup_reads checks them); assign returns (centre[R] in the dtype of its ranks, has_centre bool[R]).  Nothing of size R or
-    N crosses PCIe in add or assign; with high_sens the patched node -> centre array is uploaded once, by finish."""
+    as dedup_reads checks them); assign returns (centre[R] in the dtype of its ranks, has_centre bool[R]).  finish takes
+    whitelist_sorted as a tensor on the first device and true_barcodes as an iterable or a tensor.  Nothing of size R or N
+    crosses PCIe in add or assign; with high_sens the patched node -> centre array is uploaded once, by finish."""
 
     _centres_above = staticmethod(centres_above)
+    _rows = staticmethod(_rows)
+    _zeros = staticmethod(_zeros)
 
     def __init__(self):
         _ready()
         super().__init__()
 
     def add(self, ranks: torch.Tensor, valid: torch.Tensor | None = None) -> int:
-        _check(ranks, "ranks", BARCODE_DTYPES)
+        _rows(ranks, valid)
         R = ranks.numel()
-        _check_valid(valid, R)
         nv = C.c_size_t(0)
         check(lib().bdg_dev_tally_add(self._handle(), _ptr(ranks), _ptr(valid), R, C.byref(nv), _stream()))
         self.rows += R
         return int(nv.value)
 
-    def finish(self, *, true_barcodes=None, **kw) -> dict:
-        """pipeline.Tally.finish; whitelist_sorted is a tensor on the first device, true_barcodes an iterable or a tensor."""
-        if isinstance(true_barcodes, torch.Tensor):
-            true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
-        return super().finish(true_barcodes=true_barcodes, **kw)
+    def _close(self, stages, T, args):
+        args["true_barcodes"] = _true_barcodes(args["true_barcodes"])
+        return super()._close(stages, T, args)
 
     def _finish_call(self, n, nv, tok):
         check(lib().bdg_dev_tally_finish(self._handle(), C.byref(n), C.byref(nv), C.byref(tok), _stream()))
 
     def _upload(self, ci):
-        return torch.from_numpy(np.ascontiguousarray(ci, dtype=np.int32)).to(_device())
+        return torch.as_tensor(ci, dtype=torch.int32, device=_device())
 
-    def assign(self, ranks: torch.Tensor, valid: torch.Tensor | None = None):
-        rm = self._ready_to_assign()
-        _check(ranks, "ranks", BARCODE_DTYPES)
+    def _lookup(self, rm, ranks, valid):
         R, dev = ranks.numel(), ranks.device
-        _check_valid(valid, R)
-        if rm is None:                                        # nothing was counted: only rows without a barcode can be assigned
-            n_valid = R if valid is None else int(torch.count_nonzero(valid))
-            if n_valid:
-                raise ValueError("%d valid rows have a barcode that was never added" % n_valid)
-            return torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)
         centre = torch.empty(R, dtype=ranks.dtype, device=dev)
         has = torch.empty(R, dtype=torch.bool, device=dev)
         na, nm = C.c_size_t(0), C.c_size_t(0)
         check(lib().bdg_dev_assign_lookup32(rm.token, _ptr(self._ci), rm.n_distinct, _ptr(ranks), _ptr(valid), R, _ptr(centre), _ptr(has),
                                             C.byref(na), C.byref(nm), _stream()))
-        if nm.value:
-            raise ValueError("%d valid rows have a barcode that was never added" % nm.value)
-        self.info["assigned_reads"] += int(na.value)
-        return centre, has
-
-
-def _check_valid(valid, R):
-    if valid is not None:
-        _check(valid, "valid", MASK_DTYPES)
-        if valid.numel() != R:
-            raise ValueError("valid has %d rows, ranks %d" % (valid.numel(), R))
+        return centre, has, int(na.value), int(nm.value)
 
 
 # ---------------------------------------------------------------------------------------------- the whitelist operators

@@ -158,55 +158,30 @@ def cluster_levels(sorted_distinct: torch.Tensor, ea: torch.Tensor, eb: torch.Te
     return ci, lv
 
 
-def _ticker(timings):
-    """tick(name, t0): adds the host time since t0 to timings[name], after a device synchronise (nothing without timings)."""
-    T = timings if timings is not None else {}
+class _GroupStages:
+    """The stages of pipeline.run_stages over the group: part `rank` of `world` of the edges on every rank and an all-reduce of
+    their count, the clustering rounds of cluster_levels, --high_sens on rank 0 and a broadcast.  `g` holds the group of one
+    call; with timings, every stage ends in a device synchronise."""
 
-    def tick(name, t0):
-        if timings is not None:
-            torch.cuda.synchronize(bd._device())
-        pipeline._tick(T, name, t0)
-    return tick
+    def __init__(self, group, timings):
+        self.g = _Group(group, timings.setdefault("collective_bytes", {}) if timings is not None else None)
+        self.sync = (lambda: torch.cuda.synchronize(bd._device())) if timings is not None else None
 
+    def edges(self, rm, threshold):
+        g = self.g
+        self.a, self.b, _ = bd.edges(rm.sorted_distinct, threshold, part=g.rank, nparts=g.world)
+        n_edges = g.all_reduce(torch.tensor([self.a.numel()], dtype=torch.int64, device=bd._device()), dist.ReduceOp.SUM, "counts")
+        return int(n_edges.item())
 
-def run_stages(merged, g, info, timings, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order):
-    """The stages after the merge of the ranks' barcodes, over the global read map `merged` (a DeviceReadMap with at least one
-    valid read, the same on every rank): edges (part `rank` of `world`), centres, the clustering rounds and --high_sens on rank 0.
-    Collective over `g` (a _Group).  Fills `info` and the timings; returns (centre_idx int32[N] tensor, info), centre_idx the same
-    on every rank."""
-    tick = _ticker(timings)
-    dev = bd._device()
-    N = merged.n_distinct
+    def rounds(self, rm, centres, want_ci):
+        ci, lv = cluster_levels(rm.sorted_distinct, self.a, self.b, centres, _g=self.g)
+        del self.a, self.b
+        return ci, int(((lv != 255) & (lv != 0)).sum().item())
 
-    t0 = time.perf_counter()
-    s = merged.sorted_distinct                                        # the global nodes, ascending, on every rank
-    a, b, _ = bd.edges(s, threshold, part=g.rank, nparts=g.world)
-    n_edges = g.all_reduce(torch.tensor([a.numel()], dtype=torch.int64, device=dev), dist.ReduceOp.SUM, "counts")
-    info.update(distinct=int(N), edges=int(n_edges.item()))
-    tick("edges", t0)
-
-    t0 = time.perf_counter()
-    centres = np.asarray(list(dict.fromkeys(pipeline.select_centres(merged, n_cells, interval, whitelist_sorted, true_barcodes,
-                                                                    bd.centres_above))), dtype=np.uint32)
-    info["centres"] = int(centres.size)
-    tick("centres", t0)
-
-    t0 = time.perf_counter()
-    ci, lv = cluster_levels(s, a, b, centres, _g=g)
-    del a, b
-    n_has_edge = int(((lv != 255) & (lv != 0)).sum().item())
-    # badger.py:131 `len(counts) - len(edges.keys())`: the keys are the nodes with an edge plus every centre cluster() touched
-    info["disconnected"] = int(N) - (n_has_edge + int(centres.size))
-    tick("cluster", t0)
-
-    if high_sens:
-        t0 = time.perf_counter()
-        if g.rank == 0:
-            patched = pipeline.high_sens_patch(ci.cpu().numpy(), merged.host.sorted_distinct, merged.host.sorted_pos, centre_order)
-            ci.copy_(torch.from_numpy(patched))
-        g.broadcast_from_first(ci, "high_sens")
-        tick("high_sens", t0)
-    return ci, info
+    def patch(self, ci, rm, centre_order):
+        if self.g.rank == 0:
+            ci.copy_(torch.from_numpy(pipeline.high_sens_patch(ci.cpu().numpy(), rm.host.sorted_distinct, rm.host.sorted_pos, centre_order)))
+        return self.g.broadcast_from_first(ci, "high_sens")
 
 
 def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, threshold, n_cells, interval=25, whitelist_sorted=None,
@@ -223,40 +198,36 @@ def assign_packed(ranks: torch.Tensor, valid: torch.Tensor | None = None, *, thr
     stage ended by a device synchronise, and under "collective_bytes" the bytes each kind of collective delivered to this rank."""
     bd._ready()
     bd._check(ranks, "ranks", bd.BARCODE_DTYPES)
-    if whitelist_sorted is not None:
-        bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
-    if isinstance(true_barcodes, torch.Tensor):
-        true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+    bd._check_whitelist(whitelist_sorted)
+    true_barcodes = bd._true_barcodes(true_barcodes)
     T = timings if timings is not None else {}
-    g = _Group(group, T.setdefault("collective_bytes", {}) if timings is not None else None)
-    R, dev = ranks.numel(), ranks.device
-    tick = _ticker(timings)
+    stages = _GroupStages(group, timings)
+    g, R, dev = stages.g, ranks.numel(), ranks.device
 
     t0 = time.perf_counter()
     rm = bd.dedup_reads(ranks, valid)
-    tick("dedup_first_seen", t0)
+    pipeline._tick(T, "dedup_first_seen", t0, stages.sync)
 
     t0 = time.perf_counter()
     merged, total_valid, total_rows = dedup_merge(rm, _g=g)
-    tick("exchange_merge", t0)
+    pipeline._tick(T, "exchange_merge", t0, stages.sync)
     info = {"reads": total_rows, "valid_reads": total_valid}
     if merged is None:
-        return (torch.zeros(R, dtype=ranks.dtype, device=dev), torch.zeros(R, dtype=torch.bool, device=dev)), info
-    N = merged.n_distinct
+        return bd._zeros(ranks), info
 
-    ci, info = run_stages(merged, g, info, timings, threshold=threshold, n_cells=n_cells, interval=interval,
-                          whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order)
+    def gather(ci):
+        centre, has = bd._zeros(ranks)
+        if rm.n_valid:
+            with torch.cuda.device(dev):
+                check(lib().bdg_dev_assign_reads32(merged.token, ci.data_ptr(), merged.n_distinct, centre.data_ptr(), has.data_ptr(), R, None,
+                                                   bd._stream()))
+        n_assigned = g.all_reduce(has.sum(dtype=torch.int64).reshape(1), dist.ReduceOp.SUM, "counts")
+        return (centre, has), int(n_assigned.item())
 
-    t0 = time.perf_counter()
-    centre = torch.zeros(R, dtype=ranks.dtype, device=dev)
-    has = torch.zeros(R, dtype=torch.bool, device=dev)
-    if rm.n_valid:
-        with torch.cuda.device(dev):
-            check(lib().bdg_dev_assign_reads32(merged.token, ci.data_ptr(), N, centre.data_ptr(), has.data_ptr(), R, None, bd._stream()))
-    n_assigned = g.all_reduce(has.sum(dtype=torch.int64).reshape(1), dist.ReduceOp.SUM, "counts")
-    info["assigned_reads"] = int(n_assigned.item())
-    tick("gather", t0)
-    return (centre, has), info
+    out = pipeline.run_stages(merged, info, T, stages, gather, threshold=threshold, n_cells=n_cells, interval=interval,
+                              whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens,
+                              centre_order=centre_order, centres_above=bd.centres_above)
+    return out, info
 
 
 class Tally(bd.Tally):
@@ -270,7 +241,8 @@ class Tally(bd.Tally):
     first-seen order, count ties and the n_cells cutoff start with rank 0's first batch; with high_sens, rank 0 patches and
     broadcasts, and centre_order="set" is the set order of rank 0's process.  `info` is that process's info on every rank, except
     "assigned_reads": 0 after finish, then the rows with a centre of this rank's assign calls (summed over the ranks: the
-    one-process figure).
+    one-process figure).  finish's timings: as for assign_packed, with "exchange_merge", "tally_finish", "edges", "centres",
+    "cluster", "high_sens", "gather" and "collective_bytes".
 
     A refusal is decided from data that is the same on every rank: a rank-local problem (a freed tally, a bad argument, a finish
     on some ranks only) travels in the first all-gather of finish, and every rank raises."""
@@ -280,26 +252,26 @@ class Tally(bd.Tally):
         self._group = group
         self._totals = None           # (rows, valid rows) of all ranks once finish merged the sets
 
-    def finish(self, *, threshold, n_cells, interval=25, whitelist_sorted=None, true_barcodes=None, high_sens=False, centre_order=None,
-               timings=None) -> dict:
+    def _stages(self, timings):
+        return _GroupStages(self._group, timings)
+
+    def _read_map(self, n_distinct, n_valid, token):
+        return bd.DeviceReadMap(n_distinct, n_valid, 0, token, torch.int32)
+
+    def _close(self, stages, T, args):
         """Steps: (1) all-gather of every rank's status, set size, rows and scalar arguments; (2) all-gather of the sets
-        (bdg_dev_tally_copy, padded to the longest); (3) bdg_dev_tally_merge_parts; (4) bdg_dev_tally_finish; (5) run_stages.  The
-        node -> centre array stays on the device for assign.  timings: as for assign_packed, with "exchange_merge",
-        "tally_finish", "edges", "centres", "cluster", "high_sens" and "collective_bytes"."""
-        T = timings if timings is not None else {}
-        g = _Group(self._group, T.setdefault("collective_bytes", {}) if timings is not None else None)
-        dev, tick, L = bd._device(), _ticker(timings), lib()
+        (bdg_dev_tally_copy, padded to the longest); (3) bdg_dev_tally_merge_parts; (4) bdg_dev_tally_finish.  Returns the rows
+        and valid rows of all ranks."""
+        g, dev, L = stages.g, bd._device(), lib()
 
         t0 = time.perf_counter()
         err, status, own = None, 0, [0, 0, 0]
         scalars = [0, 0, 0, 0]
         try:
             h = self._handle()
-            scalars = [int(threshold), int(n_cells), int(interval), int(bool(high_sens))]
-            if whitelist_sorted is not None:
-                bd._check(whitelist_sorted, "whitelist_sorted", bd.BARCODE_DTYPES)
-            if isinstance(true_barcodes, torch.Tensor):
-                true_barcodes = (true_barcodes.to(torch.int64) & 0xFFFFFFFF).tolist()
+            scalars = [int(args["threshold"]), int(args["n_cells"]), int(args["interval"]), int(bool(args["high_sens"]))]
+            bd._check_whitelist(args["whitelist_sorted"])
+            args["true_barcodes"] = bd._true_barcodes(args["true_barcodes"])
             n, rows, valid = C.c_size_t(0), C.c_ulonglong(0), C.c_ulonglong(0)
             check(L.bdg_tally_info(h, C.byref(n), C.byref(rows), C.byref(valid)))
             own = [int(n.value), int(rows.value), int(valid.value)] if self._totals is None else [0, *self._totals]
@@ -342,19 +314,7 @@ class Tally(bd.Tally):
                                                       (C.c_size_t * g.world)(*sizes), (C.c_ulonglong * g.world)(*offsets), g.world,
                                                       g.rank, total_rows, total_valid, bd._stream()))
             self._totals = (total_rows, total_valid)
-        tick("exchange_merge", t0)
+        pipeline._tick(T, "exchange_merge", t0, stages.sync)
 
-        t0 = time.perf_counter()
-        n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
-        self._finish_call(n, nv, tok)                                 # a merged count of 2^32 or more: refused on every rank
-        tick("tally_finish", t0)
-        self.info = info = {"reads": total_rows, "valid_reads": total_valid}
-        self._rm, self._ci = None, None
-        if total_valid == 0:
-            return info
-        rm = bd.DeviceReadMap(int(n.value), int(nv.value), 0, int(tok.value), torch.int32)
-        ci, info = run_stages(rm, g, info, timings, threshold=threshold, n_cells=n_cells, interval=interval,
-                              whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order)
-        info["assigned_reads"] = 0
-        self._rm, self._ci = rm, ci
-        return info
+        _, _, n_distinct, token = super()._close(stages, T, args)    # a merged count of 2^32 or more: refused on every rank
+        return total_rows, total_valid, n_distinct, token

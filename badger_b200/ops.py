@@ -91,15 +91,21 @@ class ReadMap:
     sorted_distinct = property(lambda self: self._fetch("sorted_distinct"))
 
 
+def _mask(valid, n):
+    """A validity mask for n rows as uint8 for the C ABI (a bool mask is used in place), or None."""
+    if valid is None:
+        return None
+    v = np.ascontiguousarray(valid)
+    if v.size != n:
+        raise ValueError("valid has %d rows, ranks %d" % (v.size, n))
+    return v.view(np.uint8) if v.dtype == np.bool_ else (v != 0).view(np.uint8)
+
+
 def dedup_reads(ranks: np.ndarray, valid=None) -> ReadMap:
     """barcode_graph.py:192-204 over the rows with valid[i] (None: all), compacted on the device; everything it produces is
     kept there for edges_handle_resident / centres_above / assign_reads (include/badger_b200.h bdg_dedup_reads)."""
     r = np.ascontiguousarray(ranks, dtype=np.uint32)
-    if valid is None:
-        v = None
-    else:
-        v = np.ascontiguousarray(valid)
-        v = v.view(np.uint8) if v.dtype == np.bool_ else (v != 0).view(np.uint8)     # a bool mask is used in place
+    v = _mask(valid, r.size)
     n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
     if r.size:
         check(lib().bdg_dedup_reads(ptr(r), ptr(v) if v is not None else None, r.size, None, None, None, None,

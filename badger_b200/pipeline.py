@@ -78,30 +78,37 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
 
     ranks = np.ascontiguousarray(ranks, dtype=np.uint32)
     R = ranks.size
-    if valid is not None:
-        valid = np.ascontiguousarray(valid, dtype=bool)
     info = {"reads": int(R)}
     if R == 0:
         info["valid_reads"] = 0
-        return result(np.zeros(0, np.uint32), np.zeros(0, np.uint8)), info
+        return result(*_zeros(ranks)), info
 
     t0 = time.perf_counter()
     rm = ops.dedup_reads(ranks, valid)                    # valid rows compacted on the device; everything stays there
     _tick(T, "dedup_first_seen", t0)
     info["valid_reads"] = int(rm.n_valid)
     if rm.n_valid == 0:
-        return result(np.zeros(R, np.uint32), np.zeros(R, np.uint8)), info
+        return result(*_zeros(ranks)), info
 
     def gather(ci):
         c32, has, n_assigned = ops.assign_reads32(rm, ci)     # per-read gather on the device
         return result(c32, has), n_assigned
 
-    return run_stages(rm, info, T, gather, threshold=threshold, n_cells=n_cells, interval=interval, whitelist_sorted=whitelist_sorted,
-                      true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order, centres_above=ops.centres_above), info
+    return run_stages(rm, info, T, _OneProcess(), gather, threshold=threshold, n_cells=n_cells, interval=interval,
+                      whitelist_sorted=whitelist_sorted, true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order,
+                      centres_above=ops.centres_above), info
 
 
-def _tick(T, name, t0):
+def _tick(T, name, t0, sync=None):
+    """Adds the host time since t0 to T[name]; sync, when given, waits for the device first."""
+    if sync is not None:
+        sync()
     T[name] = T.get(name, 0.0) + time.perf_counter() - t0
+
+
+def _zeros(ranks):
+    """The result of rows none of which has a centre: (centre uint32[R], has_centre uint8[R]), all zero."""
+    return np.zeros(ranks.size, np.uint32), np.zeros(ranks.size, np.uint8)
 
 
 class Tally:
@@ -116,6 +123,7 @@ class Tally:
     (another tally's add, assign_packed, ...) makes `assign` raise until `finish` runs again."""
 
     _centres_above = staticmethod(ops.centres_above)
+    _zeros = staticmethod(_zeros)
 
     def __init__(self):
         self._h = C.c_void_p()
@@ -130,72 +138,90 @@ class Tally:
             raise ValueError("the tally was freed")
         return self._h
 
+    @staticmethod
+    def _rows(ranks, valid):
+        r = np.ascontiguousarray(ranks, dtype=np.uint32)
+        return r, ops._mask(valid, r.size)
+
     def add(self, ranks, valid=None) -> int:
         """Count one batch (packed barcodes per row; valid: mask or None for all rows).  Returns its number of valid rows."""
-        r = np.ascontiguousarray(ranks, dtype=np.uint32)
-        v = _mask(valid, r.size)
+        r, v = self._rows(ranks, valid)
         nv = C.c_size_t(0)
         check(lib().bdg_tally_add(self._handle(), ptr(r), ptr(v) if v is not None else None, r.size, C.byref(nv)))
         self.rows += r.size
         return int(nv.value)
-
-    def _finish_call(self, n, nv, tok):
-        check(lib().bdg_tally_finish(self._handle(), C.byref(n), C.byref(nv), C.byref(tok)))
 
     def finish(self, *, threshold, n_cells, interval=25, whitelist_sorted=None, true_barcodes=None, high_sens=False, centre_order=None,
                timings=None) -> dict:
         """The stages after the dedup (run_stages, arguments as for assign_packed) over the counted batches.  The clustering
         result stays for `assign`.  Returns `info`; no batch can be added afterwards."""
         T = timings if timings is not None else {}
-        t0 = time.perf_counter()
-        n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
-        self._finish_call(n, nv, tok)
-        _tick(T, "tally_finish", t0)
-        self.info = info = {"reads": int(self.rows), "valid_reads": int(nv.value)}
+        args = dict(threshold=threshold, n_cells=n_cells, interval=interval, whitelist_sorted=whitelist_sorted,
+                    true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order)
+        stages = self._stages(timings)
+        rows, n_valid, n_distinct, token = self._close(stages, T, args)
+        self.info = info = {"reads": int(rows), "valid_reads": int(n_valid)}
         self._rm, self._ci = None, None
-        if nv.value == 0:
+        if n_valid == 0:
             return info
-        rm = ops.ReadMap(int(n.value), int(nv.value), 0, int(tok.value))
+        rm = self._read_map(n_distinct, n_valid, token)
 
         def keep(ci):
             self._ci = None if ci is None else self._upload(ci)
             return None, 0
 
-        run_stages(rm, info, T, keep, threshold=threshold, n_cells=n_cells, interval=interval, whitelist_sorted=whitelist_sorted,
-                   true_barcodes=true_barcodes, high_sens=high_sens, centre_order=centre_order, centres_above=self._centres_above)
+        run_stages(rm, info, T, stages, keep, centres_above=self._centres_above, **args)
         self._rm = rm
         return info
 
+    def _stages(self, timings):
+        return _OneProcess()
+
+    def _close(self, stages, T, args):
+        """Ends the counting: (rows, valid rows, distinct barcodes, token of the read map) of the counted batches.  args: the
+        arguments of finish, which a form may check and normalise in place."""
+        t0 = time.perf_counter()
+        n, nv, tok = C.c_size_t(0), C.c_size_t(0), C.c_ulonglong(0)
+        self._finish_call(n, nv, tok)
+        _tick(T, "tally_finish", t0, stages.sync)
+        return self.rows, int(nv.value), int(n.value), int(tok.value)
+
+    def _finish_call(self, n, nv, tok):
+        check(lib().bdg_tally_finish(self._handle(), C.byref(n), C.byref(nv), C.byref(tok)))
+
+    def _read_map(self, n_distinct, n_valid, token):
+        return ops.ReadMap(n_distinct, n_valid, 0, token)
+
     def _upload(self, ci):
         return np.ascontiguousarray(ci, dtype=np.int32)
-
-    def _ready_to_assign(self):
-        if self.info is None:
-            raise ValueError("assign before finish")
-        return self._rm
 
     def assign(self, ranks, valid=None):
         """(centre uint32[R], has_centre uint8[R]) for the rows of `ranks`, any batching.  ValueError when a valid row's barcode
         was never added.  With high_sens the patched node -> centre array is copied to the device with every call (the tensor
         form, device.Tally, uploads it once)."""
-        rm = self._ready_to_assign()
-        r = np.ascontiguousarray(ranks, dtype=np.uint32)
-        v = _mask(valid, r.size)
-        R = r.size
-        if rm is None:                                        # nothing was counted: only rows without a barcode can be assigned
-            if R and (v is None or v.any()):
-                raise ValueError("%d valid rows have a barcode that was never added" % (R if v is None else int(np.count_nonzero(v))))
-            return np.zeros(R, np.uint32), np.zeros(R, np.uint8)
-        out = ops._pinned.array(R, np.uint32, eager=False)
-        has = ops._pinned.array(R, np.uint8, eager=False)
+        if self.info is None:
+            raise ValueError("assign before finish")
+        r, v = self._rows(ranks, valid)
+        if self._rm is None:                                  # nothing was counted: only rows without a barcode can be assigned
+            n_valid = len(r) if v is None else int((v != 0).sum())
+            if n_valid:
+                raise ValueError("%d valid rows have a barcode that was never added" % n_valid)
+            return self._zeros(r)
+        centre, has, n_assigned, n_missing = self._lookup(self._rm, r, v)
+        if n_missing:
+            raise ValueError("%d valid rows have a barcode that was never added" % n_missing)
+        self.info["assigned_reads"] += n_assigned
+        return centre, has
+
+    def _lookup(self, rm, r, v):
+        """(centre, has_centre, rows with a centre, valid rows whose barcode is not a node)."""
+        out = ops._pinned.array(r.size, np.uint32, eager=False)
+        has = ops._pinned.array(r.size, np.uint8, eager=False)
         na, nm = C.c_size_t(0), C.c_size_t(0)
         ci = self._ci
         check(lib().bdg_assign_lookup32(rm.token, ptr(ci) if ci is not None else None, rm.n_distinct, ptr(r), ptr(v) if v is not None else None,
-                                        R, ptr(out), ptr(has), C.byref(na), C.byref(nm)))
-        if nm.value:
-            raise ValueError("%d valid rows have a barcode that was never added" % nm.value)
-        self.info["assigned_reads"] += int(na.value)
-        return out, has
+                                        r.size, ptr(out), ptr(has), C.byref(na), C.byref(nm)))
+        return out, has, int(na.value), int(nm.value)
 
     def free(self):
         if self._h is not None and self._h.value and _lib._lib is not None:
@@ -209,61 +235,68 @@ class Tally:
             pass
 
 
-def _mask(valid, n):
-    """A validity mask as uint8 for the C ABI (a bool mask is used in place), or None."""
-    if valid is None:
-        return None
-    v = np.ascontiguousarray(valid)
-    if v.size != n:
-        raise ValueError("valid has %d rows, ranks %d" % (v.size, n))
-    return v.view(np.uint8) if v.dtype == np.bool_ else (v != 0).view(np.uint8)
-
-
-def run_stages(rm, info, T, gather, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order,
+def run_stages(rm, info, T, stages, gather, *, threshold, n_cells, interval, whitelist_sorted, true_barcodes, high_sens, centre_order,
                centres_above):
-    """The stages after the dedup of a read map `rm` with at least one valid read: edges, centres, clustering, --high_sens,
-    and last `gather(centre_idx)` -> (result, rows with a centre) over the read map, with centre_idx None for the clustering
-    left on the device.  Fills `info` and the timings `T`; returns what `gather` returned first.  centres_above is
-    ops.centres_above or a function of the same signature that takes the whitelist in another form."""
+    """The stages after the dedup (or the merge of the ranks' barcodes) of a read map `rm` with at least one valid read: edges,
+    centres, clustering, --high_sens, and last `gather(centre_idx)` -> (result, rows with a centre) over the read map, with
+    centre_idx None for the clustering left on the device.  `stages` builds the edges and runs the rounds and the patch:
+    _OneProcess, or distributed._GroupStages over a process group; its `sync` (None: none) ends every timed stage.  Fills `info`
+    and the timings `T`; returns what `gather` returned first.  centres_above is ops.centres_above or a function of the same
+    signature that takes the whitelist in another form."""
+    def tick(name, t0):
+        _tick(T, name, t0, stages.sync)
+
     t0 = time.perf_counter()
-    handle = ops.edges_handle_resident(rm, threshold)     # the ascending array is already on the device: no upload, peer copies to the other GPUs
-    _tick(T, "edges", t0)
-    info.update(distinct=int(rm.n_distinct), edges=int(handle.count))
+    n_edges = stages.edges(rm, threshold)
+    info.update(distinct=int(rm.n_distinct), edges=int(n_edges))
+    tick("edges", t0)
 
     t0 = time.perf_counter()
     centres = np.asarray(list(dict.fromkeys(select_centres(rm, n_cells, interval, whitelist_sorted, true_barcodes, centres_above))),
                          dtype=np.uint32)
-    _tick(T, "centres", t0)
     info["centres"] = int(centres.size)
-
-    if not high_sens:
-        t0 = time.perf_counter()
-        n_has_edge = handle.cluster_resident(centres, 2)  # consumes the handle's edges; the node -> centre array stays on the device
-        handle.free()
-        # badger.py:131 `len(counts) - len(edges.keys())`: the keys are the nodes with an edge plus every centre cluster() touched
-        info["disconnected"] = int(rm.n_distinct) - (int(n_has_edge) + int(centres.size))
-        _tick(T, "cluster", t0)
-        t0 = time.perf_counter()
-        out, n_assigned = gather(None)
-        _tick(T, "gather", t0)
-        info["assigned_reads"] = int(n_assigned)
-        return out
+    tick("centres", t0)
 
     t0 = time.perf_counter()
-    s, spos = rm.sorted_distinct, rm.sorted_pos
-    ci, lv, has_edge = handle.cluster_levels(centres, 2, want_has_edge=True)   # consumes the handle's edges (no copy to the host)
-    handle.free()
-    info["disconnected"] = int(rm.n_distinct) - (int(has_edge.sum()) + int(centres.size))
-    _tick(T, "cluster", t0)
-    t0 = time.perf_counter()
-    ci = high_sens_patch(ci, s, spos, centre_order)
-    _tick(T, "high_sens", t0)
+    ci, n_has_edge = stages.rounds(rm, centres, high_sens)
+    # badger.py:131 `len(counts) - len(edges.keys())`: the keys are the nodes with an edge plus every centre cluster() touched
+    info["disconnected"] = int(rm.n_distinct) - (int(n_has_edge) + int(centres.size))
+    tick("cluster", t0)
+
+    if high_sens:
+        t0 = time.perf_counter()
+        ci = stages.patch(ci, rm, centre_order)
+        tick("high_sens", t0)
 
     t0 = time.perf_counter()
     out, n_assigned = gather(ci)
-    _tick(T, "gather", t0)
     info["assigned_reads"] = int(n_assigned)
+    tick("gather", t0)
     return out
+
+
+class _OneProcess:
+    """The stages of run_stages in one process: the edges built on every claimed GPU from the distinct barcodes the read map
+    keeps on the first one, the rounds over them (the node -> centre array stays on the device unless --high_sens patches it
+    on the host).  The timings do not wait for the device."""
+
+    sync = None
+
+    def edges(self, rm, threshold):
+        self.handle = ops.edges_handle_resident(rm, threshold)    # the ascending array is already on the device: no upload, peer copies to the other GPUs
+        return self.handle.count
+
+    def rounds(self, rm, centres, want_ci):
+        if want_ci:
+            ci, _, has_edge = self.handle.cluster_levels(centres, 2, want_has_edge=True)
+            n_has_edge = int(has_edge.sum())
+        else:
+            ci, n_has_edge = None, self.handle.cluster_resident(centres, 2)
+        self.handle.free()
+        return ci, n_has_edge
+
+    def patch(self, ci, rm, centre_order):
+        return high_sens_patch(ci, rm.sorted_distinct, rm.sorted_pos, centre_order)
 
 
 def high_sens_patch(ci, s, spos, centre_order):

@@ -24,26 +24,11 @@ import test_step_vs_oracle_gpu as sv
 from badger_b200 import device as bd
 from badger_b200 import ops, pipeline, synth
 from badger_b200._lib import BDG_ERR_ARG, BadgerB200Error
+from gpu_helpers import claimed, cuda, dataset, host
 
-pytestmark = pytest.mark.gpu
-cuda, host = sv.cuda, sv.host
+pytestmark = [pytest.mark.gpu, pytest.mark.usefixtures("claimed")]
 TESTS = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(TESTS)
-
-
-@pytest.fixture(autouse=True)
-def claimed():
-    assert badger_b200.init() >= 1
-    yield
-    badger_b200.init()
-
-
-def dataset(seed, n_reads, n_cells=600, err=0.08):
-    rng = synth.rng_for(seed)
-    wl = synth.make_whitelist(20000, rng)
-    cells = synth.pick_cells(wl, n_cells, rng)
-    obs, valid = synth.simulate_reads(cells, n_reads, err, rng)
-    return np.sort(wl), cells, obs, valid
 
 
 def cuts(R, kind, seed):

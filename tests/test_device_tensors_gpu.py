@@ -12,35 +12,9 @@ import torch
 import badger_b200
 from badger_b200 import device as bd
 from badger_b200 import ops, pipeline, synth
+from gpu_helpers import claimed, cuda, dataset, host
 
-pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(autouse=True)
-def claimed():
-    assert badger_b200.init() >= 1
-    yield
-    badger_b200.init()
-
-
-def dataset(seed, n_reads, n_cells=600, err=0.08):
-    rng = synth.rng_for(seed)
-    wl = synth.make_whitelist(20000, rng)
-    cells = synth.pick_cells(wl, n_cells, rng)
-    obs, valid = synth.simulate_reads(cells, n_reads, err, rng)
-    return wl, cells, obs, valid
-
-
-def cuda(a, dtype=torch.int32):
-    """A numpy barcode array (uint32 bits kept) or mask as a tensor on the first device."""
-    if dtype in (torch.bool, torch.uint8):
-        return torch.from_numpy(np.ascontiguousarray(a)).to(bd._device()).to(dtype)
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).to(bd._device()).view(dtype)
-
-
-def host(t):
-    t = t.cpu()
-    return t.view(torch.int32).numpy().view(np.uint32) if t.dtype in (torch.int32, torch.uint32) else t.numpy()
+pytestmark = [pytest.mark.gpu, pytest.mark.usefixtures("claimed")]
 
 
 def assert_same_assignment(dev_out, host_out):

@@ -13,29 +13,12 @@ import torch
 import badger_b200
 from badger_b200 import device as bd
 from badger_b200 import ops, synth
+from gpu_helpers import claimed, cuda, host
 from oracle import oracle as orc
 
-pytestmark = pytest.mark.gpu
+pytestmark = [pytest.mark.gpu, pytest.mark.usefixtures("claimed")]
 
 LOW_COMPLEXITY = np.asarray([0, 0x55555555, 0xAAAAAAAA, 0xFFFFFFFF, 0x11111111, 0x1B1B1B1B, 0xE4E4E4E4, 0x0F0F0F0F], np.uint32)
-
-
-@pytest.fixture(autouse=True)
-def claimed():
-    assert badger_b200.init() >= 1
-    yield
-    badger_b200.init()
-
-
-def cuda(a, dtype=torch.int32):
-    """A numpy barcode array (uint32 bits kept) as a tensor on the first device."""
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).to(bd._device()).view(dtype)
-
-
-def host(t):
-    """A barcode tensor as uint32 numpy (the same bits), any other tensor as numpy of its own dtype."""
-    t = t.cpu()
-    return t.view(torch.int32).numpy().view(np.uint32) if t.dtype in (torch.int32, torch.uint32) else t.numpy()
 
 
 def npy(t):

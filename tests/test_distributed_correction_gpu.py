@@ -5,12 +5,6 @@ Worlds of 2 and 3 ranks run on gloo with every rank on the first GPU; a world of
 per rank.  Each world is one set of spawned processes that runs every check and reports to the test; the reference runs on
 rank 0 in the same process as that rank's distributed call, so that centre_order="set" meets the same set order."""
 import ctypes as C
-import os
-import queue
-import socket
-import sys
-import time
-import traceback
 
 import numpy as np
 import pytest
@@ -19,9 +13,9 @@ import torch
 import badger_b200
 from badger_b200 import device as bd
 from badger_b200 import distributed as bdist
-from badger_b200 import ops, pipeline, synth
+from badger_b200 import ops, pipeline
+from gpu_helpers import assert_world, claimed_without_group, cuda, dataset, host, run_world
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 pytestmark = pytest.mark.gpu
 
 N_READS = 100000
@@ -36,26 +30,6 @@ CASES = [  # threshold, whitelist, valid mask, true barcodes, high_sens, centre_
 ]
 
 
-def dataset(seed, n_reads=N_READS, n_cells=N_CELLS, err=0.08):
-    rng = synth.rng_for(seed)
-    wl = synth.make_whitelist(20000, rng)
-    cells = synth.pick_cells(wl, n_cells, rng)
-    obs, valid = synth.simulate_reads(cells, n_reads, err, rng)
-    return wl, cells, obs, valid
-
-
-def cuda(a, dtype=torch.int32):
-    """A numpy barcode array (uint32 bits kept) or mask as a tensor on the first claimed device."""
-    if dtype in (torch.bool, torch.uint8):
-        return torch.from_numpy(np.ascontiguousarray(a)).to(bd._device()).to(dtype)
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).to(bd._device()).view(dtype)
-
-
-def host(t):
-    t = t.cpu()
-    return t.view(torch.int32).numpy().view(np.uint32) if t.dtype in (torch.int32, torch.uint32) else t.numpy()
-
-
 def bounds(split, world, n):
     """[lo, hi) of every rank: uneven weights 3, 1, 2, 3, 1, 2, ...; "first_empty" gives rank 0 no rows."""
     w = np.array([0 if (split == "first_empty" and r == 0) else (3, 1, 2)[r % 3] for r in range(world)], float)
@@ -68,7 +42,7 @@ def bounds(split, world, n):
 # ---------------------------------------------------------------------------------------------------------------- the checks
 def check_cases(rank, world, gather, record):
     for k, (t, use_wl, use_valid, use_tb, high_sens, order, dtype, split) in enumerate(CASES):
-        wl, cells, obs, valid = dataset(900 + k)
+        wl, cells, obs, valid = dataset(900 + k, N_READS, N_CELLS)
         b = bounds(split, world, obs.size)
         v = valid.copy()
         if split == "last_invalid":
@@ -94,7 +68,7 @@ def check_cases(rank, world, gather, record):
 
 
 def check_edge_cases(rank, world, gather, record):
-    _, _, obs, valid = dataset(5, 3000)
+    _, _, obs, valid = dataset(5, 3000, N_CELLS)
     lo, hi = bounds("uneven", world, obs.size)[rank]
     (c, h), info = bdist.assign_packed(cuda(obs[lo:hi]), torch.zeros(hi - lo, dtype=torch.bool, device=bd._device()),
                                        threshold=2, n_cells=10)
@@ -106,7 +80,7 @@ def check_edge_cases(rank, world, gather, record):
 
 
 def check_merge_centres_rounds(rank, world, gather, record):
-    wl, cells, obs, valid = dataset(77, 120000)
+    wl, cells, obs, valid = dataset(77, 120000, N_CELLS)
     wls = np.sort(wl)
     for split in ("uneven", "first_empty"):
         lo, hi = bounds(split, world, obs.size)[rank]
@@ -148,71 +122,9 @@ def battery(rank, world, gather):
 
 
 # ---------------------------------------------------------------------------------------------------------------- the worlds
-def _worker(rank, world, backend, port, q):
-    import torch.distributed as dist
-    sys.path.insert(0, ROOT)
-    try:
-        os.environ["MASTER_ADDR"] = "127.0.0.1"
-        os.environ["MASTER_PORT"] = str(port)
-        dev = rank if backend == "nccl" else 0
-        torch.cuda.set_device(dev)
-        dist.init_process_group(backend, rank=rank, world_size=world)
-        badger_b200.init([dev])
-
-        def gather(obj):
-            out = [None] * world
-            dist.all_gather_object(out, obj)
-            return out
-        q.put((rank, battery(rank, world, gather)))
-        dist.barrier()
-        dist.destroy_process_group()
-    except BaseException:
-        q.put((rank, [("rank %d raised" % rank, False, traceback.format_exc())]))
-
-
-def run_world(world, backend, timeout=1200):
-    import torch.multiprocessing as mp
-    with socket.socket() as sk:
-        sk.bind(("127.0.0.1", 0))
-        port = sk.getsockname()[1]
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    procs = [ctx.Process(target=_worker, args=(r, world, backend, port, q)) for r in range(world)]
-    for p in procs:
-        p.start()
-    deadline = time.monotonic() + timeout
-    got = {}
-    try:
-        while len(got) < world:
-            rank, res = q.get(timeout=max(1.0, deadline - time.monotonic()))
-            got[rank] = res
-            if any(not ok for _, ok, _ in res):
-                break                      # a failed rank may leave the others waiting in a collective
-    except queue.Empty:
-        pass
-    finally:
-        for p in procs:
-            p.join(max(1.0, min(120.0, deadline - time.monotonic())))
-        for p in procs:
-            if p.is_alive():
-                p.terminate()
-                p.join(30)
-            if p.is_alive():
-                p.kill()
-                p.join()
-    return got
-
-
-def assert_world(got, world):
-    failed = [(r, name, detail) for r, res in sorted(got.items()) for name, ok, detail in res if not ok]
-    assert not failed, failed
-    assert sorted(got) == list(range(world)), "ranks that did not report: %s" % sorted(set(range(world)) - set(got))
-    print({r: len(res) for r, res in got.items()})
-
-
 @pytest.mark.parametrize("world", [2, 3])
 def test_gloo_world_on_one_gpu(world):
-    assert_world(run_world(world, "gloo"), world)
+    assert_world(run_world(battery, world, "gloo", timeout=1200), world)
 
 
 def test_nccl_world_one_gpu_per_rank():
@@ -220,22 +132,13 @@ def test_nccl_world_one_gpu_per_rank():
     if n < 2:
         pytest.skip("an NCCL world needs two GPUs")
     world = min(4, n)
-    assert_world(run_world(world, "nccl"), world)
+    assert_world(run_world(battery, world, "nccl", timeout=1200), world)
 
 
 # ------------------------------------------------------------------------------------ a world of one, in this process
-@pytest.fixture
-def claimed():
-    import torch.distributed as dist
-    assert not dist.is_initialized()
-    assert badger_b200.init([0]) == 1
-    yield
-    badger_b200.init()
-
-
-def test_world_of_one_without_a_process_group(claimed):
+def test_world_of_one_without_a_process_group(claimed_without_group):
     for t, use_wl, use_valid, use_tb, high_sens, order, dtype, _ in CASES[2:5]:
-        wl, cells, obs, valid = dataset(300 + t)
+        wl, cells, obs, valid = dataset(300 + t, N_READS, N_CELLS)
         wls = np.sort(wl)
         args = (cuda(obs, dtype), cuda(valid, torch.bool) if use_valid else None)
         kw = dict(threshold=t, n_cells=N_CELLS, high_sens=high_sens, centre_order=order, whitelist_sorted=cuda(wls, dtype) if use_wl else None,
@@ -247,8 +150,8 @@ def test_world_of_one_without_a_process_group(claimed):
         assert T["collective_bytes"]["lists"] == 12 * info["distinct"] and T["gather"] > 0
 
 
-def test_argument_errors_leave_it_usable(claimed):
-    _, _, obs, valid = dataset(3, 20000)
+def test_argument_errors_leave_it_usable(claimed_without_group):
+    _, _, obs, valid = dataset(3, 20000, N_CELLS)
     d_obs, d_valid = cuda(obs), cuda(valid, torch.bool)
     kw = dict(threshold=1, n_cells=100)
     with pytest.raises(ValueError):

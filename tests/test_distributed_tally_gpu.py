@@ -8,12 +8,8 @@ rank 0 in the same process as that rank's tally, so that centre_order="set" meet
 import ctypes as C
 import json
 import os
-import queue
-import socket
 import subprocess
 import sys
-import time
-import traceback
 
 import numpy as np
 import pytest
@@ -24,8 +20,8 @@ from badger_b200 import device as bd
 from badger_b200 import distributed as bdist
 from badger_b200 import ops, pipeline, synth
 from badger_b200._lib import BDG_ERR_ARG, BDG_OK, BadgerB200Error
+from gpu_helpers import ROOT, assert_world, claimed_without_group, cuda, dataset, host, run_world
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 TESTS = os.path.dirname(os.path.abspath(__file__))
 pytestmark = pytest.mark.gpu
 
@@ -39,26 +35,6 @@ CASES = [  # threshold, whitelist, valid mask, true barcodes, high_sens, centre_
     (3, True, True, False, False, None, torch.uint32, "uneven"),
     (3, False, True, True, False, None, torch.int32, "late_new"),
 ]
-
-
-def dataset(seed, n_reads=N_READS, n_cells=N_CELLS, err=0.08):
-    rng = synth.rng_for(seed)
-    wl = synth.make_whitelist(20000, rng)
-    cells = synth.pick_cells(wl, n_cells, rng)
-    obs, valid = synth.simulate_reads(cells, n_reads, err, rng)
-    return wl, cells, obs, valid
-
-
-def cuda(a, dtype=torch.int32):
-    """A numpy barcode array (uint32 bits kept) or mask as a tensor on the first claimed device."""
-    if dtype in (torch.bool, torch.uint8):
-        return torch.from_numpy(np.ascontiguousarray(a)).to(bd._device()).to(dtype)
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).to(bd._device()).view(dtype)
-
-
-def host(t):
-    t = t.cpu()
-    return t.view(torch.int32).numpy().view(np.uint32) if t.dtype in (torch.int32, torch.uint32) else t.numpy()
 
 
 def bounds(split, world, n):
@@ -87,7 +63,7 @@ def without_assigned(info):
 # ---------------------------------------------------------------------------------------------------------------- the checks
 def check_cases(rank, world, gather, record):
     for k, (t, use_wl, use_valid, use_tb, high_sens, order, dtype, split) in enumerate(CASES):
-        wl, cells, obs, valid = dataset(700 + k)
+        wl, cells, obs, valid = dataset(700 + k, N_READS, N_CELLS)
         if split == "late_new":                               # barcodes first seen in the last rank's last batch
             fresh = synth.rng_for(5).integers(0, 1 << 32, 40, dtype=np.uint64).astype(np.uint32)
             obs = np.concatenate([obs, np.repeat(fresh, 3)])
@@ -135,7 +111,7 @@ def check_cases(rank, world, gather, record):
 
 
 def check_no_valid_row(rank, world, gather, record):
-    _, _, obs, valid = dataset(5, 3000)
+    _, _, obs, valid = dataset(5, 3000, N_CELLS)
     lo, hi = bounds("uneven", world, obs.size)[rank]
     tl = bdist.Tally()
     none = torch.zeros(hi - lo, dtype=torch.bool, device=bd._device())
@@ -176,7 +152,7 @@ def check_merged_set(rank, world, gather, record):
 
 def check_refusals(rank, world, gather, record):
     """A rank-local problem in finish makes every rank raise, and a correct finish works afterwards."""
-    _, cells, obs, valid = dataset(11, 30000)
+    _, cells, obs, valid = dataset(11, 30000, N_CELLS)
     lo, hi = bounds("uneven", world, obs.size)[rank]
     kw = dict(threshold=1, n_cells=100)
     want = None
@@ -270,71 +246,9 @@ def battery(rank, world, gather, which):
 
 
 # ---------------------------------------------------------------------------------------------------------------- the worlds
-def _worker(rank, world, backend, port, q, which):
-    import torch.distributed as dist
-    sys.path.insert(0, ROOT)
-    try:
-        os.environ["MASTER_ADDR"] = "127.0.0.1"
-        os.environ["MASTER_PORT"] = str(port)
-        dev = rank if backend == "nccl" else 0
-        torch.cuda.set_device(dev)
-        dist.init_process_group(backend, rank=rank, world_size=world)
-        badger_b200.init([dev])
-
-        def gather(obj):
-            out = [None] * world
-            dist.all_gather_object(out, obj)
-            return out
-        q.put((rank, battery(rank, world, gather, which)))
-        dist.barrier()
-        dist.destroy_process_group()
-    except BaseException:
-        q.put((rank, [("rank %d raised" % rank, False, traceback.format_exc())]))
-
-
-def run_world(world, backend, which="all", timeout=1500):
-    import torch.multiprocessing as mp
-    with socket.socket() as sk:
-        sk.bind(("127.0.0.1", 0))
-        port = sk.getsockname()[1]
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    procs = [ctx.Process(target=_worker, args=(r, world, backend, port, q, which)) for r in range(world)]
-    for p in procs:
-        p.start()
-    deadline = time.monotonic() + timeout
-    got = {}
-    try:
-        while len(got) < world:
-            rank, res = q.get(timeout=max(1.0, deadline - time.monotonic()))
-            got[rank] = res
-            if any(not ok for _, ok, _ in res):
-                break                      # a failed rank may leave the others waiting in a collective
-    except queue.Empty:
-        pass
-    finally:
-        for p in procs:
-            p.join(max(1.0, min(120.0, deadline - time.monotonic())))
-        for p in procs:
-            if p.is_alive():
-                p.terminate()
-                p.join(30)
-            if p.is_alive():
-                p.kill()
-                p.join()
-    return got
-
-
-def assert_world(got, world):
-    failed = [(r, name, detail) for r, res in sorted(got.items()) for name, ok, detail in res if not ok]
-    assert not failed, failed
-    assert sorted(got) == list(range(world)), "ranks that did not report: %s" % sorted(set(range(world)) - set(got))
-    print({r: [name for name, _, _ in res] for r, res in got.items()})
-
-
 @pytest.mark.parametrize("world", [2, 3])
 def test_gloo_world_on_one_gpu(world):
-    assert_world(run_world(world, "gloo"), world)
+    assert_world(run_world(battery, world, "gloo", "all"), world)
 
 
 def test_nccl_world_one_gpu_per_rank():
@@ -343,26 +257,17 @@ def test_nccl_world_one_gpu_per_rank():
         print("skipped: an NCCL world needs two GPUs, this box has %d" % n)
         pytest.skip("an NCCL world needs two GPUs, this box has %d" % n)
     world = min(4, n)
-    assert_world(run_world(world, "nccl"), world)
+    assert_world(run_world(battery, world, "nccl", "all"), world)
 
 
 def test_a_merged_count_of_2_32_is_refused_on_every_rank():
-    assert_world(run_world(2, "gloo", "count"), 2)
+    assert_world(run_world(battery, 2, "gloo", "count"), 2)
 
 
 # ------------------------------------------------------------------------------------ a world of one, in this process
-@pytest.fixture
-def claimed():
-    import torch.distributed as dist
-    assert not dist.is_initialized()
-    assert badger_b200.init([0]) == 1
-    yield
-    badger_b200.init()
-
-
-def test_world_of_one_without_a_process_group(claimed):
+def test_world_of_one_without_a_process_group(claimed_without_group):
     for t, use_wl, use_valid, use_tb, high_sens, order, dtype, _ in CASES:
-        wl, cells, obs, valid = dataset(300 + t)
+        wl, cells, obs, valid = dataset(300 + t, N_READS, N_CELLS)
         wls = np.sort(wl)
         kw = dict(threshold=t, n_cells=N_CELLS, high_sens=high_sens, centre_order=order, whitelist_sorted=cuda(wls, dtype) if use_wl else None,
                   true_barcodes=cuda(cells[:200], dtype) if use_tb else None)
@@ -397,11 +302,11 @@ def raw_parts(tallies, dev):
     return keys, cnts, firsts, info
 
 
-def test_merge_parts_refusals_each_followed_by_a_working_call(claimed):
+def test_merge_parts_refusals_each_followed_by_a_working_call(claimed_without_group):
     """bdg_dev_tally_merge_parts refuses, leaving the set as it was: a part that is not ascending, an own part that is not the
     handle's set, a wrong size; then the correct call gives the tally of the rank-major concatenation."""
     L, dev = badger_b200.lib(), bd._device()
-    _, _, obs, valid = dataset(21, 40000)
+    _, _, obs, valid = dataset(21, 40000, N_CELLS)
     half = 25000
     ta, tb = bd.Tally(), bd.Tally()
     ta.add(cuda(obs[:10000]), cuda(valid[:10000], torch.bool))
@@ -450,7 +355,7 @@ def pcie_probe(out_dir):
     from torch.profiler import ProfilerActivity, profile
     from test_device_tensors_gpu import memcpy_bytes
     badger_b200.init()
-    wl, _, obs, valid = dataset(123, 1000000)
+    wl, _, obs, valid = dataset(123, 1000000, N_CELLS)
     d_obs, d_valid = cuda(obs), cuda(valid, torch.bool)
     moved = {}
 

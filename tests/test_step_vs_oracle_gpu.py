@@ -19,28 +19,10 @@ import badger_b200
 import cpu_ops
 from badger_b200 import device as bd
 from badger_b200 import ops, pipeline, synth
+from gpu_helpers import claimed, cuda, host
 from oracle import oracle as orc
 
 gpu = pytest.mark.gpu
-
-
-def cuda(a, dtype=torch.int32):
-    """A numpy barcode array (uint32 bits kept), mask or byte array as a tensor on the first device."""
-    if dtype in (torch.bool, torch.uint8):
-        return torch.from_numpy(np.ascontiguousarray(a)).to(bd._device()).to(dtype)
-    return torch.from_numpy(np.ascontiguousarray(a, dtype=np.uint32).view(np.int32)).to(bd._device()).view(dtype)
-
-
-def host(t):
-    t = t.cpu()
-    return t.view(torch.int32).numpy().view(np.uint32) if t.dtype in (torch.int32, torch.uint32) else t.numpy()
-
-
-@pytest.fixture
-def claimed():
-    assert badger_b200.init() >= 1
-    yield
-    badger_b200.init()
 
 
 def contexts():

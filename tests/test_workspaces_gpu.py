@@ -11,15 +11,9 @@ import badger_b200
 from badger_b200 import _lib, ops, pipeline, synth
 from badger_b200 import device as bd
 from badger_b200 import distributed as bdist
+from gpu_helpers import claimed
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture
-def claimed():
-    assert badger_b200.init() >= 1
-    yield
-    badger_b200.init()
 
 
 def reads(seed, n_reads=200000, n_cells=300):
