@@ -54,7 +54,6 @@ def lib():
     L.bdg_tsv_write_assignments32.argtypes = [_vp, C.c_char_p, _vp, _vp, _i]
     L.bdg_dedup_first_seen.argtypes = [_vp, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz)]
     L.bdg_dedup_reads.argtypes = [_vp, _vp, _sz, _vp, _vp, _vp, _vp, C.POINTER(_sz), C.POINTER(_sz), C.POINTER(C.c_ulonglong)]
-    L.bdg_assign_reads.argtypes = [C.c_ulonglong, _vp, _sz, _vp, _sz, C.POINTER(_sz)]
     L.bdg_edges_build.argtypes = [_vp, _sz, _i, C.POINTER(_vp)]
     L.bdg_edges_build_part.argtypes = [_vp, _sz, _i, _i, _i, C.POINTER(_vp)]
     L.bdg_edges_build_resident.argtypes = [C.c_ulonglong, _i, C.POINTER(_vp)]
@@ -130,7 +129,7 @@ def lib():
     L.bdg_lines16_close.restype = None
     for name in ("bdg_init", "bdg_host_alloc", "bdg_pack16", "bdg_dedup_first_seen", "bdg_edges_build", "bdg_edges_build_part", "bdg_edges_build_resident", "bdg_edges_build_into", "bdg_edges_copy", "bdg_cluster_levels", "bdg_cluster_levels_from_edges", "bdg_member_sorted",
                  "bdg_nearest_bounded", "bdg_kmer_score", "bdg_kmer_index_create", "bdg_kmer_index_query", "bdg_dev_edges_build", "bdg_set_edge_mode", "bdg_dev_edges_stats", "bdg_dev_edges_stats_raw", "bdg_dev_edges_balance", "bdg_join_lane_stats", "bdg_dev_pack16", "bdg_dev_member_sorted",
-                 "bdg_dev_nearest_bounded", "bdg_dev_pipe_probe", "bdg_tsv_open", "bdg_tsv_barcodes", "bdg_tsv_write_assignments", "bdg_lines16_open", "bdg_dedup_reads", "bdg_assign_reads", "bdg_pack16_sorted", "bdg_assign_reads32", "bdg_dedup_fetch", "bdg_centres_above", "bdg_centres_rest", "bdg_cluster_resident",
+                 "bdg_dev_nearest_bounded", "bdg_dev_pipe_probe", "bdg_tsv_open", "bdg_tsv_barcodes", "bdg_tsv_write_assignments", "bdg_lines16_open", "bdg_dedup_reads", "bdg_pack16_sorted", "bdg_assign_reads32", "bdg_dedup_fetch", "bdg_centres_above", "bdg_centres_rest", "bdg_cluster_resident",
                  "bdg_tsv_write_assignments32", "bdg_dev_dedup_reads", "bdg_dev_dedup_fetch", "bdg_dev_pack16_sorted", "bdg_dev_centres_above",
                  "bdg_dev_edges_copy", "bdg_dev_assign_reads32", "bdg_dev_dedup_merge", "bdg_dev_index_edges", "bdg_dev_cluster_init",
                  "bdg_dev_cluster_mark", "bdg_dev_cluster_claim", "bdg_dev_cluster_resolve", "bdg_dev_whitelist_check",

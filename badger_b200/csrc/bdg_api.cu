@@ -140,16 +140,27 @@ struct DevCtx {
     unsigned long long host_stats[bdg::MAX_PASSES][2] = {};   // interval tests done / tiles listed per pass of the last launch
     unsigned long long generation = 0;                        // bumped by every host-buffer edge build on this device
     ReadMap map;                                              // the read map of the last dedup call (first device)
-    Buf cl[4];                                                // clustering: centres, claim min / max, flags + count (result: map.centre / map.level)
-    Buf ce[9];                                                // centre selection: positions above the cutoff, sort keys / values, results, scratch
-    Buf as[6];                                                // masked dedup + per-read gather: all ranks, scan scratch, centre idx upload, centre values, result, counter
-    Buf mg[12];                                               // merge of the parts' dedup results (bdg_dev_dedup_merge), see there
-    Buf lk[5];                                                // per-read lookup (bdg_assign_lookup32): counters, and the host form's ranks, valid bytes, result, centre idx
+    Buf io;                                                   // one call's uploads, outputs and per-read scratch, carved by stage() (see there)
+    Buf sort_flag;                                            // whitelist check: index of the first entry not above its predecessor
+    Buf cl_centres, cl_min, cl_max, cl_flags;                 // clustering: centres, claim min / max, flags + count (result: map.centre / map.level)
+    // centre selection (centres_above, centres_rest) and pack16_sorted, which runs in the same buffers
+    Buf sel;                                                  // positions above the cutoff | pack16_sorted: the valid records' ranks
+    Buf sel_keys;                                             // their sort keys | the ranks sorted
+    Buf sel_sorted;                                           // the sort keys sorted | the distinct ranks (pack16_sorted's result)
+    Buf sel_scalars;                                          // count sum and selection size | the number of ranks kept
+    Buf sel_tmp;                                              // cub scratch of both
+    Buf sel_pos, head_ranks, head_counts, head_hits;          // centre selection: positions in count order, the head, its counts and hits
+    Buf mask_tmp;                                             // masked dedup: cub scratch of the scan of the valid bytes
+    Buf centre_val;                                           // per-read gathers: centre value + has byte per distinct barcode
+    Buf counters;                                             // per-read gathers: rows with a centre (assign_reads32) | assigned, missing (assign_lookup32)
+    struct {                                                  // merge of the parts' dedup results (bdg_dev_dedup_merge), see there
+        Buf starts, offs, key, idx, sorted_key, sorted_idx, cnt, first, head, scan, runs, tmp;
+    } mg;
     Buf gather_a, gather_b;                                   // node indices of the edge ends: this device's own, and (first device) those of ALL devices, gathered for cluster()
     Buf top16;                                                // first node of every high half of the barcode (the node of an edge end is searched in that run)
-    Buf io[4];                                                // host-buffer calls: pack16 letters / ranks / valid; membership whitelist / queries / hits;
-                                                              // nearest queries / targets / keys | argmin | distance; [3] check flag
-    Buf nn[9];                                                // sparse nearest: rotated keys + payload (in/out) of queries and targets, scratch
+    struct NearSide { Buf key, pay, key_sorted, pay_sorted; };
+    NearSide nn_q, nn_t;                                      // sparse nearest: rotated keys + payload (in / sorted) of the queries and the targets
+    Buf nn_tmp;                                               // sparse nearest: radix-sort scratch
     // join form of the t = 2 and t = 3 edge construction (bdg_join.cuh): barcodes in the key order of every condition's row side /
     // column side, first column of every key, bucket sizes and every barcode's place in its bucket, scan scratch, units per slab
     // and their prefix sums (one set per stream: the conditions of a block set run back to back on one stream); the t = 2
@@ -732,15 +743,14 @@ int launch_nearest_sparse(const uint32_t* d_q, size_t Q, const uint32_t* d_t, si
 {
     const int T_ = max_d <= 1 ? 1 : 2;
     const int passes = bdg::n_passes(T_);
-    // nn[0..3]: query keys in / payload in / keys sorted / payload sorted; nn[4..7]: the same for the targets; nn[8]: sort scratch
-    for (int k = 0; k < 4; k++) if (int e = ws->nn[k].ensure(Q * 4)) return e;
-    for (int k = 4; k < 8; k++) if (int e = ws->nn[k].ensure(W * 4)) return e;
-    uint32_t *qk = (uint32_t*)ws->nn[0].p, *qp = (uint32_t*)ws->nn[1].p, *qks = (uint32_t*)ws->nn[2].p, *qps = (uint32_t*)ws->nn[3].p;
-    uint32_t *tk = (uint32_t*)ws->nn[4].p, *tp = (uint32_t*)ws->nn[5].p, *tks = (uint32_t*)ws->nn[6].p, *tps = (uint32_t*)ws->nn[7].p;
+    for (Buf* b : {&ws->nn_q.key, &ws->nn_q.pay, &ws->nn_q.key_sorted, &ws->nn_q.pay_sorted}) if (int e = b->ensure(Q * 4)) return e;
+    for (Buf* b : {&ws->nn_t.key, &ws->nn_t.pay, &ws->nn_t.key_sorted, &ws->nn_t.pay_sorted}) if (int e = b->ensure(W * 4)) return e;
+    uint32_t *qk = (uint32_t*)ws->nn_q.key.p, *qp = (uint32_t*)ws->nn_q.pay.p, *qks = (uint32_t*)ws->nn_q.key_sorted.p, *qps = (uint32_t*)ws->nn_q.pay_sorted.p;
+    uint32_t *tk = (uint32_t*)ws->nn_t.key.p, *tp = (uint32_t*)ws->nn_t.pay.p, *tks = (uint32_t*)ws->nn_t.key_sorted.p, *tps = (uint32_t*)ws->nn_t.pay_sorted.p;
     size_t tmp_q = 0, tmp_t = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_q, qk, qks, qp, qps, (int)Q, 0, 32, st));
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp_t, tk, tks, tp, tps, (int)W, 0, 32, st));
-    if (int e = ws->nn[8].ensure(std::max(tmp_q, tmp_t))) return e;
+    if (int e = ws->nn_tmp.ensure(std::max(tmp_q, tmp_t))) return e;
     const uint32_t NS = (uint32_t)((W + bdg::SSB - 1) / bdg::SSB);
     const uint32_t K = (uint32_t)((Q + bdg::GROUP - 1) / bdg::GROUP);
     if (int e = ws->tile_bnd[0].ensure((size_t)NS * sizeof(uint2))) return e;
@@ -757,8 +767,8 @@ int launch_nearest_sparse(const uint32_t* d_q, size_t Q, const uint32_t* d_t, si
         const int qb = (int)std::min<size_t>((Q + 255) / 256, (size_t)ws->sms * 8), tb = (int)std::min<size_t>((W + 255) / 256, (size_t)ws->sms * 8);
         bdg::rotate_keys_iota_kernel<<<qb, 256, 0, st>>>(d_q, qk, qp, (uint32_t)Q, rot);
         bdg::rotate_keys_iota_kernel<<<tb, 256, 0, st>>>(d_t, tk, tp, (uint32_t)W, rot);
-        CU_TRY(cub::DeviceRadixSort::SortPairs(ws->nn[8].p, tmp_q, qk, qks, qp, qps, (int)Q, 0, 32, st));
-        CU_TRY(cub::DeviceRadixSort::SortPairs(ws->nn[8].p, tmp_t, tk, tks, tp, tps, (int)W, 0, 32, st));
+        CU_TRY(cub::DeviceRadixSort::SortPairs(ws->nn_tmp.p, tmp_q, qk, qks, qp, qps, (int)Q, 0, 32, st));
+        CU_TRY(cub::DeviceRadixSort::SortPairs(ws->nn_tmp.p, tmp_t, tk, tks, tp, tps, (int)W, 0, 32, st));
         bdg::tile_bounds_kernel<<<std::min<uint32_t>((NS + 255) / 256, (uint32_t)ws->sms * 8), 256, 0, st>>>(tks, (uint32_t)W, (uint2*)ws->tile_bnd[0].p, NS);
         g_launches += 3;
         bdg::EdgeWork w{};
@@ -876,6 +886,7 @@ int check_on_first(const void* p, const char* what)
 // work the caller queued on its own stream so far is done (it produces the inputs and frees the output buffers); the
 // destructor, on every return path, holds the caller's stream until the library's work is done (it writes the outputs and
 // reads the inputs).
+// A host-buffer call passes the library's own stream: there is nothing to order.
 struct CallerOrder {
     DevCtx& c;
     cudaStream_t caller;
@@ -883,6 +894,7 @@ struct CallerOrder {
     CallerOrder(DevCtx& c_, void* stream) : c(c_), caller((cudaStream_t)stream) {}
     int begin()
     {
+        if (caller == c.stream) return BDG_OK;
         CU_TRY(cudaEventRecord(c.ev_caller, caller));
         CU_TRY(cudaStreamWaitEvent(c.stream, c.ev_caller, 0));
         armed = true;
@@ -893,6 +905,61 @@ struct CallerOrder {
         if (armed && cudaEventRecord(c.ev_caller, c.stream) == cudaSuccess) cudaStreamWaitEvent(caller, c.ev_caller, 0);
     }
 };
+
+// The correction step runs on the first claimed context; its device is made current.
+int first_ctx(DevCtx** out)
+{
+    if (int rc = need_ctx()) return rc;
+    *out = &g_ctx[0];
+    CU_TRY(cudaSetDevice(g_ctx[0].dev));
+    return BDG_OK;
+}
+
+// What the argument check of an entry point returns when the call has nothing to do (an empty input); the entry point then
+// returns BDG_OK (every error code is negative).
+constexpr int EMPTY = 1;
+int done(int rc) { return rc == EMPTY ? BDG_OK : rc; }
+
+// c.io carved into consecutive pieces (256-byte aligned), grown first to their sum: the uploads, outputs and per-read scratch of
+// one call.  Every call that stages there ends with a synchronise or runs in stream order on c.stream, so the next call finds
+// it free.  Example: stage(c, {piece(d_q, Q * 4), piece(d_hit, Q)}).
+struct Piece { void** at; size_t bytes; };
+template <typename T> Piece piece(T*& p, size_t bytes) { return {(void**)&p, bytes}; }
+
+int stage(DevCtx& c, std::initializer_list<Piece> parts)
+{
+    auto round = [](size_t b) { return (b + 255) / 256 * 256; };
+    size_t total = 0;
+    for (const Piece& x : parts) total += round(x.bytes);
+    if (int e = c.io.ensure(std::max<size_t>(total, 1))) return e;
+    char* at = (char*)c.io.p;
+    for (const Piece& x : parts) { *x.at = at; at += round(x.bytes); }
+    return BDG_OK;
+}
+
+// The sort check of a whitelist on the device: sort_check launches it on c.stream, sort_check_result reads the index of the first
+// entry that is not above its predecessor back (waiting for everything queued on c.stream) and refuses the whitelist if there is one.
+int sort_check(DevCtx& c, const uint32_t* d_wl, size_t W)
+{
+    if (int e = c.sort_flag.ensure(8)) return e;
+    CU_TRY(cudaMemsetAsync(c.sort_flag.p, 0xFF, 8, c.stream));
+    if (W > 1) {
+        bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, c.stream>>>(
+            d_wl, (uint32_t)W, (unsigned long long*)c.sort_flag.p);
+        g_launches++;
+    }
+    CU_TRY(cudaGetLastError());
+    return BDG_OK;
+}
+
+int sort_check_result(DevCtx& c)
+{
+    unsigned long long first_bad = ~0ull;
+    CU_TRY(cudaMemcpyAsync(&first_bad, c.sort_flag.p, 8, cudaMemcpyDeviceToHost, c.stream));
+    CU_TRY(cudaStreamSynchronize(c.stream));
+    if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "whitelist not sorted at index %llu", first_bad);
+    return BDG_OK;
+}
 
 }  // namespace
 
@@ -911,8 +978,10 @@ struct bdg_kmer_index {
     int dev = -1;
     size_t W = 0;
     Buf wl;
-    Buf outb[6];
-    Buf kstart, post, scratch;        // posting lists: first posting of every 6-mer (4097 words), string ids grouped by 6-mer
+    Buf hit_q, hit_w, hit_cnt;        // host-buffer queries: the hits before they are copied out
+    Buf mult;                         // packed 6-mer positions per hit (the device form unpacks them)
+    Buf total;                        // hit counter
+    Buf kstart, post, scratch;       // posting lists: first posting of every 6-mer (4097 words), string ids grouped by 6-mer
     bool posted = false;
     cudaEvent_t ev[2] = {nullptr, nullptr};   // around the last query's kernel
     bool timed = false;
@@ -1116,19 +1185,31 @@ int bdg_dev_pack16(const char* d_seqs, size_t R, uint32_t* d_out, uint8_t* d_val
     return BDG_OK;
 }
 
-int bdg_dev_member_sorted(const uint32_t* d_wl, size_t W, const uint32_t* d_q, size_t Q, uint8_t* d_hit, void* stream)
+static int member_sorted_args(const uint32_t* wl, size_t W, const uint32_t* q, size_t Q, const uint8_t* hit)
 {
-    if (Q == 0) return BDG_OK;
-    if (!d_q || !d_hit || (W && !d_wl)) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (Q == 0) return EMPTY;
+    if (!q || !hit || (W && !wl)) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (W > 0xFFFFFFFFull || Q > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (W == 0) { CU_TRY(cudaMemsetAsync(d_hit, 0, Q, (cudaStream_t)stream)); return BDG_OK; }
+    return BDG_OK;
+}
+
+// Membership of Q > 0 queries in the sorted whitelist, on the current device and the given stream.
+static int member_sorted_body(const uint32_t* d_wl, size_t W, const uint32_t* d_q, size_t Q, uint8_t* d_hit, cudaStream_t st)
+{
+    if (W == 0) { CU_TRY(cudaMemsetAsync(d_hit, 0, Q, st)); return BDG_OK; }
     int grid = 0;
     if (int rc = grid_for((const void*)bdg::member_kernel, &grid)) return rc;
     const int blocks = (int)std::min<uint64_t>((uint64_t)grid, (Q + bdg::NT - 1) / bdg::NT);
-    bdg::member_kernel<<<blocks, bdg::NT, 0, (cudaStream_t)stream>>>(d_wl, (uint32_t)W, d_q, (uint32_t)Q, d_hit);
+    bdg::member_kernel<<<blocks, bdg::NT, 0, st>>>(d_wl, (uint32_t)W, d_q, (uint32_t)Q, d_hit);
     g_launches++;
     CU_TRY(cudaGetLastError());
     return BDG_OK;
+}
+
+int bdg_dev_member_sorted(const uint32_t* d_wl, size_t W, const uint32_t* d_q, size_t Q, uint8_t* d_hit, void* stream)
+{
+    if (int rc = member_sorted_args(d_wl, W, d_q, Q, d_hit)) return done(rc);
+    return member_sorted_body(d_wl, W, d_q, Q, d_hit, (cudaStream_t)stream);
 }
 
 int bdg_dev_nearest_bounded(const uint32_t* d_q, size_t Q, const uint32_t* d_t, size_t W, int max_d, uint32_t* d_keys,
@@ -1254,7 +1335,8 @@ int bdg_dedup_first_seen(const uint32_t* ranks, size_t R, uint32_t* distinct, ui
 
 // ---- f-1 + f-2 on the device: masked dedup that keeps the read map resident, and the per-read gather that uses it ------
 // ranks / valid are host arrays (kind = cudaMemcpyHostToDevice) or device arrays on c.dev (cudaMemcpyDeviceToDevice): the masked
-// compaction reads device ranks in place; the valid bytes are always copied, because the per-read gather reads them again.
+// compaction reads device ranks in place (host ranks are uploaded into c.io first); the valid bytes are always copied, because
+// the per-read gather reads them again.
 static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* valid, size_t R_all, cudaMemcpyKind kind, uint32_t* distinct,
                             uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid,
                             unsigned long long* token)
@@ -1266,8 +1348,7 @@ static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* val
     size_t n_reads = R_all;
     m.masked = valid != nullptr;
     if (valid) {
-        // as[0] all ranks (host input), as[1] scan scratch; the valid bytes and their scan stay with the read map
-        if (int e = c.as[0].ensure(R_all * 4)) return e;
+        // the valid bytes and their scan stay with the read map
         if (int e = m.valid.ensure(R_all)) return e;
         if (int e = m.valid_scan.ensure((R_all + 1) * 4)) return e;
         const uint8_t* d_valid = (const uint8_t*)m.valid.p;
@@ -1275,14 +1356,16 @@ static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* val
         auto flags = thrust::make_transform_iterator(d_valid, bdg::NonZero());
         size_t tmp = 0;
         CU_TRY(cub::DeviceScan::ExclusiveSum(nullptr, tmp, flags, d_excl, (int)R_all, st));
-        if (int e = c.as[1].ensure(tmp)) return e;
+        if (int e = c.mask_tmp.ensure(tmp)) return e;
         const uint32_t* d_ranks = ranks;
         if (kind == cudaMemcpyHostToDevice) {
-            CU_TRY(cudaMemcpyAsync(c.as[0].p, ranks, R_all * 4, kind, st));
-            d_ranks = (const uint32_t*)c.as[0].p;
+            uint32_t* up = nullptr;
+            if (int e = stage(c, {piece(up, R_all * 4)})) return e;
+            CU_TRY(cudaMemcpyAsync(up, ranks, R_all * 4, kind, st));
+            d_ranks = up;
         }
         CU_TRY(cudaMemcpyAsync(m.valid.p, valid, R_all, kind, st));
-        CU_TRY(cub::DeviceScan::ExclusiveSum(c.as[1].p, tmp, flags, d_excl, (int)R_all, st));
+        CU_TRY(cub::DeviceScan::ExclusiveSum(c.mask_tmp.p, tmp, flags, d_excl, (int)R_all, st));
         const int blocks = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
         bdg::compact_valid_kernel<<<blocks, 256, 0, st>>>(d_ranks, d_valid, d_excl, (uint32_t)R_all, (uint32_t*)m.keys().p);
         g_launches++;
@@ -1302,42 +1385,53 @@ static int dedup_reads_core(DevCtx& c, const uint32_t* ranks, const uint8_t* val
     return m.install(*n_distinct, nullptr, nullptr, nullptr, nullptr, st, token);       // dedup_core left the arrays in place
 }
 
-int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos,
-                    uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+static int dedup_reads_args(const uint32_t* ranks, size_t R_all, size_t* n_distinct, size_t* n_valid, unsigned long long* token, DevCtx** c)
 {
     if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
     *n_distinct = 0; *n_valid = 0; *token = 0;
-    if (R_all == 0) return BDG_OK;
+    if (R_all == 0) return EMPTY;
     if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (R_all > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
-    return dedup_reads_core(c, ranks, valid, R_all, cudaMemcpyHostToDevice, distinct, counts, sorted_pos, sorted_distinct, n_distinct, n_valid, token);
+    return first_ctx(c);
+}
+
+// The host form downloads the outputs it was given (kind = cudaMemcpyHostToDevice; see dedup_reads_core), the device form has none.
+static int dedup_reads_body(DevCtx& c, const uint32_t* ranks, const uint8_t* valid, size_t R_all, cudaMemcpyKind kind, uint32_t* distinct,
+                            uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid,
+                            unsigned long long* token, cudaStream_t caller)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
+    return dedup_reads_core(c, ranks, valid, R_all, kind, distinct, counts, sorted_pos, sorted_distinct, n_distinct, n_valid, token);
+}
+
+int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos,
+                    uint32_t* sorted_distinct, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+{
+    DevCtx* c = nullptr;
+    if (int rc = dedup_reads_args(ranks, R_all, n_distinct, n_valid, token, &c)) return done(rc);
+    return dedup_reads_body(*c, ranks, valid, R_all, cudaMemcpyHostToDevice, distinct, counts, sorted_pos, sorted_distinct, n_distinct, n_valid,
+                            token, c->stream);
 }
 
 int bdg_dev_dedup_reads(const uint32_t* d_ranks, const uint8_t* d_valid, size_t R_all, size_t* n_distinct, size_t* n_valid,
                         unsigned long long* token, void* stream)
 {
-    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_distinct = 0; *n_valid = 0; *token = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!d_ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R_all > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = dedup_reads_args(d_ranks, R_all, n_distinct, n_valid, token, &c)) return done(rc);
     if (int rc = check_on_first(d_ranks, "ranks")) return rc;
     if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
-    CallerOrder order(c, stream);
-    if (int rc = order.begin()) return rc;
-    return dedup_reads_core(c, d_ranks, d_valid, R_all, cudaMemcpyDeviceToDevice, nullptr, nullptr, nullptr, nullptr, n_distinct, n_valid, token);
+    return dedup_reads_body(*c, d_ranks, d_valid, R_all, cudaMemcpyDeviceToDevice, nullptr, nullptr, nullptr, nullptr, n_distinct, n_valid, token,
+                            (cudaStream_t)stream);
 }
 
 // What bdg_dedup_reads left on the device, on demand (any pointer may be NULL): the arrays of its output list, to the host
 // (kind = cudaMemcpyDeviceToHost, the call waits for the copies) or to device memory on c.dev (stream-ordered, no wait).
-static int dedup_fetch_core(DevCtx& c, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, cudaMemcpyKind kind)
+static int dedup_fetch_body(DevCtx& c, uint32_t* distinct, uint32_t* counts, uint32_t* sorted_pos, uint32_t* sorted_distinct, cudaMemcpyKind kind,
+                            cudaStream_t caller)
 {
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     const ReadMap& m = c.map;
     const size_t n = m.distinct;
     if (distinct) CU_TRY(cudaMemcpyAsync(distinct, m.first_seen(), n * 4, kind, c.stream));
@@ -1352,7 +1446,7 @@ int bdg_dedup_fetch(unsigned long long token, uint32_t* distinct, uint32_t* coun
 {
     DevCtx* c = nullptr;
     if (int rc = map_ctx(token, &c)) return rc;
-    return dedup_fetch_core(*c, distinct, counts, sorted_pos, sorted_distinct, cudaMemcpyDeviceToHost);
+    return dedup_fetch_body(*c, distinct, counts, sorted_pos, sorted_distinct, cudaMemcpyDeviceToHost, c->stream);
 }
 
 int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t* d_counts, uint32_t* d_sorted_pos, uint32_t* d_sorted_distinct,
@@ -1360,16 +1454,13 @@ int bdg_dev_dedup_fetch(unsigned long long token, uint32_t* d_distinct, uint32_t
 {
     DevCtx* c = nullptr;
     if (int rc = map_ctx(token, &c)) return rc;
-    uint32_t* outs[4] = {d_distinct, d_counts, d_sorted_pos, d_sorted_distinct};
-    for (uint32_t* p : outs)
+    for (uint32_t* p : {d_distinct, d_counts, d_sorted_pos, d_sorted_distinct})
         if (p && c->map.distinct) if (int rc = check_on_first(p, "output")) return rc;
-    CallerOrder order(*c, stream);
-    if (int rc = order.begin()) return rc;
-    return dedup_fetch_core(*c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice);
+    return dedup_fetch_body(*c, d_distinct, d_counts, d_sorted_pos, d_sorted_distinct, cudaMemcpyDeviceToDevice, (cudaStream_t)stream);
 }
 
 // ---- the dedup results of P parts (one process per GPU) reduced to the global distinct set (bdg_kernels.cuh, merge_*) ----
-// The work arrays live in mg[] until the end, so that a failed check leaves the token's read map as it was; only then are the
+// The work arrays live in c.mg until the end, so that a failed check leaves the token's read map as it was; only then are the
 // global arrays installed as the read map (counts, order, first-seen, ascending) and its read_pos rewritten in place.  The valid
 // rows are not touched.
 static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d_counts, const uint32_t* d_first, const size_t* starts,
@@ -1388,30 +1479,30 @@ static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d
     h_offs[n_parts] = (uint32_t)total;
     if (total == 0) return fail(BDG_ERR_ARG, "no part holds a barcode");
     const uint32_t T = (uint32_t)total, n_mine = (uint32_t)sizes[my_part], off_mine = h_offs[my_part];
-    // mg[0] part starts, [1] part offsets, [2] keys, [3] entry index, [4] sorted keys, [5] sorted index, [6] counts, [7] first keys,
-    // [8] heads / run order, [9] scan / sorted first keys, [10] run key | count | first | own run | position of run | local -> global, [11] scratch
-    if (int e = c.mg[0].ensure((size_t)n_parts * 8)) return e;
-    if (int e = c.mg[1].ensure(((size_t)n_parts + 1) * 4 + 4)) return e;
-    for (int k = 2; k < 10; k++) if (int e = c.mg[k].ensure(total * 4)) return e;
-    if (int e = c.mg[10].ensure((5 * total + std::max<size_t>(n_mine, 1)) * 4)) return e;
-    uint32_t *d_key = (uint32_t*)c.mg[2].p, *d_idx = (uint32_t*)c.mg[3].p, *d_sk = (uint32_t*)c.mg[4].p, *d_si = (uint32_t*)c.mg[5].p;
-    uint32_t *d_cnt = (uint32_t*)c.mg[6].p, *d_fst = (uint32_t*)c.mg[7].p, *d_head = (uint32_t*)c.mg[8].p, *d_scan = (uint32_t*)c.mg[9].p;
-    uint32_t *d_rk = (uint32_t*)c.mg[10].p, *d_rc = d_rk + total, *d_rf = d_rc + total, *d_mrun = d_rf + total, *d_prun = d_mrun + total,
+    // mg.head also holds the run order, mg.scan the sorted first keys; mg.runs: run key | count | first | own run | position of run | local -> global
+    auto& g = c.mg;
+    if (int e = g.starts.ensure((size_t)n_parts * 8)) return e;
+    if (int e = g.offs.ensure(((size_t)n_parts + 1) * 4 + 4)) return e;
+    for (Buf* b : {&g.key, &g.idx, &g.sorted_key, &g.sorted_idx, &g.cnt, &g.first, &g.head, &g.scan}) if (int e = b->ensure(total * 4)) return e;
+    if (int e = g.runs.ensure((5 * total + std::max<size_t>(n_mine, 1)) * 4)) return e;
+    uint32_t *d_key = (uint32_t*)g.key.p, *d_idx = (uint32_t*)g.idx.p, *d_sk = (uint32_t*)g.sorted_key.p, *d_si = (uint32_t*)g.sorted_idx.p;
+    uint32_t *d_cnt = (uint32_t*)g.cnt.p, *d_fst = (uint32_t*)g.first.p, *d_head = (uint32_t*)g.head.p, *d_scan = (uint32_t*)g.scan.p;
+    uint32_t *d_rk = (uint32_t*)g.runs.p, *d_rc = d_rk + total, *d_rf = d_rc + total, *d_mrun = d_rf + total, *d_prun = d_mrun + total,
              *d_loc = d_prun + total;
-    unsigned int* d_bad = (unsigned int*)((uint32_t*)c.mg[1].p + n_parts + 1);
+    unsigned int* d_bad = (unsigned int*)((uint32_t*)g.offs.p + n_parts + 1);
     size_t tmp1 = 0, tmp2 = 0;
     CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
     CU_TRY(cub::DeviceScan::InclusiveSum(nullptr, tmp2, d_head, d_scan, (int)T, st));
-    if (int e = c.mg[11].ensure(std::max(tmp1, tmp2))) return e;
-    CU_TRY(cudaMemcpyAsync(c.mg[0].p, h_starts.data(), (size_t)n_parts * 8, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemcpyAsync(c.mg[1].p, h_offs.data(), ((size_t)n_parts + 1) * 4, cudaMemcpyHostToDevice, st));
+    if (int e = g.tmp.ensure(std::max(tmp1, tmp2))) return e;
+    CU_TRY(cudaMemcpyAsync(g.starts.p, h_starts.data(), (size_t)n_parts * 8, cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(g.offs.p, h_offs.data(), ((size_t)n_parts + 1) * 4, cudaMemcpyHostToDevice, st));
     CU_TRY(cudaMemsetAsync(d_bad, 0, 4, st));
     const int blocks = (int)std::min<size_t>((total + 255) / 256, (size_t)c.sms * 8);
-    bdg::merge_gather_kernel<<<blocks, 256, 0, st>>>(d_keys, d_counts, d_first, (const uint64_t*)c.mg[0].p, (const uint32_t*)c.mg[1].p, (uint32_t)n_parts,
+    bdg::merge_gather_kernel<<<blocks, 256, 0, st>>>(d_keys, d_counts, d_first, (const uint64_t*)g.starts.p, (const uint32_t*)g.offs.p, (uint32_t)n_parts,
                                                      T, (uint32_t)my_part, c.map.ascending(), d_key, d_idx, d_cnt, d_fst, d_bad);
-    CU_TRY(cub::DeviceRadixSort::SortPairs(c.mg[11].p, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
+    CU_TRY(cub::DeviceRadixSort::SortPairs(g.tmp.p, tmp1, d_key, d_sk, d_idx, d_si, (int)T, 0, 32, st));
     bdg::dedup_heads_kernel<<<blocks, 256, 0, st>>>(d_sk, T, d_head);
-    CU_TRY(cub::DeviceScan::InclusiveSum(c.mg[11].p, tmp2, d_head, d_scan, (int)T, st));
+    CU_TRY(cub::DeviceScan::InclusiveSum(g.tmp.p, tmp2, d_head, d_scan, (int)T, st));
     bdg::merge_runs_kernel<<<blocks, 256, 0, st>>>(d_sk, d_si, d_head, d_scan, T, d_cnt, d_fst, off_mine, n_mine, d_rk, d_rc, d_rf, d_mrun);
     g_launches += 3;
     CU_TRY(cudaGetLastError());
@@ -1423,7 +1514,7 @@ static int dedup_merge_core(DevCtx& c, const uint32_t* d_keys, const uint32_t* d
     if (bad) return fail(BDG_ERR_ARG, "the list of part %d is not the distinct list of the read map the token names", my_part);
     // runs by first key (unique: every key names one barcode of one part): d_scan := sorted first keys, d_head := order
     bdg::iota_kernel<<<blocks, 256, 0, st>>>(d_idx, n_runs);
-    CU_TRY(cub::DeviceRadixSort::SortPairs(c.mg[11].p, tmp1, d_rf, d_scan, d_idx, d_head, (int)n_runs, 0, 32, st));
+    CU_TRY(cub::DeviceRadixSort::SortPairs(g.tmp.p, tmp1, d_rf, d_scan, d_idx, d_head, (int)n_runs, 0, 32, st));
     // d_key / d_cnt are free: distinct and counts in first-seen order
     bdg::merge_finish_kernel<<<blocks, 256, 0, st>>>(d_head, d_rk, d_rc, n_runs, d_key, d_cnt, d_prun);
     g_launches += 2;
@@ -1533,10 +1624,23 @@ int tally_merge_step(DevCtx& c, bdg_tally* h, int src, size_t src_n, int dst, co
     return BDG_OK;
 }
 
-int tally_add_core(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, cudaMemcpyKind kind, size_t* n_valid)
+int tally_add_args(bdg_tally* h, const uint32_t* ranks, size_t R, size_t* n_valid, DevCtx** c)
 {
+    if (n_valid) *n_valid = 0;
+    if (int rc = tally_ready(h, c)) return rc;
     if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
+    if (R == 0) return EMPTY;
+    if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    return BDG_OK;
+}
+
+// ranks / valid as for dedup_reads_core
+int tally_add_body(DevCtx& c, bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, cudaMemcpyKind kind, size_t* n_valid,
+                   cudaStream_t caller)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     size_t nb = 0, nv = 0;
     unsigned long long tok = 0;
     const int rc = dedup_reads_core(c, ranks, valid, R, kind, nullptr, nullptr, nullptr, nullptr, &nb, &nv, &tok);
@@ -1627,8 +1731,17 @@ int tally_merge_parts_core(DevCtx& c, bdg_tally* h, const uint32_t* d_keys, cons
     return BDG_OK;
 }
 
-int tally_finish_core(DevCtx& c, bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
+int tally_finish_args(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, DevCtx** c)
 {
+    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_distinct = 0; *n_valid = 0; *token = 0;
+    return tally_ready(h, c);
+}
+
+int tally_finish_body(DevCtx& c, bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, cudaStream_t caller)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     if (h->over) return fail(BDG_ERR_ARG, "a barcode was counted 2^32 times or more; the counts of a read map are uint32");
     *n_valid = h->valid;
     h->finished = true;
@@ -1692,49 +1805,32 @@ void bdg_tally_free(bdg_tally* h)
 
 int bdg_tally_add(bdg_tally* h, const uint32_t* ranks, const uint8_t* valid, size_t R, size_t* n_valid)
 {
-    if (n_valid) *n_valid = 0;
     DevCtx* c = nullptr;
-    if (int rc = tally_ready(h, &c)) return rc;
-    if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
-    if (R == 0) return BDG_OK;
-    if (!ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    return tally_add_core(*c, h, ranks, valid, R, cudaMemcpyHostToDevice, n_valid);
+    if (int rc = tally_add_args(h, ranks, R, n_valid, &c)) return done(rc);
+    return tally_add_body(*c, h, ranks, valid, R, cudaMemcpyHostToDevice, n_valid, c->stream);
 }
 
 int bdg_dev_tally_add(bdg_tally* h, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R, size_t* n_valid, void* stream)
 {
-    if (n_valid) *n_valid = 0;
     DevCtx* c = nullptr;
-    if (int rc = tally_ready(h, &c)) return rc;
-    if (h->finished) return fail(BDG_ERR_ARG, "add after finish: the tally is closed");
-    if (R == 0) return BDG_OK;
-    if (!d_ranks) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 reads in one call");
+    if (int rc = tally_add_args(h, d_ranks, R, n_valid, &c)) return done(rc);
     if (int rc = check_on_first(d_ranks, "ranks")) return rc;
     if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
-    CallerOrder order(*c, stream);
-    if (int rc = order.begin()) return rc;
-    return tally_add_core(*c, h, d_ranks, d_valid, R, cudaMemcpyDeviceToDevice, n_valid);
+    return tally_add_body(*c, h, d_ranks, d_valid, R, cudaMemcpyDeviceToDevice, n_valid, (cudaStream_t)stream);
 }
 
 int bdg_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token)
 {
-    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_distinct = 0; *n_valid = 0; *token = 0;
     DevCtx* c = nullptr;
-    if (int rc = tally_ready(h, &c)) return rc;
-    return tally_finish_core(*c, h, n_distinct, n_valid, token);
+    if (int rc = tally_finish_args(h, n_distinct, n_valid, token, &c)) return rc;
+    return tally_finish_body(*c, h, n_distinct, n_valid, token, c->stream);
 }
 
 int bdg_dev_tally_finish(bdg_tally* h, size_t* n_distinct, size_t* n_valid, unsigned long long* token, void* stream)
 {
-    if (!n_distinct || !n_valid || !token) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_distinct = 0; *n_valid = 0; *token = 0;
     DevCtx* c = nullptr;
-    if (int rc = tally_ready(h, &c)) return rc;
-    CallerOrder order(*c, stream);
-    if (int rc = order.begin()) return rc;
-    return tally_finish_core(*c, h, n_distinct, n_valid, token);
+    if (int rc = tally_finish_args(h, n_distinct, n_valid, token, &c)) return rc;
+    return tally_finish_body(*c, h, n_distinct, n_valid, token, (cudaStream_t)stream);
 }
 
 int bdg_tally_info(bdg_tally* h, size_t* n_distinct, unsigned long long* rows, unsigned long long* valid)
@@ -1798,20 +1894,21 @@ int bdg_dev_tally_merge_parts(bdg_tally* h, const uint32_t* d_keys, const unsign
 // cutoff = max(mean(counts of the first n_cells barcodes in first-seen order) / 5, 5) (:255-256); the barcodes with
 // count > cutoff in count-descending order, ties in first-seen order (the head of `bc_by_counts`, :253), with their counts and
 // - when a whitelist is given - their membership (:264).  The short walk over that head stays with the caller.
-// sorted_wl is a host array (wl_on_device false: uploaded into io[0]) or device memory on c.dev, read in place.
-static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_wl, bool wl_on_device, size_t W, uint32_t* top_ranks,
-                              uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
+// sorted_wl is a host array (wl_on_device false: uploaded into c.io) or device memory on c.dev, read in place.
+static int centres_above_body(DevCtx& c, size_t n_cells, const uint32_t* sorted_wl, bool wl_on_device, size_t W, uint32_t* top_ranks,
+                              uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff, cudaStream_t caller)
 {
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     const size_t N = c.map.distinct;
     const size_t first = std::min(n_cells, N);
     if (first == 0) return fail(BDG_ERR_ARG, "mean requires at least one data point");
     cudaStream_t st = c.stream;
     const uint32_t* d_distinct = c.map.first_seen();
     const uint32_t* d_counts = c.map.counts();
-    // ce[0] selected positions, [1] keys, [2] sorted keys, [3] sorted positions, [4] top ranks, [5] top counts, [6] hits, [7] scalars + cub scratch
-    if (int e = c.ce[7].ensure(64)) return e;
-    unsigned long long* d_sum = (unsigned long long*)c.ce[7].p;
-    uint32_t* d_nsel = (uint32_t*)((char*)c.ce[7].p + 8);
+    if (int e = c.sel_scalars.ensure(64)) return e;
+    unsigned long long* d_sum = (unsigned long long*)c.sel_scalars.p;
+    uint32_t* d_nsel = (uint32_t*)((char*)c.sel_scalars.p + 8);
     CU_TRY(cudaMemsetAsync(d_sum, 0, 16, st));
     bdg::sum_first_kernel<<<(int)std::min<size_t>((first + 255) / 256, (size_t)c.sms * 4), 256, 0, st>>>(d_counts, (uint32_t)first, d_sum);
     g_launches++;
@@ -1821,13 +1918,13 @@ static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_
     const double cut = std::max(((double)sum / (double)first) / 5.0, 5.0);
     *cutoff = cut;
     const uint32_t thr = (uint32_t)std::floor(cut);          // counts are integers: count > cutoff <=> count > floor(cutoff)
-    if (int e = c.ce[0].ensure(N * 4)) return e;
+    if (int e = c.sel.ensure(N * 4)) return e;
     thrust::counting_iterator<uint32_t> all(0);
     bdg::CountAbove pred{d_counts, thr};
     size_t tmp = 0;
-    CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, pred, st));
-    if (int e = c.ce[8].ensure(tmp)) return e;
-    CU_TRY(cub::DeviceSelect::If(c.ce[8].p, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, pred, st));
+    CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.sel.p, d_nsel, (int)N, pred, st));
+    if (int e = c.sel_tmp.ensure(tmp)) return e;
+    CU_TRY(cub::DeviceSelect::If(c.sel_tmp.p, tmp, all, (uint32_t*)c.sel.p, d_nsel, (int)N, pred, st));
     uint32_t nsel = 0;
     CU_TRY(cudaMemcpyAsync(&nsel, d_nsel, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
@@ -1835,70 +1932,62 @@ static int centres_above_core(DevCtx& c, size_t n_cells, const uint32_t* sorted_
     if (nsel == 0) return BDG_OK;
     if (nsel > cap) return fail(BDG_ERR_CAPACITY, "%u barcodes above the cutoff but room for %zu", nsel, cap);
     if (!top_ranks || !top_counts) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    for (int k = 1; k <= 5; k++) if (int e = c.ce[k].ensure((size_t)nsel * 4)) return e;
-    if (int e = c.ce[6].ensure(nsel)) return e;
+    for (Buf* b : {&c.sel_keys, &c.sel_sorted, &c.sel_pos, &c.head_ranks, &c.head_counts}) if (int e = b->ensure((size_t)nsel * 4)) return e;
+    if (int e = c.head_hits.ensure(nsel)) return e;
+    const uint32_t *sel = (const uint32_t*)c.sel.p, *keys = (const uint32_t*)c.sel_keys.p;
+    uint32_t *ranks = (uint32_t*)c.head_ranks.p, *counts = (uint32_t*)c.head_counts.p;
     const int nb = (int)std::min<size_t>(((size_t)nsel + 255) / 256, (size_t)c.sms * 4);
-    bdg::centres_keys_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.ce[0].p, d_counts, nsel, (uint32_t*)c.ce[1].p);
+    bdg::centres_keys_kernel<<<nb, 256, 0, st>>>(sel, d_counts, nsel, (uint32_t*)c.sel_keys.p);
     size_t tmp2 = 0;
-    CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp2, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[3].p, (int)nsel, 0, 32, st));
-    if (int e = c.ce[8].ensure(tmp2)) return e;
-    CU_TRY(cub::DeviceRadixSort::SortPairs(c.ce[8].p, tmp2, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[3].p, (int)nsel, 0, 32, st));
-    bdg::centres_gather_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.ce[3].p, d_distinct, d_counts, nsel, (uint32_t*)c.ce[4].p, (uint32_t*)c.ce[5].p);
+    CU_TRY(cub::DeviceRadixSort::SortPairs(nullptr, tmp2, keys, (uint32_t*)c.sel_sorted.p, sel, (uint32_t*)c.sel_pos.p, (int)nsel, 0, 32, st));
+    if (int e = c.sel_tmp.ensure(tmp2)) return e;
+    CU_TRY(cub::DeviceRadixSort::SortPairs(c.sel_tmp.p, tmp2, keys, (uint32_t*)c.sel_sorted.p, sel, (uint32_t*)c.sel_pos.p, (int)nsel, 0, 32, st));
+    bdg::centres_gather_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.sel_pos.p, d_distinct, d_counts, nsel, ranks, counts);
     g_launches += 2;
     CU_TRY(cudaGetLastError());
     if (top_hits) {
         if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
         if (W && !sorted_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
-        if (int e = c.io[3].ensure(8)) return e;
-        unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
         const uint32_t* d_wl = sorted_wl;
         if (!wl_on_device) {
-            if (int e = c.io[0].ensure(std::max<size_t>(W, 1) * 4)) return e;
-            CU_TRY(cudaMemcpyAsync(c.io[0].p, sorted_wl, W * 4, cudaMemcpyHostToDevice, st));
-            d_wl = (const uint32_t*)c.io[0].p;
+            uint32_t* up = nullptr;
+            if (int e = stage(c, {piece(up, std::max<size_t>(W, 1) * 4)})) return e;
+            CU_TRY(cudaMemcpyAsync(up, sorted_wl, W * 4, cudaMemcpyHostToDevice, st));
+            d_wl = up;
         }
-        CU_TRY(cudaMemsetAsync(d_bad, 0xFF, 8, st));
-        if (W > 1) {
-            bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, st>>>(d_wl, (uint32_t)W, d_bad);
-            g_launches++;
-        }
-        if (int rc = bdg_dev_member_sorted(d_wl, W, (const uint32_t*)c.ce[4].p, nsel, (uint8_t*)c.ce[6].p, st)) return rc;
-        unsigned long long first_bad = ~0ull;
-        CU_TRY(cudaMemcpyAsync(top_hits, c.ce[6].p, nsel, cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaMemcpyAsync(&first_bad, d_bad, 8, cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaMemcpyAsync(top_ranks, c.ce[4].p, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaMemcpyAsync(top_counts, c.ce[5].p, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
-        CU_TRY(cudaStreamSynchronize(st));
-        if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "whitelist not sorted at index %llu", first_bad);
-        return BDG_OK;
+        if (int rc = sort_check(c, d_wl, W)) return rc;
+        if (int rc = member_sorted_body(d_wl, W, ranks, nsel, (uint8_t*)c.head_hits.p, st)) return rc;
+        CU_TRY(cudaMemcpyAsync(top_hits, c.head_hits.p, nsel, cudaMemcpyDeviceToHost, st));
     }
-    CU_TRY(cudaMemcpyAsync(top_ranks, c.ce[4].p, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(top_counts, c.ce[5].p, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(top_ranks, ranks, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cudaMemcpyAsync(top_counts, counts, (size_t)nsel * 4, cudaMemcpyDeviceToHost, st));
+    if (top_hits) return sort_check_result(c);               // (waits for the copies too)
     CU_TRY(cudaStreamSynchronize(st));
     return BDG_OK;
+}
+
+static int centres_above_args(unsigned long long token, size_t* n_above, double* cutoff, DevCtx** c)
+{
+    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n_above = 0; *cutoff = 0.0;
+    return map_ctx(token, c);
 }
 
 int bdg_centres_above(unsigned long long token, size_t n_cells, const uint32_t* sorted_wl, size_t W, uint32_t* top_ranks, uint32_t* top_counts,
                       uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff)
 {
-    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_above = 0; *cutoff = 0.0;
     DevCtx* c = nullptr;
-    if (int rc = map_ctx(token, &c)) return rc;
-    return centres_above_core(*c, n_cells, sorted_wl, false, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
+    if (int rc = centres_above_args(token, n_above, cutoff, &c)) return rc;
+    return centres_above_body(*c, n_cells, sorted_wl, false, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff, c->stream);
 }
 
 int bdg_dev_centres_above(unsigned long long token, size_t n_cells, const uint32_t* d_sorted_wl, size_t W, uint32_t* top_ranks,
                           uint32_t* top_counts, uint8_t* top_hits, size_t cap, size_t* n_above, double* cutoff, void* stream)
 {
-    if (!n_above || !cutoff) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n_above = 0; *cutoff = 0.0;
     DevCtx* c = nullptr;
-    if (int rc = map_ctx(token, &c)) return rc;
+    if (int rc = centres_above_args(token, n_above, cutoff, &c)) return rc;
     if (top_hits && W) if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
-    CallerOrder order(*c, stream);
-    if (int rc = order.begin()) return rc;
-    return centres_above_core(*c, n_cells, d_sorted_wl, true, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff);
+    return centres_above_body(*c, n_cells, d_sorted_wl, true, W, top_ranks, top_counts, top_hits, cap, n_above, cutoff, (cudaStream_t)stream);
 }
 
 // The stretch of `bc_by_counts` right behind the head bdg_centres_above returns (barcode_graph.py:273-276 runs into it when too few
@@ -1917,27 +2006,28 @@ int bdg_centres_rest(unsigned long long token, double cutoff, size_t need, uint3
     cudaStream_t st = c.stream;
     const uint32_t* d_distinct = c.map.first_seen();
     const uint32_t* d_counts = c.map.counts();
-    if (int e = c.ce[0].ensure(N * 4)) return e;
-    if (int e = c.ce[4].ensure(std::min(need, N) * 4)) return e;
-    if (int e = c.ce[5].ensure(std::min(need, N) * 4)) return e;
-    if (int e = c.ce[7].ensure(64)) return e;
-    uint32_t* d_nsel = (uint32_t*)((char*)c.ce[7].p + 8);
+    if (int e = c.sel.ensure(N * 4)) return e;
+    if (int e = c.head_ranks.ensure(std::min(need, N) * 4)) return e;
+    if (int e = c.head_counts.ensure(std::min(need, N) * 4)) return e;
+    if (int e = c.sel_scalars.ensure(64)) return e;
+    uint32_t* d_nsel = (uint32_t*)((char*)c.sel_scalars.p + 8);
     thrust::counting_iterator<uint32_t> all(0);
     size_t tmp = 0;
-    CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, bdg::CountIs{d_counts, 0u}, st));
-    if (int e = c.ce[8].ensure(tmp)) return e;
+    CU_TRY(cub::DeviceSelect::If(nullptr, tmp, all, (uint32_t*)c.sel.p, d_nsel, (int)N, bdg::CountIs{d_counts, 0u}, st));
+    if (int e = c.sel_tmp.ensure(tmp)) return e;
     size_t got = 0;
     for (long long v = (long long)std::floor(cutoff); v >= 1 && got < need; v--) {
-        CU_TRY(cub::DeviceSelect::If(c.ce[8].p, tmp, all, (uint32_t*)c.ce[0].p, d_nsel, (int)N, bdg::CountIs{d_counts, (uint32_t)v}, st));
+        CU_TRY(cub::DeviceSelect::If(c.sel_tmp.p, tmp, all, (uint32_t*)c.sel.p, d_nsel, (int)N, bdg::CountIs{d_counts, (uint32_t)v}, st));
         uint32_t nsel = 0;
         CU_TRY(cudaMemcpyAsync(&nsel, d_nsel, 4, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         const size_t take = std::min<size_t>(nsel, need - got);
         if (take == 0) continue;
         const int nb = (int)std::min<size_t>((take + 255) / 256, (size_t)c.sms * 4);
-        bdg::centres_gather_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.ce[0].p, d_distinct, d_counts, (uint32_t)take, (uint32_t*)c.ce[4].p, (uint32_t*)c.ce[5].p);
+        bdg::centres_gather_kernel<<<nb, 256, 0, st>>>((const uint32_t*)c.sel.p, d_distinct, d_counts, (uint32_t)take, (uint32_t*)c.head_ranks.p,
+                                                       (uint32_t*)c.head_counts.p);
         g_launches++;
-        CU_TRY(cudaMemcpyAsync(out_ranks + got, c.ce[4].p, take * 4, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaMemcpyAsync(out_ranks + got, c.head_ranks.p, take * 4, cudaMemcpyDeviceToHost, st));
         CU_TRY(cudaStreamSynchronize(st));
         got += take;
     }
@@ -1945,27 +2035,35 @@ int bdg_centres_rest(unsigned long long token, double cutoff, size_t need, uint3
     return BDG_OK;
 }
 
-// c: the context map_ctx returned for the token
-static int check_assign_args(const DevCtx& c, bool resident, size_t N, size_t R_all)
+// ---- f-2  the per-read gather: the 5-byte result per row (centre barcode + "has a centre" byte) ----------------------------
+static int assign_reads32_args(unsigned long long token, bool resident, size_t N, const uint32_t* centre_per_row, const uint8_t* has_centre,
+                               size_t R_all, size_t* n_assigned, DevCtx** c)
 {
-    if (N != c.map.distinct || R_all != c.map.rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
-    if (resident && N && c.map.cl_token != c.map.token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
+    if (n_assigned) *n_assigned = 0;
+    if (R_all == 0) return EMPTY;
+    if (!centre_per_row || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (int rc = map_ctx(token, c)) return rc;
+    const ReadMap& m = (*c)->map;
+    if (N != m.distinct || R_all != m.rows) return fail(BDG_ERR_ARG, "sizes do not match the dedup call the token came from");
+    if (resident && N && m.cl_token != m.token) return fail(BDG_ERR_ARG, "no clustering result of this dedup call is resident on the device (bdg_cluster_resident)");
     return BDG_OK;
 }
 
-// The per-read gather on c.stream: d_ci (device, on c.dev) is the centre index per node, NULL for the resident clustering result;
-// the 5-byte result goes to d_out / d_oh (device, R_all rows) and the number of rows with a centre to the counter in as[5].
-static int assign_reads32_core(DevCtx& c, const int32_t* d_ci, size_t N, uint32_t* d_out, uint8_t* d_oh, size_t R_all)
+// d_ci (device, on c.dev) is the centre index per node, NULL for the resident clustering result; the 5-byte result goes to d_out /
+// d_oh (device, R_all rows), the number of rows with a centre to *n_assigned (optional: the call then waits for it).
+static int assign_reads32_body(DevCtx& c, const int32_t* d_ci, size_t N, uint32_t* d_out, uint8_t* d_oh, size_t R_all, size_t* n_assigned,
+                               cudaStream_t caller)
 {
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     cudaStream_t st = c.stream;
     const ReadMap& m = c.map;
-    // as[3] centre value + has byte per distinct barcode, as[5] counter
-    if (int e = c.as[3].ensure(std::max<size_t>(N, 1) * 5)) return e;
-    if (int e = c.as[5].ensure(8)) return e;
+    if (int e = c.centre_val.ensure(std::max<size_t>(N, 1) * 5)) return e;
+    if (int e = c.counters.ensure(16)) return e;
     if (!d_ci) d_ci = (const int32_t*)m.centre.p;
-    CU_TRY(cudaMemsetAsync(c.as[5].p, 0, 8, st));
-    uint32_t* d_cv = (uint32_t*)c.as[3].p;
-    uint8_t* d_ch = (uint8_t*)c.as[3].p + std::max<size_t>(N, 1) * 4;
+    CU_TRY(cudaMemsetAsync(c.counters.p, 0, 8, st));
+    uint32_t* d_cv = (uint32_t*)c.centre_val.p;
+    uint8_t* d_ch = (uint8_t*)c.centre_val.p + std::max<size_t>(N, 1) * 4;
     if (N) {
         const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
         bdg::centre_of_distinct32_kernel<<<nb, 256, 0, st>>>(d_ci, m.order() /* first-seen -> node */, m.ascending() /* node -> barcode */,
@@ -1974,289 +2072,210 @@ static int assign_reads32_core(DevCtx& c, const int32_t* d_ci, size_t N, uint32_
     const int rb = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
     bdg::assign_reads32_kernel<<<rb, 256, 0, st>>>(d_cv, d_ch, m.read_pos(), m.masked ? (const uint8_t*)m.valid.p : nullptr,
                                                    m.masked ? (const uint32_t*)m.valid_scan.p : nullptr, (uint32_t)R_all, d_out, d_oh,
-                                                   (unsigned long long*)c.as[5].p);
+                                                   (unsigned long long*)c.counters.p);
     g_launches += 2;
     CU_TRY(cudaGetLastError());
+    if (n_assigned) {
+        unsigned long long cnt = 0;
+        CU_TRY(cudaMemcpyAsync(&cnt, c.counters.p, 8, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        *n_assigned = (size_t)cnt;
+    }
     return BDG_OK;
 }
 
-// bdg_assign_reads with a 5-byte result per row (centre barcode + "has a centre" byte).  centre_idx == NULL: the clustering a
-// bdg_cluster_resident call left on the device is used in place (nothing is uploaded).
+// centre_idx == NULL: the clustering a bdg_cluster_resident call left on the device is used in place (nothing is uploaded).
 int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size_t N, uint32_t* centre_per_row, uint8_t* has_centre, size_t R_all,
                        size_t* n_assigned)
 {
-    if (n_assigned) *n_assigned = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!centre_per_row || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    DevCtx* cp = nullptr;
-    if (int rc = map_ctx(token, &cp)) return rc;
-    DevCtx& c = *cp;
-    if (int rc = check_assign_args(c, !centre_idx, N, R_all)) return rc;
-    cudaStream_t st = c.stream;
-    // as[2] centre index per node (upload), as[4] result per row
-    if (int e = c.as[4].ensure(R_all * 5)) return e;
-    const int32_t* d_ci = nullptr;
-    if (centre_idx) {
-        if (int e = c.as[2].ensure(std::max<size_t>(N, 1) * 4)) return e;
-        CU_TRY(cudaMemcpyAsync(c.as[2].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-        d_ci = (const int32_t*)c.as[2].p;
-    }
-    uint32_t* d_out = (uint32_t*)c.as[4].p;
-    uint8_t* d_oh = (uint8_t*)c.as[4].p + R_all * 4;
-    if (int rc = assign_reads32_core(c, d_ci, N, d_out, d_oh, R_all)) return rc;
-    unsigned long long cnt = 0;
+    DevCtx* c = nullptr;
+    if (int rc = assign_reads32_args(token, !centre_idx, N, centre_per_row, has_centre, R_all, n_assigned, &c)) return done(rc);
+    cudaStream_t st = c->stream;
+    int32_t* d_ci = nullptr;
+    uint32_t* d_out = nullptr;
+    uint8_t* d_oh = nullptr;
+    if (int e = stage(*c, {piece(d_out, R_all * 4), piece(d_oh, R_all), piece(d_ci, centre_idx ? N * 4 : 0)})) return e;
+    if (centre_idx) CU_TRY(cudaMemcpyAsync(d_ci, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+    if (int rc = assign_reads32_body(*c, centre_idx ? d_ci : nullptr, N, d_out, d_oh, R_all, n_assigned, st)) return rc;
     CU_TRY(cudaMemcpyAsync(centre_per_row, d_out, R_all * 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(has_centre, d_oh, R_all, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    if (n_assigned) *n_assigned = (size_t)cnt;
     return BDG_OK;
 }
 
 int bdg_dev_assign_reads32(unsigned long long token, const int32_t* d_centre_idx, size_t N, uint32_t* d_centre_per_row, uint8_t* d_has_centre,
                            size_t R_all, size_t* n_assigned, void* stream)
 {
-    if (n_assigned) *n_assigned = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!d_centre_per_row || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    DevCtx* cp = nullptr;
-    if (int rc = map_ctx(token, &cp)) return rc;
-    DevCtx& c = *cp;
-    if (int rc = check_assign_args(c, !d_centre_idx, N, R_all)) return rc;
+    DevCtx* c = nullptr;
+    if (int rc = assign_reads32_args(token, !d_centre_idx, N, d_centre_per_row, d_has_centre, R_all, n_assigned, &c)) return done(rc);
     if (d_centre_idx && N) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
     if (int rc = check_on_first(d_centre_per_row, "centre_per_row")) return rc;
     if (int rc = check_on_first(d_has_centre, "has_centre")) return rc;
-    CallerOrder order(c, stream);
-    if (int rc = order.begin()) return rc;
-    if (int rc = assign_reads32_core(c, N ? d_centre_idx : nullptr, N, d_centre_per_row, d_has_centre, R_all)) return rc;
-    if (n_assigned) {
-        unsigned long long cnt = 0;
-        CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, c.stream));
-        CU_TRY(cudaStreamSynchronize(c.stream));
-        *n_assigned = (size_t)cnt;
-    }
-    return BDG_OK;
+    return assign_reads32_body(*c, N ? d_centre_idx : nullptr, N, d_centre_per_row, d_has_centre, R_all, n_assigned, (cudaStream_t)stream);
 }
 
 // The per-read gather for rows outside any read map: every valid row's barcode is looked up among the token's nodes (the
-// ascending array); d_ci as for assign_reads32_core.  Counters (assigned, missing) go to lk[0].
-static int assign_lookup32_core(DevCtx& c, const int32_t* d_ci, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R,
-                                uint32_t* d_out, uint8_t* d_oh)
+// ascending array).
+static int assign_lookup32_args(unsigned long long token, bool resident, size_t N, const uint32_t* ranks, size_t R, const uint32_t* centre,
+                                const uint8_t* has_centre, size_t* n_assigned, size_t* n_missing, DevCtx** c)
 {
+    if (n_assigned) *n_assigned = 0;
+    if (n_missing) *n_missing = 0;
+    if (int rc = map_ctx(token, c)) return rc;
+    const ReadMap& m = (*c)->map;
+    if (N != m.distinct) return fail(BDG_ERR_ARG, "N does not match the read map the token names");
+    if (resident && m.cl_token != m.token) return fail(BDG_ERR_ARG, "no clustering result of this read map is resident on the device (bdg_cluster_resident)");
+    if (R == 0) return EMPTY;
+    if (!ranks || !centre || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    return BDG_OK;
+}
+
+// d_ci as for assign_reads32_body; the counters (assigned, missing) go to *n_assigned / *n_missing (optional: the call then waits).
+static int assign_lookup32_body(DevCtx& c, const int32_t* d_ci, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid, size_t R,
+                                uint32_t* d_out, uint8_t* d_oh, size_t* n_assigned, size_t* n_missing, cudaStream_t caller)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     cudaStream_t st = c.stream;
-    if (int e = c.lk[0].ensure(16)) return e;
+    if (int e = c.counters.ensure(16)) return e;
     if (!d_ci) d_ci = (const int32_t*)c.map.centre.p;
-    CU_TRY(cudaMemsetAsync(c.lk[0].p, 0, 16, st));
+    CU_TRY(cudaMemsetAsync(c.counters.p, 0, 16, st));
     const int rb = (int)std::min<size_t>((R + bdg::NT - 1) / bdg::NT, (size_t)c.sms * 8);
     bdg::lookup_assign32_kernel<<<rb, bdg::NT, 0, st>>>(c.map.ascending(), (uint32_t)N, d_ci, d_ranks, d_valid, R, d_out, d_oh,
-                                                         (unsigned long long*)c.lk[0].p);
+                                                         (unsigned long long*)c.counters.p);
     g_launches++;
     CU_TRY(cudaGetLastError());
-    return BDG_OK;
-}
-
-// c: the context map_ctx returned for the token
-static int check_lookup_args(const DevCtx& c, bool resident, size_t N)
-{
-    if (N != c.map.distinct) return fail(BDG_ERR_ARG, "N does not match the read map the token names");
-    if (resident && c.map.cl_token != c.map.token) return fail(BDG_ERR_ARG, "no clustering result of this read map is resident on the device (bdg_cluster_resident)");
-    return BDG_OK;
-}
-
-static int read_lookup_counters(DevCtx& c, size_t* n_assigned, size_t* n_missing)
-{
-    unsigned long long cnt[2] = {0, 0};
-    CU_TRY(cudaMemcpyAsync(cnt, c.lk[0].p, 16, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
-    if (n_assigned) *n_assigned = (size_t)cnt[0];
-    if (n_missing) *n_missing = (size_t)cnt[1];
+    if (n_assigned || n_missing) {
+        unsigned long long cnt[2] = {0, 0};
+        CU_TRY(cudaMemcpyAsync(cnt, c.counters.p, 16, cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        if (n_assigned) *n_assigned = (size_t)cnt[0];
+        if (n_missing) *n_missing = (size_t)cnt[1];
+    }
     return BDG_OK;
 }
 
 int bdg_assign_lookup32(unsigned long long token, const int32_t* centre_idx, size_t N, const uint32_t* ranks, const uint8_t* valid, size_t R,
                         uint32_t* centre, uint8_t* has_centre, size_t* n_assigned, size_t* n_missing)
 {
-    if (n_assigned) *n_assigned = 0;
-    if (n_missing) *n_missing = 0;
-    DevCtx* cp = nullptr;
-    if (int rc = map_ctx(token, &cp)) return rc;
-    DevCtx& c = *cp;
-    if (int rc = check_lookup_args(c, !centre_idx, N)) return rc;
-    if (R == 0) return BDG_OK;
-    if (!ranks || !centre || !has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    cudaStream_t st = c.stream;
-    // lk[1] ranks, lk[2] valid bytes, lk[3] result (R x 5 bytes), lk[4] centre index per node
-    if (int e = c.lk[1].ensure(R * 4)) return e;
-    if (int e = c.lk[3].ensure(R * 5)) return e;
-    CU_TRY(cudaMemcpyAsync(c.lk[1].p, ranks, R * 4, cudaMemcpyHostToDevice, st));
-    if (valid) {
-        if (int e = c.lk[2].ensure(R)) return e;
-        CU_TRY(cudaMemcpyAsync(c.lk[2].p, valid, R, cudaMemcpyHostToDevice, st));
-    }
-    const int32_t* d_ci = nullptr;
-    if (centre_idx) {
-        if (int e = c.lk[4].ensure(N * 4)) return e;
-        CU_TRY(cudaMemcpyAsync(c.lk[4].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-        d_ci = (const int32_t*)c.lk[4].p;
-    }
-    uint32_t* d_out = (uint32_t*)c.lk[3].p;
-    uint8_t* d_oh = (uint8_t*)c.lk[3].p + R * 4;
-    if (int rc = assign_lookup32_core(c, d_ci, N, (const uint32_t*)c.lk[1].p, valid ? (const uint8_t*)c.lk[2].p : nullptr, R, d_out, d_oh)) return rc;
+    DevCtx* c = nullptr;
+    if (int rc = assign_lookup32_args(token, !centre_idx, N, ranks, R, centre, has_centre, n_assigned, n_missing, &c)) return done(rc);
+    cudaStream_t st = c->stream;
+    uint32_t *d_ranks = nullptr, *d_out = nullptr;
+    uint8_t *d_valid = nullptr, *d_oh = nullptr;
+    int32_t* d_ci = nullptr;
+    if (int e = stage(*c, {piece(d_ranks, R * 4), piece(d_valid, valid ? R : 0), piece(d_out, R * 4), piece(d_oh, R),
+                           piece(d_ci, centre_idx ? N * 4 : 0)})) return e;
+    CU_TRY(cudaMemcpyAsync(d_ranks, ranks, R * 4, cudaMemcpyHostToDevice, st));
+    if (valid) CU_TRY(cudaMemcpyAsync(d_valid, valid, R, cudaMemcpyHostToDevice, st));
+    if (centre_idx) CU_TRY(cudaMemcpyAsync(d_ci, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
+    if (int rc = assign_lookup32_body(*c, centre_idx ? d_ci : nullptr, N, d_ranks, valid ? d_valid : nullptr, R, d_out, d_oh, n_assigned,
+                                      n_missing, st)) return rc;
     CU_TRY(cudaMemcpyAsync(centre, d_out, R * 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(has_centre, d_oh, R, cudaMemcpyDeviceToHost, st));
-    return read_lookup_counters(c, n_assigned, n_missing);
+    CU_TRY(cudaStreamSynchronize(st));
+    return BDG_OK;
 }
 
 int bdg_dev_assign_lookup32(unsigned long long token, const int32_t* d_centre_idx, size_t N, const uint32_t* d_ranks, const uint8_t* d_valid,
                             size_t R, uint32_t* d_centre, uint8_t* d_has_centre, size_t* n_assigned, size_t* n_missing, void* stream)
 {
-    if (n_assigned) *n_assigned = 0;
-    if (n_missing) *n_missing = 0;
-    DevCtx* cp = nullptr;
-    if (int rc = map_ctx(token, &cp)) return rc;
-    DevCtx& c = *cp;
-    if (int rc = check_lookup_args(c, !d_centre_idx, N)) return rc;
-    if (R == 0) return BDG_OK;
-    if (!d_ranks || !d_centre || !d_has_centre) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    DevCtx* c = nullptr;
+    if (int rc = assign_lookup32_args(token, !d_centre_idx, N, d_ranks, R, d_centre, d_has_centre, n_assigned, n_missing, &c)) return done(rc);
     if (d_centre_idx) if (int rc = check_on_first(d_centre_idx, "centre_idx")) return rc;
     if (int rc = check_on_first(d_ranks, "ranks")) return rc;
     if (d_valid) if (int rc = check_on_first(d_valid, "valid")) return rc;
     if (int rc = check_on_first(d_centre, "centre")) return rc;
     if (int rc = check_on_first(d_has_centre, "has_centre")) return rc;
-    CallerOrder order(c, stream);
-    if (int rc = order.begin()) return rc;
-    if (int rc = assign_lookup32_core(c, d_centre_idx, N, d_ranks, d_valid, R, d_centre, d_has_centre)) return rc;
-    if (n_assigned || n_missing) return read_lookup_counters(c, n_assigned, n_missing);
-    return BDG_OK;
-}
-
-int bdg_assign_reads(unsigned long long token, const int32_t* centre_idx, size_t N, uint64_t* centre_per_row, size_t R_all, size_t* n_assigned)
-{
-    if (n_assigned) *n_assigned = 0;
-    if (R_all == 0) return BDG_OK;
-    if (!centre_per_row || (N && !centre_idx)) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    DevCtx* cp = nullptr;
-    if (int rc = map_ctx(token, &cp)) return rc;
-    DevCtx& c = *cp;
-    if (int rc = check_assign_args(c, false, N, R_all)) return rc;
-    const ReadMap& m = c.map;
-    cudaStream_t st = c.stream;
-    // as[2] centre index per node (upload), as[3] centre value per distinct barcode in first-seen order, as[4] result per row, as[5] counter
-    if (int e = c.as[2].ensure(std::max<size_t>(N, 1) * 4)) return e;
-    if (int e = c.as[3].ensure(std::max<size_t>(N, 1) * 8)) return e;
-    if (int e = c.as[4].ensure(R_all * 8)) return e;
-    if (int e = c.as[5].ensure(8)) return e;
-    CU_TRY(cudaMemcpyAsync(c.as[2].p, centre_idx, N * 4, cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemsetAsync(c.as[5].p, 0, 8, st));
-    if (N) {
-        const int nb = (int)std::min<size_t>((N + 255) / 256, (size_t)c.sms * 8);
-        bdg::centre_of_distinct_kernel<<<nb, 256, 0, st>>>((const int32_t*)c.as[2].p, m.order() /* first-seen -> node */,
-                                                           m.ascending() /* node -> barcode */, (uint32_t)N, (uint64_t*)c.as[3].p);
-    }
-    const int rb = (int)std::min<size_t>((R_all + 255) / 256, (size_t)c.sms * 8);
-    bdg::assign_reads_kernel<<<rb, 256, 0, st>>>((const uint64_t*)c.as[3].p, m.read_pos(), m.masked ? (const uint8_t*)m.valid.p : nullptr,
-                                                 m.masked ? (const uint32_t*)m.valid_scan.p : nullptr, (uint32_t)R_all, (uint64_t*)c.as[4].p,
-                                                 (unsigned long long*)c.as[5].p);
-    g_launches += 2;
-    CU_TRY(cudaGetLastError());
-    unsigned long long cnt = 0;
-    CU_TRY(cudaMemcpyAsync(centre_per_row, c.as[4].p, R_all * 8, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaMemcpyAsync(&cnt, c.as[5].p, 8, cudaMemcpyDeviceToHost, st));
-    CU_TRY(cudaStreamSynchronize(st));
-    if (n_assigned) *n_assigned = (size_t)cnt;
-    return BDG_OK;
+    return assign_lookup32_body(*c, d_centre_idx, N, d_ranks, d_valid, R, d_centre, d_has_centre, n_assigned, n_missing, (cudaStream_t)stream);
 }
 
 int bdg_pack16(const char* seqs, size_t R, uint32_t* out, uint8_t* valid)
 {
     if (R == 0) return BDG_OK;
     if (!seqs || !out || !valid) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
-    const size_t sizes[3] = {R * 16, R * 4, R};               // grow-only workspaces: letters, ranks, validity
-    for (int k = 0; k < 3; k++)
-        if (int e = c.io[k].ensure(sizes[k])) return e;
-    CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, c.stream));
-    if (int rc = bdg_dev_pack16((const char*)c.io[0].p, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, c.stream)) return rc;
-    CU_TRY(cudaMemcpyAsync(out, c.io[1].p, R * 4, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaMemcpyAsync(valid, c.io[2].p, R, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
+    DevCtx* c = nullptr;
+    if (int rc = first_ctx(&c)) return rc;
+    char* d_seqs = nullptr;
+    uint32_t* d_out = nullptr;
+    uint8_t* d_valid = nullptr;
+    if (int e = stage(*c, {piece(d_seqs, R * 16), piece(d_out, R * 4), piece(d_valid, R)})) return e;
+    CU_TRY(cudaMemcpyAsync(d_seqs, seqs, R * 16, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = bdg_dev_pack16(d_seqs, R, d_out, d_valid, c->stream)) return rc;
+    CU_TRY(cudaMemcpyAsync(out, d_out, R * 4, cudaMemcpyDeviceToHost, c->stream));
+    CU_TRY(cudaMemcpyAsync(valid, d_valid, R, cudaMemcpyDeviceToHost, c->stream));
+    CU_TRY(cudaStreamSynchronize(c->stream));
     return BDG_OK;
 }
 
-
 // badger.py:82-88 for the array pipeline: the whitelist records packed (a-1), the invalid ones dropped, sorted and made
 // distinct on the device (cub radix sort + unique); out_sorted has room for R entries, *n receives the number kept.
-// d_seqs: the R records on c.dev; the distinct packed barcodes stay in ce[2], *n receives their number.
-static int pack16_sorted_core(DevCtx& c, const char* d_seqs, size_t R, size_t* n)
+static int pack16_sorted_args(const char* seqs, size_t R, const uint32_t* out_sorted, size_t* n, DevCtx** c)
 {
+    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
+    *n = 0;
+    if (R == 0) return EMPTY;
+    if (!seqs || !out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
+    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
+    return first_ctx(c);
+}
+
+// d_seqs: the R records on c.dev; ranks / valid: scratch for R entries; the distinct packed barcodes are copied to out_sorted
+// (kind: to the host or to device memory on c.dev; the host form waits for the copy).
+static int pack16_sorted_body(DevCtx& c, const char* d_seqs, size_t R, uint32_t* ranks, uint8_t* valid, uint32_t* out_sorted, cudaMemcpyKind kind,
+                              size_t* n, cudaStream_t caller)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     cudaStream_t st = c.stream;
-    // io[1] ranks, io[2] validity; ce[0] kept ranks, ce[1] sorted, ce[2] distinct, ce[7] count, ce[8] cub scratch
-    if (int e = c.io[1].ensure(R * 4)) return e;
-    if (int e = c.io[2].ensure(R)) return e;
-    for (int k = 0; k < 3; k++) if (int e = c.ce[k].ensure(R * 4)) return e;
-    if (int e = c.ce[7].ensure(64)) return e;
-    uint32_t* d_n = (uint32_t*)c.ce[7].p;
-    if (int rc = bdg_dev_pack16(d_seqs, R, (uint32_t*)c.io[1].p, (uint8_t*)c.io[2].p, st)) return rc;
+    for (Buf* b : {&c.sel, &c.sel_keys, &c.sel_sorted}) if (int e = b->ensure(R * 4)) return e;
+    if (int e = c.sel_scalars.ensure(64)) return e;
+    uint32_t *kept_ranks = (uint32_t*)c.sel.p, *sorted = (uint32_t*)c.sel_keys.p, *distinct = (uint32_t*)c.sel_sorted.p;
+    uint32_t* d_n = (uint32_t*)c.sel_scalars.p;
+    if (int rc = bdg_dev_pack16(d_seqs, R, ranks, valid, st)) return rc;
     size_t t1 = 0, t2 = 0, t3 = 0;
-    CU_TRY(cub::DeviceSelect::Flagged(nullptr, t1, (const uint32_t*)c.io[1].p, (const uint8_t*)c.io[2].p, (uint32_t*)c.ce[0].p, d_n, (int)R, st));
-    CU_TRY(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[1].p, (int)R, 0, 32, st));
-    CU_TRY(cub::DeviceSelect::Unique(nullptr, t3, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, d_n, (int)R, st));
-    if (int e = c.ce[8].ensure(std::max(t1, std::max(t2, t3)))) return e;
-    CU_TRY(cub::DeviceSelect::Flagged(c.ce[8].p, t1, (const uint32_t*)c.io[1].p, (const uint8_t*)c.io[2].p, (uint32_t*)c.ce[0].p, d_n, (int)R, st));
+    CU_TRY(cub::DeviceSelect::Flagged(nullptr, t1, (const uint32_t*)ranks, (const uint8_t*)valid, kept_ranks, d_n, (int)R, st));
+    CU_TRY(cub::DeviceRadixSort::SortKeys(nullptr, t2, (const uint32_t*)kept_ranks, sorted, (int)R, 0, 32, st));
+    CU_TRY(cub::DeviceSelect::Unique(nullptr, t3, (const uint32_t*)sorted, distinct, d_n, (int)R, st));
+    if (int e = c.sel_tmp.ensure(std::max(t1, std::max(t2, t3)))) return e;
+    CU_TRY(cub::DeviceSelect::Flagged(c.sel_tmp.p, t1, (const uint32_t*)ranks, (const uint8_t*)valid, kept_ranks, d_n, (int)R, st));
     uint32_t kept = 0;
     CU_TRY(cudaMemcpyAsync(&kept, d_n, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     if (kept == 0) return BDG_OK;
-    CU_TRY(cub::DeviceRadixSort::SortKeys(c.ce[8].p, t2, (const uint32_t*)c.ce[0].p, (uint32_t*)c.ce[1].p, (int)kept, 0, 32, st));
-    CU_TRY(cub::DeviceSelect::Unique(c.ce[8].p, t3, (const uint32_t*)c.ce[1].p, (uint32_t*)c.ce[2].p, d_n, (int)kept, st));
-    uint32_t distinct = 0;
-    CU_TRY(cudaMemcpyAsync(&distinct, d_n, 4, cudaMemcpyDeviceToHost, st));
+    CU_TRY(cub::DeviceRadixSort::SortKeys(c.sel_tmp.p, t2, (const uint32_t*)kept_ranks, sorted, (int)kept, 0, 32, st));
+    CU_TRY(cub::DeviceSelect::Unique(c.sel_tmp.p, t3, (const uint32_t*)sorted, distinct, d_n, (int)kept, st));
+    uint32_t n_distinct = 0;
+    CU_TRY(cudaMemcpyAsync(&n_distinct, d_n, 4, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
-    *n = distinct;
+    CU_TRY(cudaMemcpyAsync(out_sorted, distinct, (size_t)n_distinct * 4, kind, st));
+    if (kind == cudaMemcpyDeviceToHost) CU_TRY(cudaStreamSynchronize(st));
+    *n = n_distinct;
     return BDG_OK;
 }
 
 int bdg_pack16_sorted(const char* seqs, size_t R, uint32_t* out_sorted, size_t* n)
 {
-    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n = 0;
-    if (R == 0) return BDG_OK;
-    if (!seqs || !out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
-    if (int e = c.io[0].ensure(R * 16)) return e;     // io[0] letters
-    CU_TRY(cudaMemcpyAsync(c.io[0].p, seqs, R * 16, cudaMemcpyHostToDevice, c.stream));
-    size_t kept = 0;
-    if (int rc = pack16_sorted_core(c, (const char*)c.io[0].p, R, &kept)) return rc;
-    CU_TRY(cudaMemcpyAsync(out_sorted, c.ce[2].p, kept * 4, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
-    *n = kept;
-    return BDG_OK;
+    DevCtx* c = nullptr;
+    if (int rc = pack16_sorted_args(seqs, R, out_sorted, n, &c)) return done(rc);
+    char* d_seqs = nullptr;
+    uint32_t* ranks = nullptr;
+    uint8_t* valid = nullptr;
+    if (int e = stage(*c, {piece(d_seqs, R * 16), piece(ranks, R * 4), piece(valid, R)})) return e;
+    CU_TRY(cudaMemcpyAsync(d_seqs, seqs, R * 16, cudaMemcpyHostToDevice, c->stream));
+    return pack16_sorted_body(*c, d_seqs, R, ranks, valid, out_sorted, cudaMemcpyDeviceToHost, n, c->stream);
 }
 
 int bdg_dev_pack16_sorted(const char* d_seqs, size_t R, uint32_t* d_out_sorted, size_t* n, void* stream)
 {
-    if (!n) return fail(BDG_ERR_ARG, "NULL result pointer");
-    *n = 0;
-    if (R == 0) return BDG_OK;
-    if (!d_seqs || !d_out_sorted) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (R > 0x7FFFFFFFull) return fail(BDG_ERR_ARG, "more than 2^31 records in one call");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = pack16_sorted_args(d_seqs, R, d_out_sorted, n, &c)) return done(rc);
     if (int rc = check_on_first(d_seqs, "records")) return rc;
     if (int rc = check_on_first(d_out_sorted, "out_sorted")) return rc;
-    CallerOrder order(c, stream);
-    if (int rc = order.begin()) return rc;
-    size_t kept = 0;
-    if (int rc = pack16_sorted_core(c, d_seqs, R, &kept)) return rc;
-    CU_TRY(cudaMemcpyAsync(d_out_sorted, c.ce[2].p, kept * 4, cudaMemcpyDeviceToDevice, c.stream));
-    *n = kept;
-    return BDG_OK;
+    uint32_t* ranks = nullptr;
+    uint8_t* valid = nullptr;
+    if (int e = stage(*c, {piece(ranks, R * 4), piece(valid, R)})) return e;
+    return pack16_sorted_body(*c, d_seqs, R, ranks, valid, d_out_sorted, cudaMemcpyDeviceToDevice, n, (cudaStream_t)stream);
 }
 
 // One device's share of a host-buffer edge build: upload, launch, read the count back (re-run once with the exact
@@ -2610,16 +2629,16 @@ static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint
 {
     cudaStream_t st = c.stream;
     c.map.cl_token = 0;                                    // the resident result is about to be overwritten
-    if (int e = c.cl[0].ensure(std::max<size_t>(C, 1) * 4)) return e;
+    if (int e = c.cl_centres.ensure(std::max<size_t>(C, 1) * 4)) return e;
     if (int e = c.map.centre.ensure(N * 4)) return e;
     if (int e = c.map.level.ensure(N)) return e;
-    if (int e = c.cl[1].ensure(N * 4)) return e;
-    if (int e = c.cl[2].ensure(N * 4)) return e;
-    if (int e = c.cl[3].ensure(16)) return e;
-    unsigned int* d_bad = (unsigned int*)c.cl[3].p;
+    if (int e = c.cl_min.ensure(N * 4)) return e;
+    if (int e = c.cl_max.ensure(N * 4)) return e;
+    if (int e = c.cl_flags.ensure(16)) return e;
+    unsigned int* d_bad = (unsigned int*)c.cl_flags.p;
     CU_TRY(cudaMemsetAsync(d_bad, 0, 4, c.stream));
-    uint32_t* d_cen = (uint32_t*)c.cl[0].p;
-    int32_t *d_ci = (int32_t*)c.map.centre.p, *d_min = (int32_t*)c.cl[1].p, *d_max = (int32_t*)c.cl[2].p;
+    uint32_t* d_cen = (uint32_t*)c.cl_centres.p;
+    int32_t *d_ci = (int32_t*)c.map.centre.p, *d_min = (int32_t*)c.cl_min.p, *d_max = (int32_t*)c.cl_max.p;
     uint8_t* d_lv = (uint8_t*)c.map.level.p;
     const int nb = node_blocks(N, c.sms);
     const bool trace = getenv("BDG_TRACE") != nullptr;
@@ -2643,7 +2662,7 @@ static int cluster_on_device(DevCtx& c, const uint32_t* d_sorted, size_t N, uint
     if (level) CU_TRY(cudaMemcpyAsync(level, d_lv, N, cudaMemcpyDeviceToHost, st));
     unsigned long long has_edge = 0;
     if (n_has_edge) {
-        unsigned long long* d_cnt = (unsigned long long*)((char*)c.cl[3].p + 8);
+        unsigned long long* d_cnt = (unsigned long long*)((char*)c.cl_flags.p + 8);
         CU_TRY(cudaMemsetAsync(d_cnt, 0, 8, st));
         bdg::count_has_edge_kernel<<<nb, 256, 0, st>>>(d_lv, (uint32_t)N, d_cnt);
         g_launches++;
@@ -2706,9 +2725,7 @@ static int cluster_from_edges(bdg_edges* e, size_t N, const uint32_t* centres, s
     if (C && !centres) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (e->ctx.empty()) return fail(BDG_ERR_ARG, "empty edge handle");
     if (N > 0x7FFFFFFFull || rounds < 0 || rounds > 253) return fail(BDG_ERR_ARG, "N must be < 2^31 and 0 <= rounds <= 253");
-    for (size_t g = 0; g < e->ctx.size(); g++)
-        if (e->ctx[g] < 0 || (size_t)e->ctx[g] >= g_ctx.size() || g_ctx[e->ctx[g]].generation != e->gen[g])
-            return fail(BDG_ERR_ARG, "stale edge handle: a later edge build on the same device has reused its buffers");
+    if (int rc = check_edges_handle(e)) return rc;
     DevCtx& c = g_ctx[e->ctx[0]];
     if (c.sorted.cap < N * 4) return fail(BDG_ERR_ARG, "N does not match the array the edges were built from");
     CU_TRY(cudaSetDevice(c.dev));
@@ -2815,32 +2832,18 @@ int bdg_dev_cluster_resolve(int32_t* d_centre_idx, uint8_t* d_level, int32_t* d_
 
 int bdg_member_sorted(const uint32_t* sorted_wl, size_t W, const uint32_t* q, size_t Q, uint8_t* hit)
 {
-    if (Q == 0) return BDG_OK;
-    if (!q || !hit || (W && !sorted_wl)) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (W > 0xFFFFFFFFull || Q > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
-    const size_t sizes[4] = {std::max<size_t>(W, 1) * 4, Q * 4, Q, 8};       // grow-only workspaces: whitelist, queries, hits, check flag
-    for (int k = 0; k < 4; k++)
-        if (int e = c.io[k].ensure(sizes[k])) return e;
-    uint32_t *d_wl = (uint32_t*)c.io[0].p, *d_q = (uint32_t*)c.io[1].p;
-    uint8_t* d_hit = (uint8_t*)c.io[2].p;
-    unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
-    CU_TRY(cudaMemcpyAsync(d_wl, sorted_wl, W * 4, cudaMemcpyHostToDevice, c.stream));
-    CU_TRY(cudaMemcpyAsync(d_q, q, Q * 4, cudaMemcpyHostToDevice, c.stream));
-    CU_TRY(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
-    if (W > 1) {                                            // the whitelist must be sorted: checked on the device, read back with the hits
-        bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, c.stream>>>(d_wl, (uint32_t)W, d_bad);
-        g_launches++;
-    }
-    if (int rc = bdg_dev_member_sorted(d_wl, W, d_q, Q, d_hit, c.stream)) return rc;
-    unsigned long long first_bad = ~0ull;
-    CU_TRY(cudaMemcpyAsync(hit, d_hit, Q, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaMemcpyAsync(&first_bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
-    if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "whitelist not sorted at index %llu", first_bad);
-    return BDG_OK;
+    if (int rc = member_sorted_args(sorted_wl, W, q, Q, hit)) return done(rc);
+    DevCtx* c = nullptr;
+    if (int rc = first_ctx(&c)) return rc;
+    uint32_t *d_wl = nullptr, *d_q = nullptr;
+    uint8_t* d_hit = nullptr;
+    if (int e = stage(*c, {piece(d_wl, std::max<size_t>(W, 1) * 4), piece(d_q, Q * 4), piece(d_hit, Q)})) return e;
+    CU_TRY(cudaMemcpyAsync(d_wl, sorted_wl, W * 4, cudaMemcpyHostToDevice, c->stream));
+    CU_TRY(cudaMemcpyAsync(d_q, q, Q * 4, cudaMemcpyHostToDevice, c->stream));
+    if (int rc = sort_check(*c, d_wl, W)) return rc;        // the whitelist must be sorted: checked on the device, read back with the hits
+    if (int rc = member_sorted_body(d_wl, W, d_q, Q, d_hit, c->stream)) return rc;
+    CU_TRY(cudaMemcpyAsync(hit, d_hit, Q, cudaMemcpyDeviceToHost, c->stream));
+    return sort_check_result(*c);
 }
 
 // The check bdg_member_sorted makes on its whitelist, for a whitelist in device memory (bdg_dev_member_sorted does not check).
@@ -2849,23 +2852,13 @@ int bdg_dev_whitelist_check(const uint32_t* d_sorted_wl, size_t W, void* stream)
     if (W <= 1) return BDG_OK;
     if (!d_sorted_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
     if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = first_ctx(&c)) return rc;
     if (int rc = check_on_first(d_sorted_wl, "whitelist")) return rc;
-    if (int e = c.io[3].ensure(8)) return e;
-    unsigned long long* d_bad = (unsigned long long*)c.io[3].p;
-    CallerOrder order(c, stream);
+    CallerOrder order(*c, stream);
     if (int rc = order.begin()) return rc;
-    CU_TRY(cudaMemsetAsync(d_bad, 0xFF, 8, c.stream));
-    bdg::sorted_check_kernel<false><<<(int)std::min<size_t>((W + 255) / 256, (size_t)c.sms * 8), 256, 0, c.stream>>>(d_sorted_wl, (uint32_t)W, d_bad);
-    g_launches++;
-    CU_TRY(cudaGetLastError());
-    unsigned long long first_bad = ~0ull;
-    CU_TRY(cudaMemcpyAsync(&first_bad, d_bad, 8, cudaMemcpyDeviceToHost, c.stream));
-    CU_TRY(cudaStreamSynchronize(c.stream));
-    if (first_bad != ~0ull) return fail(BDG_ERR_ARG, "whitelist not sorted at index %llu", first_bad);
-    return BDG_OK;
+    if (int rc = sort_check(*c, d_sorted_wl, W)) return rc;
+    return sort_check_result(*c);
 }
 
 int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, size_t W, int max_d, int32_t* argmin, uint8_t* dist)
@@ -2883,13 +2876,11 @@ int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, si
         DevCtx& c = g_ctx[g];
         rc = [&]() -> int {
             CU_TRY(cudaSetDevice(c.dev));
-            // io[0] queries, io[1] targets, io[2] keys | argmin | distance
-            if (int e = c.io[0].ensure(n * 4)) return e;
-            if (int e = c.io[1].ensure(std::max<size_t>(W, 1) * 4)) return e;
-            if (int e = c.io[2].ensure(n * 9)) return e;
-            uint32_t *d_q = (uint32_t*)c.io[0].p, *d_t = (uint32_t*)c.io[1].p, *d_keys = (uint32_t*)c.io[2].p;
-            int32_t* d_arg = (int32_t*)(d_keys + n);
-            uint8_t* d_dist = (uint8_t*)(d_arg + n);
+            uint32_t *d_q = nullptr, *d_t = nullptr, *d_keys = nullptr;
+            int32_t* d_arg = nullptr;
+            uint8_t* d_dist = nullptr;
+            if (int e = stage(c, {piece(d_q, n * 4), piece(d_t, std::max<size_t>(W, 1) * 4), piece(d_keys, n * 4), piece(d_arg, n * 4),
+                                  piece(d_dist, n)})) return e;
             CU_TRY(cudaMemcpyAsync(d_q, q + lo, n * 4, cudaMemcpyHostToDevice, c.stream));
             CU_TRY(cudaMemcpyAsync(d_t, targets, W * 4, cudaMemcpyHostToDevice, c.stream));
             if (int e = bdg_dev_nearest_bounded(d_q, n, d_t, W, max_d, d_keys, d_arg, d_dist, c.stream)) return e;
@@ -2910,32 +2901,37 @@ int bdg_nearest_bounded(const uint32_t* q, size_t Q, const uint32_t* targets, si
 }
 
 // ---- a-5  KmerIndexer / QGramIndex: the known strings stay on the device between queries ------------------
-// wl: the W strings in host memory (kind = cudaMemcpyHostToDevice) or in device memory on the first claimed device
-// (cudaMemcpyDeviceToDevice, read on that device's stream, which the device form has ordered after the caller's).
-static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, cudaMemcpyKind kind, bdg_kmer_index** out)
+static int kmer_index_args(const uint32_t* wl, size_t W, bdg_kmer_index** out, DevCtx** c)
 {
     if (!out || (W && !wl)) return fail(BDG_ERR_ARG, "NULL pointer argument");
     *out = nullptr;
     if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (int rc = need_ctx()) return rc;
+    return first_ctx(c);
+}
+
+// wl: the W strings in host memory (kind = cudaMemcpyHostToDevice) or in device memory on the first claimed device
+// (cudaMemcpyDeviceToDevice, read on that device's stream, which is ordered after the caller's); copied straight into the index.
+static int kmer_index_body(DevCtx& c, const uint32_t* wl, size_t W, bool postings, cudaMemcpyKind kind, cudaStream_t caller, bdg_kmer_index** out)
+{
+    CallerOrder order(c, caller);
+    if (int rc = order.begin()) return rc;
     bdg_kmer_index* ix = new (std::nothrow) bdg_kmer_index();
     if (!ix) return fail(BDG_ERR_OOM, "host allocation failed");
-    ix->dev = g_ctx[0].dev;
+    ix->dev = c.dev;
     ix->W = W;
-    CU_TRY(cudaSetDevice(ix->dev));
     if (int e = ix->wl.ensure(std::max<size_t>(W, 1) * 4)) {
         delete ix;
         return e;
     }
-    cudaError_t e = cudaMemcpyAsync(ix->wl.p, wl, W * 4, kind, g_ctx[0].stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(g_ctx[0].stream);
+    cudaError_t e = cudaMemcpyAsync(ix->wl.p, wl, W * 4, kind, c.stream);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(c.stream);
     if (e != cudaSuccess) { bdg_kmer_index_free(ix); return fail(BDG_ERR_CUDA, "upload of the index failed: %s", cudaGetErrorString(e)); }
     // posting lists of the strings' 6-mers (kmer_indexer.py:29-32): worth it once a bucket is a small share of the strings
     size_t min_w = 4096;
     if (const char* v = getenv("BDG_KMER_POST_MIN_W")) min_w = (size_t)std::max(0ll, atoll(v));
     if (postings && W >= min_w && W > 0 && W <= 0xFFFFFFFFull / 11) {          // (the postings are counted in 32 bits)
-        cudaStream_t st = g_ctx[0].stream;
-        const int sms = g_ctx[0].sms;
+        cudaStream_t st = c.stream;
+        const int sms = c.sms;
         size_t tmp = 0;
         bool ok = ix->kstart.ensure(4097 * 4) == BDG_OK && ix->scratch.ensure(2 * 4097 * 4) == BDG_OK;
         ok = ok && cub::DeviceScan::ExclusiveSum(nullptr, tmp, (const uint32_t*)nullptr, (uint32_t*)nullptr, 4097, st) == cudaSuccess;
@@ -2971,21 +2967,17 @@ static int kmer_index_create(const uint32_t* wl, size_t W, bool postings, cudaMe
 
 int bdg_kmer_index_create(const uint32_t* wl, size_t W, bdg_kmer_index** out)
 {
-    return kmer_index_create(wl, W, true, cudaMemcpyHostToDevice, out);
+    DevCtx* c = nullptr;
+    if (int rc = kmer_index_args(wl, W, out, &c)) return rc;
+    return kmer_index_body(*c, wl, W, true, cudaMemcpyHostToDevice, c->stream, out);
 }
 
 int bdg_dev_kmer_index_create(const uint32_t* d_known, size_t W, void* stream, bdg_kmer_index** out)
 {
-    if (!out || (W && !d_known)) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    *out = nullptr;
-    if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
+    DevCtx* c = nullptr;
+    if (int rc = kmer_index_args(d_known, W, out, &c)) return rc;
     if (W) if (int rc = check_on_first(d_known, "known")) return rc;
-    CallerOrder order(c, stream);
-    if (int rc = order.begin()) return rc;
-    return kmer_index_create(d_known, W, true, cudaMemcpyDeviceToDevice, out);
+    return kmer_index_body(*c, d_known, W, true, cudaMemcpyDeviceToDevice, (cudaStream_t)stream, out);
 }
 
 int bdg_kmer_index_info(const bdg_kmer_index* ix, int* posted, double* kernel_ms)
@@ -3014,8 +3006,8 @@ static int kmer_query_core(bdg_kmer_index* ix, DevCtx& c, const uint32_t* d_q, s
                            uint32_t* d_hw, uint8_t* d_cnt, unsigned long long* d_mult, unsigned long long* tot)
 {
     const size_t W = ix->W;
-    if (int e = ix->outb[5].ensure(8)) return e;
-    unsigned long long* d_total = (unsigned long long*)ix->outb[5].p;
+    if (int e = ix->total.ensure(8)) return e;
+    unsigned long long* d_total = (unsigned long long*)ix->total.p;
     CU_TRY(cudaMemsetAsync(d_total, 0, 8, c.stream));
     CU_TRY(cudaEventRecord(ix->ev[0], c.stream));
     if (ix->posted) {                                       // walk the buckets of the queries' own 6-mers
@@ -3054,12 +3046,14 @@ int bdg_kmer_index_query(bdg_kmer_index* ix, const uint32_t* q, size_t Q, int mi
     if (!c) return fail(BDG_ERR_NODEVICE, "the device the index lives on is no longer claimed (bdg_shutdown?)");
     CU_TRY(cudaSetDevice(c->dev));
     const size_t capa = std::max<size_t>(cap, 1);
-    const size_t sizes[5] = {Q * 4, capa * 4, capa * 4, capa, capa * 8};     // queries, hit_q, hit_w, cnt, mult
-    for (int k = 0; k < 5; k++)
-        if (int e = ix->outb[k].ensure(sizes[k])) return e;
-    uint32_t *d_q = (uint32_t*)ix->outb[0].p, *d_hq = (uint32_t*)ix->outb[1].p, *d_hw = (uint32_t*)ix->outb[2].p;
-    uint8_t* d_cnt = (uint8_t*)ix->outb[3].p;
-    unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
+    for (Buf* b : {&ix->hit_q, &ix->hit_w}) if (int e = b->ensure(capa * 4)) return e;
+    if (int e = ix->hit_cnt.ensure(capa)) return e;
+    if (int e = ix->mult.ensure(capa * 8)) return e;
+    uint32_t* d_q = nullptr;
+    if (int e = stage(*c, {piece(d_q, Q * 4)})) return e;
+    uint32_t *d_hq = (uint32_t*)ix->hit_q.p, *d_hw = (uint32_t*)ix->hit_w.p;
+    uint8_t* d_cnt = (uint8_t*)ix->hit_cnt.p;
+    unsigned long long* d_mult = (unsigned long long*)ix->mult.p;
     CU_TRY(cudaMemcpyAsync(d_q, q, Q * 4, cudaMemcpyHostToDevice, c->stream));
     unsigned long long tot = 0;
     if (int rc = kmer_query_core(ix, *c, d_q, Q, min_kmers, cap, d_hq, d_hw, d_cnt, d_mult, &tot)) return rc;
@@ -3095,8 +3089,8 @@ int bdg_dev_kmer_index_query(bdg_kmer_index* ix, const uint32_t* d_q, size_t Q, 
         for (const void* p : outs) if (int rc = check_on_first(p, "output")) return rc;
     }
     // the position counts are unpacked from library scratch into d_pos; the other outputs are written by the kernels in place
-    if (int e = ix->outb[4].ensure(std::max<size_t>(cap, 1) * 8)) return e;
-    unsigned long long* d_mult = (unsigned long long*)ix->outb[4].p;
+    if (int e = ix->mult.ensure(std::max<size_t>(cap, 1) * 8)) return e;
+    unsigned long long* d_mult = (unsigned long long*)ix->mult.p;
     CallerOrder order(c, stream);
     if (int rc = order.begin()) return rc;
     unsigned long long tot = 0;
@@ -3120,7 +3114,9 @@ int bdg_kmer_score(const uint32_t* q, size_t Q, const uint32_t* wl, size_t W, in
     if (Q == 0 || W == 0) return BDG_OK;
     if (!q || !wl || (cap && (!hit_q || !hit_w || !cnt || !mult))) return fail(BDG_ERR_ARG, "NULL pointer argument");
     bdg_kmer_index* ix = nullptr;
-    if (int rc = kmer_index_create(wl, W, Q >= 64, cudaMemcpyHostToDevice, &ix)) return rc;       // a one-off call with few queries: the scan costs less than the lists
+    DevCtx* c = nullptr;
+    if (int rc = kmer_index_args(wl, W, &ix, &c)) return rc;
+    if (int rc = kmer_index_body(*c, wl, W, Q >= 64, cudaMemcpyHostToDevice, c->stream, &ix)) return rc;   // a one-off call with few queries: the scan costs less than the lists
     const int rc = bdg_kmer_index_query(ix, q, Q, min_kmers, cap, hit_q, hit_w, cnt, mult, total);
     bdg_kmer_index_free(ix);
     return rc;
@@ -3133,17 +3129,11 @@ int bdg_dev_kmer_score(const uint32_t* d_q, size_t Q, const uint32_t* d_wl, size
     *total = 0;
     if (Q == 0 || W == 0) return BDG_OK;
     if (!d_q || !d_wl) return fail(BDG_ERR_ARG, "NULL pointer argument");
-    if (W > 0xFFFFFFFFull) return fail(BDG_ERR_ARG, "size exceeds 2^32");
-    if (int rc = need_ctx()) return rc;
-    DevCtx& c = g_ctx[0];
-    CU_TRY(cudaSetDevice(c.dev));
-    if (int rc = check_on_first(d_wl, "wl")) return rc;
     bdg_kmer_index* ix = nullptr;
-    {
-        CallerOrder order(c, stream);
-        if (int rc = order.begin()) return rc;
-        if (int rc = kmer_index_create(d_wl, W, Q >= 64, cudaMemcpyDeviceToDevice, &ix)) return rc;   // the rule of bdg_kmer_score
-    }
+    DevCtx* c = nullptr;
+    if (int rc = kmer_index_args(d_wl, W, &ix, &c)) return rc;
+    if (int rc = check_on_first(d_wl, "wl")) return rc;
+    if (int rc = kmer_index_body(*c, d_wl, W, Q >= 64, cudaMemcpyDeviceToDevice, (cudaStream_t)stream, &ix)) return rc;   // the rule of bdg_kmer_score
     const int rc = bdg_dev_kmer_index_query(ix, d_q, Q, min_kmers, cap, d_hit_q, d_hit_w, d_cnt, d_pos, total, stream);
     bdg_kmer_index_free(ix);          // cudaFree waits for the unpack kernel that still reads the index's scratch
     return rc;

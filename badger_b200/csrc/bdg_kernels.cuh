@@ -704,9 +704,9 @@ __global__ void __launch_bounds__(NT) lookup_assign32_kernel(const uint32_t* __r
 
 // ---------------------------------------------------------------------------------------------------
 // Rows f-1 / f-2 with the per-read arrays staying on the device: bdg_dedup_reads compacts the valid rows (valid bytes +
-// their exclusive scan), dedups them as above and keeps read -> first-seen position resident; bdg_assign_reads then
+// their exclusive scan), dedups them as above and keeps read -> first-seen position resident; bdg_assign_reads32 then
 // turns the clustering result into the centre of every input row (barcode_graph.py:322-329 + 395-404) with two
-// gathers.  HBM bound: 4 + 1 + 4 B in and 8 B out per row plus one random 8-byte read of the per-barcode table.
+// gathers.  HBM bound: 4 + 1 + 4 B in and 5 B out per row plus one random 5-byte read of the per-barcode table.
 // ---------------------------------------------------------------------------------------------------
 struct NonZero {
     __host__ __device__ __forceinline__ uint32_t operator()(const uint8_t& v) const { return v ? 1u : 0u; }
@@ -719,34 +719,8 @@ __global__ void compact_valid_kernel(const uint32_t* __restrict__ ranks, const u
         if (__ldg(&valid[i])) out[__ldg(&excl[i])] = __ldg(&ranks[i]);
 }
 
-constexpr uint64_t NO_CENTRE = 1ull << 32;
-
-// centre value of every distinct barcode in first-seen order: node = order[p]; centre_idx[node] >= 0 -> barcode of that node
-__global__ void centre_of_distinct_kernel(const int32_t* __restrict__ centre_idx, const uint32_t* __restrict__ order,
-                                          const uint32_t* __restrict__ node_key, uint32_t n, uint64_t* __restrict__ out)
-{
-    for (uint32_t p = blockIdx.x * blockDim.x + threadIdx.x; p < n; p += gridDim.x * blockDim.x) {
-        const int32_t c = __ldg(&centre_idx[__ldg(&order[p])]);
-        out[p] = (c >= 0 && (uint32_t)c < n) ? (uint64_t)__ldg(&node_key[c]) : NO_CENTRE;
-    }
-}
-
-__global__ void assign_reads_kernel(const uint64_t* __restrict__ centre_of_distinct, const uint32_t* __restrict__ read_to_distinct,
-                                    const uint8_t* __restrict__ valid, const uint32_t* __restrict__ excl, uint32_t n_rows,
-                                    uint64_t* __restrict__ out, unsigned long long* __restrict__ n_assigned)
-{
-    unsigned long long mine = 0;
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_rows; i += gridDim.x * blockDim.x) {
-        uint64_t v = NO_CENTRE;
-        if (!valid || __ldg(&valid[i])) v = __ldg(&centre_of_distinct[__ldg(&read_to_distinct[valid ? __ldg(&excl[i]) : i])]);
-        out[i] = v;
-        mine += v != NO_CENTRE ? 1 : 0;
-    }
-    for (int o = 16; o; o >>= 1) mine += __shfl_down_sync(0xffffffffu, mine, o);
-    if ((threadIdx.x & 31) == 0 && mine) atomicAdd(n_assigned, mine);
-}
-
-// The same with a 5-byte result per row: centre barcode + "has a centre" byte.
+// centre value + "has a centre" byte of every distinct barcode in first-seen order: node = order[p]; centre_idx[node] >= 0 ->
+// barcode of that node
 __global__ void centre_of_distinct32_kernel(const int32_t* __restrict__ centre_idx, const uint32_t* __restrict__ order,
                                             const uint32_t* __restrict__ node_key, uint32_t n, uint32_t* __restrict__ out, uint8_t* __restrict__ has)
 {

@@ -157,18 +157,21 @@ def pack16_sorted(records) -> np.ndarray:
     return out[:int(n.value)].copy()
 
 
+NONE = np.uint64(1) << np.uint64(32)      # "no centre" in a uint64 per-read result (every uint32 is a valid barcode)
+
+
+def widen(centre, has_centre) -> np.ndarray:
+    """A 5-byte per-read result (assign_reads32) as one uint64 per row: the centre barcode, or NONE where has_centre is 0."""
+    out = centre.astype(np.uint64)
+    out[has_centre == 0] = NONE
+    return out
+
+
 def assign_reads(rmap: ReadMap, centre_idx: np.ndarray):
     """barcode_graph.py:322-329 + 395-404 on the device: centre barcode of every input row of the dedup call (uint64, 2^32 =
-    none) from the clustering result on node positions; returns (centre_per_row, rows with a centre)."""
-    ci = np.ascontiguousarray(centre_idx, dtype=np.int32)
-    out = np.empty(rmap.rows, np.uint64)
-    n = C.c_size_t(0)
-    if rmap.rows:
-        if rmap.token == 0:                                   # no valid row at all: nothing was deduplicated
-            out[:] = np.uint64(1) << np.uint64(32)
-        else:
-            check(lib().bdg_assign_reads(rmap.token, ptr(ci), ci.size, ptr(out), out.size, C.byref(n)))
-    return out, int(n.value)
+    none) from the clustering result on node positions; returns (centre_per_row, rows with a centre).  assign_reads32, widened."""
+    centre, has, n = assign_reads32(rmap, np.ascontiguousarray(centre_idx, dtype=np.int32))
+    return widen(centre, has), n
 
 
 def assign_reads32(rmap: ReadMap, centre_idx=None):

@@ -27,7 +27,7 @@ from ._lib import check, lib, ptr
 from .barcode_graph import _unrank_many
 from .common import rank
 
-NONE = np.uint64(1) << np.uint64(32)      # "no centre" marker in the uint64 result (every uint32 is a valid barcode)
+NONE = ops.NONE                           # "no centre" marker in the uint64 result (every uint32 is a valid barcode)
 
 
 class _Token:
@@ -70,11 +70,7 @@ def assign_packed(ranks, valid=None, *, threshold, n_cells, interval=25, whiteli
     T = timings if timings is not None else {}
 
     def result(c32, has):
-        if form == "u32":
-            return c32, has
-        out = c32.astype(np.uint64)
-        out[has == 0] = NONE
-        return out
+        return (c32, has) if form == "u32" else ops.widen(c32, has)
 
     ranks = np.ascontiguousarray(ranks, dtype=np.uint32)
     R = ranks.size

@@ -85,18 +85,17 @@ int bdg_dedup_first_seen(const uint32_t* ranks, size_t R, uint32_t* distinct, ui
 /* ---- f-1 / f-2 with the per-read arrays resident on the device -------------------------------------------------- */
 /* bdg_dedup_reads = bdg_dedup_first_seen over the rows with valid[i] != 0 (valid == NULL: all rows), compacted on the
  * device; the read -> barcode map is NOT copied out but kept on the first device, and *token names it.
- * bdg_assign_reads is the per-read half of assign_by_cluster + output_file (barcode_graph.py:322-329, 395-404):
- * centre_idx[N] is the clustering result on node positions of the ascending array (bdg_cluster_levels*, possibly patched
- * by the caller, e.g. for --high_sens); centre_per_row[R_all] receives, for every input row of the dedup call, the
- * barcode of the centre its barcode was assigned to, or 2^32 (rows with valid == 0, unassigned / evicted barcodes:
- * the reference writes '*').  *n_assigned = rows with a centre.  The token dies with the next dedup call. */
+ * bdg_assign_reads32 is the per-read half of assign_by_cluster + output_file (barcode_graph.py:322-329, 395-404), and the
+ * library's only per-read gather: centre_idx[N] is the clustering result on node positions of the ascending array
+ * (bdg_cluster_levels*, possibly patched by the caller, e.g. for --high_sens); for every input row of the dedup call,
+ * centre_per_row[R_all] receives the barcode of the centre its barcode was assigned to and has_centre[R_all] 1, or both 0
+ * (rows with valid == 0, unassigned / evicted barcodes: the reference writes '*').  *n_assigned = rows with a centre.
+ * centre_idx == NULL: the clustering result a bdg_cluster_resident call left on the device is used in place - no per-node
+ * array crosses PCIe in either direction.  The token dies with the next dedup call.  (A caller that wants one uint64 per row,
+ * 2^32 for "no centre", widens this result on the host, as badger_b200.ops.widen does.) */
 int bdg_dedup_reads(const uint32_t* ranks, const uint8_t* valid, size_t R_all, uint32_t* distinct, uint32_t* counts,
                     uint32_t* sorted_pos, uint32_t* sorted_distinct /* optional: the distinct barcodes ascending */,
                     size_t* n_distinct, size_t* n_valid, unsigned long long* token);
-int bdg_assign_reads(unsigned long long token, const int32_t* centre_idx, size_t N, uint64_t* centre_per_row, size_t R_all,
-                     size_t* n_assigned);
-/* The same with a 5-byte result per row (centre barcode + "has a centre" byte).  centre_idx == NULL: the clustering result a
- * bdg_cluster_resident call left on the device is used in place - no per-node array crosses PCIe in either direction. */
 int bdg_assign_reads32(unsigned long long token, const int32_t* centre_idx, size_t N, uint32_t* centre_per_row, uint8_t* has_centre,
                        size_t R_all, size_t* n_assigned);
 /* bdg_dedup_reads accepts NULL for distinct / counts / sorted_pos / sorted_distinct (nothing is downloaded then);

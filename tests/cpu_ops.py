@@ -100,11 +100,9 @@ def dedup_reads(ranks, valid=None):
 
 
 def assign_reads(rm, centre_idx):
-    none = np.uint64(1) << np.uint64(32)
+    from badger_b200 import ops
     c32, has, n = assign_reads32(rm, centre_idx)
-    out = c32.astype(np.uint64)
-    out[has == 0] = none
-    return out, n
+    return ops.widen(c32, has), n
 
 
 def assign_reads32(rm, centre_idx=None):
